@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — causal-OT loss forward+backward evaluations per second (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one eval = `compute_sinkhorn_loss` value + gradients w.r.t. f_fake, h_fake, m_real,
@@ -54,6 +54,8 @@ def parse():
     ap.add_argument("--cpu-budget-s", type=float, default=25.0)
     ap.add_argument("--configs", default="cfg1_mmnist,cfg2_shared_ctx,cfg3_bair,cfg4_batched,cfg5_large",
                     help="comma list of the other BASELINE configs carried in the line ('' = headline only)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss and gradients of the last timed headline step as DIR/<name>.npy (rank 0)")
     return ap.parse_args()
 
 
@@ -252,6 +254,32 @@ def golden_terms(name):
         return None
     with np.load(path, allow_pickle=False) as z:
         return {k: z[k] for k in z.files}
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_SAMPLE = 1 << 20          # elements kept of each large output when the whole set would exceed the limit
+GRAD_OUTPUTS = ("fake", "h_fake", "m_real", "h_real", "m_fake")     # the leaves the headline step differentiates
+
+
+def host_outputs(loss, grads):
+    """The arrays a caller of the headline step receives: the loss and the gradients w.r.t. GRAD_OUTPUTS (in that
+    order), copied to host memory in their compute dtype (float32)."""
+    out = {"loss": loss.detach().cpu().numpy()}
+    out.update({"grad_" + n: g.detach().cpu().numpy() for n, g in zip(GRAD_OUTPUTS, grads)})
+    return out
+
+
+def dump_outputs(path, arrays):
+    """DIR/<name>.npy for every array.  If the set exceeds DUMP_LIMIT_BYTES, each array larger than DUMP_SAMPLE
+    elements is replaced by the same seeded sample of its flattened elements on every run (indices ascending)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    sample = sum(a.nbytes for a in arrays.values()) > DUMP_LIMIT_BYTES
+    for name, a in arrays.items():
+        if sample and a.size > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def peaks():
@@ -653,6 +681,7 @@ def main():
     cfg, K, config = workload_config(args.workload, args.kind)
     B, T = cfg["B"], cfg["T"]
     notes = {}
+    dump = bool(args.dump_outputs) and rank == 0
 
     cx = Ctx()
     cx.torch, cx.dist, cx.world, cx.rank, cx.dev, cx.lib = torch, dist, world, rank, dev, lib
@@ -702,6 +731,7 @@ def main():
     progress("graphs captured; timing the headline")
     launches0 = lib.kccot_launch_count()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    last_eager = []                                 # (loss, grads) of the last eager step, kept only for the dump
 
     def timed_serial(n):
         barrier(cx)
@@ -710,6 +740,8 @@ def main():
         for i in range(n):
             if graphs is not None:
                 graphs[i % nsets].step()
+            elif dump and i == n - 1:
+                last_eager[:] = [step(sets[i % nsets])]
             else:
                 step(sets[i % nsets])
         e1.record()
@@ -737,6 +769,9 @@ def main():
 
         timed_lanes(max(3, args.warmup))
         ms, t0, t1 = timed_lanes(args.steps)
+        if dump:                                    # before the serial leg replays the graphs again
+            last = graphs[(args.steps - 1) % nsets]
+            dumped = host_outputs(last.loss, [last.grads[n] for n in GRAD_OUTPUTS])
         ms_serial, _, _ = timed_serial(min(args.steps, 400))
         serial_evals = world * min(args.steps, 400) / (ms_serial * 1e-3)
         # the overlapped replays must leave the same results as a serial replay
@@ -748,6 +783,8 @@ def main():
     else:
         ms, t0, t1 = timed_serial(args.steps)
         serial_evals = None
+        if dump:
+            dumped = host_outputs(*last_eager[0])
     launches = lib.kccot_launch_count() - launches0
     if graphs is not None:
         launches = args.steps * graphs[0].kernels_per_replay      # replays do not pass through the C-ABI counter
@@ -915,6 +952,8 @@ def main():
             "roofline": roofline, "cpu_baseline": cpu, "eager_evals_per_s": eager_evals,
             "serial_evals_per_s": serial_evals, "lanes": NLANES if serial_evals is not None else 1, "notes": notes,
             "configs": other}
+    if dump:
+        dump_outputs(args.dump_outputs, dumped)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -6,6 +6,7 @@ running on torch CPU through `oracle/tf_shim`, in fp64 unless the key ends in `_
 gradients from autograd through the reference's unrolled graph.  Inputs are fp32-representable
 (drawn in fp32, then widened), so the CUDA path sees bit-identical inputs.
 """
+import hashlib
 import os
 import sys
 import warnings
@@ -40,8 +41,28 @@ def _loss_case(g, inp, dtype):
     return loss, grads, terms, C
 
 
+F32_SAMPLE = 4096
+
+
+def reduced_record(d, seed, J):
+    """What a reduced-size case stores, so that each file stays below 1 MB: instead of the inputs their SHA-256
+    digests (`sha256_<input>`; the tests re-draw the inputs with synthetic.make_inputs from `seed` and check them),
+    every fp64 result in full, and of the fp32 gradients of the two videos the same fixed seeded sample of elements
+    (`grad_f_real_f32_sample`, `grad_f_fake_f32_sample` at the flat indices `grad_f32_sample_index`).  `d` holds
+    the inputs and every result in full."""
+    out = {k: v for k, v in d.items() if k not in INPUT_ORDER}
+    out.update({"sha256_" + k: np.str_(hashlib.sha256(np.ascontiguousarray(d[k]).tobytes()).hexdigest())
+                for k in INPUT_ORDER})
+    out.update(seed=seed, J=J)
+    idx = np.sort(np.random.default_rng(0).choice(d["real"].size, F32_SAMPLE, replace=False)).astype(np.int32)
+    out["grad_f32_sample_index"] = idx
+    for n in ("f_real", "f_fake"):
+        out[f"grad_{n}_f32_sample"] = out.pop(f"grad_{n}_f32").reshape(-1)[idx]
+    return out
+
+
 def gen_loss_reduced(g):
-    """BASELINE configs 1-3 at reduced frame size (full B, T, J), inputs stored."""
+    """BASELINE configs 1-3 at reduced frame size (full B, T, J); see reduced_record for what is stored."""
     cases = {"cfg1": dict(B=32, T=20, ctx=10, H=8, W=8, C=1), "cfg2": dict(B=64, T=10, ctx=3, H=4, W=4, C=3),
              "cfg3": dict(B=64, T=12, ctx=2, H=4, W=4, C=3)}
     for name, c in cases.items():
@@ -55,7 +76,7 @@ def gen_loss_reduced(g):
             d.update({k: _np(v) for k, v in C.items()})
             d.update({"grad_" + n: _np(gr) for n, gr in zip(GRAD_NAMES, grads)})
             d.update({"grad_" + n + "_f32": _np(gr) for n, gr in zip(GRAD_NAMES, grads32)})
-            np.savez_compressed(os.path.join(OUT, f"loss_{name}_reduced_{kind}.npz"), **d)
+            np.savez_compressed(os.path.join(OUT, f"loss_{name}_reduced_{kind}.npz"), **reduced_record(d, seed=1, J=8))
             print(name, kind, float(loss), flush=True)
 
 

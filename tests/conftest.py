@@ -33,6 +33,18 @@ def load_golden(name):
         return {k: z[k] for k in z.files}
 
 
+def golden_inputs(g):
+    """The inputs of a reduced-size golden case (CPU tensors), re-drawn by synthetic.make_inputs from the stored
+    seed and checked bit for bit against the stored SHA-256 of the inputs the golden results were computed on."""
+    import hashlib
+    from kccotgan_b200.synthetic import INPUT_ORDER, make_inputs
+    inp = make_inputs(int(g["B"]), int(g["T"]), int(g["H"]), int(g["W"]), int(g["C"]), J=int(g["J"]), ctx=int(g["ctx"]),
+                      kind=str(g["kind"]), seed=int(g["seed"]))
+    for k in INPUT_ORDER:
+        assert hashlib.sha256(inp[k].numpy().tobytes()).hexdigest() == str(g["sha256_" + k]), k
+    return inp
+
+
 def rel_l2(a, b):
     a = np.asarray(a, dtype=np.float64)
     b = np.asarray(b, dtype=np.float64)

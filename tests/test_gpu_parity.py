@@ -11,7 +11,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import load_golden, rel_l2
+from conftest import golden_inputs, load_golden, rel_l2
 from kccotgan_b200.synthetic import CONFIGS, GRAD_NAMES, INPUT_ORDER, make_inputs
 
 pytestmark = pytest.mark.gpu
@@ -149,7 +149,7 @@ def test_mixed_loss_reduced(gu, cfg, kind, path):
     functional.set_path(path)
     g = load_golden(f"loss_{cfg}_reduced_{kind}.npz")
     s = float(g["scaling_coef"])
-    inp = {k: torch.from_numpy(g[k]) for k in INPUT_ORDER}
+    inp = golden_inputs(g)
     loss, terms, grads = _run_loss(gu, inp, s)
     ref_terms = np.array([float(g["loss_xy"]), float(g["loss_xx"]), float(g["loss_yy"])])
     scale = np.abs(ref_terms).max()

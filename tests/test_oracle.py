@@ -4,10 +4,10 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import load_golden, rel_l2
+from conftest import golden_inputs, load_golden, rel_l2
 from oracle import closed_form as cf
 from oracle import port_torch as pt
-from kccotgan_b200.synthetic import INPUT_ORDER, GRAD_NAMES, make_inputs
+from kccotgan_b200.synthetic import INPUT_ORDER, GRAD_NAMES
 
 TOL = 1e-11   # fp64 restatement vs fp64 execution of the reference source
 
@@ -100,7 +100,8 @@ def test_pm(small):
 def test_mixed_loss_reduced(cfg, kind):
     g = load_golden(f"loss_{cfg}_reduced_{kind}.npz")
     s = float(g["scaling_coef"])
-    args = [g[k] for k in INPUT_ORDER]
+    inp = golden_inputs(g)          # the golden inputs are exactly what synthetic.make_inputs re-draws from the seed
+    args = [inp[k].numpy() for k in INPUT_ORDER]
     loss, grads, det = cf.compute_sinkhorn_loss(args[0], args[1], s, 0.8, 100, *args[2:], grad=True)
     scale = max(abs(float(g[k])) for k in ("loss_xy", "loss_xx", "loss_yy"))
     assert abs(loss - float(g["loss"])) <= 1e-10 * scale
@@ -110,28 +111,30 @@ def test_mixed_loss_reduced(cfg, kind):
         assert rel_l2(det[k], g[k]) < TOL
     for n in GRAD_NAMES:
         assert rel_l2(grads[n], g["grad_" + n]) < 1e-8, n
-    # the golden inputs are exactly what synthetic.make_inputs re-draws from the seed
-    re = make_inputs(int(g["B"]), int(g["T"]), int(g["H"]), int(g["W"]), int(g["C"]), J=8, ctx=int(g["ctx"]),
-                     kind=kind, seed=1)
-    for k in INPUT_ORDER:
-        assert np.array_equal(re[k].numpy(), g[k]), k
 
 
 def test_port_matches_golden_fp64_and_fp32():
     """The torch port of the reference formulation (the CPU baseline that bench.py times)."""
     g = load_golden("loss_cfg2_reduced_uniform.npz")
     s = float(g["scaling_coef"])
-    t64 = [torch.from_numpy(g[k]).double() for k in INPUT_ORDER]
+    inp = golden_inputs(g)
+    t64 = [inp[k].double() for k in INPUT_ORDER]
     loss, grads = pt.mixed_loss_fwd_bwd(t64[0], t64[1], s, *t64[2:])
     assert abs(float(loss) - float(g["loss"])) < 1e-9 * abs(float(g["loss_xy"]))
     for n in GRAD_NAMES[1:]:
         assert rel_l2(grads[n].numpy(), g["grad_" + n]) < 1e-8, n
-    t32 = [torch.from_numpy(g[k]).float() for k in INPUT_ORDER]
+    t32 = [inp[k].float() for k in INPUT_ORDER]
     loss32, grads32 = pt.mixed_loss_fwd_bwd(t32[0], t32[1], s, *t32[2:])
-    # fp32 run of the same formulation reproduces the reference's own fp32 numbers closely
+    # fp32 run of the same formulation reproduces the reference's own fp32 numbers closely; of the video gradient
+    # the golden keeps a fixed sample of elements
     assert abs(float(loss32) - float(g["loss_f32"])) < 2e-4 * abs(float(g["loss_xy"]))
+    idx = g["grad_f32_sample_index"]
     for n in GRAD_NAMES[1:]:
-        assert rel_l2(grads32[n].numpy(), g["grad_" + n + "_f32"]) < 2e-3, n
+        got = grads32[n].numpy()
+        ref = g.get("grad_" + n + "_f32")
+        if ref is None:
+            got, ref = got.reshape(-1)[idx], g["grad_" + n + "_f32_sample"]
+        assert rel_l2(got, ref) < 2e-3, n
 
 
 def test_smoothing_golden():
