@@ -7,7 +7,7 @@ import ctypes
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("KCCOT_LIB", os.path.join(_HERE, "libkccot.so"))
+LIB_PATH = os.path.join(_HERE, "libkccot.so")
 
 PATH_AUTO, PATH_SIMT, PATH_TCGEN05, FLAG_ACCUMULATE = 0, 1, 2, 16
 SHARD_FLAGS_PER_RANK = 256          # KCCOT_SHARD_FLAGS_PER_RANK of include/kccot.h

@@ -1,10 +1,6 @@
 """Build libkccot.so (all CUDA sources under csrc/) for sm_100a, in-tree.
 
-    python -m kccotgan_b200.build [--force] [--verbose] [--dev]
-
-`--dev` builds libkccot_dev.so instead: the same sources with -DKCCOT_DEV, which adds the development probes
-(csrc/debug_probe.cu: kccot_debug_*), the clock64 timeline of the gradient GEMM and the A/B switches.  The
-product library carries none of them.  Scripts select it with KCCOT_LIB=kccotgan_b200/libkccot_dev.so.
+    python -m kccotgan_b200.build [--force] [--verbose]
 
 nvcc cross-compiles without a GPU; the .so is git-ignored but travels to the GPU box with the
 repo snapshot.  Objects are rebuilt only when their source (or any header) is newer.
@@ -18,7 +14,6 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 BUILD = os.path.join(HERE, "csrc", "build")
 LIB = os.path.join(HERE, "libkccot.so")
-LIB_DEV = os.path.join(HERE, "libkccot_dev.so")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo",
          "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr", "-Xptxas", "-v"]
@@ -34,9 +29,9 @@ def _headers_mtime():
     return max(os.path.getmtime(h) for h in hs)
 
 
-def _compile(src, verbose, dev=False):
-    obj = os.path.join(BUILD, src[:-3] + (".dev.o" if dev else ".o"))
-    cmd = [NVCC, *FLAGS, *(["-DKCCOT_DEV"] if dev else []), "-c", os.path.join(CSRC, src), "-o", obj]
+def _compile(src, verbose):
+    obj = os.path.join(BUILD, src[:-3] + ".o")
+    cmd = [NVCC, *FLAGS, "-c", os.path.join(CSRC, src), "-o", obj]
     r = subprocess.run(cmd, capture_output=True, text=True)
     log = r.stdout + r.stderr
     with open(obj + ".log", "w") as f:
@@ -48,27 +43,26 @@ def _compile(src, verbose, dev=False):
     return obj
 
 
-def build(force=False, verbose=False, dev=False):
+def build(force=False, verbose=False):
     os.makedirs(BUILD, exist_ok=True)
     hm = _headers_mtime()
     todo, objs = [], []
-    lib = LIB_DEV if dev else LIB
     for src in _sources():
-        obj = os.path.join(BUILD, src[:-3] + (".dev.o" if dev else ".o"))
+        obj = os.path.join(BUILD, src[:-3] + ".o")
         objs.append(obj)
         newest = max(os.path.getmtime(os.path.join(CSRC, src)), hm)
         if force or not os.path.exists(obj) or os.path.getmtime(obj) < newest:
             todo.append(src)
     if todo:
         with ThreadPoolExecutor(max_workers=min(8, len(todo))) as ex:
-            list(ex.map(lambda s: _compile(s, verbose, dev), todo))
-    if todo or not os.path.exists(lib):
-        cmd = [NVCC, "-shared", "-o", lib, *objs, "-lcudart"]
+            list(ex.map(lambda s: _compile(s, verbose), todo))
+    if todo or not os.path.exists(LIB):
+        cmd = [NVCC, "-shared", "-o", LIB, *objs, "-lcudart"]
         r = subprocess.run(cmd, capture_output=True, text=True)
         if r.returncode != 0:
             raise RuntimeError("link failed:\n" + r.stdout + r.stderr)
-    return lib
+    return LIB
 
 
 if __name__ == "__main__":
-    print(build(force="--force" in sys.argv, verbose="--verbose" in sys.argv, dev="--dev" in sys.argv))
+    print(build(force="--force" in sys.argv, verbose="--verbose" in sys.argv))

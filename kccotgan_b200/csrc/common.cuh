@@ -32,27 +32,9 @@ inline void count_launch(int n = 1) { g_launches.fetch_add((unsigned long long)n
     }                                                                                     \
   } while (0)
 
-#ifdef KCCOT_DEV
-// development build: KCCOT_SYNC_EACH=1 synchronises after every launch and logs its source line (finds the kernel
-// that does not come back)
-inline void dev_sync_each(const char* file, int line) {
-  static const bool on = getenv("KCCOT_SYNC_EACH") != nullptr;
-  if (!on) return;
-  fprintf(stderr, "[kccot] launched %s:%d ...", file, line);
-  fflush(stderr);
-  cudaError_t e = cudaDeviceSynchronize();
-  fprintf(stderr, " done (%s)\n", cudaGetErrorString(e));
-  fflush(stderr);
-}
-#define KCCOT_DEV_SYNC() ::kccot::dev_sync_each(__FILE__, __LINE__)
-#else
-#define KCCOT_DEV_SYNC() do { } while (0)
-#endif
-
 #define KCCOT_LAUNCH_CHECK()                                                             \
   do {                                                                                   \
     ::kccot::count_launch();                                                             \
-    KCCOT_DEV_SYNC();                                                                    \
     cudaError_t _e = cudaGetLastError();                                                 \
     if (_e != cudaSuccess) {                                                             \
       ::kccot::set_error("kernel launch failed: %s (%s:%d)", cudaGetErrorString(_e),      \
@@ -96,10 +78,6 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-#ifdef KCCOT_DEV
-  static const bool no_pdl = getenv("KCCOT_NO_PDL") != nullptr;      // development build: A/B switch
-  if (no_pdl) cfg.numAttrs = 0;
-#endif
   return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
 }
 int num_sms();

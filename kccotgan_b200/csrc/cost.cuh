@@ -66,9 +66,6 @@ int launch_sqdist_partials_tc(const float* x, const float* y, int nprob, int Bx,
 
 // grad_tcgen05.cu — tensor-core adjoint over the stacked rows z = [x; y] (see the file header).
 // Wws: tc_grad_ws_bytes(nprob) of scratch for the W' images.  gx / gy may be null.
-#ifdef KCCOT_DEV
-void set_grad_trace(long long* b);
-#endif
 bool tc_grad_supported(const float* x, const float* y, int Bx, int By, long long K, const float* gx,
                        const float* gy);
 size_t tc_grad_ws_bytes(int nprob);      // scratch of the two launchers below (W' images)
@@ -80,13 +77,12 @@ int launch_grad_pair_tc(const float* Cbar, const float* x, const float* y, int n
 // ------------------------------------------------------------------------------------------------
 // Large-batch path (B > 64): gemm_f16x3.cu / large_prep.cu / large_abi.cu
 // ------------------------------------------------------------------------------------------------
-#define G3_BM 128
-#define G3_BN 256
+#define G3_BN 256        // square output tile of gemm_f16x3.cu (large_prep.cu reads it for the symmetric blocks)
 #define G3_BK 64
 struct G3Job {
   int a_row0, b_row0;      // first row of this block in the A / B operand arrays
   int m, n;                // valid rows / columns of the block
-  int tm, tn, ntiles;      // filled by g3_count_tiles
+  int tm, tn, ntiles;      // filled by g3_count_tiles_pair
   int tri;                 // symmetric block (a_row0 == b_row0): only tiles touching the upper triangle
   float* out;              // [ksplit][m][ld]
   long long ld, ks_stride;
@@ -100,17 +96,13 @@ struct G3Params {
   const float* alpha_dev;  // optional device scalar multiplied into alpha
   int accumulate;          // add into `out` instead of overwriting it
 };
-int g3_count_tiles(G3Job* jb);
-int g3_count_tiles_pair(G3Job* jb);     // 256 x 256 tiles of the CTA-pair kernel (gemm_f16x3_2cta.cu)
-// `units`: CTAs (single-CTA kernel) or clusters (pair kernel) to fill
+int g3_count_tiles_pair(G3Job* jb);     // 256 x 256 tiles of the CTA-pair kernel
+// `units`: clusters to fill
 void g3_plan_split(int ntiles, int nkb, int units, int* ksplit, int* kb_per_split);
+// A*: [a_rows][a_pitch] fp16 (hi, lo), B*: [b_rows][b_pitch]; contraction over `kdim` leading columns
 int launch_gemm_f16x3_pair(const __half* A1, const __half* A2, long long a_rows, long long a_pitch_elems,
                            const __half* B1, const __half* B2, long long b_rows, long long b_pitch_elems, long long kdim,
                            G3Params P, cudaStream_t st);
-// A*: [a_rows][a_pitch] fp16 (hi, lo), B*: [b_rows][b_pitch]; contraction over `kdim` leading columns
-int launch_gemm_f16x3(const __half* A1, const __half* A2, long long a_rows, long long a_pitch_elems,
-                      const __half* B1, const __half* B2, long long b_rows, long long b_pitch_elems, long long kdim,
-                      G3Params P, cudaStream_t st);
 
 // large_abi.cu: true when the large-batch path takes the shape
 bool large_path_wanted(int Bx, int By, bool same);
@@ -134,7 +126,5 @@ int large_shard_cost_bwd(const float* Cbar3rows, const float* XYcol, const float
                          int Brows, const float* h_fake, const float* m_real, const float* h_real, const float* m_fake,
                          int T, int J, float s, float* g_fake_rows, float* gh_fake_rows, float* gm_real_part,
                          float* gh_real_rows, float* gm_fake_part, void* ws, size_t ws_bytes, cudaStream_t st);
-void large_set_drain(int k_blocks);
-void large_set_pair(int use_pair);
 
 }  // namespace kccot

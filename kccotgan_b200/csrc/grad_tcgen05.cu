@@ -113,8 +113,7 @@ __global__ void __launch_bounds__(128) build_w_image_kernel(const float* __restr
 __global__ void __launch_bounds__(kThreads, 1)
 grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUtensorMap tmy,
                const __grid_constant__ CUtensorMap tmo, int Bx, int By, long long K, const float* __restrict__ Wimg,
-               int rb, int N, float neg2s, int accumulate, int nstages, int ctx_period, int ctx_len,
-               long long* __restrict__ trace) {
+               int rb, int N, float neg2s, int accumulate, int nstages, int ctx_period, int ctx_len) {
   extern __shared__ uint8_t smem_raw[];
   // align by OFFSET so that the compiler keeps the shared address space (LDS/STS, not generic LD/ST)
   uint8_t* base = smem_raw + ((1024u - (tc::smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -128,14 +127,6 @@ grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ 
   Bars& bars = *reinterpret_cast<Bars*>(obuf + 2 * kObufBytes);
 
   const int p = blockIdx.y;
-#ifdef KCCOT_DEV
-  const bool tr = (trace != nullptr) && blockIdx.x == 1 && blockIdx.y == 0;   // development timeline of one CTA
-#define KTRACE(role, ev) do { if (tr && trn < 64) trace[((role) * 64 + trn) * 2 + (ev)] = clock64(); } while (0)
-#else
-  (void)trace;                  // the timeline exists only in the development build (python -m kccotgan_b200.build --dev)
-#define KTRACE(role, ev) do { } while (0)
-#endif
-  int trn = 0;
   // Shared-context hint (ctx_len != 0): the column tiles whose index modulo ctx_period is below ctx_len are skipped
   // altogether (their gradient rows are constants of the caller); the loops run over the ACTIVE tiles and
   // tile_of() maps an active index to its column tile.
@@ -216,10 +207,8 @@ grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ 
           if (rows == 0) continue;
           const CUtensorMap* tm = half ? &tmy : &tmx;
           tc::mbar_wait(&bars.empty[stage], phase ^ 1);
-          KTRACE(0, 0);
           tc::mbar_arrive_expect_tx(&bars.full[stage], (uint32_t)(rows * 128));
           tc::tma_load_3d(tm, &bars.full[stage], st_hi + (size_t)stage * stage_bytes, col0, 0, p);
-          KTRACE(0, 1); ++trn;
           if (++stage == nstages) { stage = 0; phase ^= 1; }
         }
       }
@@ -249,7 +238,6 @@ grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ 
           if (rows == 0) continue;
           const uint32_t a_w = tmem + (uint32_t)(half ? Bx : 0);           // W' columns of this half
           tc::mbar_wait(&bars.conv[stage], phase);
-          KTRACE(1, 0);
           tc::tc_fence_after();
           // N-major B over two atoms: columns 0-31 = Zhi box, 32-63 = Zlo box (LBO apart); 4-row swizzle
           // atoms 512 B apart, 8 contraction rows per k-step
@@ -264,7 +252,6 @@ grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ 
             }
           }
           tc::umma_commit(&bars.empty[stage]);
-          KTRACE(1, 1); ++trn;
           if (++stage == nstages) { stage = 0; phase ^= 1; }
         }
         tc::umma_commit(&bars.acc_full[ab]);
@@ -281,7 +268,7 @@ grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ 
     // converted before box n - 1 had landed, full[slot(n-1)] still showed the phase before box n - 1, whose parity is
     // the one box n + 8 waits for: the wait passed, the warp converted a slot that was being filled and arrived on
     // conv[] a pass early, and the barriers of the ring went out of step for good (the kernel hung about once in a
-    // few hundred thousand CTAs, found with the development build's bounded waits).
+    // few hundred thousand CTAs; DESIGN.md records how it was found).
     const int cw = warp - 2;
     if (cw < nstages) {
       const int nhalves = (Bx ? 1 : 0) + (By ? 1 : 0);
@@ -293,7 +280,6 @@ grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ 
         const int half = nhalves == 2 ? (int)(n & 1) : (Bx ? 0 : 1);
         const int rows = half ? By : Bx;
         tc::mbar_wait(&bars.full[cw], phase);
-        if (cw == 0 && lane == 0) KTRACE(2, 0);
         const int n16 = rows * 8;                           // 16-byte units in this box (multiple of 64)
         for (int e0 = lane; e0 < n16; e0 += 32 * 4) {
           float4 v[4];
@@ -322,7 +308,6 @@ grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ 
         tc::fence_proxy_async_smem();
         __syncwarp();
         if (lane == 0) tc::mbar_arrive(&bars.conv[cw]);
-        if (cw == 0 && lane == 0) { KTRACE(2, 1); ++trn; }
       }
     }
   } else {
@@ -340,7 +325,6 @@ grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ 
     int ob = 0;
     for (long long t = t_begin; t < t_end; ++t) {
       tc::mbar_wait(&bars.acc_full[ab], ab_phase);
-      if (issuer) KTRACE(3, 0);
       tc::tc_fence_after();
       float d[32];
       if (active) {
@@ -355,32 +339,25 @@ grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ 
           d[j] = neg2s * (mine + __shfl_down_sync(0xffffffffu, mine, 16));
         }
       }
-      if (issuer) KTRACE(4, 0);      // tmem loaded
       tc::tc_fence_before();
       __syncwarp();
       if (lane == 0) tc::mbar_arrive(&bars.acc_empty[ab]); // the accumulator is free as soon as it is in registers
       // the staging buffer `ob` was last read by the TMA store issued two tiles ago
       if (issuer) tc::tma_store_wait_read<1>();
-      if (issuer) KTRACE(4, 1);      // wait_read done
       tc::named_bar_sync(2, kEpiWarps * 32);
-      if (issuer) KTRACE(5, 0);      // barrier A passed
       if (active && hi_lane && r < N) {
         const uint32_t row = tc::smem_u32(obuf + ob * kObufBytes) + r * 128;
 #pragma unroll
         for (int j = 0; j < 8; ++j)
           tc::sts128(row + ((j ^ (r & 7)) << 4), make_float4(d[4 * j], d[4 * j + 1], d[4 * j + 2], d[4 * j + 3]));
       }
-      if (issuer) KTRACE(5, 1);      // staged
       tc::fence_proxy_async_smem();
-      if (issuer) KTRACE(6, 0);      // fenced
       tc::named_bar_sync(2, kEpiWarps * 32);
-      if (issuer) KTRACE(6, 1);      // barrier B passed
       if (issuer) {
         const int col0 = (int)(tile_of(t) * kCols);
         if (accumulate) tc::tma_reduce_add_3d(&tmo, obuf + ob * kObufBytes, col0, 0, p);
         else tc::tma_store_3d(&tmo, obuf + ob * kObufBytes, col0, 0, p);
         tc::tma_store_commit();
-        KTRACE(3, 1); ++trn;
       }
       ob ^= 1;
       if (++ab == kAccBufs) { ab = 0; ab_phase ^= 1; }
@@ -392,11 +369,6 @@ grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ 
   if (warp == 1) tc::tmem_dealloc(tmem, kTmemCols);
 }
 
-#ifdef KCCOT_DEV
-static long long* g_grad_trace = nullptr;     // set through kccot_debug_set_grad_trace (development build only)
-#else
-static constexpr long long* g_grad_trace = nullptr;
-#endif
 struct GradPlan { int nstages; size_t smem; };
 GradPlan plan_grad(int Bx, int By, int N) {
   (void)N;
@@ -411,10 +383,6 @@ GradPlan plan_grad(int Bx, int By, int N) {
   return g;
 }
 }  // namespace
-
-#ifdef KCCOT_DEV
-void set_grad_trace(long long* b) { g_grad_trace = b; }
-#endif
 
 bool tc_grad_supported(const float* x, const float* y, int Bx, int By, long long K, const float* gx, const float* gy) {
   if (Bx % 8 || By % 8 || Bx + By > 128 || Bx > kMaxN || By > kMaxN || Bx < 8 || By < 8) return false;
@@ -462,7 +430,7 @@ static int launch_grad_rows(const CUtensorMap& tmx, const CUtensorMap& tmy, cons
   if (gx < 1) gx = 1;
   dim3 grid(gx, nprob);
   KCCOT_CUDA(launch_pdl(grad_tc_kernel, grid, dim3(kThreads), g.smem, st, tmx, tmy, tmo, Bx, By, K, img, rb, N,
-                        -2.f * s, accumulate, g.nstages, ctx_period, ctx_len, g_grad_trace));
+                        -2.f * s, accumulate, g.nstages, ctx_period, ctx_len));
   KCCOT_LAUNCH_CHECK();
   return KCCOT_OK;
 }
@@ -502,12 +470,3 @@ int launch_grad_pair_tc(const float* Cbar, const float* x, const float* y, int n
 }
 
 }  // namespace kccot
-
-#ifdef KCCOT_DEV
-// development build only: device buffer of 4 roles x 64 records x 2 timestamps (clock64) filled by CTA 1
-extern "C" void kccot_debug_set_grad_trace(long long* buf) { kccot::set_grad_trace(buf); }
-// development build only: bounded barrier waits of THIS translation unit report into `buf` (see tc_common.cuh)
-extern "C" int kccot_debug_set_wait_log(unsigned long long* buf) {
-  return (int)cudaMemcpyToSymbol(kccot::tc::s_wait_log, &buf, sizeof(buf));
-}
-#endif

@@ -7,9 +7,6 @@
 namespace kccot {
 
 namespace {
-int g_drain = 0;        // k-blocks per accumulation chunk of the GEMM; 0 = the kernel's default (development knob)
-bool g_pair = true;     // CTA-pair kernel (gemm_f16x3_2cta.cu); false: single-CTA 128 x 256 tiles (development knob)
-
 struct Carver {
   char* base;
   size_t off = 0;
@@ -61,8 +58,8 @@ FwdWs carve_fwd(void* ws, int Bx, int By, long long K, bool same, bool mixed) {
     w.job[0] = G3Job{0, Bx, Bx, By, 0, 0, 0, 0, nullptr, By, 0};
   }
   int ntiles = 0;
-  for (int j = 0; j < w.njobs; ++j) ntiles += g_pair ? g3_count_tiles_pair(&w.job[j]) : g3_count_tiles(&w.job[j]);
-  g3_plan_split(ntiles, (int)(w.Kp / G3_BK), g_pair ? num_sms() / 2 : num_sms(), &w.ksplit, &w.kb_per_split);
+  for (int j = 0; j < w.njobs; ++j) ntiles += g3_count_tiles_pair(&w.job[j]);
+  g3_plan_split(ntiles, (int)(w.Kp / G3_BK), num_sms() / 2, &w.ksplit, &w.kb_per_split);
   Carver c(ws);
   w.scal = c.take<float>(kScalCount);
   w.part = c.take<float>((size_t)w.nseg * K);
@@ -121,11 +118,9 @@ int run_fwd(const FwdWs& w, const float* x, const float* y, int Bx, int By, long
   P.njobs = w.njobs;
   P.ksplit = w.ksplit;
   P.kb_per_split = w.kb_per_split;
-  P.drain = g_drain;
   P.alpha = 1.f;
   P.alpha_dev = nullptr;
-  if (g_pair) return launch_gemm_f16x3_pair(w.Zh1, w.Zh2, R, w.Kp, w.Zh1, w.Zh2, R, w.Kp, K, P, st);
-  return launch_gemm_f16x3(w.Zh1, w.Zh2, R, w.Kp, w.Zh1, w.Zh2, R, w.Kp, K, P, st);
+  return launch_gemm_f16x3_pair(w.Zh1, w.Zh2, R, w.Kp, w.Zh1, w.Zh2, R, w.Kp, K, P, st);
 }
 
 int run_bwd_rows(const BwdWs& w, const float* Cxx, const float* Cxy, const float* Cyy, int Bx, int By, long long K, float s,
@@ -136,22 +131,16 @@ int run_bwd_rows(const BwdWs& w, const float* Cxx, const float* Cxy, const float
     return rc;
   G3Params P{};
   P.job[0] = G3Job{0, 0, nrows, (int)K, 0, 0, 0, 0, g, K, 0};
-  if (g_pair) g3_count_tiles_pair(&P.job[0]);
-  else g3_count_tiles(&P.job[0]);
+  g3_count_tiles_pair(&P.job[0]);
   P.njobs = 1;
   P.ksplit = 1;
   P.kb_per_split = (int)(w.Rp / G3_BK);
-  P.drain = g_drain;
   P.alpha = -2.f * s;
   P.alpha_dev = w.scal + kScalGradAlpha;
   P.accumulate = accumulate;
-  if (g_pair) return launch_gemm_f16x3_pair(w.Wh1, w.Wh2, nrows, w.Rp, w.ZT1, w.ZT2, K, w.Rp, R, P, st);
-  return launch_gemm_f16x3(w.Wh1, w.Wh2, nrows, w.Rp, w.ZT1, w.ZT2, K, w.Rp, R, P, st);
+  return launch_gemm_f16x3_pair(w.Wh1, w.Wh2, nrows, w.Rp, w.ZT1, w.ZT2, K, w.Rp, R, P, st);
 }
 }  // namespace
-
-void large_set_drain(int k_blocks) { g_drain = k_blocks > 0 ? k_blocks : 0; }
-void large_set_pair(int use_pair) { g_pair = use_pair != 0; }
 
 bool large_path_wanted(int Bx, int By, bool same) { return (same ? Bx : Bx + By) > 128; }
 
@@ -284,16 +273,11 @@ int large_shard_cost_fwd(const float* real, const float* fake, int B, long long 
   P.job[1] = G3Job{row0, 0, Brows, B, 0, 0, 0, 0, w.P[1], B, 0};
   P.job[2] = G3Job{B + row0, B, Brows, B, 0, 0, 0, 0, w.P[2], B, 0};
   P.njobs = 3;
-  int ntiles = 0;
-  for (int j = 0; j < 3; ++j) ntiles += g_pair ? g3_count_tiles_pair(&P.job[j]) : g3_count_tiles(&P.job[j]);
-  (void)ntiles;
+  for (int j = 0; j < 3; ++j) g3_count_tiles_pair(&P.job[j]);
   P.ksplit = 1;
   P.kb_per_split = (int)(w.Kp / G3_BK);
-  P.drain = g_drain;
   P.alpha = 1.f;
-  if (int rc = g_pair ? launch_gemm_f16x3_pair(w.Zh1, w.Zh2, R, w.Kp, w.Zh1, w.Zh2, R, w.Kp, K, P, st)
-                      : launch_gemm_f16x3(w.Zh1, w.Zh2, R, w.Kp, w.Zh1, w.Zh2, R, w.Kp, K, P, st))
-    return rc;
+  if (int rc = launch_gemm_f16x3_pair(w.Zh1, w.Zh2, R, w.Kp, w.Zh1, w.Zh2, R, w.Kp, K, P, st)) return rc;
   const long long RB = (long long)Brows * B, hm = (long long)T * J;
   LargeFin F{};
   F.b[0] = LargeFinBlock{w.P[0], B, RB, 1, 0, w.norms + row0, w.norms + B, h_fake + row0 * hm, m_real, nullptr, nullptr,
@@ -329,17 +313,14 @@ int large_shard_cost_bwd(const float* Cbar3rows, const float* XYcol, const float
     return rc;
   G3Params P{};
   P.job[0] = G3Job{0, 0, Brows, (int)K, 0, 0, 0, 0, g_fake_rows, K, 0};
-  if (g_pair) g3_count_tiles_pair(&P.job[0]);
-  else g3_count_tiles(&P.job[0]);
+  g3_count_tiles_pair(&P.job[0]);
   P.njobs = 1;
   P.ksplit = 1;
   P.kb_per_split = (int)(w.Rp / G3_BK);
-  P.drain = g_drain;
   P.alpha = -2.f * s;
   P.alpha_dev = w.scal + kScalGradAlpha;
   const int R = 2 * B;
-  if (g_pair) return launch_gemm_f16x3_pair(w.Wh1, w.Wh2, Brows, w.Rp, w.ZT1, w.ZT2, K, w.Rp, R, P, st);
-  return launch_gemm_f16x3(w.Wh1, w.Wh2, Brows, w.Rp, w.ZT1, w.ZT2, K, w.Rp, R, P, st);
+  return launch_gemm_f16x3_pair(w.Wh1, w.Wh2, Brows, w.Rp, w.ZT1, w.ZT2, K, w.Rp, R, P, st);
 }
 
 }  // namespace kccot

@@ -22,25 +22,12 @@
 // back one iteration and continues, for the rest of the solve, with the plain log-domain updates with
 // max subtraction — the reference's formulation.  The backward switches to direct exponentials before
 // any rank-one factor would leave 2^+-60.
-#include <stdlib.h>
-
 #include <type_traits>
 
 #include "common.cuh"
 #include "sinkhorn.cuh"
 
 namespace kccot {
-
-// Development-only phase timeline (build with -DKCCOT_SK_TRACE; scripts/sk_trace.py reads it).
-#ifdef KCCOT_SK_TRACE
-__device__ long long g_sk_trace[2][16];
-#define SK_STAMP(kern, idx)                                                          \
-  do {                                                                               \
-    if (blockIdx.x == 0 && threadIdx.x == 0) g_sk_trace[kern][idx] = clock64();      \
-  } while (0)
-#else
-#define SK_STAMP(kern, idx)
-#endif
 
 namespace {
 constexpr float kBig = 1e30f;      // padding cost: exp2(anything - kBig) == 0, and 0 * kBig == 0
@@ -49,9 +36,9 @@ constexpr float kHi = 1.2e27f;     // ~2^90
 constexpr float kExpLim = 60.f;    // |log2| allowed for a backward rank-one factor
 
 // Lanes per row (and per column): a row of the B x B problem is split over LPR adjacent lanes, EPT elements
-// each.  EPT = 8 / 16: four lanes (B <= 32 / 64); EPT = 32: two lanes (B <= 64) — one shuffle instead of two
-// and a 4-warp barrier instead of an 8-warp one: 478 against 569 cycles per iteration in
-// scripts/matvec_probe.py.
+// each.  EPT = 8: four lanes (B <= 32); EPT = 16: four lanes (B <= 64, backward); EPT = 32: two lanes (B <= 64,
+// forward) — one shuffle instead of two and a 4-warp barrier instead of an 8-warp one: 478 against 569 cycles
+// per iteration of a bare mat-vec loop on a B200 (DESIGN.md §5).
 __host__ __device__ constexpr int lpr_of(int ept) { return ept == 32 ? 2 : 4; }
 
 template <int LPR>
@@ -269,14 +256,12 @@ __global__ void __launch_bounds__(lpr_of(EPT) * lpr_of(EPT) * EPT) sinkhorn_fwd_
   const float ahat = -log2f((float)B);
   const float two_ahat = 1.f / (float)B;
   float Cr[EPT], Cc[EPT], Kr[EPT], Kc[EPT];
-  SK_STAMP(0, 0);
   pdl_wait();                    // C comes from the kernel before (cost_finalize_kernel in the fused path)
   pdl_launch_dependents();       // the backward kernel may load its cost slices while this one iterates
   const float* Cn = C + (long long)n * B * B;
   const bool via_tile = HS && (B & 3) == 0 && (reinterpret_cast<uintptr_t>(Cn) & 15) == 0;
   const float c0 = via_tile ? load_slices_tile<EPT>(Cn, B, kscale, red, Cr, Cc, hist)      // the history region is still free
                             : load_slices<EPT>(Cn, B, kscale, red, Cr, Cc);
-  SK_STAMP(0, 1);
   float* uh = u_hist + (long long)n * (L + 1) * B;
   float* vh = v_hist + (long long)n * (L + 1) * B;
   float* Uh = hist;
@@ -316,7 +301,6 @@ __global__ void __launch_bounds__(lpr_of(EPT) * lpr_of(EPT) * EPT) sinkhorn_fwd_
 
   const float ahat_alpha = ahat + alpha;
   float u_cur = 0.f;            // uhat of this thread's row (all four lanes of a row hold it)
-  SK_STAMP(0, 2);
   bool slow = false;
   int it = 0, nits = 0;
   // iterations before `first_check` can never stop (gan_utils.py:159 needs nits >= Lmin, :116 needs the
@@ -484,7 +468,6 @@ __global__ void __launch_bounds__(lpr_of(EPT) * lpr_of(EPT) * EPT) sinkhorn_fwd_
     }
     break;
   }
-  SK_STAMP(0, 3);
   // ---- sharp cost sum(pi * C) ---------------------------------------------------------------
   float s1 = 0.f, s0 = 0.f;
   {
@@ -514,7 +497,6 @@ __global__ void __launch_bounds__(lpr_of(EPT) * lpr_of(EPT) * EPT) sinkhorn_fwd_
       }
     }
   }
-  SK_STAMP(0, 4);
   if (HS) {
     const int total = (nits + 1) * B;
     if (B == BM && ((reinterpret_cast<uintptr_t>(uh) | reinterpret_cast<uintptr_t>(vh)) & 15) == 0) {
@@ -537,7 +519,6 @@ __global__ void __launch_bounds__(lpr_of(EPT) * lpr_of(EPT) * EPT) sinkhorn_fwd_
       }
     }
   }
-  SK_STAMP(0, 5);
 }
 
 // HS = true: the whole potential history (nits+1 rows of u and v) is copied to shared memory up
@@ -571,11 +552,9 @@ __global__ void __launch_bounds__(lpr_of(EPT) * lpr_of(EPT) * EPT, MINB) sinkhor
   const float kscale = kLog2e / eps;
   const float ahat = -log2f((float)B);
   float Cr[EPT], Cc[EPT], Kr[EPT], Kc[EPT], Gr[EPT], Gc[EPT];
-  SK_STAMP(1, 0);
   load_slices<EPT>(C + (long long)n * B * B, B, kscale, red, Cr, Cc);   // C predates the forward kernel: safe before the wait
   pdl_wait();                    // history, nits, upstream gradient come from the kernels before
   pdl_launch_dependents();       // the gradient GEMM may start streaming the videos now
-  SK_STAMP(1, 1);
   const float* uh = u_hist + (long long)n * (L + 1) * B;
   const float* vh = v_hist + (long long)n * (L + 1) * B;
   const int nits = nits_in[n];
@@ -594,7 +573,6 @@ __global__ void __launch_bounds__(lpr_of(EPT) * lpr_of(EPT) * EPT, MINB) sinkhor
     vn_s[tp] = vh[(long long)nits * B + tid];
   }
   __syncthreads();
-  SK_STAMP(1, 2);
   if (HS) {
     // copy the history; remember the last step whose potentials are further than 2^60 from the
     // absorption reference (steps k <= k_slow + 1 use direct exponentials).  All loads of a thread are
@@ -672,7 +650,6 @@ __global__ void __launch_bounds__(lpr_of(EPT) * lpr_of(EPT) * EPT, MINB) sinkhor
     }
   }
   __syncthreads();
-  SK_STAMP(1, 3);
   const float un_i = un_s[ip], vn_i = vn_s[ip];    // row i / column i of this thread
   // ---- adjoint seeds.  cost = sum(pi*C) = sum(pi*(C - c0)) + c0*sum(pi), and sum(pi) == 1 identically
   // in the inputs (the last v-update normalises every column of pi to 1/B), so the c0 term has zero
@@ -709,7 +686,6 @@ __global__ void __launch_bounds__(lpr_of(EPT) * lpr_of(EPT) * EPT, MINB) sinkhor
   const uint32_t ga_i = pin_u32(sa(&ga[ip])), gb_i = pin_u32(sa(&gb[ip]));
   const uint32_t Uh_i = pin_u32(sa(HS ? &Uh[ip] : &Us[0][ip])), Vh_i = pin_u32(sa(HS ? &Vh[ip] : &Vs[0][ip]));
 
-  SK_STAMP(1, 4);
   int k = nits;
   if (HS) {
     // ---- fast steps (all potentials within 2^60 of the absorption reference): a loop with nothing but
@@ -762,7 +738,6 @@ __global__ void __launch_bounds__(lpr_of(EPT) * lpr_of(EPT) * EPT, MINB) sinkhor
       __syncthreads();
     }
   }
-  SK_STAMP(1, 5);
   bool slow = false;
   for (; k >= 1; --k) {
     const int b = k & 1;
@@ -863,7 +838,6 @@ __global__ void __launch_bounds__(lpr_of(EPT) * lpr_of(EPT) * EPT, MINB) sinkhor
     }
     __syncthreads();
   }
-  SK_STAMP(1, 6);
   // ---- Cbar = g * (Gr + Gc^T) ---------------------------------------------------------------
   float* out = Cbar + (long long)n * B * B;
   if (HS) {
@@ -906,18 +880,6 @@ __global__ void __launch_bounds__(lpr_of(EPT) * lpr_of(EPT) * EPT, MINB) sinkhor
       }
     }
   }
-  SK_STAMP(1, 7);
-}
-
-// forward, 32 < B <= 64: two lanes per row; the development build (KCCOT_DEV) can select the four-lane mapping
-// with KCCOT_SK_LANES=4 for A/B timing
-static bool four_lanes() {
-#ifdef KCCOT_DEV
-  static const bool v = [] { const char* e = getenv("KCCOT_SK_LANES"); return e && atoi(e) == 4; }();
-  return v;
-#else
-  return false;
-#endif
 }
 
 template <int EPT>
@@ -947,8 +909,6 @@ int launch_sinkhorn_fwd_small(const float* C, int nsolve, int B, float eps, int 
   const int t4 = ((4 * B + 31) / 32) * 32, t2 = ((2 * B + 31) / 32) * 32;
   if (B <= 32)
     return launch_fwd_t<8>(C, nsolve, B, eps, L, Lmin, thresh, exit_on_index, u_hist, v_hist, nits, cost, t4, st, mix);
-  if (four_lanes())
-    return launch_fwd_t<16>(C, nsolve, B, eps, L, Lmin, thresh, exit_on_index, u_hist, v_hist, nits, cost, t4, st, mix);
   return launch_fwd_t<32>(C, nsolve, B, eps, L, Lmin, thresh, exit_on_index, u_hist, v_hist, nits, cost, t2, st, mix);
 }
 
@@ -990,9 +950,3 @@ int launch_sinkhorn_bwd_small(const float* C, int nsolve, int B, float eps, int 
 }
 
 }  // namespace kccot
-
-#ifdef KCCOT_SK_TRACE
-extern "C" int kccot_debug_sk_trace(long long* host_out) {
-  return (int)cudaMemcpyFromSymbol(host_out, kccot::g_sk_trace, sizeof(kccot::g_sk_trace));
-}
-#endif

@@ -48,65 +48,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
       "r"(parity)
       : "memory");
 }
-#ifdef KCCOT_DEV
-// Development build: bounded waits.  When a wait-log buffer is set (kccot_debug_set_wait_log, per translation unit),
-// a wait that has not completed after 0.3 s records {globaltimer, block/thread, barrier address/parity, source line,
-// raw barrier word} and returns; log[1] becomes an abort flag that makes every later wait give up at once.  The
-// kernel then finishes with garbage and the host reads where it was stuck.  log[0] = number of records (6 words each,
-// from word 8).
-static __device__ unsigned long long* s_wait_log = nullptr;
-__device__ __forceinline__ unsigned long long globaltimer_ns() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
-static __device__ __noinline__ void wait_log_record(uint32_t a, uint32_t parity, int line, unsigned long long now, int aborted) {
-  unsigned long long* log = s_wait_log;
-  unsigned long long raw;
-  asm volatile("ld.shared.b64 %0, [%1];" : "=l"(raw) : "r"(a));
-  const unsigned long long slot = atomicAdd(log, 1ull);
-  if (slot < 4000) {
-    unsigned long long* r = log + 8 + slot * 6;
-    r[0] = now;
-    r[1] = (unsigned long long)blockIdx.x | ((unsigned long long)blockIdx.y << 16) | ((unsigned long long)threadIdx.x << 32) |
-           ((unsigned long long)aborted << 48);
-    r[2] = (unsigned long long)a | ((unsigned long long)parity << 32);
-    r[3] = (unsigned long long)line;
-    r[4] = raw;
-    unsigned smid;
-    asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-    r[5] = smid;
-  }
-  atomicExch(log + 1, 1ull);
-  __threadfence();
-}
-__device__ __forceinline__ void mbar_wait_dev(uint64_t* bar, uint32_t parity, int line) {
-  const uint32_t a = smem_u32(bar);
-  unsigned long long t0 = 0;
-  for (uint32_t spins = 0;; ++spins) {
-    uint32_t done;
-    asm volatile(
-        "{\n\t.reg .pred P;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 P, [%1], %2;\n\t"
-        "selp.b32 %0, 1, 0, P;\n\t}"
-        : "=r"(done)
-        : "r"(a), "r"(parity)
-        : "memory");
-    if (done) return;
-    if ((spins & 255u) == 255u && s_wait_log != nullptr) {
-      const unsigned long long now = globaltimer_ns();
-      if (t0 == 0) t0 = now;
-      const bool abort_seen = *reinterpret_cast<volatile unsigned long long*>(s_wait_log + 1) != 0ull;
-      if (now - t0 > 300000000ull || (abort_seen && now - t0 > 1000000ull)) {
-        wait_log_record(a, parity, line, now, abort_seen ? 1 : 0);
-        return;
-      }
-      if (abort_seen && spins > 100000u) return;
-    }
-  }
-}
-#define mbar_wait(bar, par) mbar_wait_dev(bar, par, __LINE__)
-#endif
 // generic-proxy smem writes -> visible to the async proxy (TMA / tcgen05 operand reads)
 __device__ __forceinline__ void fence_proxy_async_smem() {
   asm volatile("fence.proxy.async.shared::cta;" ::: "memory");

@@ -6,7 +6,6 @@ Prints ms and algorithmic TFLOP/s of: mixed cost forward (pre-pass + GEMM + fina
 Sinkhorn backward, mixed cost backward (W' build + transposed split + GEMM + martingale adjoint); checks a
 256 x 256 corner of C_xy against the CUDA-core direct-form kernels.
 """
-import ctypes
 import os
 import sys
 
@@ -25,12 +24,6 @@ def main():
     T, J, L = 20, 8, 100
     dev = torch.device("cuda", 0)
     lib = _lib.load()
-    # development library only (KCCOT_LIB=kccotgan_b200/libkccot_dev.so): KCCOT_G3_DRAIN / KCCOT_G3_PAIR knobs
-    if os.environ.get("KCCOT_G3_DRAIN") or os.environ.get("KCCOT_G3_PAIR"):
-        import ctypes as _c
-        fn = _c.CDLL(_lib.LIB_PATH).kccot_debug_large_config
-        fn(int(os.environ.get("KCCOT_G3_DRAIN", "0")), int(os.environ.get("KCCOT_G3_PAIR", "1")))
-        print("large config: drain", os.environ.get("KCCOT_G3_DRAIN", "0"), "pair", os.environ.get("KCCOT_G3_PAIR", "1"))
     g = torch.Generator(device=dev).manual_seed(1)
     real = torch.rand((B, K), generator=g, device=dev)
     fake = torch.rand((B, K), generator=g, device=dev)
