@@ -21,15 +21,16 @@
 //               B = [Zhi | Zlo]: two N-atoms, LBO = distance between the hi and lo rings.  kind::tf32 reads fp32
 //               words and IGNORES the low 13 mantissa bits, so the raw box serves as Zhi = trunc(Z) as it stands; the
 //               converter warps only write Zlo = Z - trunc(Z) (exact in fp32) into the lo ring.
-//   Stage     = ONE box (8 KB + 8 KB lo at 64 rows): the ring is up to 9 deep, which is what hides the
-//               HBM latency (the first version used two 64 KB stages and starved 44 % of the time).
+//   Stage     = ONE box (8 KB + 8 KB lo at 64 rows): the ring is 5 deep, and with two CTAs per SM 10 boxes are in
+//               flight per SM, which is what hides the HBM latency (the first version used two 64 KB stages and
+//               starved 44 % of the time).
 //   3xTF32 in ONE instruction per k-step (M = 128, N = 64, K = 8).  The elected lane needs ~30-40 cycles per
 //               tcgen05.mma (descriptor moves to uniform registers; measured with the clock64 timeline) and the
 //               earlier two-instruction form (N = 64 for W'hi, N = 32 for W'lo, converter rewriting the hi box
 //               rounded) was shared-memory bound: 136 KB through the port per 24 KB tile (TMA write, converter read /
 //               write, operand reads, output staging), 1 420 cycles per tile.  This one moves 96 KB and its steady
 //               state is the HBM itself: ~1 100 cycles per tile = 22 B/clk per SM = the measured copy peak.  fp32
-//               accumulate in TMEM, 6 accumulator buffers of 64 columns.
+//               accumulate in TMEM, 2 accumulator buffers of 64 columns (256 columns with W': half of an SM's).
 //   Epilogue:   each of the four epilogue warps owns one quadrant: lanes 0-15 add their two column halves, lanes
 //               16-31 hand W'lo.Zhi down by shuffle; 16 rows per warp are staged in 128-byte-swizzled shared memory
 //               and one TMA store (or reduce-add) writes the [N x 32] box as full 128-byte row segments.
@@ -42,20 +43,24 @@ namespace {
 constexpr int kCols = 32;                  // video columns per work tile (UMMA N) = one TMA box
 constexpr int kBoxCols = 32;               // fp32 columns per TMA box (128-byte swizzle row)
 constexpr int kMaxN = 64;                  // output rows per launch
-constexpr int kMaxStages = 9;               // 162 KB: leaves room for a martingale CTA (44 KB) on the same SM; 12 measured no faster
-constexpr int kConvWarps = kMaxStages;      // ONE converter warp per ring slot (see the converter branch for why)
+// Half-SM footprint: two CTAs fit on one SM (shared memory, registers and tensor memory), so a CTA of another
+// evaluation streams while this one sets up or drains.  Two CTAs keep 2 x 5 boxes in flight per SM.
+constexpr int kStages = 5;
+constexpr int kConvWarps = kStages;         // ONE converter warp per ring slot (see the converter branch for why)
 constexpr int kConvThreads = kConvWarps * 32;
 constexpr int kEpiWarps = 4;
-constexpr int kThreads = 64 + kConvThreads + kEpiWarps * 32;   // 480
-constexpr int kAccBufs = 6;
+constexpr int kThreads = 64 + kConvThreads + kEpiWarps * 32;   // 352
+constexpr int kCtasPerSm = 2;
+constexpr int kAccBufs = 2;                // the epilogue needs ~1 000 of a tile's ~1 100 cycles: two buffers keep up
 constexpr int kAccCols = 64;               // per tile: [W.Zhi | W.Zlo], 32 columns each
-constexpr int kTmemCols = 512;             // W' (hi / lo interleaved by lane) [0,128) | 6 accumulator buffers x 64 columns
+constexpr int kTmemCols = 256;             // W' (hi / lo interleaved by lane) [0,128) | 2 accumulator buffers x 64 columns
 constexpr int kTmemAcc0 = 128;
 constexpr bool kRawHi = true;              // the MMA truncates the raw box itself; converters write only the lo box
 constexpr int kObufBytes = kMaxN * 128;     // one staged output tile
+static_assert(kTmemCols >= kTmemAcc0 + kAccBufs * kAccCols && kTmemCols * kCtasPerSm <= 512, "tensor memory");
 
 struct Bars {
-  uint64_t full[kMaxStages], conv[kMaxStages], empty[kMaxStages];
+  uint64_t full[kStages], conv[kStages], empty[kStages];
   uint64_t acc_full[kAccBufs], acc_empty[kAccBufs];
   uint64_t w_ready;                          // W' is in tensor memory (4 loader warps arrive)
   uint32_t tmem_base;
@@ -110,20 +115,20 @@ __global__ void __launch_bounds__(128) build_w_image_kernel(const float* __restr
   im[(lane_hi + 16) * 4] = lo;
 }
 
-__global__ void __launch_bounds__(kThreads, 1)
+__global__ void __launch_bounds__(kThreads, kCtasPerSm)
 grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUtensorMap tmy,
                const __grid_constant__ CUtensorMap tmo, int Bx, int By, long long K, const float* __restrict__ Wimg,
-               int rb, int N, float neg2s, int accumulate, int nstages, int ctx_period, int ctx_len) {
+               int rb, int N, float neg2s, int accumulate, int ctx_period, int ctx_len) {
   extern __shared__ uint8_t smem_raw[];
   // align by OFFSET so that the compiler keeps the shared address space (LDS/STS, not generic LD/ST)
   uint8_t* base = smem_raw + ((1024u - (tc::smem_u32(smem_raw) & 1023u)) & 1023u);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int rows_max = max(Bx, By);
   const int stage_bytes = rows_max * 128;           // one [rows x 32] box
-  // layout: hi[nstages] | lo[nstages] | output staging | barriers   (W' lives in tensor memory)
+  // layout: hi[kStages] | lo[kStages] | output staging | barriers   (W' lives in tensor memory)
   uint8_t* st_hi = base;
-  uint8_t* st_lo = st_hi + (size_t)nstages * stage_bytes;
-  uint8_t* obuf = st_lo + (size_t)nstages * stage_bytes;      // 2 x [64 rows x 128 B] output staging (swizzled)
+  uint8_t* st_lo = st_hi + (size_t)kStages * stage_bytes;
+  uint8_t* obuf = st_lo + (size_t)kStages * stage_bytes;      // 2 x [64 rows x 128 B] output staging (swizzled)
   Bars& bars = *reinterpret_cast<Bars*>(obuf + 2 * kObufBytes);
 
   const int p = blockIdx.y;
@@ -145,7 +150,7 @@ grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ 
     tc::prefetch_tmap(&tmx);
     tc::prefetch_tmap(&tmy);
     tc::prefetch_tmap(&tmo);
-    for (int s = 0; s < nstages; ++s) {
+    for (int s = 0; s < kStages; ++s) {
       tc::mbar_init(&bars.full[s], 1);
       tc::mbar_init(&bars.conv[s], 1);                      // one converter warp per box
       tc::mbar_init(&bars.empty[s], 1);
@@ -209,21 +214,21 @@ grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ 
           tc::mbar_wait(&bars.empty[stage], phase ^ 1);
           tc::mbar_arrive_expect_tx(&bars.full[stage], (uint32_t)(rows * 128));
           tc::tma_load_3d(tm, &bars.full[stage], st_hi + (size_t)stage * stage_bytes, col0, 0, p);
-          if (++stage == nstages) { stage = 0; phase ^= 1; }
+          if (++stage == kStages) { stage = 0; phase ^= 1; }
         }
       }
       // Drain: the tcgen05.commit arrivals on empty[] are asynchronous and nobody else waits for the last ones; an
       // arrival must not land after the CTA has exited (the shared memory then belongs to the next CTA on this SM).
-      for (int i = 0; i < nstages; ++i) {
+      for (int i = 0; i < kStages; ++i) {
         tc::mbar_wait(&bars.empty[stage], phase ^ 1);
-        if (++stage == nstages) { stage = 0; phase ^= 1; }
+        if (++stage == kStages) { stage = 0; phase ^= 1; }
       }
     }
   } else if (warp == 1) {
     // ------------------------------- MMA issuer -----------------------------------------------
     if (tc::elect_one()) {
       const uint32_t idesc = tc::make_idesc_tf32(128, kAccCols, /*A K-major*/ 0, /*B MN-major*/ 1);
-      const uint32_t lbo = (uint32_t)((size_t)nstages * stage_bytes);     // hi box -> lo box of the same stage
+      const uint32_t lbo = (uint32_t)((size_t)kStages * stage_bytes);     // hi box -> lo box of the same stage
       int stage = 0, phase = 0;
       int ab = 0, ab_phase = 0;
       tc::mbar_wait(&bars.w_ready, 0);
@@ -252,7 +257,7 @@ grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ 
             }
           }
           tc::umma_commit(&bars.empty[stage]);
-          if (++stage == nstages) { stage = 0; phase ^= 1; }
+          if (++stage == kStages) { stage = 0; phase ^= 1; }
         }
         tc::umma_commit(&bars.acc_full[ab]);
         if (++ab == kAccBufs) { ab = 0; ab_phase ^= 1; }
@@ -260,7 +265,7 @@ grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ 
     }
   } else if (warp < 2 + kConvWarps) {
     // ------------------------------- tf32 hi / lo split ---------------------------------------
-    // Warp-per-SLOT: converter warp cw owns ring slot cw, i.e. the boxes cw, cw + nstages, ... — up to nstages boxes
+    // Warp-per-SLOT: converter warp cw owns ring slot cw, i.e. the boxes cw, cw + kStages, ... — up to kStages boxes
     // are being converted at once (all warps on one box serialised the boxes at ~600 cycles each).
     // The owner sees EVERY phase of full[cw] in order, which the parity wait needs.  An earlier version dealt the
     // boxes round-robin over 8 warps with 9 slots: after box n a warp went on to box n + 8, which lives in the slot of
@@ -270,45 +275,43 @@ grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ 
     // conv[] a pass early, and the barriers of the ring went out of step for good (the kernel hung about once in a
     // few hundred thousand CTAs; DESIGN.md records how it was found).
     const int cw = warp - 2;
-    if (cw < nstages) {
-      const int nhalves = (Bx ? 1 : 0) + (By ? 1 : 0);
-      const long long nbox = (t_end - t_begin) * nhalves;
-      const uint32_t hi = tc::smem_u32(st_hi + (size_t)cw * stage_bytes);
-      const uint32_t lo = tc::smem_u32(st_lo + (size_t)cw * stage_bytes);
-      int phase = 0;
-      for (long long n = cw; n < nbox; n += nstages, phase ^= 1) {
-        const int half = nhalves == 2 ? (int)(n & 1) : (Bx ? 0 : 1);
-        const int rows = half ? By : Bx;
-        tc::mbar_wait(&bars.full[cw], phase);
-        const int n16 = rows * 8;                           // 16-byte units in this box (multiple of 64)
-        for (int e0 = lane; e0 < n16; e0 += 32 * 4) {
-          float4 v[4];
+    const int nhalves = (Bx ? 1 : 0) + (By ? 1 : 0);
+    const long long nbox = (t_end - t_begin) * nhalves;
+    const uint32_t hi = tc::smem_u32(st_hi + (size_t)cw * stage_bytes);
+    const uint32_t lo = tc::smem_u32(st_lo + (size_t)cw * stage_bytes);
+    int phase = 0;
+    for (long long n = cw; n < nbox; n += kStages, phase ^= 1) {
+      const int half = nhalves == 2 ? (int)(n & 1) : (Bx ? 0 : 1);
+      const int rows = half ? By : Bx;
+      tc::mbar_wait(&bars.full[cw], phase);
+      const int n16 = rows * 8;                           // 16-byte units in this box (multiple of 64)
+      for (int e0 = lane; e0 < n16; e0 += 32 * 4) {
+        float4 v[4];
 #pragma unroll
-          for (int u = 0; u < 4; ++u)
-            if (e0 + 32 * u < n16) v[u] = tc::lds128(hi + (e0 + 32 * u) * 16);
+        for (int u = 0; u < 4; ++u)
+          if (e0 + 32 * u < n16) v[u] = tc::lds128(hi + (e0 + 32 * u) * 16);
 #pragma unroll
-          for (int u = 0; u < 4; ++u) {
-            const int e = e0 + 32 * u;
-            if (e < n16) {
-              float4 h, l;
-              if (kRawHi) {            // the MMA reads trunc(v) out of the raw box; lo = v - trunc(v) is exact
-                h.x = tc::trunc_tf32(v[u].x); h.y = tc::trunc_tf32(v[u].y);
-                h.z = tc::trunc_tf32(v[u].z); h.w = tc::trunc_tf32(v[u].w);
-                l.x = v[u].x - h.x; l.y = v[u].y - h.y; l.z = v[u].z - h.z; l.w = v[u].w - h.w;
-              } else {
-                h.x = tc::to_tf32(v[u].x); h.y = tc::to_tf32(v[u].y); h.z = tc::to_tf32(v[u].z); h.w = tc::to_tf32(v[u].w);
-                l.x = tc::to_tf32(v[u].x - h.x); l.y = tc::to_tf32(v[u].y - h.y);
-                l.z = tc::to_tf32(v[u].z - h.z); l.w = tc::to_tf32(v[u].w - h.w);
-                tc::sts128(hi + e * 16, h);
-              }
-              tc::sts128(lo + e * 16, l);
+        for (int u = 0; u < 4; ++u) {
+          const int e = e0 + 32 * u;
+          if (e < n16) {
+            float4 h, l;
+            if (kRawHi) {            // the MMA reads trunc(v) out of the raw box; lo = v - trunc(v) is exact
+              h.x = tc::trunc_tf32(v[u].x); h.y = tc::trunc_tf32(v[u].y);
+              h.z = tc::trunc_tf32(v[u].z); h.w = tc::trunc_tf32(v[u].w);
+              l.x = v[u].x - h.x; l.y = v[u].y - h.y; l.z = v[u].z - h.z; l.w = v[u].w - h.w;
+            } else {
+              h.x = tc::to_tf32(v[u].x); h.y = tc::to_tf32(v[u].y); h.z = tc::to_tf32(v[u].z); h.w = tc::to_tf32(v[u].w);
+              l.x = tc::to_tf32(v[u].x - h.x); l.y = tc::to_tf32(v[u].y - h.y);
+              l.z = tc::to_tf32(v[u].z - h.z); l.w = tc::to_tf32(v[u].w - h.w);
+              tc::sts128(hi + e * 16, h);
             }
+            tc::sts128(lo + e * 16, l);
           }
         }
-        tc::fence_proxy_async_smem();
-        __syncwarp();
-        if (lane == 0) tc::mbar_arrive(&bars.conv[cw]);
       }
+      tc::fence_proxy_async_smem();
+      __syncwarp();
+      if (lane == 0) tc::mbar_arrive(&bars.conv[cw]);
     }
   } else {
     // ------------------------------- epilogue --------------------------------------------------
@@ -369,19 +372,13 @@ grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ 
   if (warp == 1) tc::tmem_dealloc(tmem, kTmemCols);
 }
 
-struct GradPlan { int nstages; size_t smem; };
-GradPlan plan_grad(int Bx, int By, int N) {
-  (void)N;
-  const size_t wbytes = 0;                                                 // W' lives in tensor memory
-  const size_t stage = (size_t)2 * (Bx > By ? Bx : By) * 128;              // hi + lo of one box
-  const size_t budget = 227 * 1024 - 2048 - sizeof(Bars) - 2 * kObufBytes;
-  int ns = (int)((budget - wbytes) / stage);
-  if (ns > kMaxStages) ns = kMaxStages;
-  GradPlan g;
-  g.nstages = ns;
-  g.smem = wbytes + ns * stage + 2 * kObufBytes + sizeof(Bars) + 1024;
-  return g;
+// dynamic shared memory: hi[kStages] | lo[kStages] | 2 output staging tiles | barriers, + 1 KB for the alignment
+constexpr size_t grad_smem_bytes(int rows_max) {
+  return (size_t)kStages * 2 * rows_max * 128 + 2 * kObufBytes + sizeof(Bars) + 1024;
 }
+// per SM: 228 KB of shared memory, of which the hardware reserves 1 KB per CTA
+static_assert(grad_smem_bytes(kMaxN) + 1024 <= 228 * 1024 / kCtasPerSm, "two CTAs per SM");
+
 }  // namespace
 
 bool tc_grad_supported(const float* x, const float* y, int Bx, int By, long long K, const float* gx, const float* gy) {
@@ -389,21 +386,25 @@ bool tc_grad_supported(const float* x, const float* y, int Bx, int By, long long
   if (K % 4 != 0 || K < 128) return false;
   if ((reinterpret_cast<uintptr_t>(x) & 15) || (reinterpret_cast<uintptr_t>(y) & 15)) return false;
   if ((gx && (reinterpret_cast<uintptr_t>(gx) & 15)) || (gy && (reinterpret_cast<uintptr_t>(gy) & 15))) return false;
-  return plan_grad(Bx, By, Bx > By ? Bx : By).nstages >= 2;
+  return true;
 }
 
 // img: the W' images of build_w_image_kernel ([nprob][2][128 x 128] floats); rb = 0: gradient of the x rows, 1: y rows
 static int launch_grad_rows(const CUtensorMap& tmx, const CUtensorMap& tmy, const float* img, int rb, int nprob, int Bx,
                             int By, long long K, float s, float* out, int accumulate, cudaStream_t st) {
   const int N = rb ? By : Bx;
-  const GradPlan g = plan_grad(Bx, By, N);
+  const size_t smem = grad_smem_bytes(Bx > By ? Bx : By);
   CUtensorMap tmo;     // output [nprob][N][K], box [N x 32], 128-byte swizzle (matches the staging tile)
   if (int rc = encode_tmap_3d(&tmo, out, (uint64_t)K, (uint64_t)N, (uint64_t)nprob, (uint64_t)K * 4, (uint64_t)K * 4 * N,
                               kBoxCols, (uint32_t)N))
     return rc;
   static size_t attr_smem[kMaxDevices] = {};
-  if (smem_attr_needed(attr_smem, g.smem))
-    KCCOT_CUDA(cudaFuncSetAttribute(grad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g.smem));
+  if (smem_attr_needed(attr_smem, smem)) {
+    KCCOT_CUDA(cudaFuncSetAttribute(grad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    // the whole 228 KB as shared memory, so that a second CTA (of this or another kernel) still finds its seat
+    KCCOT_CUDA(cudaFuncSetAttribute(grad_tc_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
+                                    (int)cudaSharedmemCarveoutMaxShared));
+  }
   long long ntiles = (K + kCols - 1) / kCols;
   // shared-context hint: only the gradient of the y rows (the fake video) skips the context tiles (the skipped
   // columns are left untouched)
@@ -416,7 +417,9 @@ static int launch_grad_rows(const CUtensorMap& tmx, const CUtensorMap& tmy, cons
   int gx = (sms + nprob - 1) / nprob;
   if ((long long)gx * nprob > sms) {
     // several waves of CTAs (more problems than SMs): pick the column split whose last wave wastes the fewest SMs,
-    // keeping at least 32 tiles per CTA (256 problems on 148 SMs: 1 range each = 2 waves at 86 %, 4 ranges = 7 at 99 %)
+    // keeping at least 32 tiles per CTA (256 problems on 148 SMs: 1 range each = 2 waves at 86 %, 4 ranges = 7 at 99 %).
+    // A wave counts one CTA per SM although two fit: counting two (8 ranges for 256 problems) was measured 0.15 %
+    // slower on config 4.
     int best = gx;
     double best_eff = 0.0;
     for (int g = gx; g <= gx + 7 && (long long)g * 32 <= ntiles; ++g) {
@@ -429,8 +432,8 @@ static int launch_grad_rows(const CUtensorMap& tmx, const CUtensorMap& tmy, cons
   if (gx > ntiles) gx = (int)ntiles;
   if (gx < 1) gx = 1;
   dim3 grid(gx, nprob);
-  KCCOT_CUDA(launch_pdl(grad_tc_kernel, grid, dim3(kThreads), g.smem, st, tmx, tmy, tmo, Bx, By, K, img, rb, N,
-                        -2.f * s, accumulate, g.nstages, ctx_period, ctx_len));
+  KCCOT_CUDA(launch_pdl(grad_tc_kernel, grid, dim3(kThreads), smem, st, tmx, tmy, tmo, Bx, By, K, img, rb, N,
+                        -2.f * s, accumulate, ctx_period, ctx_len));
   KCCOT_LAUNCH_CHECK();
   return KCCOT_OK;
 }
