@@ -9,7 +9,8 @@
  * the stub for the reference's own TensorFlow training loop.
  *
  * Conventions
- *   - All pointers are DEVICE pointers to contiguous fp32 unless stated; the caller owns every
+ *   - All pointers are DEVICE pointers to contiguous fp32 unless stated (the *_bf16 mixed-loss
+ *     entries take bf16 videos); the caller owns every
  *     buffer (inputs, outputs, saved state, workspace).  The library allocates nothing per call
  *     and keeps no pointer after return.
  *   - `stream` is a cudaStream_t passed as void*.  Calls only enqueue work; none synchronises.
@@ -226,6 +227,30 @@ int kccot_mixed_loss_bwd_ctx(const float* gloss, const float* real, const float*
                              float* g_real, float* g_fake, float* gh_fake, float* gm_real, float* gh_real,
                              float* gm_fake, void* ws, size_t ws_bytes, int flags, void* stream,
                              long long ctx_period, long long ctx_len);
+
+/* bf16 videos — the mixed loss for callers that keep their videos in bf16 (e.g. under bf16 autocast).
+ * real / fake and g_real / g_fake are raw bf16 bits (uint16_t), 16-byte aligned; h, M, their gradients, `saved`,
+ * loss, terms and gloss stay fp32, and `saved` is sized by kccot_mixed_loss_saved_bytes as for fp32.  Arguments as
+ * in the _ctx entries above (ctx_period = ctx_len = 0: no hint).
+ * Contract: the results are EXACTLY those of the fp32 entries on the widened videos (a bf16 value is exact in fp32):
+ * loss, terms and the h / M gradients bit for bit, g_real / g_fake the fp32 gradient rounded to nearest even.
+ * Paths: with B <= 64, B % 8 == 0, K % 8 == 0, K >= 128 and a path flag other than KCCOT_PATH_SIMT the tcgen05
+ * kernels read and write bf16 directly (no fp32 copy; the workspace is that of the fp32 call).  Every other shape
+ * widens the videos into the workspace, runs the fp32 chain and rounds the gradients.
+ * KCCOT_FLAG_ACCUMULATE is rejected (KCCOT_EINVAL): accumulating in bf16 would round at every call.  So is a video
+ * or gradient pointer that is not 16-byte aligned. */
+size_t kccot_mixed_loss_workspace_bytes_bf16(int nprob, int B, long long K, int L, int flags);
+int kccot_mixed_loss_fwd_bf16(const uint16_t* real, const uint16_t* fake, int nprob, int B, long long K,
+                              const float* h_fake, const float* m_real, const float* h_real,
+                              const float* m_fake, int T, int J, float s, float eps, int L, void* saved,
+                              float* loss, float* terms, void* ws, size_t ws_bytes, int flags, void* stream,
+                              long long ctx_period, long long ctx_len);
+int kccot_mixed_loss_bwd_bf16(const float* gloss, const uint16_t* real, const uint16_t* fake, int nprob,
+                              int B, long long K, const float* h_fake, const float* m_real,
+                              const float* h_real, const float* m_fake, int T, int J, float s, float eps,
+                              int L, const void* saved, uint16_t* g_real, uint16_t* g_fake, float* gh_fake,
+                              float* gm_real, float* gh_real, float* gm_fake, void* ws, size_t ws_bytes,
+                              int flags, void* stream, long long ctx_period, long long ctx_len);
 
 /* ------------------------------------------------------------------------------------------
  * Martingale penalty p_M — gan_utils.py:179-201.  M [B,T,J]; pm [1]; gM [B,T,J] = gpm * dpm/dM.

@@ -63,6 +63,11 @@ SIGNATURES = {
                                       _LL, _LL]),
     "kccot_mixed_loss_bwd_ctx": (_I, [_P, _P, _P, _I, _I, _LL, _P, _P, _P, _P, _I, _I, _F, _F, _I, _P, _P, _P, _P, _P, _P,
                                       _P, _P, _SZ, _I, _P, _LL, _LL]),
+    "kccot_mixed_loss_workspace_bytes_bf16": (_SZ, [_I, _I, _LL, _I, _I]),
+    "kccot_mixed_loss_fwd_bf16": (_I, [_P, _P, _I, _I, _LL, _P, _P, _P, _P, _I, _I, _F, _F, _I, _P, _P, _P, _P, _SZ, _I,
+                                       _P, _LL, _LL]),
+    "kccot_mixed_loss_bwd_bf16": (_I, [_P, _P, _P, _I, _I, _LL, _P, _P, _P, _P, _I, _I, _F, _F, _I, _P, _P, _P, _P, _P,
+                                       _P, _P, _P, _SZ, _I, _P, _LL, _LL]),
     "kccot_pm_fwd": (_I, [_P, _I, _I, _I, _F, _F, _P, _P, _P]),
     "kccot_pm_bwd": (_I, [_P, _I, _I, _I, _F, _F, _P, _P, _P, _P]),
     "kccot_smooth_workspace_bytes": (_SZ, [_I, _I, _I, _I, _I, _I]),

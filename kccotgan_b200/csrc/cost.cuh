@@ -48,6 +48,15 @@ int launch_sqdist_partials_simt(const float* x, const float* y, int nprob, int B
 int mixed_cost_fwd_impl(const float* real, const float* fake, int nprob, int B, long long K, const float* h_fake,
                         const float* m_real, const float* h_real, const float* m_fake, int T, int J, float s,
                         float* C3, void* ws, size_t ws_bytes, int flags, void* stream, int* zero_counters);
+// the tensor-core path of kccot_mixed_cost_fwd / _bwd for bf16 videos and gradients (raw bits; cost_abi.cu)
+int mixed_cost_fwd_bf16_tc(const uint16_t* real, const uint16_t* fake, int nprob, int B, long long K,
+                           const float* h_fake, const float* m_real, const float* h_real, const float* m_fake, int T,
+                           int J, float s, float* C3, void* ws, size_t ws_bytes, cudaStream_t st, int* zero_counters);
+int mixed_cost_bwd_bf16_tc(const float* Cbar3, const uint16_t* real, const uint16_t* fake, int nprob, int B,
+                           long long K, const float* h_fake, const float* m_real, const float* h_real,
+                           const float* m_fake, int T, int J, float s, uint16_t* g_real, uint16_t* g_fake,
+                           float* gh_fake, float* gm_real, float* gh_real, float* gm_fake, void* ws, size_t ws_bytes,
+                           cudaStream_t st);
 int launch_cost_finalize(const CostBlocks& blocks, int nblocks, int nprob, int T, int J, float s,
                          cudaStream_t st);
 int launch_cost_bwd_simt(const float* W, long long sr, long long sc, long long wprob, const float* a,
@@ -63,6 +72,10 @@ bool tc_sqdist_supported(const float* x, const float* y, int Bx, int By, long lo
 void tc_sqdist_plan(int nprob, int R, long long K, int* ksplit, int* kblocks_per_slab);
 int launch_sqdist_partials_tc(const float* x, const float* y, int nprob, int Bx, int By, long long K,
                               int ksplit, int kblocks_per_slab, float* part, cudaStream_t st);
+// bf16 videos (raw bits, K % 8 == 0, 16-byte aligned): the same partials as the fp32 launcher on widened copies
+bool tc_sqdist_bf16_supported(int Bx, int By, long long K);
+int launch_sqdist_partials_tc_bf16(const uint16_t* x, const uint16_t* y, int nprob, int Bx, int By, long long K,
+                                   int ksplit, int kblocks_per_slab, float* part, cudaStream_t st);
 
 // grad_tcgen05.cu — tensor-core adjoint over the stacked rows z = [x; y] (see the file header).
 // Wws: tc_grad_ws_bytes(nprob) of scratch for the W' images.  gx / gy may be null.
@@ -71,6 +84,10 @@ bool tc_grad_supported(const float* x, const float* y, int Bx, int By, long long
 size_t tc_grad_ws_bytes(int nprob);      // scratch of the two launchers below (W' images)
 int launch_grad_tc(const float* Cbar3, const float* x, const float* y, int nprob, int Bx, int By, long long K,
                    float s, float* gx, float* gy, int accumulate, float* Wws, cudaStream_t st);
+// bf16 videos and gradients of the mixed loss (B <= 64, K % 8 == 0, 16-byte aligned): gx / gy equal the fp32
+// launcher's result on the widened videos rounded to nearest even; no accumulation
+int launch_grad_tc_bf16(const float* Cbar3, const uint16_t* x, const uint16_t* y, int nprob, int B, long long K,
+                        float s, uint16_t* gx, uint16_t* gy, float* Wws, cudaStream_t st);
 int launch_grad_pair_tc(const float* Cbar, const float* x, const float* y, int nprob, int Bx, int By, long long K,
                         float s, float* gx, float* gy, int accumulate, float* Wws, cudaStream_t st);
 

@@ -29,6 +29,59 @@ int check_common(int nprob, int Bx, int By, long long K) {
                   By, K);
   return KCCOT_OK;
 }
+// the three blocks (xy, xx, yy — gan_utils.py:221-223) of the mixed cost, without their partials
+void mixed_blocks(CostBlocks& blocks, const float* h_fake, const float* m_real, const float* h_real, const float* m_fake,
+                  int B, float* C3, int* zero_counters) {
+  blocks.zero = zero_counters;
+  const long long BB = (long long)B * B;
+  const float* hs[3] = {h_fake, h_real, h_fake};
+  const float* Ms[3] = {m_real, m_real, m_fake};
+  for (int q = 0; q < 3; ++q) {
+    CostBlock& b = blocks.b[q];
+    b.h1 = hs[q]; b.M1 = Ms[q]; b.h2 = nullptr; b.M2 = nullptr;
+    b.C = C3 + q * BB; b.C_prob_stride = 3 * BB; b.Bx = B; b.By = B; b.zero_diag = q > 0;
+  }
+}
+// the partials of the stacked-row tensor-core kernel: blocks of the [2B x 2B] tile
+void mixed_blocks_tc(CostBlocks& blocks, const float* part, int B, int ks) {
+  const int roff[3] = {0, 0, B}, coff[3] = {B, 0, B};
+  for (int q = 0; q < 3; ++q) {
+    CostBlock& b = blocks.b[q];
+    b.part = part; b.prob_stride = (long long)ks * kTcTile; b.ks_stride = kTcTile; b.ld = 128;
+    b.nks = ks; b.row_off = roff[q]; b.col_off = coff[q]; b.sym = 1; b.tiled = 1;
+  }
+}
+// martingale terms of the mixed adjoint: xy = (h_fake, m_real), xx = (h_real, m_real), yy = (h_fake, m_fake)
+MartJobs mixed_mart_jobs(const float* Cbar3, int B, const float* h_fake, const float* m_real, const float* h_real,
+                         const float* m_fake, float* gh_fake, float* gm_real, float* gh_real, float* gm_fake, int acc) {
+  const long long BB = (long long)B * B, cprob = 3 * BB;
+  const float* Cxy = Cbar3;
+  const float* Cxx = Cbar3 + BB;
+  const float* Cyy = Cbar3 + 2 * BB;
+  MartJobs jobs{};
+  jobs.j[0] = MartJob{gh_fake, Cxy, m_real, Cyy, m_fake, cprob, B, B, B, 0, 0, acc};
+  jobs.j[1] = MartJob{gm_real, Cxy, h_fake, Cxx, h_real, cprob, B, B, B, 1, 1, acc};
+  jobs.j[2] = MartJob{gh_real, Cxx, m_real, nullptr, nullptr, cprob, B, B, B, 0, 0, acc};
+  jobs.j[3] = MartJob{gm_fake, Cyy, h_fake, nullptr, nullptr, cprob, B, B, B, 1, 1, acc};
+  return jobs;
+}
+// The martingale adjoint (a few MFLOP, ~10 us of latency) and the gradient GEMM both depend on Cbar3 only: the
+// small kernel goes first on the side stream and the persistent GEMM CTAs (`grad`) fill in around it.
+template <typename Grad>
+int mart_beside_grad(const MartJobs& jobs, int nprob, int T, int J, float s, cudaStream_t st, Grad grad) {
+  SideLane* lane = side_lane();
+  cudaStream_t ms = st;
+  if (lane) {
+    KCCOT_CUDA(cudaEventRecord(lane->fork, st));
+    KCCOT_CUDA(cudaStreamWaitEvent(lane->stream, lane->fork, 0));
+    ms = lane->stream;
+  }
+  if (int rc = launch_martingale_jobs(jobs, 4, nprob, T, J, s, ms)) return rc;
+  if (lane) KCCOT_CUDA(cudaEventRecord(lane->join, lane->stream));
+  if (int rc = grad()) return rc;
+  if (lane) KCCOT_CUDA(cudaStreamWaitEvent(st, lane->join, 0));
+  return KCCOT_OK;
+}
 
 }  // namespace
 }  // namespace kccot
@@ -152,27 +205,14 @@ int mixed_cost_fwd_impl(const float* real, const float* fake, int nprob, int B, 
     return KCCOT_EUNSUPPORTED;
   }
   CostBlocks blocks{};
-  blocks.zero = zero_counters;
   const long long BB = (long long)B * B;
-  // order xy, xx, yy — gan_utils.py:221-223
-  const float* hs[3] = {h_fake, h_real, h_fake};
-  const float* Ms[3] = {m_real, m_real, m_fake};
-  for (int q = 0; q < 3; ++q) {
-    CostBlock& b = blocks.b[q];
-    b.h1 = hs[q]; b.M1 = Ms[q]; b.h2 = nullptr; b.M2 = nullptr;
-    b.C = C3 + q * BB; b.C_prob_stride = 3 * BB; b.Bx = B; b.By = B; b.zero_diag = q > 0;
-  }
+  mixed_blocks(blocks, h_fake, m_real, h_real, m_fake, B, C3, zero_counters);
   if (path == KCCOT_PATH_TCGEN05) {
     int ks, kbps;
     tc_sqdist_plan(nprob, 2 * B, K, &ks, &kbps);
     KCCOT_CHECK_ARG(ws_bytes >= (size_t)nprob * ks * kTcTile * 4, "workspace too small");
     if (int rc = launch_sqdist_partials_tc(real, fake, nprob, B, B, K, ks, kbps, (float*)ws, st)) return rc;
-    const int roff[3] = {0, 0, B}, coff[3] = {B, 0, B};
-    for (int q = 0; q < 3; ++q) {
-      CostBlock& b = blocks.b[q];
-      b.part = (const float*)ws; b.prob_stride = (long long)ks * kTcTile; b.ks_stride = kTcTile; b.ld = 128;
-      b.nks = ks; b.row_off = roff[q]; b.col_off = coff[q]; b.sym = 1; b.tiled = 1;
-    }
+    mixed_blocks_tc(blocks, (const float*)ws, B, ks);
   } else {
     int ks;
     long long slab;
@@ -190,6 +230,37 @@ int mixed_cost_fwd_impl(const float* real, const float* fake, int nprob, int B, 
     }
   }
   return launch_cost_finalize(blocks, 3, nprob, T, J, s, st);
+}
+
+int mixed_cost_fwd_bf16_tc(const uint16_t* real, const uint16_t* fake, int nprob, int B, long long K,
+                           const float* h_fake, const float* m_real, const float* h_real, const float* m_fake, int T,
+                           int J, float s, float* C3, void* ws, size_t ws_bytes, cudaStream_t st, int* zero_counters) {
+  if (int rc = check_common(nprob, B, B, K)) return rc;
+  KCCOT_CHECK_ARG(real && fake && h_fake && m_real && h_real && m_fake && C3 && ws, "null pointer");
+  KCCOT_CHECK_ARG(T >= 2 && J >= 1, "martingale term needs T >= 2, J >= 1 (T=%d J=%d)", T, J);
+  KCCOT_CHECK_ARG(tc_sqdist_bf16_supported(B, B, K), "bf16 tensor-core path unsupported for B=%d K=%lld", B, K);
+  CostBlocks blocks{};
+  mixed_blocks(blocks, h_fake, m_real, h_real, m_fake, B, C3, zero_counters);
+  int ks, kbps;
+  tc_sqdist_plan(nprob, 2 * B, K, &ks, &kbps);
+  KCCOT_CHECK_ARG(ws_bytes >= (size_t)nprob * ks * kTcTile * 4, "workspace too small");
+  if (int rc = launch_sqdist_partials_tc_bf16(real, fake, nprob, B, B, K, ks, kbps, (float*)ws, st)) return rc;
+  mixed_blocks_tc(blocks, (const float*)ws, B, ks);
+  return launch_cost_finalize(blocks, 3, nprob, T, J, s, st);
+}
+
+int mixed_cost_bwd_bf16_tc(const float* Cbar3, const uint16_t* real, const uint16_t* fake, int nprob, int B,
+                           long long K, const float* h_fake, const float* m_real, const float* h_real,
+                           const float* m_fake, int T, int J, float s, uint16_t* g_real, uint16_t* g_fake,
+                           float* gh_fake, float* gm_real, float* gh_real, float* gm_fake, void* ws, size_t ws_bytes,
+                           cudaStream_t st) {
+  if (int rc = check_common(nprob, B, B, K)) return rc;
+  KCCOT_CHECK_ARG(Cbar3 && real && fake && h_fake && m_real && h_real && m_fake, "null pointer");
+  KCCOT_CHECK_ARG(ws && ws_bytes >= tc_grad_ws_bytes(nprob), "workspace too small");
+  const MartJobs jobs = mixed_mart_jobs(Cbar3, B, h_fake, m_real, h_real, m_fake, gh_fake, gm_real, gh_real, gm_fake, 0);
+  return mart_beside_grad(jobs, nprob, T, J, s, st, [&] {
+    return launch_grad_tc_bf16(Cbar3, real, fake, nprob, B, K, s, g_real, g_fake, (float*)ws, st);
+  });
 }
 }  // namespace kccot
 
@@ -296,13 +367,8 @@ int kccot_mixed_cost_bwd(const float* Cbar3, const float* real, const float* fak
     set_error("tcgen05 gradient path requested but unsupported for B=%d K=%lld", B, K);
     return KCCOT_EUNSUPPORTED;
   }
-  // martingale terms: xy = (h_fake, m_real), xx = (h_real, m_real), yy = (h_fake, m_fake) — one launch
-  MartJobs jobs{};
-  const int Bi = B;
-  jobs.j[0] = MartJob{gh_fake, Cxy, m_real, Cyy, m_fake, cprob, Bi, Bi, Bi, 0, 0, acc};
-  jobs.j[1] = MartJob{gm_real, Cxy, h_fake, Cxx, h_real, cprob, Bi, Bi, Bi, 1, 1, acc};
-  jobs.j[2] = MartJob{gh_real, Cxx, m_real, nullptr, nullptr, cprob, Bi, Bi, Bi, 0, 0, acc};
-  jobs.j[3] = MartJob{gm_fake, Cyy, h_fake, nullptr, nullptr, cprob, Bi, Bi, Bi, 1, 1, acc};
+  // martingale terms: one launch
+  const MartJobs jobs = mixed_mart_jobs(Cbar3, B, h_fake, m_real, h_real, m_fake, gh_fake, gm_real, gh_real, gm_fake, acc);
   if (want_tc && real != fake && large_path_wanted(B, B, false) && ws && ws_bytes >= large_cost_bwd_ws_bytes(B, B, K, true)) {
     if (int rc = launch_martingale_jobs(jobs, 4, nprob, T, J, s, st)) return rc;
     for (int p = 0; p < nprob; ++p)
@@ -312,22 +378,10 @@ int kccot_mixed_cost_bwd(const float* Cbar3, const float* real, const float* fak
         return rc;
     return KCCOT_OK;
   }
-  if (tc_ok) {
-    // The martingale adjoint (a few MFLOP, ~10 us of latency) and the gradient GEMM both depend on Cbar3
-    // only: the small kernel goes first on the side stream and the persistent GEMM CTAs fill in around it.
-    SideLane* lane = side_lane();
-    cudaStream_t ms = st;
-    if (lane) {
-      KCCOT_CUDA(cudaEventRecord(lane->fork, st));
-      KCCOT_CUDA(cudaStreamWaitEvent(lane->stream, lane->fork, 0));
-      ms = lane->stream;
-    }
-    if (int rc = launch_martingale_jobs(jobs, 4, nprob, T, J, s, ms)) return rc;
-    if (lane) KCCOT_CUDA(cudaEventRecord(lane->join, lane->stream));
-    if (int rc = launch_grad_tc(Cbar3, real, fake, nprob, B, B, K, s, g_real, g_fake, acc, (float*)ws, st)) return rc;
-    if (lane) KCCOT_CUDA(cudaStreamWaitEvent(st, lane->join, 0));
-    return KCCOT_OK;
-  }
+  if (tc_ok)
+    return mart_beside_grad(jobs, nprob, T, J, s, st, [&] {
+      return launch_grad_tc(Cbar3, real, fake, nprob, B, B, K, s, g_real, g_fake, acc, (float*)ws, st);
+    });
   if (g_fake) {
     if (int rc = launch_cost_bwd_simt(Cxy, 1, B, cprob, fake, real, nprob, B, B, K, s, g_fake, acc, st)) return rc;
     if (int rc = launch_cost_bwd_simt(Cyy, B, 1, cprob, fake, fake, nprob, B, B, K, s, g_fake, 1, st)) return rc;

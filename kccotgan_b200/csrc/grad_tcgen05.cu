@@ -34,6 +34,8 @@
 //   Epilogue:   each of the four epilogue warps owns one quadrant: lanes 0-15 add their two column halves, lanes
 //               16-31 hand W'lo.Zhi down by shuffle; 16 rows per warp are staged in 128-byte-swizzled shared memory
 //               and one TMA store (or reduce-add) writes the [N x 32] box as full 128-byte row segments.
+#include <cuda_bf16.h>
+
 #include "cost.cuh"
 #include "tc_common.cuh"
 
@@ -115,10 +117,25 @@ __global__ void __launch_bounds__(128) build_w_image_kernel(const float* __restr
   im[(lane_hi + 16) * 4] = lo;
 }
 
-__global__ void __launch_bounds__(kThreads, kCtasPerSm)
-grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUtensorMap tmy,
-               const __grid_constant__ CUtensorMap tmo, int Bx, int By, long long K, const float* __restrict__ Wimg,
-               int rb, int N, float neg2s, int accumulate, int ctx_period, int ctx_len) {
+// bf16 videos (grad_tc_bf16_kernel): the [rows x 32] bf16 box (rows x 64 B, unswizzled) lands in the LO slot of its
+// stage, which is free because a widened bf16 value has Zlo = Z - trunc_tf32(Z) = 0 exactly: the W'hi.Zlo block of
+// the fp32 instruction is zero and is not computed.  The slot's converter warp widens the box into the hi slot at the
+// SWIZZLE_128B_BASE32B positions the fp32 TMA box would have had, the MMA is M128 x N32 x K8 over Zhi only, and the
+// epilogue rounds to bf16 (nearest even) and stores a [N x 32] bf16 box (64-byte swizzle).
+__device__ __forceinline__ uint2 lds64(uint32_t saddr) {
+  uint2 v;
+  asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(v.x), "=r"(v.y) : "r"(saddr));
+  return v;
+}
+__device__ __forceinline__ uint32_t pack_bf16x2_rn(float lo, float hi) {
+  const __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
+  return *reinterpret_cast<const uint32_t*>(&h);
+}
+
+template <bool kBf16>
+__device__ __forceinline__ void grad_tc_body(const CUtensorMap& tmx, const CUtensorMap& tmy, const CUtensorMap& tmo,
+                                             int Bx, int By, long long K, const float* __restrict__ Wimg, int rb, int N,
+                                             float neg2s, int accumulate, int ctx_period, int ctx_len) {
   extern __shared__ uint8_t smem_raw[];
   // align by OFFSET so that the compiler keeps the shared address space (LDS/STS, not generic LD/ST)
   uint8_t* base = smem_raw + ((1024u - (tc::smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -212,8 +229,8 @@ grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ 
           if (rows == 0) continue;
           const CUtensorMap* tm = half ? &tmy : &tmx;
           tc::mbar_wait(&bars.empty[stage], phase ^ 1);
-          tc::mbar_arrive_expect_tx(&bars.full[stage], (uint32_t)(rows * 128));
-          tc::tma_load_3d(tm, &bars.full[stage], st_hi + (size_t)stage * stage_bytes, col0, 0, p);
+          tc::mbar_arrive_expect_tx(&bars.full[stage], (uint32_t)(rows * (kBf16 ? 64 : 128)));
+          tc::tma_load_3d(tm, &bars.full[stage], (kBf16 ? st_lo : st_hi) + (size_t)stage * stage_bytes, col0, 0, p);
           if (++stage == kStages) { stage = 0; phase ^= 1; }
         }
       }
@@ -227,7 +244,7 @@ grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ 
   } else if (warp == 1) {
     // ------------------------------- MMA issuer -----------------------------------------------
     if (tc::elect_one()) {
-      const uint32_t idesc = tc::make_idesc_tf32(128, kAccCols, /*A K-major*/ 0, /*B MN-major*/ 1);
+      const uint32_t idesc = tc::make_idesc_tf32(128, kBf16 ? kCols : kAccCols, /*A K-major*/ 0, /*B MN-major*/ 1);
       const uint32_t lbo = (uint32_t)((size_t)kStages * stage_bytes);     // hi box -> lo box of the same stage
       int stage = 0, phase = 0;
       int ab = 0, ab_phase = 0;
@@ -285,27 +302,48 @@ grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ 
       const int rows = half ? By : Bx;
       tc::mbar_wait(&bars.full[cw], phase);
       const int n16 = rows * 8;                           // 16-byte units in this box (multiple of 64)
-      for (int e0 = lane; e0 < n16; e0 += 32 * 4) {
-        float4 v[4];
+      if (kBf16) {
+        // unit e = (row r, fp32 chunk j): 8 bytes of bf16 in, 16 bytes of fp32 out at the SWIZZLE_128B_BASE32B
+        // position of the fp32 box (32-byte chunk j / 2 of row r XOR r % 4)
+        for (int e0 = lane; e0 < n16; e0 += 32 * 4) {
+          uint2 v[4];
 #pragma unroll
-        for (int u = 0; u < 4; ++u)
-          if (e0 + 32 * u < n16) v[u] = tc::lds128(hi + (e0 + 32 * u) * 16);
+          for (int u = 0; u < 4; ++u)
+            if (e0 + 32 * u < n16) v[u] = lds64(lo + (e0 + 32 * u) * 8);
 #pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          const int e = e0 + 32 * u;
-          if (e < n16) {
-            float4 h, l;
-            if (kRawHi) {            // the MMA reads trunc(v) out of the raw box; lo = v - trunc(v) is exact
-              h.x = tc::trunc_tf32(v[u].x); h.y = tc::trunc_tf32(v[u].y);
-              h.z = tc::trunc_tf32(v[u].z); h.w = tc::trunc_tf32(v[u].w);
-              l.x = v[u].x - h.x; l.y = v[u].y - h.y; l.z = v[u].z - h.z; l.w = v[u].w - h.w;
-            } else {
-              h.x = tc::to_tf32(v[u].x); h.y = tc::to_tf32(v[u].y); h.z = tc::to_tf32(v[u].z); h.w = tc::to_tf32(v[u].w);
-              l.x = tc::to_tf32(v[u].x - h.x); l.y = tc::to_tf32(v[u].y - h.y);
-              l.z = tc::to_tf32(v[u].z - h.z); l.w = tc::to_tf32(v[u].w - h.w);
-              tc::sts128(hi + e * 16, h);
+          for (int u = 0; u < 4; ++u) {
+            const int e = e0 + 32 * u;
+            if (e < n16) {
+              const int r = e >> 3, j = e & 7;
+              const float4 f = make_float4(__uint_as_float(v[u].x << 16), __uint_as_float(v[u].x & 0xffff0000u),
+                                           __uint_as_float(v[u].y << 16), __uint_as_float(v[u].y & 0xffff0000u));
+              tc::sts128(hi + r * 128 + ((((j >> 1) ^ (r & 3)) << 5) | ((j & 1) << 4)), f);
             }
-            tc::sts128(lo + e * 16, l);
+          }
+        }
+      } else {
+        for (int e0 = lane; e0 < n16; e0 += 32 * 4) {
+          float4 v[4];
+#pragma unroll
+          for (int u = 0; u < 4; ++u)
+            if (e0 + 32 * u < n16) v[u] = tc::lds128(hi + (e0 + 32 * u) * 16);
+#pragma unroll
+          for (int u = 0; u < 4; ++u) {
+            const int e = e0 + 32 * u;
+            if (e < n16) {
+              float4 h, l;
+              if (kRawHi) {            // the MMA reads trunc(v) out of the raw box; lo = v - trunc(v) is exact
+                h.x = tc::trunc_tf32(v[u].x); h.y = tc::trunc_tf32(v[u].y);
+                h.z = tc::trunc_tf32(v[u].z); h.w = tc::trunc_tf32(v[u].w);
+                l.x = v[u].x - h.x; l.y = v[u].y - h.y; l.z = v[u].z - h.z; l.w = v[u].w - h.w;
+              } else {
+                h.x = tc::to_tf32(v[u].x); h.y = tc::to_tf32(v[u].y); h.z = tc::to_tf32(v[u].z); h.w = tc::to_tf32(v[u].w);
+                l.x = tc::to_tf32(v[u].x - h.x); l.y = tc::to_tf32(v[u].y - h.y);
+                l.z = tc::to_tf32(v[u].z - h.z); l.w = tc::to_tf32(v[u].w - h.w);
+                tc::sts128(hi + e * 16, h);
+              }
+              tc::sts128(lo + e * 16, l);
+            }
           }
         }
       }
@@ -331,15 +369,22 @@ grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ 
       tc::tc_fence_after();
       float d[32];
       if (active) {
-        float e[32];
         const uint32_t ta = tmem + ((uint32_t)(quad * 32) << 16) + (uint32_t)(kTmemAcc0 + ab * kAccCols);
-        tc::tmem_ld_32x32(ta, d);
-        tc::tmem_ld_32x32(ta + 32, e);
-        tc::tmem_ld_wait();
+        if (kBf16) {                                                  // W'hi.Zhi  |  W'lo.Zhi  (Zlo = 0)
+          tc::tmem_ld_32x32(ta, d);
+          tc::tmem_ld_wait();
 #pragma unroll
-        for (int j = 0; j < 32; ++j) {
-          const float mine = hi_lane ? d[j] + e[j] : d[j];             // W'hi.(Zhi + Zlo)  |  W'lo.Zhi
-          d[j] = neg2s * (mine + __shfl_down_sync(0xffffffffu, mine, 16));
+          for (int j = 0; j < 32; ++j) d[j] = neg2s * (d[j] + __shfl_down_sync(0xffffffffu, d[j], 16));
+        } else {
+          float e[32];
+          tc::tmem_ld_32x32(ta, d);
+          tc::tmem_ld_32x32(ta + 32, e);
+          tc::tmem_ld_wait();
+#pragma unroll
+          for (int j = 0; j < 32; ++j) {
+            const float mine = hi_lane ? d[j] + e[j] : d[j];             // W'hi.(Zhi + Zlo)  |  W'lo.Zhi
+            d[j] = neg2s * (mine + __shfl_down_sync(0xffffffffu, mine, 16));
+        }
         }
       }
       tc::tc_fence_before();
@@ -349,10 +394,21 @@ grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ 
       if (issuer) tc::tma_store_wait_read<1>();
       tc::named_bar_sync(2, kEpiWarps * 32);
       if (active && hi_lane && r < N) {
-        const uint32_t row = tc::smem_u32(obuf + ob * kObufBytes) + r * 128;
+        if (kBf16) {                      // 64-byte rows, 64-byte swizzle: 16-byte chunk q at q ^ ((r / 2) % 4)
+          const uint32_t row = tc::smem_u32(obuf + ob * kObufBytes) + r * 64;
 #pragma unroll
-        for (int j = 0; j < 8; ++j)
-          tc::sts128(row + ((j ^ (r & 7)) << 4), make_float4(d[4 * j], d[4 * j + 1], d[4 * j + 2], d[4 * j + 3]));
+          for (int q = 0; q < 4; ++q)
+            tc::sts128(row + ((q ^ ((r >> 1) & 3)) << 4),
+                       make_float4(__uint_as_float(pack_bf16x2_rn(d[8 * q], d[8 * q + 1])),
+                                   __uint_as_float(pack_bf16x2_rn(d[8 * q + 2], d[8 * q + 3])),
+                                   __uint_as_float(pack_bf16x2_rn(d[8 * q + 4], d[8 * q + 5])),
+                                   __uint_as_float(pack_bf16x2_rn(d[8 * q + 6], d[8 * q + 7]))));
+        } else {
+          const uint32_t row = tc::smem_u32(obuf + ob * kObufBytes) + r * 128;
+#pragma unroll
+          for (int j = 0; j < 8; ++j)
+            tc::sts128(row + ((j ^ (r & 7)) << 4), make_float4(d[4 * j], d[4 * j + 1], d[4 * j + 2], d[4 * j + 3]));
+        }
       }
       tc::fence_proxy_async_smem();
       tc::named_bar_sync(2, kEpiWarps * 32);
@@ -370,6 +426,21 @@ grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ 
   tc::tc_fence_before();
   __syncthreads();
   if (warp == 1) tc::tmem_dealloc(tmem, kTmemCols);
+}
+
+__global__ void __launch_bounds__(kThreads, kCtasPerSm)
+grad_tc_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUtensorMap tmy,
+               const __grid_constant__ CUtensorMap tmo, int Bx, int By, long long K, const float* __restrict__ Wimg,
+               int rb, int N, float neg2s, int accumulate, int ctx_period, int ctx_len) {
+  grad_tc_body<false>(tmx, tmy, tmo, Bx, By, K, Wimg, rb, N, neg2s, accumulate, ctx_period, ctx_len);
+}
+
+// bf16 videos and gradient (see grad_tc_body): same shared memory, registers and tensor memory as grad_tc_kernel
+__global__ void __launch_bounds__(kThreads, kCtasPerSm)
+grad_tc_bf16_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUtensorMap tmy,
+                    const __grid_constant__ CUtensorMap tmo, int Bx, int By, long long K, const float* __restrict__ Wimg,
+                    int rb, int N, float neg2s, int accumulate, int ctx_period, int ctx_len) {
+  grad_tc_body<true>(tmx, tmy, tmo, Bx, By, K, Wimg, rb, N, neg2s, accumulate, ctx_period, ctx_len);
 }
 
 // dynamic shared memory: hi[kStages] | lo[kStages] | 2 output staging tiles | barriers, + 1 KB for the alignment
@@ -390,19 +461,26 @@ bool tc_grad_supported(const float* x, const float* y, int Bx, int By, long long
 }
 
 // img: the W' images of build_w_image_kernel ([nprob][2][128 x 128] floats); rb = 0: gradient of the x rows, 1: y rows
+// bf16: videos and `out` are bf16 (grad_tc_bf16_kernel), no accumulation
 static int launch_grad_rows(const CUtensorMap& tmx, const CUtensorMap& tmy, const float* img, int rb, int nprob, int Bx,
-                            int By, long long K, float s, float* out, int accumulate, cudaStream_t st) {
+                            int By, long long K, float s, void* out, int accumulate, bool bf16, cudaStream_t st) {
   const int N = rb ? By : Bx;
   const size_t smem = grad_smem_bytes(Bx > By ? Bx : By);
-  CUtensorMap tmo;     // output [nprob][N][K], box [N x 32], 128-byte swizzle (matches the staging tile)
-  if (int rc = encode_tmap_3d(&tmo, out, (uint64_t)K, (uint64_t)N, (uint64_t)nprob, (uint64_t)K * 4, (uint64_t)K * 4 * N,
-                              kBoxCols, (uint32_t)N))
+  // output [nprob][N][K], box [N x 32]: fp32 with the 128-byte swizzle, bf16 with the 64-byte swizzle (each matches
+  // its staging tile)
+  CUtensorMap tmo;
+  if (int rc = bf16 ? encode_tmap_3d(&tmo, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, CU_TENSOR_MAP_SWIZZLE_64B, out, (uint64_t)K,
+                                     (uint64_t)N, (uint64_t)nprob, (uint64_t)K * 2, (uint64_t)K * 2 * N, kBoxCols,
+                                     (uint32_t)N)
+                    : encode_tmap_3d(&tmo, out, (uint64_t)K, (uint64_t)N, (uint64_t)nprob, (uint64_t)K * 4,
+                                     (uint64_t)K * 4 * N, kBoxCols, (uint32_t)N))
     return rc;
-  static size_t attr_smem[kMaxDevices] = {};
-  if (smem_attr_needed(attr_smem, smem)) {
-    KCCOT_CUDA(cudaFuncSetAttribute(grad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  auto kernel = bf16 ? grad_tc_bf16_kernel : grad_tc_kernel;
+  static size_t attr_smem[2][kMaxDevices] = {};
+  if (smem_attr_needed(attr_smem[bf16 ? 1 : 0], smem)) {
+    KCCOT_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     // the whole 228 KB as shared memory, so that a second CTA (of this or another kernel) still finds its seat
-    KCCOT_CUDA(cudaFuncSetAttribute(grad_tc_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
+    KCCOT_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
                                     (int)cudaSharedmemCarveoutMaxShared));
   }
   long long ntiles = (K + kCols - 1) / kCols;
@@ -432,8 +510,8 @@ static int launch_grad_rows(const CUtensorMap& tmx, const CUtensorMap& tmy, cons
   if (gx > ntiles) gx = (int)ntiles;
   if (gx < 1) gx = 1;
   dim3 grid(gx, nprob);
-  KCCOT_CUDA(launch_pdl(grad_tc_kernel, grid, dim3(kThreads), smem, st, tmx, tmy, tmo, Bx, By, K, img, rb, N,
-                        -2.f * s, accumulate, ctx_period, ctx_len));
+  KCCOT_CUDA(launch_pdl(kernel, grid, dim3(kThreads), smem, st, tmx, tmy, tmo, Bx, By, K, img, rb, N, -2.f * s,
+                        accumulate, ctx_period, ctx_len));
   KCCOT_LAUNCH_CHECK();
   return KCCOT_OK;
 }
@@ -455,9 +533,30 @@ static int launch_grad_common(const float* C, const float* x, const float* y, in
                               kBoxCols, (uint32_t)By, true))
     return rc;
   if (gy)
-    if (int rc = launch_grad_rows(tmx, tmy, img, 1, nprob, Bx, By, K, s, gy, accumulate, st)) return rc;
+    if (int rc = launch_grad_rows(tmx, tmy, img, 1, nprob, Bx, By, K, s, gy, accumulate, false, st)) return rc;
   if (gx)
-    if (int rc = launch_grad_rows(tmx, tmy, img, 0, nprob, Bx, By, K, s, gx, accumulate, st)) return rc;
+    if (int rc = launch_grad_rows(tmx, tmy, img, 0, nprob, Bx, By, K, s, gx, accumulate, false, st)) return rc;
+  return KCCOT_OK;
+}
+
+int launch_grad_tc_bf16(const float* Cbar3, const uint16_t* x, const uint16_t* y, int nprob, int B, long long K,
+                        float s, uint16_t* gx, uint16_t* gy, float* Wws, cudaStream_t st) {
+  if (!gx && !gy) return KCCOT_OK;
+  const int rb_first = gx ? 0 : 1, nrb = (gx ? 1 : 0) + (gy ? 1 : 0);
+  KCCOT_CUDA(launch_pdl(build_w_image_kernel<true>, dim3(kMaxN, nrb, nprob), dim3(128), 0, st, Cbar3, B, B, rb_first,
+                        Wws));
+  KCCOT_LAUNCH_CHECK();
+  CUtensorMap tmx, tmy;     // [rows x 32] bf16 boxes, unswizzled (the converters place them)
+  if (int rc = encode_tmap_3d(&tmx, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, CU_TENSOR_MAP_SWIZZLE_NONE, x, (uint64_t)K,
+                              (uint64_t)B, (uint64_t)nprob, (uint64_t)K * 2, (uint64_t)K * 2 * B, kBoxCols, (uint32_t)B))
+    return rc;
+  if (int rc = encode_tmap_3d(&tmy, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, CU_TENSOR_MAP_SWIZZLE_NONE, y, (uint64_t)K,
+                              (uint64_t)B, (uint64_t)nprob, (uint64_t)K * 2, (uint64_t)K * 2 * B, kBoxCols, (uint32_t)B))
+    return rc;
+  if (gy)
+    if (int rc = launch_grad_rows(tmx, tmy, Wws, 1, nprob, B, B, K, s, gy, 0, true, st)) return rc;
+  if (gx)
+    if (int rc = launch_grad_rows(tmx, tmy, Wws, 0, nprob, B, B, K, s, gx, 0, true, st)) return rc;
   return KCCOT_OK;
 }
 

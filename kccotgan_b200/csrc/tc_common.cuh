@@ -252,6 +252,10 @@ __device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
 // with 16-byte atoms (K-major operands), true: 128-byte swizzle with 32-byte atoms (MN-major tf32 operands)
 int encode_tmap_3d(CUtensorMap* out, const void* base, uint64_t d0, uint64_t d1, uint64_t d2, uint64_t stride1_bytes,
                    uint64_t stride2_bytes, uint32_t b0, uint32_t b1, bool atom32 = false, bool noswizzle = false);
+// host: the same with an explicit element type and swizzle mode (bf16 videos)
+int encode_tmap_3d(CUtensorMap* out, CUtensorMapDataType dtype, CUtensorMapSwizzle swizzle, const void* base,
+                   uint64_t d0, uint64_t d1, uint64_t d2, uint64_t stride1_bytes, uint64_t stride2_bytes, uint32_t b0,
+                   uint32_t b1);
 // host: 2-D fp16 tensor map [rows][cols] (row pitch in bytes), box (box_cols, box_rows), 128-byte swizzle
 int encode_tmap_2d_f16(CUtensorMap* out, const void* base, uint64_t cols, uint64_t rows, uint64_t pitch_bytes,
                        uint32_t box_cols, uint32_t box_rows);

@@ -1,7 +1,11 @@
 """torch.autograd glue between the reference-shaped Python functions and the C ABI.
 
 PyTorch supplies device memory, streams and the tape only; every arithmetic step is a libkccot
-kernel.  Tensors must be CUDA fp32 — anything else raises ValueError (no fallback).
+kernel.  Tensors must be CUDA fp32 — anything else raises ValueError (no fallback) — except in the mixed loss
+(MixedLossFn, MixedLossBatchedFn), which also takes bf16 videos and h / m: two bf16 videos run the bf16 entry points
+of the library (the result is exactly the fp32 one on the widened videos, video gradients rounded to bf16); a bf16
+video next to an fp32 one, and bf16 h / m, are widened with .float() (exact).  Gradients come back in the dtype of
+their input.
 """
 import ctypes
 
@@ -58,6 +62,37 @@ def _check(t, name, ndim=None):
     if ndim is not None and t.dim() != ndim:
         raise ValueError(f"{name}: expected {ndim} dimensions, got shape {tuple(t.shape)}")
     return t.contiguous()
+
+
+def _check_video(t, name):
+    """A CUDA video of the mixed loss: fp32 or bf16, made contiguous."""
+    if isinstance(t, torch.Tensor) and t.dtype == torch.bfloat16:
+        if not t.is_cuda:
+            raise ValueError(f"{name}: expected a CUDA tensor (kccotgan_b200 has no CPU path), got {t.device}")
+        return t.contiguous()
+    return _check(t, name)
+
+
+def _videos(real, fake):
+    """-> (real, fake, bf16).  Two bf16 videos stay bf16 (cloned if a view is not 16-byte aligned, as the bf16 entry
+    points require); otherwise a bf16 one is widened to fp32, which is exact."""
+    real, fake = _check_video(real, "f_real"), _check_video(fake, "f_fake")
+    if real.dtype == fake.dtype == torch.bfloat16:
+        return (real if real.data_ptr() % 16 == 0 else real.clone(),
+                fake if fake.data_ptr() % 16 == 0 else fake.clone(), True)
+    return real.float(), fake.float(), False
+
+
+def _check_hm(t, name, ndim):
+    """h / m of the mixed loss: fp32, or bf16 widened to fp32 (exact)."""
+    if isinstance(t, torch.Tensor) and t.dtype == torch.bfloat16:
+        t = t.float()
+    return _check(t, name, ndim)
+
+
+def _as_dtypes(grads, dtypes):
+    """each gradient in the dtype of its input (the fp32 gradient of a widened bf16 input rounded to nearest even)"""
+    return [g.to(dt) if g is not None and g.dtype != dt else g for g, dt in zip(grads, dtypes)]
 
 
 def _ws(nbytes, dev):
@@ -200,28 +235,37 @@ class SinkhornFn(torch.autograd.Function):
 _SIZES = {}
 
 
-def _mixed_sizes(B, K, L, nprob=1):
-    key = (B, K, L, nprob)
+def _mixed_sizes(B, K, L, nprob=1, dtype=torch.float32):
+    """(saved, workspace) bytes; bf16 videos: the workspace depends on the path flag (native or widened path)"""
+    bf16 = dtype == torch.bfloat16
+    flags = _PATH["flags"] if bf16 else 0
+    key = (B, K, L, nprob, dtype, flags)
     if key not in _SIZES:
         lib = _lib.load()
-        _SIZES[key] = (int(lib.kccot_mixed_loss_saved_bytes(nprob, B, L)),
-                       int(lib.kccot_mixed_loss_workspace_bytes(nprob, B, K, L)))
+        ws = (lib.kccot_mixed_loss_workspace_bytes_bf16(nprob, B, K, L, flags) if bf16
+              else lib.kccot_mixed_loss_workspace_bytes(nprob, B, K, L))
+        _SIZES[key] = (int(lib.kccot_mixed_loss_saved_bytes(nprob, B, L)), int(ws))
     return _SIZES[key]
 
 
 class MixedLossFn(torch.autograd.Function):
-    """One C-ABI call per direction (kccot_mixed_loss_fwd / _bwd)."""
+    """One C-ABI call per direction (kccot_mixed_loss_fwd_ctx / _bwd_ctx, or their _bf16 forms for bf16 videos)."""
 
     @staticmethod
     def forward(ctx, real, fake, h_fake, m_real, h_real, m_fake, s, eps, L, shared=(0, 0)):
         """shared = (period, len) in flattened columns: the shared-context hint of kccot_mixed_loss_*_ctx."""
-        R, F = _flat_rows(real, "f_real"), _flat_rows(fake, "f_fake")
+        dtypes = [t.dtype if isinstance(t, torch.Tensor) else None for t in (real, fake, h_fake, m_real, h_real, m_fake)]
+        R, F, bf16 = _videos(real, fake)
+        if R.dim() < 2 or F.dim() < 2:
+            raise ValueError(f"f_real / f_fake: expected [batch, ...], got shapes {tuple(real.shape)} / "
+                             f"{tuple(fake.shape)}")
+        R, F = R.reshape(R.shape[0], -1), F.reshape(F.shape[0], -1)
         if R.shape != F.shape:
             raise ValueError(f"f_real and f_fake must have the same shape, got {tuple(real.shape)} vs "
                              f"{tuple(fake.shape)}")
         B, K = R.shape
-        hs = [_check(t, n, 3) for t, n in ((h_fake, "h_fake"), (m_real, "m_real"), (h_real, "h_real"),
-                                           (m_fake, "m_fake"))]
+        hs = [_check_hm(t, n, 3) for t, n in ((h_fake, "h_fake"), (m_real, "m_real"), (h_real, "h_real"),
+                                              (m_fake, "m_fake"))]
         T, J = hs[0].shape[1], hs[0].shape[2]
         for t, n in zip(hs, ("h_fake", "m_real", "h_real", "m_fake")):
             if tuple(t.shape) != (B, T, J):
@@ -230,17 +274,17 @@ class MixedLossFn(torch.autograd.Function):
             raise ValueError(f"the martingale term needs at least 2 time steps, got T={T}")
         dev = R.device
         L = int(L)
-        saved_bytes, ws_bytes = _mixed_sizes(B, K, L)
+        saved_bytes, ws_bytes = _mixed_sizes(B, K, L, dtype=R.dtype)
         saved = torch.empty(saved_bytes, dtype=torch.uint8, device=dev)
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         out = torch.empty(4, dtype=torch.float32, device=dev)          # loss | xy, xx, yy
         with _on_device(dev):
-            _lib.call("kccot_mixed_loss_fwd_ctx", _ptr(R), _ptr(F), 1, B, K, _ptr(hs[0]), _ptr(hs[1]), _ptr(hs[2]),
-                      _ptr(hs[3]), T, J, float(s), float(eps), L, _ptr(saved), ctypes.c_void_p(out.data_ptr()),
-                      ctypes.c_void_p(out.data_ptr() + 4), _ptr(ws), ws_bytes, _PATH["flags"], _stream(dev),
-                      int(shared[0]), int(shared[1]))
+            _lib.call("kccot_mixed_loss_fwd_bf16" if bf16 else "kccot_mixed_loss_fwd_ctx", _ptr(R), _ptr(F), 1, B, K,
+                      _ptr(hs[0]), _ptr(hs[1]), _ptr(hs[2]), _ptr(hs[3]), T, J, float(s), float(eps), L, _ptr(saved),
+                      ctypes.c_void_p(out.data_ptr()), ctypes.c_void_p(out.data_ptr() + 4), _ptr(ws), ws_bytes,
+                      _PATH["flags"], _stream(dev), int(shared[0]), int(shared[1]))
         ctx.save_for_backward(R, F, *hs, saved)
-        ctx.meta = (real.shape, fake.shape, float(s), float(eps), L, (int(shared[0]), int(shared[1])))
+        ctx.meta = (real.shape, fake.shape, float(s), float(eps), L, (int(shared[0]), int(shared[1])), dtypes)
         loss, terms = out[0], out[1:]
         ctx.mark_non_differentiable(terms)
         ctx.set_materialize_grads(False)          # no zero-fill kernel for the unused gradient of `terms`
@@ -249,7 +293,8 @@ class MixedLossFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, gloss, _gterms):
         R, F, h_fake, m_real, h_real, m_fake, saved = ctx.saved_tensors
-        rshape, fshape, s, eps, L, shared = ctx.meta
+        rshape, fshape, s, eps, L, shared, dtypes = ctx.meta
+        bf16 = R.dtype == torch.bfloat16
         B, K = R.shape
         T, J = h_fake.shape[1], h_fake.shape[2]
         dev = R.device
@@ -265,16 +310,17 @@ class MixedLossFn(torch.autograd.Function):
         gm_real = torch.empty_like(m_real) if need[3] else None
         gh_real = torch.empty_like(h_real) if need[4] else None
         gm_fake = torch.empty_like(m_fake) if need[5] else None
-        _, ws_bytes = _mixed_sizes(B, K, L)
+        _, ws_bytes = _mixed_sizes(B, K, L, dtype=R.dtype)
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         with _on_device(dev):
-            _lib.call("kccot_mixed_loss_bwd_ctx", _ptr(gloss), _ptr(R), _ptr(F), 1, B, K, _ptr(h_fake), _ptr(m_real),
-                      _ptr(h_real), _ptr(m_fake), T, J, s, eps, L, _ptr(saved), _ptr(g_real), _ptr(g_fake),
-                      _ptr(gh_fake), _ptr(gm_real), _ptr(gh_real), _ptr(gm_fake), _ptr(ws), ws_bytes, _PATH["flags"],
-                      _stream(dev), shared[0], shared[1])
+            _lib.call("kccot_mixed_loss_bwd_bf16" if bf16 else "kccot_mixed_loss_bwd_ctx", _ptr(gloss), _ptr(R),
+                      _ptr(F), 1, B, K, _ptr(h_fake), _ptr(m_real), _ptr(h_real), _ptr(m_fake), T, J, s, eps, L,
+                      _ptr(saved), _ptr(g_real), _ptr(g_fake), _ptr(gh_fake), _ptr(gm_real), _ptr(gh_real),
+                      _ptr(gm_fake), _ptr(ws), ws_bytes, _PATH["flags"], _stream(dev), shared[0], shared[1])
         g_real = g_real.reshape(rshape) if g_real is not None else None
         g_fake = g_fake.reshape(fshape) if g_fake is not None else None
-        return g_real, g_fake, gh_fake, gm_real, gh_real, gm_fake, None, None, None, None
+        grads = _as_dtypes((g_real, g_fake, gh_fake, gm_real, gh_real, gm_fake), dtypes)
+        return (*grads, None, None, None, None)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -286,15 +332,16 @@ class MixedLossBatchedFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, real, fake, h_fake, m_real, h_real, m_fake, s, eps, L):
-        real, fake = _check(real, "f_real"), _check(fake, "f_fake")
+        dtypes = [t.dtype if isinstance(t, torch.Tensor) else None for t in (real, fake, h_fake, m_real, h_real, m_fake)]
+        real, fake, bf16 = _videos(real, fake)
         if real.dim() < 3 or real.shape != fake.shape:
             raise ValueError(f"f_real / f_fake: expected equal shapes [nprob, B, ...], got {tuple(real.shape)} vs "
                              f"{tuple(fake.shape)}")
         P, B = real.shape[0], real.shape[1]
         R, F = real.reshape(P, B, -1), fake.reshape(P, B, -1)
         K = R.shape[2]
-        hs = [_check(t, n, 4) for t, n in ((h_fake, "h_fake"), (m_real, "m_real"), (h_real, "h_real"),
-                                           (m_fake, "m_fake"))]
+        hs = [_check_hm(t, n, 4) for t, n in ((h_fake, "h_fake"), (m_real, "m_real"), (h_real, "h_real"),
+                                              (m_fake, "m_fake"))]
         T, J = hs[0].shape[2], hs[0].shape[3]
         for t, n in zip(hs, ("h_fake", "m_real", "h_real", "m_fake")):
             if tuple(t.shape) != (P, B, T, J):
@@ -303,17 +350,20 @@ class MixedLossBatchedFn(torch.autograd.Function):
             raise ValueError(f"the martingale term needs at least 2 time steps, got T={T}")
         dev = R.device
         L = int(L)
-        saved_bytes, ws_bytes = _mixed_sizes(B, K, L, P)
+        saved_bytes, ws_bytes = _mixed_sizes(B, K, L, P, R.dtype)
         saved = torch.empty(saved_bytes, dtype=torch.uint8, device=dev)
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         loss = torch.empty(P, dtype=torch.float32, device=dev)
         terms = torch.empty((P, 3), dtype=torch.float32, device=dev)
         with _on_device(dev):
-            _lib.call("kccot_mixed_loss_fwd", _ptr(R), _ptr(F), P, B, K, _ptr(hs[0]), _ptr(hs[1]), _ptr(hs[2]),
-                      _ptr(hs[3]), T, J, float(s), float(eps), L, _ptr(saved), _ptr(loss), _ptr(terms), _ptr(ws),
-                      ws_bytes, _PATH["flags"], _stream(dev))
+            args = (_ptr(R), _ptr(F), P, B, K, _ptr(hs[0]), _ptr(hs[1]), _ptr(hs[2]), _ptr(hs[3]), T, J, float(s),
+                    float(eps), L, _ptr(saved), _ptr(loss), _ptr(terms), _ptr(ws), ws_bytes, _PATH["flags"], _stream(dev))
+            if bf16:
+                _lib.call("kccot_mixed_loss_fwd_bf16", *args, 0, 0)
+            else:
+                _lib.call("kccot_mixed_loss_fwd", *args)
         ctx.save_for_backward(R, F, *hs, saved)
-        ctx.meta = (real.shape, fake.shape, float(s), float(eps), L)
+        ctx.meta = (real.shape, fake.shape, float(s), float(eps), L, dtypes)
         ctx.mark_non_differentiable(terms)
         ctx.set_materialize_grads(False)
         return loss, terms
@@ -321,7 +371,8 @@ class MixedLossBatchedFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, gloss, _gterms):
         R, F, h_fake, m_real, h_real, m_fake, saved = ctx.saved_tensors
-        rshape, fshape, s, eps, L = ctx.meta
+        rshape, fshape, s, eps, L, dtypes = ctx.meta
+        bf16 = R.dtype == torch.bfloat16
         P, B, K = R.shape
         T, J = h_fake.shape[2], h_fake.shape[3]
         dev = R.device
@@ -330,17 +381,20 @@ class MixedLossBatchedFn(torch.autograd.Function):
             return (None,) * 9
         gloss = gloss.reshape(P).float().contiguous()
         outs = [torch.empty_like(t) if need[i] else None for i, t in enumerate((R, F, h_fake, m_real, h_real, m_fake))]
-        _, ws_bytes = _mixed_sizes(B, K, L, P)
+        _, ws_bytes = _mixed_sizes(B, K, L, P, R.dtype)
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         with _on_device(dev):
-            _lib.call("kccot_mixed_loss_bwd", _ptr(gloss), _ptr(R), _ptr(F), P, B, K, _ptr(h_fake), _ptr(m_real),
-                      _ptr(h_real), _ptr(m_fake), T, J, s, eps, L, _ptr(saved), *[_ptr(o) for o in outs], _ptr(ws),
-                      ws_bytes, _PATH["flags"], _stream(dev))
+            args = (_ptr(gloss), _ptr(R), _ptr(F), P, B, K, _ptr(h_fake), _ptr(m_real), _ptr(h_real), _ptr(m_fake), T,
+                    J, s, eps, L, _ptr(saved), *[_ptr(o) for o in outs], _ptr(ws), ws_bytes, _PATH["flags"], _stream(dev))
+            if bf16:
+                _lib.call("kccot_mixed_loss_bwd_bf16", *args, 0, 0)
+            else:
+                _lib.call("kccot_mixed_loss_bwd", *args)
         if outs[0] is not None:
             outs[0] = outs[0].reshape(rshape)
         if outs[1] is not None:
             outs[1] = outs[1].reshape(fshape)
-        return (*outs, None, None, None)
+        return (*_as_dtypes(outs, dtypes), None, None, None)
 
 
 class MartingalePenaltyFn(torch.autograd.Function):

@@ -3,6 +3,10 @@
 Same function names, positional orders and defaults; inputs are torch CUDA fp32 tensors instead of
 TensorFlow eager tensors, outputs are tensors on the autograd tape (0-d where the reference
 returns a scalar).  All arithmetic runs in libkccot's sm_100a kernels (include/kccot.h).
+The mixed loss (compute_sinkhorn_loss and its variants below) also takes bf16 videos: the result is
+exactly that of the fp32 call on the widened videos, the video gradients come back in bf16 (the fp32
+gradient rounded to nearest even), and two bf16 videos are read as bf16 by the kernels (no fp32 copy
+at B <= 64 with B % 8 == 0 and K % 8 == 0, K >= 128).  The other functions stay fp32-only.
 
 Reference quirks are reproduced on purpose (SURVEY.md Appendix B):
   * compute_sinkhorn_loss passes `sinkhorn_eps, sinkhorn_l` positionally into compute_sinkhorn's
@@ -14,7 +18,7 @@ Reference quirks are reproduced on purpose (SURVEY.md Appendix B):
 """
 import torch
 
-from .functional import CostFn, MartingalePenaltyFn, MixedLossBatchedFn, MixedLossFn, SinkhornFn, _check
+from .functional import CostFn, MartingalePenaltyFn, MixedLossBatchedFn, MixedLossFn, SinkhornFn, _check_video
 
 __all__ = ["cost_xy", "modified_cost", "bi_causal_modified_cost", "benchmark_sinkhorn", "compute_sinkhorn",
            "compute_N", "scale_invariante_martingale_regularization", "compute_sinkhorn_loss"]
@@ -79,8 +83,8 @@ def compute_sinkhorn_loss(f_real, f_fake, scaling_coef, sinkhorn_eps, sinkhorn_l
     stacked Gram of [real; fake], the three solves run as three CTAs of one launch.
     """
     del sinkhorn_eps, sinkhorn_l      # reference quirk, see module docstring
-    f_real = _check(f_real, "f_real")
-    f_fake = _check(f_fake, "f_fake")
+    f_real = _check_video(f_real, "f_real")
+    f_fake = _check_video(f_fake, "f_fake")
     if video and (f_real.dim() != 5 or f_fake.dim() != 5):
         raise ValueError(f"video=True expects [B,H,T,W,C] tensors, got {tuple(f_real.shape)} / {tuple(f_fake.shape)}")
     if not video and (f_real.dim() != 3 or f_fake.dim() != 3):
@@ -105,8 +109,8 @@ def compute_sinkhorn_loss_shared_context(f_real, f_fake, scaling_coef, h_fake, m
     the returned gradient is ZERO there instead of the value the reference's tape would hand to the data tensor.
     Saves ctx/T of the fake video's forward traffic and ctx/T of the whole backward.  Not valid after temporal or
     3-D smoothing (it leaks predicted frames into the context frames).  Returns (loss, [xy, xx, yy])."""
-    f_real = _check(f_real, "f_real")
-    f_fake = _check(f_fake, "f_fake")
+    f_real = _check_video(f_real, "f_real")
+    f_fake = _check_video(f_fake, "f_fake")
     if f_real.dim() != 5 or f_fake.dim() != 5:
         raise ValueError(f"expected [B,H,T,W,C] videos, got {tuple(f_real.shape)} / {tuple(f_fake.shape)}")
     T, W, C = f_real.shape[2], f_real.shape[3], f_real.shape[4]

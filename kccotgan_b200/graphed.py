@@ -5,7 +5,8 @@ evaluation; at B=64 the kernels take ~200 us and the launch gaps another ~70 us.
 captures the same C-ABI launch chain once on static buffers and replays it with a single
 `cudaGraphLaunch`.  Contract (the usual static-buffer one): the caller writes the step's tensors into
 `.real, .fake, .h_fake, .m_real, .h_real, .m_fake` (or passes tensors that already live there), calls
-`step()`, and reads `.loss` and `.grads[...]`; no host synchronisation is involved.
+`step()`, and reads `.loss` and `.grads[...]`; no host synchronisation is involved.  `real` and `fake` may both be
+bf16 (the gradients of the videos are then bf16 too); h / m are fp32.
 """
 import torch
 
@@ -22,8 +23,11 @@ class GraphedSinkhornLoss:
         (zero copies: later steps must overwrite them in place); adopt=False clones them."""
         srcs = (real, fake, h_fake, m_real, h_real, m_fake)
         for t, n in zip(srcs, _NAMES):
-            if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float32):
+            if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype in (torch.float32, torch.bfloat16)):
                 raise ValueError(f"{n}: expected a CUDA float32 tensor")
+        # bf16 videos (the bf16 entry points of the library) when both are bf16; h / m stay fp32
+        if real.dtype != fake.dtype or any(t.dtype != torch.float32 for t in srcs[2:]):
+            raise ValueError("real / fake: expected both float32 or both bfloat16; h / m: expected float32")
         self.scaling_coef = float(scaling_coef)
         self.ctx_frames = int(ctx_frames)       # > 0: gan_utils.compute_sinkhorn_loss_shared_context
         bufs = [t.detach() if adopt else t.detach().clone() for t in srcs]
