@@ -9,8 +9,8 @@
  * the stub for the reference's own TensorFlow training loop.
  *
  * Conventions
- *   - All pointers are DEVICE pointers to contiguous fp32 unless stated (the *_bf16 mixed-loss
- *     entries take bf16 videos); the caller owns every
+ *   - All pointers are DEVICE pointers to contiguous fp32 unless stated (the *_bf16 mixed-loss and
+ *     smoothing entries take bf16 videos); the caller owns every
  *     buffer (inputs, outputs, saved state, workspace).  The library allocates nothing per call
  *     and keeps no pointer after return.
  *   - `stream` is a cudaStream_t passed as void*.  Calls only enqueue work; none synchronises.
@@ -277,6 +277,31 @@ int kccot_smooth_fwd(int mode, const float* x, int B, int H, int T, int W, int C
 int kccot_smooth_bwd(int mode, const float* gout, const float* out, const float* maxval, int B, int H,
                      int T, int W, int C, const float* taps_t, int radius_t, const float* taps_s,
                      int radius_s, float* gx, void* ws, size_t ws_bytes, void* stream);
+
+/* bf16 videos — the smoothing for callers that keep their videos in bf16.  x, out, gout and gx are raw bf16 bits
+ * (uint16_t), any alignment; maxval, the taps and the workspace (kccot_smooth_workspace_bytes: mode 3 keeps its two
+ * intermediates in fp32) are as in the fp32 entries, and so are the argument checks, error codes and limits.
+ * `ties` [kccot_smooth_ties_bytes] is a caller-owned bit mask, 4-byte aligned, written by the forward (which zeroes it
+ * first) and read by the backward: bit e % 32 of word e / 32 is set where element e is a tied maximum.
+ * Contract, for bf16 x (a bf16 value is exact in fp32):
+ *   fwd: out is kccot_smooth_fwd on the widened x rounded to nearest even, maxval bit-identical.  The kernels widen on
+ *        load, keep every intermediate in fp32 with the fp32 coefficients and FMA order, and round only at the store.
+ *   ties: the elements whose fp32 quotient conv(x) / maxval is exactly 1.0f, the set the fp32 backward finds with
+ *        out == 1.0f.  The bf16 out cannot carry it: every fp32 value in [1 - 2^-9, 1) rounds to 1.0.
+ *   bwd: gx is the fp32 backward on the widened gout rounded to nearest even, bit for bit at every element outside
+ *        the adjoint stencil's support of the tied maxima; inside it gx differs only through S = sum(gout * out),
+ *        which is formed from the bf16 out.  The tie count is the popcount of the mask.
+ * Both calls are graph-capturable (the taps travel as kernel arguments; the mask and the sums are cleared with
+ * cudaMemsetAsync). */
+size_t kccot_smooth_ties_bytes(int B, int H, int T, int W, int C);   /* ceil(B*H*T*W*C / 32) * 4 */
+int kccot_smooth_fwd_bf16(int mode, const uint16_t* x, int B, int H, int T, int W, int C,
+                          const float* taps_t, int radius_t, const float* taps_s, int radius_s,
+                          uint16_t* out, float* maxval, uint32_t* ties, void* ws, size_t ws_bytes,
+                          void* stream);
+int kccot_smooth_bwd_bf16(int mode, const uint16_t* gout, const uint16_t* out, const float* maxval,
+                          const uint32_t* ties, int B, int H, int T, int W, int C, const float* taps_t,
+                          int radius_t, const float* taps_s, int radius_s, uint16_t* gx, void* ws,
+                          size_t ws_bytes, void* stream);
 
 #ifdef __cplusplus
 }

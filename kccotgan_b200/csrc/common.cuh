@@ -1,5 +1,6 @@
 // Shared helpers for libkccot (sm_100a only).
 #pragma once
+#include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -135,6 +136,18 @@ __device__ __forceinline__ float fast_log2(float x) {
   float y;
   asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
   return y;
+}
+
+// bf16 as raw bits (uint16_t): widening to fp32 is exact, narrowing rounds to nearest even
+// four bf16 (element 0 in the low half of .x) -> fp32
+__device__ __forceinline__ float4 widen_bf16x4(uint2 v) {
+  return make_float4(__uint_as_float(v.x << 16), __uint_as_float(v.x & 0xffff0000u), __uint_as_float(v.y << 16),
+                     __uint_as_float(v.y & 0xffff0000u));
+}
+// two fp32 -> two bf16 in one word (lo in the low half)
+__device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
+  const __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
+  return *reinterpret_cast<const uint32_t*>(&h);
 }
 
 }  // namespace kccot

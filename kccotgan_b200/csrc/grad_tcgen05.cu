@@ -34,8 +34,6 @@
 //   Epilogue:   each of the four epilogue warps owns one quadrant: lanes 0-15 add their two column halves, lanes
 //               16-31 hand W'lo.Zhi down by shuffle; 16 rows per warp are staged in 128-byte-swizzled shared memory
 //               and one TMA store (or reduce-add) writes the [N x 32] box as full 128-byte row segments.
-#include <cuda_bf16.h>
-
 #include "cost.cuh"
 #include "tc_common.cuh"
 
@@ -126,10 +124,6 @@ __device__ __forceinline__ uint2 lds64(uint32_t saddr) {
   uint2 v;
   asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(v.x), "=r"(v.y) : "r"(saddr));
   return v;
-}
-__device__ __forceinline__ uint32_t pack_bf16x2_rn(float lo, float hi) {
-  const __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
-  return *reinterpret_cast<const uint32_t*>(&h);
 }
 
 template <bool kBf16>
@@ -399,10 +393,10 @@ __device__ __forceinline__ void grad_tc_body(const CUtensorMap& tmx, const CUten
 #pragma unroll
           for (int q = 0; q < 4; ++q)
             tc::sts128(row + ((q ^ ((r >> 1) & 3)) << 4),
-                       make_float4(__uint_as_float(pack_bf16x2_rn(d[8 * q], d[8 * q + 1])),
-                                   __uint_as_float(pack_bf16x2_rn(d[8 * q + 2], d[8 * q + 3])),
-                                   __uint_as_float(pack_bf16x2_rn(d[8 * q + 4], d[8 * q + 5])),
-                                   __uint_as_float(pack_bf16x2_rn(d[8 * q + 6], d[8 * q + 7]))));
+                       make_float4(__uint_as_float(pack_bf16x2(d[8 * q], d[8 * q + 1])),
+                                   __uint_as_float(pack_bf16x2(d[8 * q + 2], d[8 * q + 3])),
+                                   __uint_as_float(pack_bf16x2(d[8 * q + 4], d[8 * q + 5])),
+                                   __uint_as_float(pack_bf16x2(d[8 * q + 6], d[8 * q + 7]))));
         } else {
           const uint32_t row = tc::smem_u32(obuf + ob * kObufBytes) + r * 128;
 #pragma unroll

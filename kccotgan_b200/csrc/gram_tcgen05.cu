@@ -63,11 +63,6 @@ __device__ __forceinline__ uint2 lds64(uint32_t saddr) {
   asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(v.x), "=r"(v.y) : "r"(saddr));
   return v;
 }
-// four bf16 (raw bits, element 0 in the low half of .x) -> fp32, exact
-__device__ __forceinline__ float4 widen_bf16x4(uint2 v) {
-  return make_float4(__uint_as_float(v.x << 16), __uint_as_float(v.x & 0xffff0000u), __uint_as_float(v.y << 16),
-                     __uint_as_float(v.y & 0xffff0000u));
-}
 }  // namespace
 
 __global__ void __launch_bounds__(kThreads, 1)

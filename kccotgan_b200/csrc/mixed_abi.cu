@@ -1,16 +1,10 @@
 // Fused entry points of the mixed Sinkhorn loss (gan_utils.py:204-227): one C-ABI call enqueues the
 // whole forward (or backward) chain on the caller's stream.
-#include <cuda_bf16.h>
-
 #include "cost.cuh"
 #include "sinkhorn.cuh"
 
 namespace kccot {
 namespace {
-__device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
-  const __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
-  return *reinterpret_cast<const uint32_t*>(&h);
-}
 struct SavedLayout {
   size_t off_C3, off_uh, off_vh, off_nits, off_cost, off_cnt, total;
 };
@@ -69,10 +63,8 @@ __global__ void __launch_bounds__(256) widen_bf16_kernel(const uint16_t* __restr
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n8; i += stride) {
     const uint4 v = reinterpret_cast<const uint4*>(src)[i];
     float4* d = reinterpret_cast<float4*>(dst) + 2 * i;
-    d[0] = make_float4(__uint_as_float(v.x << 16), __uint_as_float(v.x & 0xffff0000u), __uint_as_float(v.y << 16),
-                       __uint_as_float(v.y & 0xffff0000u));
-    d[1] = make_float4(__uint_as_float(v.z << 16), __uint_as_float(v.z & 0xffff0000u), __uint_as_float(v.w << 16),
-                       __uint_as_float(v.w & 0xffff0000u));
+    d[0] = widen_bf16x4(make_uint2(v.x, v.y));
+    d[1] = widen_bf16x4(make_uint2(v.z, v.w));
   }
   for (long long i = 8 * n8 + blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += stride)
     dst[i] = __uint_as_float((uint32_t)src[i] << 16);

@@ -256,6 +256,281 @@ __global__ void __launch_bounds__(FT) tie_sums_kernel(const float* __restrict__ 
   }
 }
 
+// ---- bf16 videos ----------------------------------------------------------------------------------------------------
+// The bf16 passes are axis_col_kernel / axis_tile_kernel / tie_sums_kernel with other load and store sides, written as
+// kernels of their own so that the fp32 kernels keep their code.  TI / TO is the element type a pass reads / writes:
+// uint16_t (bf16 raw bits) on the first pass of a call and the last, float for the fp32 intermediates of mode 3, whose
+// middle passes are the fp32 kernels themselves.  Loads widen (exact), every sum is formed in fp32 with the same
+// coefficients and the same FMA order per element, whatever the vector width, and only the final store rounds (nearest
+// even): the output is the fp32 call's output rounded.
+// The backward needs the set of tied maxima, out == 1.0f in fp32, which a bf16 output cannot carry (every fp32 value in
+// [1 - 2^-9, 1) rounds to 1.0).  So the forward's last pass sets bit e of `ties` where its fp32 quotient is exactly 1.0f
+// (an atomicOr per tied element, so about one per call), and the backward reads the bit.
+struct Ties {
+  uint32_t* bits;         // bit e % 32 of bits[e / 32]: element e is a tied maximum.  Set by the forward's last pass
+                          // (MODE & 4), read by the backward's first (MODE & 8)
+  const float* maxval;
+  const float* sums;      // [0] = sum(gout*out) over the bf16 out, [1] = number of tied maxima (popcount of bits)
+};
+
+// V = 8 (16-byte bf16 / 2 x 16-byte fp32 accesses), 4 (8-byte bf16 / 16-byte fp32 accesses) or 1
+template <int V> struct VecF { float v[V]; };
+template <int V, typename T>
+__device__ __forceinline__ void load_v(VecF<V>& r, const T* p) {
+  if constexpr (V == 8 && sizeof(T) == 2) {
+    const uint4 u = *reinterpret_cast<const uint4*>(p);
+    const float4 a = widen_bf16x4(make_uint2(u.x, u.y)), b = widen_bf16x4(make_uint2(u.z, u.w));
+    r.v[0] = a.x; r.v[1] = a.y; r.v[2] = a.z; r.v[3] = a.w; r.v[4] = b.x; r.v[5] = b.y; r.v[6] = b.z; r.v[7] = b.w;
+  } else if constexpr (V == 8) {
+    const float4 a = reinterpret_cast<const float4*>(p)[0], b = reinterpret_cast<const float4*>(p)[1];
+    r.v[0] = a.x; r.v[1] = a.y; r.v[2] = a.z; r.v[3] = a.w; r.v[4] = b.x; r.v[5] = b.y; r.v[6] = b.z; r.v[7] = b.w;
+  } else if constexpr (V == 4) {
+    const float4 a = sizeof(T) == 2 ? widen_bf16x4(*reinterpret_cast<const uint2*>(p))
+                                    : *reinterpret_cast<const float4*>(p);
+    r.v[0] = a.x; r.v[1] = a.y; r.v[2] = a.z; r.v[3] = a.w;
+  } else if constexpr (sizeof(T) == 2) {
+    r.v[0] = __uint_as_float((uint32_t)*p << 16);
+  } else {
+    r.v[0] = *p;
+  }
+}
+template <int V, typename T>
+__device__ __forceinline__ void store_v(T* p, const VecF<V>& r) {
+  if constexpr (V == 8 && sizeof(T) == 2) {
+    *reinterpret_cast<uint4*>(p) = make_uint4(pack_bf16x2(r.v[0], r.v[1]), pack_bf16x2(r.v[2], r.v[3]),
+                                              pack_bf16x2(r.v[4], r.v[5]), pack_bf16x2(r.v[6], r.v[7]));
+  } else if constexpr (V == 8) {
+    reinterpret_cast<float4*>(p)[0] = make_float4(r.v[0], r.v[1], r.v[2], r.v[3]);
+    reinterpret_cast<float4*>(p)[1] = make_float4(r.v[4], r.v[5], r.v[6], r.v[7]);
+  } else if constexpr (V == 4 && sizeof(T) == 2) {
+    *reinterpret_cast<uint2*>(p) = make_uint2(pack_bf16x2(r.v[0], r.v[1]), pack_bf16x2(r.v[2], r.v[3]));
+  } else if constexpr (V == 4) {
+    *reinterpret_cast<float4*>(p) = make_float4(r.v[0], r.v[1], r.v[2], r.v[3]);
+  } else if constexpr (sizeof(T) == 2) {
+    *p = __bfloat16_as_ushort(__float2bfloat16_rn(r.v[0]));
+  } else {
+    *p = r.v[0];
+  }
+}
+// the BwdIn transform of the fp32 kernels with the tie bits in place of out == 1.0f; e % V == 0
+template <int V>
+__device__ __forceinline__ void bwd_v(VecF<V>& r, float sc, float tie, const uint32_t* bits, long long e) {
+  const uint32_t b = bits[e >> 5] >> (e & 31);
+#pragma unroll
+  for (int j = 0; j < V; ++j) r.v[j] = r.v[j] * sc + (((b >> j) & 1u) ? tie : 0.f);
+}
+// sets the tie bits of the V elements e.. whose quotient is exactly 1.0f; e % V == 0
+template <int V>
+__device__ __forceinline__ void mark_ties(uint32_t* bits, const VecF<V>& r, long long e) {
+  uint32_t b = 0;
+#pragma unroll
+  for (int j = 0; j < V; ++j) b |= (r.v[j] == 1.0f ? 1u : 0u) << j;
+  if (b) atomicOr(bits + (e >> 5), b << (e & 31));
+}
+
+// axis_col_kernel for bf16 (MODE bits as there; MODE & 4 also marks the ties, MODE & 8 reads them)
+template <typename TI, typename TO, int MODE, int V, int R>
+__global__ void __launch_bounds__(FT) axis_col_bf16_kernel(const TI* __restrict__ in, TO* __restrict__ out,
+                                                           long long outer, int n, long long inner, const Taps tp,
+                                                           float* gmax, const float* divisor, Ties tie) {
+  constexpr int kR = R, kTaps = 2 * R + 1;
+  extern __shared__ float coef[];                          // coef[p][d] = A[p][p + d - R] (0 outside the matrix)
+  for (int e = threadIdx.x; e < n * kTaps; e += FT) {
+    const int p = e / kTaps, q = p + (e % kTaps) - kR;
+    coef[e] = (q >= 0 && q < n) ? band_coef<R>(tp, n, p, q, (MODE & 16) != 0) : 0.f;
+  }
+  __syncthreads();
+  const long long iv = inner / V;
+  const long long gid = (long long)blockIdx.x * FT + threadIdx.x;
+  float lmax = -3.0e38f;
+  if (gid < outer * iv) {
+    const long long o = gid / iv;
+    const long long base = o * n * inner + (gid - o * iv) * V;
+    float gscale = 0.f, gtie = 0.f, inv = 1.f;
+    if (MODE & 8) {
+      const float m = *tie.maxval;
+      gscale = 1.f / m;
+      gtie = -(tie.sums[0] / m) / tie.sums[1];
+    }
+    if (MODE & 4) inv = *divisor;
+    auto fetch = [&](int q) {
+      VecF<V> r;
+      if (q < n) {
+        load_v<V>(r, in + base + (long long)q * inner);
+        if (MODE & 8) bwd_v<V>(r, gscale, gtie, tie.bits, base + (long long)q * inner);
+      } else {
+#pragma unroll
+        for (int j = 0; j < V; ++j) r.v[j] = 0.f;
+      }
+      return r;
+    };
+    VecF<V> win[kTaps];
+#pragma unroll
+    for (int d = 0; d < kR; ++d)
+#pragma unroll
+      for (int j = 0; j < V; ++j) win[d].v[j] = 0.f;
+#pragma unroll
+    for (int d = kR; d < kTaps; ++d) win[d] = fetch(d - kR);
+    // two rows in flight per thread where the window leaves registers for it (a bf16 pass has half the fp32 threads)
+    constexpr bool kDeep = V * kTaps <= 64;
+    VecF<V> next = fetch(kR + 1), next2;
+    for (int p = 0; p < n; ++p) {
+      if constexpr (kDeep) next2 = fetch(p + kR + 2);
+      VecF<V> acc;
+#pragma unroll
+      for (int j = 0; j < V; ++j) acc.v[j] = 0.f;
+#pragma unroll
+      for (int d = 0; d < kTaps; ++d) {
+        const float c = coef[p * kTaps + d];
+#pragma unroll
+        for (int j = 0; j < V; ++j) acc.v[j] = fmaf(c, win[d].v[j], acc.v[j]);
+      }
+      if (MODE & 4) {
+#pragma unroll
+        for (int j = 0; j < V; ++j) acc.v[j] /= inv;
+        mark_ties<V>(tie.bits, acc, base + (long long)p * inner);
+      }
+      if (MODE & 2) {
+#pragma unroll
+        for (int j = 0; j < V; ++j) lmax = fmaxf(lmax, acc.v[j]);
+      }
+      if (MODE & 1) store_v<V>(out + base + (long long)p * inner, acc);
+#pragma unroll
+      for (int d = 0; d < kTaps - 1; ++d) win[d] = win[d + 1];
+      win[kTaps - 1] = next;
+      if constexpr (kDeep) next = next2;
+      else next = fetch(p + kR + 2);
+    }
+  }
+  if (MODE & 2) {
+    lmax = warp_max(lmax);
+    if ((threadIdx.x & 31) == 0) atomic_max_float(gmax, lmax);
+  }
+}
+
+// axis_tile_kernel for bf16
+template <typename TI, typename TO, int MODE, int R>
+__global__ void __launch_bounds__(1024) axis_tile_bf16_kernel(const TI* __restrict__ in, TO* __restrict__ out,
+                                                              long long outer, int n, int inner, int o_chunk,
+                                                              const Taps tp, float* gmax, const float* divisor,
+                                                              Ties tie) {
+  constexpr int kR = R, kTaps = 2 * R + 1;
+  extern __shared__ __align__(16) float tile[];            // [o_chunk][n][inner], contiguous like global memory
+  const int ni = n * inner;
+  const long long o0 = (long long)blockIdx.x * o_chunk;
+  const int no = (int)min((long long)o_chunk, outer - o0);
+  const long long g0 = o0 * ni;
+  const int telems = no * ni;
+  float gscale = 0.f, gtie = 0.f, inv = 1.f;
+  if (MODE & 8) {
+    const float m = *tie.maxval;
+    gscale = 1.f / m;
+    gtie = -(tie.sums[0] / m) / tie.sums[1];
+  }
+  if (MODE & 4) inv = *divisor;
+  if ((ni & 7) == 0 && (reinterpret_cast<uintptr_t>(in) & 15) == 0) {
+    for (int e = threadIdx.x * 8; e < telems; e += blockDim.x * 8) {
+      VecF<8> r;
+      load_v<8>(r, in + g0 + e);
+      if (MODE & 8) bwd_v<8>(r, gscale, gtie, tie.bits, g0 + e);
+      store_v<8>(tile + e, r);
+    }
+  } else {
+    for (int e = threadIdx.x; e < telems; e += blockDim.x) {
+      VecF<1> r;
+      load_v<1>(r, in + g0 + e);
+      if (MODE & 8) bwd_v<1>(r, gscale, gtie, tie.bits, g0 + e);
+      tile[e] = r.v[0];
+    }
+  }
+  const int t = threadIdx.x;
+  float c[kTaps];
+  int off[kTaps];
+  {
+    const int p = min(t, ni - 1) / inner;
+#pragma unroll
+    for (int d = 0; d < kTaps; ++d) {
+      const int q = p + d - kR;
+      const bool ok = q >= 0 && q < n;
+      c[d] = ok ? band_coef<R>(tp, n, p, q, (MODE & 16) != 0) : 0.f;
+      off[d] = ok ? (d - kR) * inner : 0;
+    }
+  }
+  __syncthreads();
+  float lmax = -3.0e38f;
+  auto row_out = [&](int oo) {
+    const float* row = tile + oo * ni + t;
+    VecF<1> acc;
+    acc.v[0] = 0.f;
+#pragma unroll
+    for (int d = 0; d < kTaps; ++d) acc.v[0] = fmaf(c[d], row[off[d]], acc.v[0]);
+    const long long e = g0 + (long long)oo * ni + t;
+    if (MODE & 4) {
+      acc.v[0] = acc.v[0] / inv;
+      mark_ties<1>(tie.bits, acc, e);
+    }
+    if (MODE & 2) lmax = fmaxf(lmax, acc.v[0]);
+    if (MODE & 1) store_v<1>(out + e, acc);
+  };
+  if (t < ni) {
+    if constexpr ((MODE & 2) != 0) {
+#pragma unroll 1     // unrolled, the max pass spills at R = 5, 6 (64 registers per thread at 1024 threads)
+      for (int oo = 0; oo < no; ++oo) row_out(oo);
+    } else {
+      for (int oo = 0; oo < no; ++oo) row_out(oo);
+    }
+  }
+  if (MODE & 2) {
+    lmax = warp_max(lmax);
+    if ((threadIdx.x & 31) == 0) atomic_max_float(gmax, lmax);
+  }
+}
+
+// tie_sums_kernel for bf16: sums[0] = sum gout * out (bf16 out), sums[1] = popcount of the tie bits (nwords words)
+__global__ void __launch_bounds__(FT) tie_sums_bf16_kernel(const uint16_t* __restrict__ gout,
+                                                           const uint16_t* __restrict__ out,
+                                                           const uint32_t* __restrict__ bits, long long n,
+                                                           long long nwords, float* sums) {
+  float s = 0.f;
+  unsigned cnt = 0;
+  const long long stride = (long long)gridDim.x * FT;
+  const long long tid = (long long)blockIdx.x * FT + threadIdx.x;
+  const bool vec = ((reinterpret_cast<uintptr_t>(gout) | reinterpret_cast<uintptr_t>(out)) & 15) == 0;
+  const long long n8 = vec ? n / 8 : 0;
+  const uint4* g8 = reinterpret_cast<const uint4*>(gout);
+  const uint4* o8 = reinterpret_cast<const uint4*>(out);
+  auto acc8 = [&](const uint4& g, const uint4& o) {
+    const float4 g0 = widen_bf16x4(make_uint2(g.x, g.y)), g1 = widen_bf16x4(make_uint2(g.z, g.w));
+    const float4 o0 = widen_bf16x4(make_uint2(o.x, o.y)), o1 = widen_bf16x4(make_uint2(o.z, o.w));
+    s = fmaf(g0.x, o0.x, s); s = fmaf(g0.y, o0.y, s); s = fmaf(g0.z, o0.z, s); s = fmaf(g0.w, o0.w, s);
+    s = fmaf(g1.x, o1.x, s); s = fmaf(g1.y, o1.y, s); s = fmaf(g1.z, o1.z, s); s = fmaf(g1.w, o1.w, s);
+  };
+  long long i = tid;
+  for (; i + 3 * stride < n8; i += 4 * stride) {
+    uint4 g[4], o[4];
+#pragma unroll
+    for (int u = 0; u < 4; ++u) { g[u] = __ldg(g8 + i + u * stride); o[u] = __ldg(o8 + i + u * stride); }
+#pragma unroll
+    for (int u = 0; u < 4; ++u) acc8(g[u], o[u]);
+  }
+  for (; i < n8; i += stride) acc8(__ldg(g8 + i), __ldg(o8 + i));
+  for (long long k = 8 * n8 + tid; k < n; k += stride)
+    s = fmaf(__uint_as_float((uint32_t)gout[k] << 16), __uint_as_float((uint32_t)out[k] << 16), s);
+  for (long long w = tid; w < nwords; w += stride) cnt += __popc(bits[w]);
+  __shared__ float red[2][FT / 32];
+  s = warp_sum(s);
+  const float c = warp_sum((float)cnt);
+  if ((threadIdx.x & 31) == 0) { red[0][threadIdx.x >> 5] = s; red[1][threadIdx.x >> 5] = c; }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float ss = 0.f, cc = 0.f;
+#pragma unroll
+    for (int w = 0; w < FT / 32; ++w) { ss += red[0][w]; cc += red[1][w]; }
+    atomicAdd(&sums[0], ss);
+    atomicAdd(&sums[1], cc);
+  }
+}
+
 struct AxisPlan { long long outer, inner; int n, o_chunk; bool tiled; };
 AxisPlan plan_axis(long long outer, int n, long long inner) {
   AxisPlan p;
@@ -314,6 +589,71 @@ int make_taps(Taps* tp, const float* w, int radius, const char* what) {
   }
   tp->r = radius;
   for (int k = 0; k < 2 * kMaxRadius + 1; ++k) tp->w[k] = k < 2 * radius + 1 ? w[k] : 0.f;
+  return KCCOT_OK;
+}
+
+// run_axis for the bf16 passes (TI / TO as in axis_col_bf16_kernel; MODE 2 passes write nothing and take TO = uint16_t)
+template <typename TI, typename TO, int MODE, int R>
+int run_axis_bf16_r(const TI* in, TO* out, const AxisPlan& p, const Taps& tp, float* gmax, const float* divisor,
+                    Ties tie, cudaStream_t st) {
+  if (p.tiled) {
+    const int ni = p.n * (int)p.inner;
+    const int threads = (ni + 31) / 32 * 32;
+    const unsigned grid = (unsigned)((p.outer + p.o_chunk - 1) / p.o_chunk);
+    const size_t smem = (size_t)p.o_chunk * ni * sizeof(float);
+    axis_tile_bf16_kernel<TI, TO, MODE, R><<<grid, threads, smem, st>>>(in, out, p.outer, p.n, (int)p.inner, p.o_chunk,
+                                                                       tp, gmax, divisor, tie);
+  } else {
+    // widest access the shape and pointers allow, but 4 instead of 8 elements per thread while 8 would leave fewer
+    // than ~1 000 threads per SM (config 3's T pass: 98 304 threads at 8, 196 608 at 4)
+    auto fits = [&](int v) {
+      const uintptr_t a = (uintptr_t)(v * sizeof(TI) < 16 ? v * sizeof(TI) : 16) - 1;
+      const uintptr_t b = (uintptr_t)(v * sizeof(TO) < 16 ? v * sizeof(TO) : 16) - 1;
+      return p.inner % v == 0 && (reinterpret_cast<uintptr_t>(in) & a) == 0 &&
+             (!(MODE & 1) || (reinterpret_cast<uintptr_t>(out) & b) == 0);
+    };
+    const int v = fits(8) && p.outer * (p.inner / 8) >= 1024LL * num_sms() ? 8 : fits(4) ? 4 : fits(8) ? 8 : 1;
+    const long long total = p.outer * (p.inner / v);
+    const unsigned grid = (unsigned)((total + FT - 1) / FT);
+    const size_t smem = (size_t)p.n * (2 * R + 1) * sizeof(float);
+    auto kernel = v == 8 ? axis_col_bf16_kernel<TI, TO, MODE, 8, R>
+                         : v == 4 ? axis_col_bf16_kernel<TI, TO, MODE, 4, R> : axis_col_bf16_kernel<TI, TO, MODE, 1, R>;
+    if (smem > 48 * 1024)
+      KCCOT_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kernel<<<grid, FT, smem, st>>>(in, out, p.outer, p.n, p.inner, tp, gmax, divisor, tie);
+  }
+  KCCOT_LAUNCH_CHECK();
+  return KCCOT_OK;
+}
+template <typename TI, typename TO, int MODE>
+int run_axis_bf16(const TI* in, TO* out, const AxisPlan& p, const Taps& tp, float* gmax, const float* divisor, Ties tie,
+                  cudaStream_t st) {
+  switch (tp.r) {
+    case 1: return run_axis_bf16_r<TI, TO, MODE, 1>(in, out, p, tp, gmax, divisor, tie, st);
+    case 2: return run_axis_bf16_r<TI, TO, MODE, 2>(in, out, p, tp, gmax, divisor, tie, st);
+    case 3: return run_axis_bf16_r<TI, TO, MODE, 3>(in, out, p, tp, gmax, divisor, tie, st);
+    case 4: return run_axis_bf16_r<TI, TO, MODE, 4>(in, out, p, tp, gmax, divisor, tie, st);
+    case 5: return run_axis_bf16_r<TI, TO, MODE, 5>(in, out, p, tp, gmax, divisor, tie, st);
+    case 6: return run_axis_bf16_r<TI, TO, MODE, 6>(in, out, p, tp, gmax, divisor, tie, st);
+  }
+  set_error("smoothing radius %d not supported (1..%d)", tp.r, kMaxRadius);
+  return KCCOT_EUNSUPPORTED;
+}
+
+// argument checks of the bf16 entries: those of kccot_smooth_fwd, all made before any CUDA call
+int smooth_bf16_args(int mode, int B, int H, int T, int W, int C, const float* taps_t, int radius_t,
+                     const float* taps_s, int radius_s, void* ws, size_t ws_bytes, Taps* tp) {
+  KCCOT_CHECK_ARG(B >= 1 && H >= 1 && T >= 1 && W >= 1 && C >= 1, "bad sizes");
+  KCCOT_CHECK_ARG(T <= kMaxAxis && H <= kMaxAxis && W <= kMaxAxis, "axis longer than %d not supported (H=%d T=%d W=%d)", kMaxAxis,
+                  H, T, W);
+  if (int rc = mode == 1 ? make_taps(tp, taps_t, radius_t, "temporal_convolution") : make_taps(tp, taps_s, radius_s,
+                                                                                            "gaussian_convolution3D"))
+    return rc;
+  KCCOT_CHECK_ARG(T > tp->r, "REFLECT padding by %d needs T > %d (T=%d)", tp->r, tp->r, T);
+  if (mode == 3) {
+    KCCOT_CHECK_ARG(H > tp->r && W > tp->r, "3-D smoothing needs H, W > %d (H=%d W=%d)", tp->r, H, W);
+    KCCOT_CHECK_ARG(ws && ws_bytes >= kccot_smooth_workspace_bytes(mode, B, H, T, W, C), "workspace too small");
+  }
   return KCCOT_OK;
 }
 }  // namespace
@@ -391,6 +731,75 @@ int kccot_smooth_bwd(int mode, const float* gout, const float* out, const float*
   if (int rc = run_axis<1 | 8 | 16>(gout, t1, pw, tp, nullptr, nullptr, bw, st)) return rc;
   if (int rc = run_axis<1 | 16>(t1, t2, pt, tp, nullptr, nullptr, none, st)) return rc;
   return run_axis<1 | 16>(t2, gx, ph, tp, nullptr, nullptr, none, st);
+}
+
+size_t kccot_smooth_ties_bytes(int B, int H, int T, int W, int C) {
+  if (B < 1 || H < 1 || T < 1 || W < 1 || C < 1) return 0;
+  const size_t n = (size_t)B * H * T * W * C;
+  return (n + 31) / 32 * sizeof(uint32_t);
+}
+
+int kccot_smooth_fwd_bf16(int mode, const uint16_t* x, int B, int H, int T, int W, int C, const float* taps_t,
+                          int radius_t, const float* taps_s, int radius_s, uint16_t* out, float* maxval,
+                          uint32_t* ties, void* ws, size_t ws_bytes, void* stream) {
+  KCCOT_CHECK_ARG(mode == 1 || mode == 3, "smoothing mode must be 1 (temporal) or 3 (3-D); the reference's '2d' "
+                                          "branch raises (data_utils.py:537-538)");
+  KCCOT_CHECK_ARG(x && out && maxval && ties, "null pointer");
+  KCCOT_CHECK_ARG((reinterpret_cast<uintptr_t>(ties) & 3) == 0, "tie mask must be 4-byte aligned");
+  Taps tp;
+  if (int rc = smooth_bf16_args(mode, B, H, T, W, C, taps_t, radius_t, taps_s, radius_s, ws, ws_bytes, &tp)) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  KCCOT_CUDA(cudaMemsetAsync(ties, 0, kccot_smooth_ties_bytes(B, H, T, W, C), st));
+  init_max_kernel<<<1, 1, 0, st>>>(maxval);
+  KCCOT_LAUNCH_CHECK();
+  const AxisPlan pt = plan_axis((long long)B * H, T, (long long)W * C);
+  const Ties tie{ties, nullptr, nullptr};
+  if (mode == 1) {
+    if (int rc = run_axis_bf16<uint16_t, uint16_t, 2>(x, nullptr, pt, tp, maxval, nullptr, tie, st)) return rc;
+    return run_axis_bf16<uint16_t, uint16_t, 1 | 4>(x, out, pt, tp, nullptr, maxval, tie, st);
+  }
+  // mode 3: bf16 -> fp32 H pass, the fp32 T pass and W max pass, fp32 -> bf16 W pass
+  const size_t n = align_up((size_t)B * H * T * W * C * sizeof(float), 256);
+  float* t1 = (float*)((char*)ws + 256);
+  float* t2 = (float*)((char*)ws + 256 + n);
+  const AxisPlan ph = plan_axis(B, H, (long long)T * W * C);
+  const AxisPlan pw = plan_axis((long long)B * H * T, W, C);
+  BwdIn none{};
+  if (int rc = run_axis_bf16<uint16_t, float, 1>(x, t1, ph, tp, nullptr, nullptr, tie, st)) return rc;
+  if (int rc = run_axis<1>(t1, t2, pt, tp, nullptr, nullptr, none, st)) return rc;
+  if (int rc = run_axis<2>(t2, nullptr, pw, tp, maxval, nullptr, none, st)) return rc;
+  return run_axis_bf16<float, uint16_t, 1 | 4>(t2, out, pw, tp, nullptr, maxval, tie, st);
+}
+
+int kccot_smooth_bwd_bf16(int mode, const uint16_t* gout, const uint16_t* out, const float* maxval,
+                          const uint32_t* ties, int B, int H, int T, int W, int C, const float* taps_t, int radius_t,
+                          const float* taps_s, int radius_s, uint16_t* gx, void* ws, size_t ws_bytes, void* stream) {
+  KCCOT_CHECK_ARG(mode == 1 || mode == 3, "smoothing mode must be 1 or 3");
+  KCCOT_CHECK_ARG(gout && out && maxval && ties && gx && ws && ws_bytes >= 256, "null pointer / workspace");
+  KCCOT_CHECK_ARG((reinterpret_cast<uintptr_t>(ties) & 3) == 0, "tie mask must be 4-byte aligned");
+  Taps tp;
+  if (int rc = smooth_bf16_args(mode, B, H, T, W, C, taps_t, radius_t, taps_s, radius_s, ws, ws_bytes, &tp)) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  const long long nel = (long long)B * H * T * W * C;
+  const long long nwords = (nel + 31) / 32;
+  float* sums = (float*)ws;
+  KCCOT_CUDA(cudaMemsetAsync(sums, 0, 2 * sizeof(float), st));
+  tie_sums_bf16_kernel<<<(unsigned)min((long long)4 * num_sms(), (nel / 8 + FT - 1) / FT + 1), FT, 0, st>>>(
+      gout, out, ties, nel, nwords, sums);
+  KCCOT_LAUNCH_CHECK();
+  const Ties tie{const_cast<uint32_t*>(ties), maxval, sums};     // read only: MODE & 4 is not set in the backward
+  const AxisPlan pt = plan_axis((long long)B * H, T, (long long)W * C);
+  if (mode == 1) return run_axis_bf16<uint16_t, uint16_t, 1 | 8 | 16>(gout, gx, pt, tp, nullptr, nullptr, tie, st);
+  // mode 3: bf16 -> fp32 W pass with the tie transform, the fp32 T pass, fp32 -> bf16 H pass
+  const size_t n = align_up((size_t)nel * sizeof(float), 256);
+  float* t1 = (float*)((char*)ws + 256);
+  float* t2 = (float*)((char*)ws + 256 + n);
+  const AxisPlan ph = plan_axis(B, H, (long long)T * W * C);
+  const AxisPlan pw = plan_axis((long long)B * H * T, W, C);
+  BwdIn none{};
+  if (int rc = run_axis_bf16<uint16_t, float, 1 | 8 | 16>(gout, t1, pw, tp, nullptr, nullptr, tie, st)) return rc;
+  if (int rc = run_axis<1 | 16>(t1, t2, pt, tp, nullptr, nullptr, none, st)) return rc;
+  return run_axis_bf16<float, uint16_t, 1 | 16>(t2, gx, ph, tp, nullptr, nullptr, tie, st);
 }
 
 }  // extern "C"

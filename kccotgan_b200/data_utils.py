@@ -2,11 +2,15 @@
 
 Only the kernel-smoothing class is on the loss hot path; the loaders, plotting helpers and LR
 schedules of the reference's data_utils are out of scope (SURVEY.md §2).
+
+The convolutions take CUDA fp32 or bf16 videos and return the input's dtype.  A bf16 video is smoothed by bf16
+kernels with fp32 arithmetic inside: the output is the fp32 output on the widened video rounded to nearest even, and
+the gradient is bf16 (kccot_smooth_fwd_bf16 / _bwd_bf16 in include/kccot.h).  Any other dtype raises ValueError.
 """
 import numpy as np
 import torch
 
-from .functional import SmoothFn, _check
+from .functional import SmoothFn, _check_video
 
 
 class KernelSmoothing:
@@ -47,7 +51,7 @@ class KernelSmoothing:
 
     def temporal_convolution(self, inputs, sigma):
         """data_utils.py:503-521 — (2r+1)-tap REFLECT filter along T, / global max."""
-        inputs = _check(inputs, "inputs", 5)
+        inputs = _check_video(inputs, "inputs", 5)
         self._check_axis("T", inputs.shape[2], self.temporal_radius)
         return SmoothFn.apply(inputs, 1, tuple(self._weights(self.temporal_radius, sigma)), None)
 
@@ -63,7 +67,7 @@ class KernelSmoothing:
     def gaussian_convolution3D(self, inputs, sigma):
         """data_utils.py:552-582 — (2r+1)^3 REFLECT filter over (H,T,W) per channel (three separable
         passes), / global max.  Uses the SPATIAL radius for all three axes (:553,562-564)."""
-        inputs = _check(inputs, "inputs", 5)
+        inputs = _check_video(inputs, "inputs", 5)
         _, H, T, W, _ = inputs.shape
         for name, n in (("H", H), ("T", T), ("W", W)):
             self._check_axis(name, n, self.spatial_radius)

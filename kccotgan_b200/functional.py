@@ -5,7 +5,8 @@ kernel.  Tensors must be CUDA fp32 — anything else raises ValueError (no fallb
 (MixedLossFn, MixedLossBatchedFn), which also takes bf16 videos and h / m: two bf16 videos run the bf16 entry points
 of the library (the result is exactly the fp32 one on the widened videos, video gradients rounded to bf16); a bf16
 video next to an fp32 one, and bf16 h / m, are widened with .float() (exact).  Gradients come back in the dtype of
-their input.
+their input.  The smoothing (SmoothFn) also takes bf16 videos: they run the bf16 entry points, whose output is the
+fp32 output on the widened video rounded to bf16, and whose gradient is bf16 (see kccot_smooth_fwd_bf16 in kccot.h).
 """
 import ctypes
 
@@ -64,13 +65,15 @@ def _check(t, name, ndim=None):
     return t.contiguous()
 
 
-def _check_video(t, name):
-    """A CUDA video of the mixed loss: fp32 or bf16, made contiguous."""
+def _check_video(t, name, ndim=None):
+    """A CUDA video of the mixed loss or the smoothing: fp32 or bf16, made contiguous."""
     if isinstance(t, torch.Tensor) and t.dtype == torch.bfloat16:
         if not t.is_cuda:
             raise ValueError(f"{name}: expected a CUDA tensor (kccotgan_b200 has no CPU path), got {t.device}")
+        if ndim is not None and t.dim() != ndim:
+            raise ValueError(f"{name}: expected {ndim} dimensions, got shape {tuple(t.shape)}")
         return t.contiguous()
-    return _check(t, name)
+    return _check(t, name, ndim)
 
 
 def _videos(real, fake):
@@ -438,36 +441,51 @@ def _taps(w):
 
 class SmoothFn(torch.autograd.Function):
     """mode 1: `taps_t` filters T; mode 3: `taps_s` filters H, T and W.  The weights are host sequences (they become
-    kernel arguments: nothing is copied to the device, so an annealed sigma costs nothing per step)."""
+    kernel arguments: nothing is copied to the device, so an annealed sigma costs nothing per step).
+    A bf16 x runs kccot_smooth_fwd_bf16 / _bwd_bf16: output and gradient are bf16, and the tie mask of the forward (the
+    elements at the maximum, which the bf16 output cannot tell apart from values just below it) is saved for the
+    backward."""
 
     @staticmethod
     def forward(ctx, x, mode, taps_t, taps_s):
-        x = _check(x, "inputs", 5)
+        x = _check_video(x, "inputs", 5)
+        bf16 = x.dtype == torch.bfloat16
         B, H, T, W, C = x.shape
         dev = x.device
+        lib = _lib.load()
         out = torch.empty_like(x)
         maxval = torch.empty((1,), dtype=torch.float32, device=dev)
-        ws = _ws(_lib.load().kccot_smooth_workspace_bytes(mode, B, H, T, W, C), dev)
+        ws = _ws(lib.kccot_smooth_workspace_bytes(mode, B, H, T, W, C), dev)
         at, rt = _taps(taps_t)
         as_, rs = _taps(taps_s)
         with _on_device(dev):
-            _lib.call("kccot_smooth_fwd", mode, _ptr(x), B, H, T, W, C, at, rt, as_, rs, _ptr(out), _ptr(maxval), _ptr(ws),
-                      ws.numel(), _stream(dev))
-        ctx.save_for_backward(out, maxval)
+            if bf16:
+                ties = torch.empty(lib.kccot_smooth_ties_bytes(B, H, T, W, C) // 4, dtype=torch.int32, device=dev)
+                _lib.call("kccot_smooth_fwd_bf16", mode, _ptr(x), B, H, T, W, C, at, rt, as_, rs, _ptr(out), _ptr(maxval),
+                          _ptr(ties), _ptr(ws), ws.numel(), _stream(dev))
+                ctx.save_for_backward(out, maxval, ties)
+            else:
+                _lib.call("kccot_smooth_fwd", mode, _ptr(x), B, H, T, W, C, at, rt, as_, rs, _ptr(out), _ptr(maxval),
+                          _ptr(ws), ws.numel(), _stream(dev))
+                ctx.save_for_backward(out, maxval)
         ctx.mode, ctx.taps = mode, (taps_t, taps_s)
         return out
 
     @staticmethod
     def backward(ctx, gout):
-        out, maxval = ctx.saved_tensors
+        out, maxval, *ties = ctx.saved_tensors
         B, H, T, W, C = out.shape
         dev = out.device
-        gout = gout.contiguous().float()
+        gout = gout.contiguous().to(out.dtype)
         gx = torch.empty_like(out)
         ws = _ws(_lib.load().kccot_smooth_workspace_bytes(ctx.mode, B, H, T, W, C), dev)
         at, rt = _taps(ctx.taps[0])
         as_, rs = _taps(ctx.taps[1])
         with _on_device(dev):
-            _lib.call("kccot_smooth_bwd", ctx.mode, _ptr(gout), _ptr(out), _ptr(maxval), B, H, T, W, C, at, rt, as_, rs,
-                      _ptr(gx), _ptr(ws), ws.numel(), _stream(dev))
+            if ties:
+                _lib.call("kccot_smooth_bwd_bf16", ctx.mode, _ptr(gout), _ptr(out), _ptr(maxval), _ptr(ties[0]), B, H, T,
+                          W, C, at, rt, as_, rs, _ptr(gx), _ptr(ws), ws.numel(), _stream(dev))
+            else:
+                _lib.call("kccot_smooth_bwd", ctx.mode, _ptr(gout), _ptr(out), _ptr(maxval), B, H, T, W, C, at, rt, as_,
+                          rs, _ptr(gx), _ptr(ws), ws.numel(), _stream(dev))
         return gx, None, None, None

@@ -6,7 +6,9 @@ returns a scalar).  All arithmetic runs in libkccot's sm_100a kernels (include/k
 The mixed loss (compute_sinkhorn_loss and its variants below) also takes bf16 videos: the result is
 exactly that of the fp32 call on the widened videos, the video gradients come back in bf16 (the fp32
 gradient rounded to nearest even), and two bf16 videos are read as bf16 by the kernels (no fp32 copy
-at B <= 64 with B % 8 == 0 and K % 8 == 0, K >= 128).  The other functions stay fp32-only.
+at B <= 64 with B % 8 == 0 and K % 8 == 0, K >= 128).  So can a bf16 video smoothed first by
+data_utils.KernelSmoothing, which returns bf16 (the whole smoothing -> loss -> adjoints chain then makes no fp32
+copy of a video).  The other functions here stay fp32-only.
 
 Reference quirks are reproduced on purpose (SURVEY.md Appendix B):
   * compute_sinkhorn_loss passes `sinkhorn_eps, sinkhorn_l` positionally into compute_sinkhorn's
