@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define KCCOT_VERSION 202
+#define KCCOT_VERSION 203
 #define KCCOT_SHARD_FLAGS_PER_RANK 256
 
 /* error codes */
@@ -117,30 +117,6 @@ int kccot_sinkhorn_fwd(const float* C, int nsolve, int B, float eps, int L, int 
 int kccot_sinkhorn_bwd(const float* C, int nsolve, int B, float eps, int L, const float* u_hist,
                        const float* v_hist, const int32_t* nits, const float* gcost, float* Cbar,
                        void* ws, size_t ws_bytes, void* stream);
-
-/* ------------------------------------------------------------------------------------------
- * Row-sharded Sinkhorn, host-driven variant (round 1; kept for callers that bring their own exchange): one call
- * per half-iteration pair, the CALLER moves the column statistics between ranks.  The fused variant below
- * (kccot_shard_sinkhorn_*) supersedes it.  This rank owns rows
- * [row0, row0+Brows) of the B x B cost (Crows [Brows,B]).  The u-update is local; the v-update needs a
- * column log-sum-exp over all rows: each rank produces colstat [2,B] = (max, sum exp2(. - max)) over its
- * rows, the CALLER all-gathers them (NCCL over NVLink) and every rank combines.  The reverse pass
- * exchanges plain [B] sums.  Potentials are in the library's internal log2 units; `ws` (same buffer for
- * all calls of one solve) starts with the cost shift: the caller all-reduces (MIN) the float at ws+0
- * after kccot_shard_begin.  One kernel boundary per half-iteration pair is the synchronisation point.
- * ------------------------------------------------------------------------------------------ */
-size_t kccot_shard_workspace_bytes(int Brows, int B);
-int kccot_shard_begin(const float* Crows, int Brows, int B, void* ws, size_t ws_bytes, void* stream);
-int kccot_shard_fwd_rows(const float* Crows, int Brows, int B, float eps, const float* v, float* u_rows,
-                         float* colstat, void* ws, size_t ws_bytes, void* stream);
-int kccot_shard_fwd_combine(const float* colstat_all, int nranks, int B, float* v, void* ws, void* stream);
-int kccot_shard_cost_partial(const float* Crows, int Brows, int B, float eps, const float* u_rows,
-                             const float* v, float* partial, void* ws, void* stream);
-int kccot_shard_bwd_seed(const float* Crows, int Brows, int B, float eps, const float* u_rows, const float* v,
-                         float g, float* Cbar_rows, float* ubar_rows, float* colsum, void* ws, void* stream);
-int kccot_shard_bwd_rows(const float* Crows, int Brows, int B, float eps, const float* u_k_rows,
-                         const float* v_k, const float* v_km1, const float* vbar, int first,
-                         float* ubar_rows, float* Cbar_rows, float* colsum, void* ws, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Row-sharded mixed loss, fused exchange (BASELINE config 5 on N GPUs).  Videos, h and M are replicated on

@@ -36,13 +36,6 @@ SIGNATURES = {
     "kccot_sinkhorn_workspace_bytes": (_SZ, [_I, _I, _I]),
     "kccot_sinkhorn_fwd": (_I, [_P, _I, _I, _F, _I, _I, _F, _I, _P, _P, _P, _P, _P, _SZ, _P]),
     "kccot_sinkhorn_bwd": (_I, [_P, _I, _I, _F, _I, _P, _P, _P, _P, _P, _P, _SZ, _P]),
-    "kccot_shard_workspace_bytes": (_SZ, [_I, _I]),
-    "kccot_shard_begin": (_I, [_P, _I, _I, _P, _SZ, _P]),
-    "kccot_shard_fwd_rows": (_I, [_P, _I, _I, _F, _P, _P, _P, _P, _SZ, _P]),
-    "kccot_shard_fwd_combine": (_I, [_P, _I, _I, _P, _P, _P]),
-    "kccot_shard_cost_partial": (_I, [_P, _I, _I, _F, _P, _P, _P, _P, _P]),
-    "kccot_shard_bwd_seed": (_I, [_P, _I, _I, _F, _P, _P, _F, _P, _P, _P, _P, _P]),
-    "kccot_shard_bwd_rows": (_I, [_P, _I, _I, _F, _P, _P, _P, _P, _I, _P, _P, _P, _P, _P]),
     "kccot_shard_cost_workspace_bytes": (_SZ, [_I, _LL, _I]),
     "kccot_shard_cost_fwd": (_I, [_P, _P, _I, _LL, _I, _I, _P, _P, _P, _P, _I, _I, _F, _P, _P, _SZ, _P]),
     "kccot_shard_cost_bwd": (_I, [_P, _P, _P, _I, _LL, _I, _I, _P, _P, _P, _P, _I, _I, _F, _P, _P, _P, _P, _P, _P, _SZ,
@@ -93,8 +86,8 @@ def load():
             fn = getattr(lib, name)          # AttributeError if the .so does not export a declared symbol
             fn.restype = res
             fn.argtypes = args
-        if lib.kccot_version() != 202:
-            raise OSError(f"{LIB_PATH}: ABI version {lib.kccot_version()} != 202; rebuild")
+        if lib.kccot_version() != 203:
+            raise OSError(f"{LIB_PATH}: ABI version {lib.kccot_version()} != 203; rebuild")
         _lib = lib
     return _lib
 

@@ -5,7 +5,6 @@
 namespace kccot {
 
 constexpr int kSmallSinkhornMaxB = 64;   // register-resident single-CTA path
-constexpr int kRowChunk = 32;            // rows per CTA in the streamed path
 
 // Epilogue / prologue of the mixed loss folded into the small kernels (problems come in triples xy, xx, yy):
 //   forward : the CTA of a triple that finishes last writes loss[p] = 2 xy - xx - yy (gan_utils.py:225) and the
@@ -28,14 +27,7 @@ int launch_sinkhorn_bwd_small(const float* C, int nsolve, int B, float eps, int 
 
 
 // sinkhorn_stream.cu — any B; C streamed from L2/HBM; a kernel boundary per half-iteration pair.
-struct StreamState {
-  float shift;      // c0 = min(C) (over all ranks when sharded)
-  float err;        // sum |u - u_prev| of the current iteration (log2 units)
-  int done;         // 1 once the stopping rule fired
-  int nits;         // executed iterations when done
-  float s0, s1;     // sum(pi), sum(pi * Chat) accumulators of the final cost
-};
-size_t stream_workspace_bytes(int Brows, int B);
+size_t stream_workspace_bytes(int B);
 int stream_sinkhorn_fwd(const float* C, int B, float eps, int L, int Lmin, float thresh, int exit_on_index,
                         float* u_hist, float* v_hist, int32_t* nits, float* cost, void* ws, cudaStream_t st);
 int stream_sinkhorn_bwd(const float* C, int B, float eps, int L, const float* u_hist, const float* v_hist,

@@ -12,7 +12,7 @@ extern "C" {
 size_t kccot_sinkhorn_workspace_bytes(int nsolve, int B, int L) {
   (void)L;
   if (B <= kSmallSinkhornMaxB) return align_up(256 + (size_t)(nsolve > 0 ? nsolve : 1) * sizeof(int32_t), 256);
-  size_t a = stream_workspace_bytes(B, B);
+  size_t a = stream_workspace_bytes(B);
   if (persist_supported(B, B, L)) {
     const size_t b = persist_workspace_bytes(nsolve < kPersistChunk ? (nsolve > 0 ? nsolve : 1) : kPersistChunk, B, B, L);
     a = a > b ? a : b;
@@ -40,7 +40,7 @@ int kccot_sinkhorn_fwd(const float* C, int nsolve, int B, float eps, int L, int 
     }
     return KCCOT_OK;
   }
-  KCCOT_CHECK_ARG(ws && ws_bytes >= stream_workspace_bytes(B, B), "workspace too small");
+  KCCOT_CHECK_ARG(ws && ws_bytes >= stream_workspace_bytes(B), "workspace too small");
   for (int n = 0; n < nsolve; ++n) {
     const long long hs = (long long)(L + 1) * B;
     if (int rc = stream_sinkhorn_fwd(C + (long long)n * B * B, B, eps, L, Lmin, thresh, exit_on_index, u_hist + n * hs,
@@ -68,7 +68,7 @@ int kccot_sinkhorn_bwd(const float* C, int nsolve, int B, float eps, int L, cons
     }
     return KCCOT_OK;
   }
-  KCCOT_CHECK_ARG(ws && ws_bytes >= stream_workspace_bytes(B, B), "workspace too small");
+  KCCOT_CHECK_ARG(ws && ws_bytes >= stream_workspace_bytes(B), "workspace too small");
   for (int n = 0; n < nsolve; ++n) {
     const long long hs = (long long)(L + 1) * B;
     if (int rc = stream_sinkhorn_bwd(C + (long long)n * B * B, B, eps, L, u_hist + n * hs, v_hist + n * hs, nits + n,

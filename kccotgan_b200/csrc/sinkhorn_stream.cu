@@ -1,20 +1,28 @@
-// Log-domain Sinkhorn for any B (and for one rank's row block of a row-sharded problem): the cost
-// rows are streamed from L2/HBM, one launch per iteration half-pair, so a kernel boundary is the
-// grid-wide (and, sharded, the cross-rank) synchronisation point.  Same internal units as the
-// register-resident path (sinkhorn_small.cu): log2 domain, cost shifted by its global minimum.
+// Log-domain Sinkhorn for any B, the fallback of the shapes the other two paths do not take: the
+// cost rows are streamed from L2/HBM, one launch per iteration half-pair, so a kernel boundary is
+// the grid-wide synchronisation point.  Same internal units as the register-resident path
+// (sinkhorn_small.cu): log2 domain, cost shifted by its global minimum.
 //
-// A CTA owns kRowChunk consecutive rows.  Phase 1 (warp per row) does the row reduction, phase 2
-// (thread per column) the column partials over the CTA's rows; partials are combined over CTAs —
-// and over ranks — by the *_combine kernels.  gan_utils.py:151-164 and SURVEY.md Appendix A.
+// A CTA owns RC consecutive rows.  Phase 1 (warp per row) does the row reduction, phase 2 (thread
+// per column) the column partials over the CTA's rows; partials are combined over CTAs by the
+// *_combine kernels.  gan_utils.py:151-164 and SURVEY.md Appendix A.
 #include "common.cuh"
 #include "sinkhorn.cuh"
 
 namespace kccot {
 
 namespace {
-constexpr int RC = kRowChunk;
+constexpr int RC = 32;     // rows per CTA
 constexpr int NT = 256;
 constexpr float kNegBig = -3.0e38f;
+
+struct StreamState {
+  float shift;      // c0 = min(C)
+  float err;        // sum |u - u_prev| of the current iteration (log2 units)
+  int done;         // 1 once the stopping rule fired
+  int nits;         // executed iterations when done
+  float s0, s1;     // sum(pi), sum(pi * Chat) accumulators of the final cost
+};
 
 __device__ __forceinline__ void atomic_min_float(float* addr, float v) {
   if (v >= 0.f) atomicMin(reinterpret_cast<int*>(addr), __float_as_int(v));
@@ -44,12 +52,15 @@ __device__ __forceinline__ void lse_warp_merge(float& m, float& s) {
   m = M;
 }
 
-__global__ void __launch_bounds__(NT) stream_fwd_rows_kernel(const float* __restrict__ C, int Brows, int B, float kscale,
-                                                             float ahat, const float* __restrict__ v_cur,
-                                                             float* __restrict__ u_cur, float* __restrict__ u_hist_row,
-                                                             float* __restrict__ colmax_part,
-                                                             float* __restrict__ colsum_part, StreamState* state,
-                                                             int track_err) {
+// One CTA per SM is enough (the grid has B / RC CTAs): without the bound ptxas caps the kernel at 128
+// registers and spills part of t[RC].
+__global__ void __launch_bounds__(NT, 1) stream_fwd_rows_kernel(const float* __restrict__ C, int B, float kscale,
+                                                                float ahat, const float* __restrict__ v_cur,
+                                                                float* __restrict__ u_cur,
+                                                                float* __restrict__ u_hist_row,
+                                                                float* __restrict__ colmax_part,
+                                                                float* __restrict__ colsum_part, StreamState* state,
+                                                                int track_err) {
   if (state->done) return;
   __shared__ float us[RC];
   const float c0 = state->shift;
@@ -58,7 +69,7 @@ __global__ void __launch_bounds__(NT) stream_fwd_rows_kernel(const float* __rest
   float errw = 0.f;
   for (int rr = warp; rr < RC; rr += NT / 32) {
     const int r = r0 + rr;
-    if (r >= Brows) { if (lane == 0) us[rr] = kNegBig; continue; }
+    if (r >= B) { if (lane == 0) us[rr] = kNegBig; continue; }
     const float* row = C + (long long)r * B;
     float m = kNegBig, s = 0.f;
     for (int j = lane; j < B; j += 32) lse_push(v_cur[j] - (row[j] - c0) * kscale, m, s);
@@ -73,7 +84,7 @@ __global__ void __launch_bounds__(NT) stream_fwd_rows_kernel(const float* __rest
   }
   if (track_err && lane == 0 && errw != 0.f) atomicAdd(&state->err, errw);
   __syncthreads();
-  const int nrows = min(RC, Brows - r0);
+  const int nrows = min(RC, B - r0);
   for (int j = threadIdx.x; j < B; j += NT) {
     float t[RC];
     float m = kNegBig;
@@ -94,41 +105,17 @@ __global__ void __launch_bounds__(NT) stream_fwd_combine_kernel(const float* __r
                                                                 const float* __restrict__ colsum_part, int nparts,
                                                                 int B, float ahat, float* __restrict__ v_cur,
                                                                 float* __restrict__ v_hist_row,
-                                                                const StreamState* state, long long pstride) {
+                                                                const StreamState* state) {
   if (state->done) return;
-  const int j = blockIdx.x * NT + threadIdx.x;
-  if (j >= B) return;
-  float M = kNegBig;
-  for (int p = 0; p < nparts; ++p) M = fmaxf(M, colmax_part[p * pstride + j]);
-  float S = 0.f;
-  for (int p = 0; p < nparts; ++p) S += colsum_part[p * pstride + j] * fast_exp2(colmax_part[p * pstride + j] - M);
-  const float v = ahat - (M + fast_log2(S));
-  v_cur[j] = v;
-  if (v_hist_row) v_hist_row[j] = v;
-}
-
-// reduce this rank's per-chunk (max, sumexp) partials to one pair per column (what the ranks exchange)
-__global__ void __launch_bounds__(NT) stream_colstat_reduce_kernel(const float* __restrict__ colmax_part,
-                                                                   const float* __restrict__ colsum_part, int nparts,
-                                                                   int B, float* __restrict__ out_max,
-                                                                   float* __restrict__ out_sum) {
   const int j = blockIdx.x * NT + threadIdx.x;
   if (j >= B) return;
   float M = kNegBig;
   for (int p = 0; p < nparts; ++p) M = fmaxf(M, colmax_part[(long long)p * B + j]);
   float S = 0.f;
   for (int p = 0; p < nparts; ++p) S += colsum_part[(long long)p * B + j] * fast_exp2(colmax_part[(long long)p * B + j] - M);
-  out_max[j] = M;
-  out_sum[j] = S;
-}
-
-__global__ void __launch_bounds__(NT) stream_colsum_reduce_kernel(const float* __restrict__ part, int nparts, int B,
-                                                                  float* __restrict__ out) {
-  const int j = blockIdx.x * NT + threadIdx.x;
-  if (j >= B) return;
-  float acc = 0.f;
-  for (int p = 0; p < nparts; ++p) acc += part[(long long)p * B + j];
-  out[j] = acc;
+  const float v = ahat - (M + fast_log2(S));
+  v_cur[j] = v;
+  if (v_hist_row) v_hist_row[j] = v;
 }
 
 __global__ void stream_stop_kernel(StreamState* state, int iter_1based, float thresh, float kscale, int cond_ok) {
@@ -138,13 +125,13 @@ __global__ void stream_stop_kernel(StreamState* state, int iter_1based, float th
   if (cond_ok && thresh > err) { state->done = 1; state->nits = iter_1based; }
 }
 
-__global__ void __launch_bounds__(NT) stream_cost_kernel(const float* __restrict__ C, int Brows, int B, float kscale,
+__global__ void __launch_bounds__(NT) stream_cost_kernel(const float* __restrict__ C, int B, float kscale,
                                                          const float* __restrict__ u_cur,
                                                          const float* __restrict__ v_cur, StreamState* state) {
   const float c0 = state->shift;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   float s0 = 0.f, s1 = 0.f;
-  for (int r = blockIdx.x * (NT / 32) + warp; r < Brows; r += gridDim.x * (NT / 32)) {
+  for (int r = blockIdx.x * (NT / 32) + warp; r < B; r += gridDim.x * (NT / 32)) {
     const float* row = C + (long long)r * B;
     const float ui = u_cur[r];
     for (int j = lane; j < B; j += 32) {
@@ -166,8 +153,8 @@ __global__ void stream_cost_finish_kernel(StreamState* state, float kscale, int 
 
 // ------------------------------------ backward ---------------------------------------------------
 // seed:  Cbar = g pi (1 - C/eps),  ubar_i = g sum_j pi C/eps,  column partials of g pi C/eps
-__global__ void __launch_bounds__(NT) stream_bwd_seed_kernel(const float* __restrict__ C, int Brows, int row_off, int B,
-                                                             float kscale, float inv_eps,
+__global__ void __launch_bounds__(NT) stream_bwd_seed_kernel(const float* __restrict__ C, int B, float kscale,
+                                                             float inv_eps,
                                                              const float* __restrict__ u_hist,
                                                              const float* __restrict__ v_hist,
                                                              const int32_t* __restrict__ nits_p,
@@ -179,13 +166,13 @@ __global__ void __launch_bounds__(NT) stream_bwd_seed_kernel(const float* __rest
   const float shift = *shift_p;
   const int nits = *nits_p;
   const float g = *gcost;
-  const float* u = u_hist + (long long)nits * B + row_off;   // rows are indexed globally in the history
+  const float* u = u_hist + (long long)nits * B;
   const float* v = v_hist + (long long)nits * B;
   const int r0 = blockIdx.x * RC;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   for (int rr = warp; rr < RC; rr += NT / 32) {
     const int r = r0 + rr;
-    if (r >= Brows) { if (lane == 0) us[rr] = 0.f; continue; }
+    if (r >= B) { if (lane == 0) us[rr] = 0.f; continue; }
     const float* row = C + (long long)r * B;
     float* grow = Cbar + (long long)r * B;
     const float ui = u[r];
@@ -201,7 +188,7 @@ __global__ void __launch_bounds__(NT) stream_bwd_seed_kernel(const float* __rest
     if (lane == 0) { ubar[r] = acc; us[rr] = ui; }
   }
   __syncthreads();
-  const int nrows = min(RC, Brows - r0);
+  const int nrows = min(RC, B - r0);
   for (int j = threadIdx.x; j < B; j += NT) {
     float acc = 0.f;
     const float vj = v[j];
@@ -215,18 +202,28 @@ __global__ void __launch_bounds__(NT) stream_bwd_seed_kernel(const float* __rest
 
 // reverse step k:  rows: Pv -> Cbar += Pv*vbar_j, ubar_i = (first ? ubar_i : 0) - sum_j Pv vbar_j
 //                  cols: Pu -> Cbar += Pu*ubar_i, partial of sum_i Pu ubar_i
-__device__ __forceinline__ void stream_bwd_rows_core(const float* __restrict__ C, int Brows, int B, float kscale,
-                                                     float ahat, const float* __restrict__ uk,
-                                                     const float* __restrict__ vk, const float* __restrict__ vkm1,
-                                                     bool first, float shift, const float* __restrict__ vbar,
-                                                     float* __restrict__ ubar, float* __restrict__ Cbar,
-                                                     float* __restrict__ colsum_part) {
+// The operands are located in the saved history by the device-side iteration count.
+__global__ void __launch_bounds__(NT) stream_bwd_rows_kernel(const float* __restrict__ C, int B, float kscale, float ahat,
+                                                             const float* __restrict__ u_hist,
+                                                             const float* __restrict__ v_hist,
+                                                             const int32_t* __restrict__ nits_p, int k,
+                                                             const float* __restrict__ shift_p,
+                                                             const float* __restrict__ vbar, float* __restrict__ ubar,
+                                                             float* __restrict__ Cbar,
+                                                             float* __restrict__ colsum_part) {
+  const int nits = *nits_p;
+  if (k > nits) return;
+  const float* __restrict__ uk = u_hist + (long long)k * B;
+  const float* __restrict__ vk = v_hist + (long long)k * B;
+  const float* __restrict__ vkm1 = v_hist + (long long)(k - 1) * B;
+  const bool first = k == nits;
+  const float shift = *shift_p;
   __shared__ float us[RC], ubs[RC];
   const int r0 = blockIdx.x * RC;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   for (int rr = warp; rr < RC; rr += NT / 32) {
     const int r = r0 + rr;
-    if (r >= Brows) { if (lane == 0) { us[rr] = 0.f; ubs[rr] = 0.f; } continue; }
+    if (r >= B) { if (lane == 0) { us[rr] = 0.f; ubs[rr] = 0.f; } continue; }
     const float* row = C + (long long)r * B;
     float* grow = Cbar + (long long)r * B;
     const float ui = uk[r] - ahat;
@@ -245,7 +242,7 @@ __device__ __forceinline__ void stream_bwd_rows_core(const float* __restrict__ C
     }
   }
   __syncthreads();
-  const int nrows = min(RC, Brows - r0);
+  const int nrows = min(RC, B - r0);
   for (int j = threadIdx.x; j < B; j += NT) {
     float acc = 0.f;
     const float vj = vkm1[j];
@@ -257,35 +254,6 @@ __device__ __forceinline__ void stream_bwd_rows_core(const float* __restrict__ C
     }
     colsum_part[(long long)blockIdx.x * B + j] = acc;
   }
-}
-
-// single-GPU form: operands located in the saved history by the device-side iteration count
-__global__ void __launch_bounds__(NT) stream_bwd_rows_kernel(const float* __restrict__ C, int Brows, int row_off, int B,
-                                                             float kscale, float ahat,
-                                                             const float* __restrict__ u_hist,
-                                                             const float* __restrict__ v_hist,
-                                                             const int32_t* __restrict__ nits_p, int k,
-                                                             const float* __restrict__ shift_p,
-                                                             const float* __restrict__ vbar, float* __restrict__ ubar,
-                                                             float* __restrict__ Cbar,
-                                                             float* __restrict__ colsum_part) {
-  const int nits = *nits_p;
-  if (k > nits) return;
-  stream_bwd_rows_core(C, Brows, B, kscale, ahat, u_hist + (long long)k * B + row_off, v_hist + (long long)k * B,
-                       v_hist + (long long)(k - 1) * B, k == nits, *shift_p, vbar, ubar, Cbar, colsum_part);
-}
-
-// sharded form: the three potential vectors are passed directly
-__global__ void __launch_bounds__(NT) stream_bwd_rows_direct_kernel(const float* __restrict__ C, int Brows, int B,
-                                                                    float kscale, float ahat,
-                                                                    const float* __restrict__ uk,
-                                                                    const float* __restrict__ vk,
-                                                                    const float* __restrict__ vkm1, int first,
-                                                                    const float* __restrict__ shift_p,
-                                                                    const float* __restrict__ vbar,
-                                                                    float* __restrict__ ubar, float* __restrict__ Cbar,
-                                                                    float* __restrict__ colsum_part) {
-  stream_bwd_rows_core(C, Brows, B, kscale, ahat, uk, vk, vkm1, first != 0, *shift_p, vbar, ubar, Cbar, colsum_part);
 }
 
 __global__ void __launch_bounds__(NT) stream_bwd_combine_kernel(const float* __restrict__ colsum_part, int nparts, int B,
@@ -301,8 +269,8 @@ __global__ void __launch_bounds__(NT) stream_bwd_combine_kernel(const float* __r
 }  // namespace
 
 // ------------------------------------------------------------------------------------------------
-size_t stream_workspace_bytes(int Brows, int B) {
-  const size_t nchunk = (Brows + RC - 1) / RC;
+size_t stream_workspace_bytes(int B) {
+  const size_t nchunk = (B + RC - 1) / RC;
   return align_up(256 + (size_t)4 * B * 4 + 2 * nchunk * (size_t)B * 4 + 1024, 256);
 }
 
@@ -311,7 +279,7 @@ struct StreamWs {
   float *u_cur, *v_cur, *ubar, *vbar, *part_a, *part_b;
   int nchunk;
 };
-static StreamWs carve(void* ws, int Brows, int B) {
+static StreamWs carve(void* ws, int B) {
   StreamWs w;
   char* p = (char*)ws;
   w.state = (StreamState*)p; p += 256;
@@ -319,7 +287,7 @@ static StreamWs carve(void* ws, int Brows, int B) {
   w.v_cur = (float*)p; p += (size_t)B * 4;
   w.ubar = (float*)p; p += (size_t)B * 4;
   w.vbar = (float*)p; p += (size_t)B * 4;
-  w.nchunk = (Brows + RC - 1) / RC;
+  w.nchunk = (B + RC - 1) / RC;
   w.part_a = (float*)p; p += (size_t)w.nchunk * B * 4;
   w.part_b = (float*)p;
   return w;
@@ -327,7 +295,7 @@ static StreamWs carve(void* ws, int Brows, int B) {
 
 int stream_sinkhorn_fwd(const float* C, int B, float eps, int L, int Lmin, float thresh, int exit_on_index,
                         float* u_hist, float* v_hist, int32_t* nits, float* cost, void* ws, cudaStream_t st) {
-  StreamWs w = carve(ws, B, B);
+  StreamWs w = carve(ws, B);
   const float kscale = kLog2e / eps, ahat = -log2f((float)B);
   stream_state_init_kernel<<<1, 1, 0, st>>>(w.state);
   KCCOT_LAUNCH_CHECK();
@@ -339,18 +307,18 @@ int stream_sinkhorn_fwd(const float* C, int B, float eps, int L, int Lmin, float
   const int cgrid = (B + NT - 1) / NT;
   for (int it = 0; it < L; ++it) {
     const bool may_stop = (exit_on_index ? (it >= Lmin) : (it + 1 >= Lmin)) && (it + 1 < L);
-    stream_fwd_rows_kernel<<<w.nchunk, NT, 0, st>>>(C, B, B, kscale, ahat, w.v_cur, w.u_cur, u_hist + (long long)(it + 1) * B,
+    stream_fwd_rows_kernel<<<w.nchunk, NT, 0, st>>>(C, B, kscale, ahat, w.v_cur, w.u_cur, u_hist + (long long)(it + 1) * B,
                                                     w.part_a, w.part_b, w.state, may_stop ? 1 : 0);
     KCCOT_LAUNCH_CHECK();
     stream_fwd_combine_kernel<<<cgrid, NT, 0, st>>>(w.part_a, w.part_b, w.nchunk, B, ahat, w.v_cur,
-                                                    v_hist + (long long)(it + 1) * B, w.state, (long long)B);
+                                                    v_hist + (long long)(it + 1) * B, w.state);
     KCCOT_LAUNCH_CHECK();
     if (may_stop) {
       stream_stop_kernel<<<1, 1, 0, st>>>(w.state, it + 1, thresh, kscale, 1);
       KCCOT_LAUNCH_CHECK();
     }
   }
-  stream_cost_kernel<<<min(2 * num_sms(), (B + 7) / 8), NT, 0, st>>>(C, B, B, kscale, w.u_cur, w.v_cur, w.state);
+  stream_cost_kernel<<<min(2 * num_sms(), (B + 7) / 8), NT, 0, st>>>(C, B, kscale, w.u_cur, w.v_cur, w.state);
   KCCOT_LAUNCH_CHECK();
   stream_cost_finish_kernel<<<1, 1, 0, st>>>(w.state, kscale, L, cost, nits);
   KCCOT_LAUNCH_CHECK();
@@ -359,7 +327,7 @@ int stream_sinkhorn_fwd(const float* C, int B, float eps, int L, int Lmin, float
 
 int stream_sinkhorn_bwd(const float* C, int B, float eps, int L, const float* u_hist, const float* v_hist,
                         const int32_t* nits, const float* gcost, float* Cbar, void* ws, cudaStream_t st) {
-  StreamWs w = carve(ws, B, B);
+  StreamWs w = carve(ws, B);
   const float kscale = kLog2e / eps, ahat = -log2f((float)B);
   // the saved potentials contain the forward's shift (the global minimum): recompute the same value
   stream_state_init_kernel<<<1, 1, 0, st>>>(w.state);
@@ -368,13 +336,13 @@ int stream_sinkhorn_bwd(const float* C, int B, float eps, int L, const float* u_
   KCCOT_LAUNCH_CHECK();
   const float* shift_p = &w.state->shift;
   const int cgrid = (B + NT - 1) / NT;
-  stream_bwd_seed_kernel<<<w.nchunk, NT, 0, st>>>(C, B, 0, B, kscale, 1.f / eps, u_hist, v_hist, nits, gcost, shift_p,
+  stream_bwd_seed_kernel<<<w.nchunk, NT, 0, st>>>(C, B, kscale, 1.f / eps, u_hist, v_hist, nits, gcost, shift_p,
                                                   Cbar, w.ubar, w.part_a);
   KCCOT_LAUNCH_CHECK();
   stream_bwd_combine_kernel<<<cgrid, NT, 0, st>>>(w.part_a, w.nchunk, B, 1.f, w.vbar, nullptr, 0);
   KCCOT_LAUNCH_CHECK();
   for (int k = L; k >= 1; --k) {
-    stream_bwd_rows_kernel<<<w.nchunk, NT, 0, st>>>(C, B, 0, B, kscale, ahat, u_hist, v_hist, nits, k, shift_p, w.vbar,
+    stream_bwd_rows_kernel<<<w.nchunk, NT, 0, st>>>(C, B, kscale, ahat, u_hist, v_hist, nits, k, shift_p, w.vbar,
                                                     w.ubar, Cbar, w.part_a);
     KCCOT_LAUNCH_CHECK();
     stream_bwd_combine_kernel<<<cgrid, NT, 0, st>>>(w.part_a, w.nchunk, B, -1.f, w.vbar, nits, k);
@@ -384,109 +352,3 @@ int stream_sinkhorn_bwd(const float* C, int B, float eps, int L, const float* u_
 }
 
 }  // namespace kccot
-
-// ------------------------------------------------------------------------------------------------
-// Row-sharded single problem (BASELINE config 5): this rank owns rows [row0, row0 + Brows) of the
-// B x B cost.  One call per half-iteration pair; the caller exchanges the [B] column statistics
-// between ranks (NCCL all-gather / all-reduce over NVLink) between the calls.  kccotgan_b200/sharded.py.
-// ------------------------------------------------------------------------------------------------
-using namespace kccot;
-
-extern "C" {
-
-size_t kccot_shard_workspace_bytes(int Brows, int B) { return stream_workspace_bytes(Brows, B); }
-
-// state (in ws): float shift at byte 0 = min over this rank's rows; the caller all-reduces (MIN) that float
-int kccot_shard_begin(const float* Crows, int Brows, int B, void* ws, size_t ws_bytes, void* stream) {
-  KCCOT_CHECK_ARG(Crows && ws && Brows >= 1 && B >= 1 && ws_bytes >= stream_workspace_bytes(Brows, B), "bad arguments");
-  cudaStream_t st = (cudaStream_t)stream;
-  StreamWs w = carve(ws, Brows, B);
-  stream_state_init_kernel<<<1, 1, 0, st>>>(w.state);
-  KCCOT_LAUNCH_CHECK();
-  const long long n = (long long)Brows * B;
-  stream_min_kernel<<<(int)min((long long)4 * num_sms(), (n + NT - 1) / NT), NT, 0, st>>>(Crows, n, w.state);
-  KCCOT_LAUNCH_CHECK();
-  return KCCOT_OK;
-}
-
-// u for this rank's rows (written to u_rows[Brows]) from the full v[B]; then this rank's column
-// statistics colstat[2][B] = (max_i, sum_i exp2(. - max)) over its rows
-int kccot_shard_fwd_rows(const float* Crows, int Brows, int B, float eps, const float* v, float* u_rows,
-                         float* colstat, void* ws, size_t ws_bytes, void* stream) {
-  KCCOT_CHECK_ARG(Crows && v && u_rows && colstat && ws && ws_bytes >= stream_workspace_bytes(Brows, B), "bad arguments");
-  cudaStream_t st = (cudaStream_t)stream;
-  StreamWs w = carve(ws, Brows, B);
-  const float kscale = kLog2e / eps, ahat = -log2f((float)B);
-  stream_fwd_rows_kernel<<<w.nchunk, NT, 0, st>>>(Crows, Brows, B, kscale, ahat, v, u_rows, nullptr, w.part_a, w.part_b,
-                                                  w.state, 0);
-  KCCOT_LAUNCH_CHECK();
-  stream_colstat_reduce_kernel<<<(B + NT - 1) / NT, NT, 0, st>>>(w.part_a, w.part_b, w.nchunk, B, colstat, colstat + B);
-  KCCOT_LAUNCH_CHECK();
-  return KCCOT_OK;
-}
-
-// v[B] from the gathered statistics colstat_all[nranks][2][B]
-int kccot_shard_fwd_combine(const float* colstat_all, int nranks, int B, float* v, void* ws, void* stream) {
-  KCCOT_CHECK_ARG(colstat_all && v && ws && nranks >= 1, "bad arguments");
-  cudaStream_t st = (cudaStream_t)stream;
-  const float ahat = -log2f((float)B);
-  StreamState* state = (StreamState*)ws;
-  // stride between ranks is 2*B: reuse the combine kernel on interleaved views
-  stream_fwd_combine_kernel<<<(B + NT - 1) / NT, NT, 0, st>>>(colstat_all, colstat_all + B, nranks, B, ahat, v, nullptr,
-                                                             state, 2 * B);
-  KCCOT_LAUNCH_CHECK();
-  return KCCOT_OK;
-}
-
-// partial[0] = sum(pi), partial[1] = sum(pi * Chat) over this rank's rows; cost = all-reduce then
-// partial[1] * eps/log2(e) + shift * partial[0]
-int kccot_shard_cost_partial(const float* Crows, int Brows, int B, float eps, const float* u_rows, const float* v,
-                             float* partial, void* ws, void* stream) {
-  KCCOT_CHECK_ARG(Crows && u_rows && v && partial && ws, "bad arguments");
-  cudaStream_t st = (cudaStream_t)stream;
-  StreamState* state = (StreamState*)ws;
-  KCCOT_CUDA(cudaMemsetAsync(&state->s0, 0, 2 * sizeof(float), st));
-  stream_cost_kernel<<<min(2 * num_sms(), (Brows + 7) / 8), NT, 0, st>>>(Crows, Brows, B, kLog2e / eps, u_rows, v, state);
-  KCCOT_LAUNCH_CHECK();
-  KCCOT_CUDA(cudaMemcpyAsync(partial, &state->s0, 2 * sizeof(float), cudaMemcpyDeviceToDevice, st));
-  return KCCOT_OK;
-}
-
-// seeds of the reverse pass on this rank's rows: Cbar_rows, ubar_rows, and colsum[B] (this rank's
-// part of vbar; the caller all-reduces it).  g = upstream gradient (host scalar).
-int kccot_shard_bwd_seed(const float* Crows, int Brows, int B, float eps, const float* u_rows, const float* v, float g,
-                         float* Cbar_rows, float* ubar_rows, float* colsum, void* ws, void* stream) {
-  KCCOT_CHECK_ARG(Crows && u_rows && v && Cbar_rows && ubar_rows && colsum && ws, "bad arguments");
-  cudaStream_t st = (cudaStream_t)stream;
-  StreamWs w = carve(ws, Brows, B);
-  // the seed kernel reads (nits, g) through device pointers: park them in the state block
-  int32_t* zero_nits = (int32_t*)((char*)ws + 64);
-  float* gdev = (float*)((char*)ws + 68);
-  KCCOT_CUDA(cudaMemsetAsync(zero_nits, 0, 4, st));
-  KCCOT_CUDA(cudaMemcpyAsync(gdev, &g, 4, cudaMemcpyHostToDevice, st));
-  stream_bwd_seed_kernel<<<w.nchunk, NT, 0, st>>>(Crows, Brows, 0, B, kLog2e / eps, 1.f / eps, u_rows, v, zero_nits, gdev,
-                                                  &w.state->shift, Cbar_rows, ubar_rows, w.part_a);
-  KCCOT_LAUNCH_CHECK();
-  stream_colsum_reduce_kernel<<<(B + NT - 1) / NT, NT, 0, st>>>(w.part_a, w.nchunk, B, colsum);
-  KCCOT_LAUNCH_CHECK();
-  return KCCOT_OK;
-}
-
-// one reverse step on this rank's rows: needs u^k (own rows), v^k, v^{k-1}, vbar (all [B]); updates
-// Cbar_rows and ubar_rows; colsum[B] = this rank's part of sum_i Pu_ij ubar_i (vbar = -all-reduce)
-int kccot_shard_bwd_rows(const float* Crows, int Brows, int B, float eps, const float* u_k_rows, const float* v_k,
-                         const float* v_km1, const float* vbar, int first, float* ubar_rows, float* Cbar_rows,
-                         float* colsum, void* ws, void* stream) {
-  KCCOT_CHECK_ARG(Crows && u_k_rows && v_k && v_km1 && vbar && ubar_rows && Cbar_rows && colsum && ws, "bad arguments");
-  cudaStream_t st = (cudaStream_t)stream;
-  StreamWs w = carve(ws, Brows, B);
-  stream_bwd_rows_direct_kernel<<<w.nchunk, NT, 0, st>>>(Crows, Brows, B, kLog2e / eps, -log2f((float)B), u_k_rows, v_k,
-                                                         v_km1, first, &w.state->shift, vbar, ubar_rows, Cbar_rows,
-                                                         w.part_a);
-  KCCOT_LAUNCH_CHECK();
-  stream_colsum_reduce_kernel<<<(B + NT - 1) / NT, NT, 0, st>>>(w.part_a, w.nchunk, B, colsum);
-  KCCOT_LAUNCH_CHECK();
-  return KCCOT_OK;
-}
-
-}  // extern "C"

@@ -2,11 +2,11 @@
 
 1. Independent problems (BASELINE config 4, data-parallel replicas): `split_problems` deals problems
    to ranks; each rank runs the single-GPU kernels on its share; NO data-path collective.
-2. One large problem (config 5): the rows of the B x B cost are sharded (`row_range`).  The u-update
-   is local to a rank; the v-update needs a column log-sum-exp over all rows, so every iteration the
-   ranks exchange one [2, B] (max, sum-exp) pair per rank (all-gather) and combine; the reverse pass
-   exchanges plain [B] sums (all-reduce).  `ShardedSinkhorn` drives the C-ABI half-iteration kernels
-   (`kccot_shard_*`) and the collectives.  The arithmetic backend is pluggable so that the partition /
+2. One large problem (config 5): the rows of the B x B cost are sharded (`row_range`).
+   `ShardedMixedLoss` computes a rank's cost rows, runs its row block of the three Sinkhorn solves in
+   persistent kernels that exchange the [B] column sums with the other ranks through peer mailboxes
+   (no host-launched collective per iteration), and returns the gradient rows of the rank's samples;
+   NCCL carries only a few collectives per evaluation.  The backend is pluggable so that the partition /
    exchange logic is testable with `gloo` on CPU (the tests pass their own fp64 stand-in; the product
    backend is CUDA-only — there is no CPU fallback in this package).
 """
@@ -30,133 +30,6 @@ def row_range(B, rank, world):
     """Rows [r0, r1) of the cost matrix owned by `rank`."""
     r = split_problems(B, rank, world)
     return r.start, r.stop
-
-
-class CudaShardBackend:
-    """Half-iteration kernels of libkccot on this rank's row block (sinkhorn_stream.cu)."""
-
-    def __init__(self, C_rows, B, eps):
-        if not (isinstance(C_rows, torch.Tensor) and C_rows.is_cuda and C_rows.dtype == torch.float32):
-            raise ValueError("C_rows: expected a CUDA float32 tensor (kccotgan_b200 has no CPU path)")
-        self.C = C_rows.contiguous()
-        self.Brows, self.B, self.eps = int(C_rows.shape[0]), int(B), float(eps)
-        if C_rows.shape[1] != B:
-            raise ValueError(f"C_rows must be [rows, B={B}], got {tuple(C_rows.shape)}")
-        self.dev = C_rows.device
-        lib = _lib.load()
-        self.ws = torch.zeros(lib.kccot_shard_workspace_bytes(self.Brows, self.B), dtype=torch.uint8, device=self.dev)
-        self.shift = self.ws[:4].view(torch.float32)          # the float the ranks all-reduce (MIN)
-
-    def _st(self):
-        return ctypes.c_void_p(torch.cuda.current_stream(self.dev).cuda_stream)
-
-    @staticmethod
-    def _p(t):
-        return ctypes.c_void_p(t.data_ptr())
-
-    def new(self, *shape):
-        return torch.empty(*shape, dtype=torch.float32, device=self.dev)
-
-    def zeros(self, *shape):
-        return torch.zeros(*shape, dtype=torch.float32, device=self.dev)
-
-    def begin(self):
-        with torch.cuda.device(self.dev):
-            _lib.call("kccot_shard_begin", self._p(self.C), self.Brows, self.B, self._p(self.ws), self.ws.numel(), self._st())
-        return self.shift
-
-    def fwd_rows(self, v, u_rows, colstat):
-        with torch.cuda.device(self.dev):
-            _lib.call("kccot_shard_fwd_rows", self._p(self.C), self.Brows, self.B, self.eps, self._p(v), self._p(u_rows),
-                      self._p(colstat), self._p(self.ws), self.ws.numel(), self._st())
-
-    def fwd_combine(self, colstat_all, v):
-        with torch.cuda.device(self.dev):
-            _lib.call("kccot_shard_fwd_combine", self._p(colstat_all), int(colstat_all.shape[0]), self.B, self._p(v),
-                      self._p(self.ws), self._st())
-
-    def cost_partial(self, u_rows, v, partial):
-        with torch.cuda.device(self.dev):
-            _lib.call("kccot_shard_cost_partial", self._p(self.C), self.Brows, self.B, self.eps, self._p(u_rows),
-                      self._p(v), self._p(partial), self._p(self.ws), self._st())
-
-    def bwd_seed(self, u_rows, v, g, Cbar_rows, ubar_rows, colsum):
-        with torch.cuda.device(self.dev):
-            _lib.call("kccot_shard_bwd_seed", self._p(self.C), self.Brows, self.B, self.eps, self._p(u_rows), self._p(v),
-                      float(g), self._p(Cbar_rows), self._p(ubar_rows), self._p(colsum), self._p(self.ws), self._st())
-
-    def bwd_rows(self, u_k, v_k, v_km1, vbar, first, ubar_rows, Cbar_rows, colsum):
-        with torch.cuda.device(self.dev):
-            _lib.call("kccot_shard_bwd_rows", self._p(self.C), self.Brows, self.B, self.eps, self._p(u_k), self._p(v_k),
-                      self._p(v_km1), self._p(vbar), int(bool(first)), self._p(ubar_rows), self._p(Cbar_rows),
-                      self._p(colsum), self._p(self.ws), self._st())
-
-
-class ShardedSinkhorn:
-    """compute_sinkhorn's solve (gan_utils.py:138-165) on a row-sharded cost.
-
-    forward(): every rank passes its rows; returns the (replicated) sharp cost sum(pi * C).
-    backward(g): returns this rank's rows of g * d cost / d C.
-    L <= 100 runs exactly L iterations (the reference's Lmin = 100 makes the early exit unreachable);
-    for L > 100 the stopping rule needs sum|u - u_prev| over all ranks: one extra scalar all-reduce and
-    a host read per iteration past the 100th.
-    """
-
-    def __init__(self, backend, group=None):
-        self.be = backend
-        self.group = group
-        self.world = dist.get_world_size(group) if dist.is_initialized() else 1
-        self.rank = dist.get_rank(group) if dist.is_initialized() else 0
-
-    # -- collectives (no-ops on a single rank) ----------------------------------------------------
-    def _allreduce(self, t, op):
-        if self.world > 1:
-            dist.all_reduce(t, op=op, group=self.group)
-        return t
-
-    def _allgather(self, t):
-        if self.world == 1:
-            return t.unsqueeze(0)
-        out = [torch.empty_like(t) for _ in range(self.world)]
-        dist.all_gather(out, t, group=self.group)
-        return torch.stack(out, 0).contiguous()
-
-    def forward(self, L=100, Lmin=100, thresh=1e-2):
-        be = self.be
-        B, Brows = be.B, be.Brows
-        self._allreduce(be.begin(), dist.ReduceOp.MIN)          # global cost shift
-        self.u_hist = be.zeros(L + 1, Brows)                    # this rank's rows only
-        self.v_hist = be.zeros(L + 1, B)
-        colstat = be.new(2, B)
-        kscale = math.log2(math.e) / be.eps
-        nits = 0
-        for it in range(int(L)):
-            be.fwd_rows(self.v_hist[it], self.u_hist[it + 1], colstat)
-            be.fwd_combine(self._allgather(colstat), self.v_hist[it + 1])
-            nits = it + 1
-            if nits >= Lmin and nits < L:                       # gan_utils.py:157-160
-                err = (self.u_hist[it + 1] - self.u_hist[it]).abs().sum().reshape(1) / kscale
-                if thresh > float(self._allreduce(err, dist.ReduceOp.SUM)):
-                    break
-        self.nits = nits
-        partial = be.new(2)
-        be.cost_partial(self.u_hist[nits], self.v_hist[nits], partial)
-        self._allreduce(partial, dist.ReduceOp.SUM)
-        shift = be.shift if isinstance(be.shift, torch.Tensor) else torch.as_tensor(be.shift)
-        return partial[1] / kscale + shift.reshape(()) * partial[0]
-
-    def backward(self, g=1.0):
-        be = self.be
-        B, Brows, n = be.B, be.Brows, self.nits
-        Cbar = be.new(Brows, B)
-        ubar = be.new(Brows)
-        colsum = be.new(B)
-        be.bwd_seed(self.u_hist[n], self.v_hist[n], g, Cbar, ubar, colsum)
-        vbar = self._allreduce(colsum.clone(), dist.ReduceOp.SUM)
-        for k in range(n, 0, -1):
-            be.bwd_rows(self.u_hist[k], self.v_hist[k], self.v_hist[k - 1], vbar, k == n, ubar, Cbar, colsum)
-            vbar = -self._allreduce(colsum.clone(), dist.ReduceOp.SUM)
-        return Cbar
 
 
 # ------------------------------------------------------------------------------------------------

@@ -1,67 +1,8 @@
-"""CPU stand-in for the kccot_shard_* kernels (fp64 torch), TEST ONLY: lets the partition / exchange
-logic of kccotgan_b200.sharded.ShardedSinkhorn run under gloo without a GPU.  Same internal units as
-sinkhorn_stream.cu: log2 domain, cost shifted by the (all-reduced) minimum."""
+"""CPU stand-in for the stages of the fused row-sharded loss (fp64 torch), TEST ONLY: lets the partition /
+exchange logic of kccotgan_b200.sharded.ShardedMixedLoss run under gloo without a GPU."""
 import math
 
 import torch
-
-
-class CpuShardBackend:
-    def __init__(self, C_rows, B, eps):
-        self.C = C_rows.double()
-        self.Brows, self.B, self.eps = C_rows.shape[0], B, float(eps)
-        self.k = math.log2(math.e) / self.eps
-        self.ahat = -math.log2(B)
-        self.shift = torch.zeros(1, dtype=torch.float64)
-
-    def new(self, *shape):
-        return torch.zeros(*shape, dtype=torch.float64)
-
-    zeros = new
-
-    def begin(self):
-        self.shift[0] = self.C.min()
-        return self.shift
-
-    def _chat(self):
-        return (self.C - self.shift) * self.k
-
-    def fwd_rows(self, v, u_rows, colstat):
-        Ch = self._chat()
-        u_rows.copy_(self.ahat - torch.logsumexp((v[None, :] - Ch) * math.log(2), dim=1) / math.log(2))
-        t = u_rows[:, None] - Ch
-        m = t.max(dim=0).values
-        colstat[0].copy_(m)
-        colstat[1].copy_(torch.exp2(t - m[None, :]).sum(dim=0))
-
-    def fwd_combine(self, colstat_all, v):
-        M = colstat_all[:, 0].max(dim=0).values
-        S = (colstat_all[:, 1] * torch.exp2(colstat_all[:, 0] - M[None, :])).sum(dim=0)
-        v.copy_(self.ahat - (M + torch.log2(S)))
-
-    def cost_partial(self, u_rows, v, partial):
-        Ch = self._chat()
-        pi = torch.exp2(u_rows[:, None] + v[None, :] - Ch)
-        partial[0] = pi.sum()
-        partial[1] = (pi * Ch).sum()
-
-    def bwd_seed(self, u_rows, v, g, Cbar_rows, ubar_rows, colsum):
-        Ch = self._chat()
-        ce = (self.C - self.shift) / self.eps
-        pi = g * torch.exp2(u_rows[:, None] + v[None, :] - Ch)
-        Cbar_rows.copy_(pi * (1 - ce))
-        ubar_rows.copy_((pi * ce).sum(dim=1))
-        colsum.copy_((pi * ce).sum(dim=0))
-
-    def bwd_rows(self, u_k, v_k, v_km1, vbar, first, ubar_rows, Cbar_rows, colsum):
-        Ch = self._chat()
-        Pv = torch.exp2(u_k[:, None] + v_k[None, :] - self.ahat - Ch)
-        Cbar_rows.add_(Pv * vbar[None, :])
-        ub = (ubar_rows if first else torch.zeros_like(ubar_rows)) - Pv @ vbar
-        ubar_rows.copy_(ub)
-        Pu = torch.exp2(u_k[:, None] + v_km1[None, :] - self.ahat - Ch)
-        Cbar_rows.add_(Pu * ub[:, None])
-        colsum.copy_(Pu.T @ ub)
 
 
 class CpuMixedShardBackend:

@@ -29,7 +29,7 @@ def test_header_symbols_exported(lib):
 
 def test_version_and_no_cpu_fallback(lib):
     from kccotgan_b200 import _lib
-    assert lib.kccot_version() == 202
+    assert lib.kccot_version() == 203
     if not torch.cuda.is_available():
         assert lib.kccot_device_check() != 0
         assert "no CUDA device" in _lib.last_error()

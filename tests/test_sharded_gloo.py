@@ -1,7 +1,7 @@
 """T4/T5 on CPU: the multi-GPU host logic under torch.distributed `gloo`, world_size 2.
   * problem-parallel partitioning (no collective on the data path);
-  * the row-sharded Sinkhorn exchange (all-gather of (max, sum-exp) pairs, all-reduce of column sums),
-    with an fp64 CPU stand-in for the kernels, against the single-process oracle."""
+  * the fused row-sharded mixed loss (cost shift, cost partials, adjoint panels and gradient sums
+    exchanged between ranks), with an fp64 CPU stand-in for the kernels, against the single-process oracle."""
 import os
 import sys
 
@@ -25,48 +25,6 @@ def test_split_problems_covers_everything():
             sizes = [len(split_problems(nprob, r, world)) for r in range(world)]
             assert max(sizes) - min(sizes) <= 1
     assert row_range(8192, 3, 8) == (3072, 4096)
-
-
-def _worker(rank, world, port, B, eps, L, C, out):
-    os.environ["MASTER_ADDR"] = "127.0.0.1"
-    os.environ["MASTER_PORT"] = str(port)
-    dist.init_process_group("gloo", rank=rank, world_size=world)
-    try:
-        from kccotgan_b200.sharded import ShardedSinkhorn, row_range, split_problems
-        from _shard_cpu_backend import CpuShardBackend
-        r0, r1 = row_range(B, rank, world)
-        sk = ShardedSinkhorn(CpuShardBackend(torch.from_numpy(C[r0:r1]), B, eps))
-        cost = sk.forward(L=L)
-        Cbar = sk.backward(g=1.5)
-        # problem-parallel mode: each rank "solves" its share; only the scalars are gathered at the end
-        mine = torch.zeros(5, dtype=torch.float64)
-        for p in split_problems(5, rank, world):
-            mine[p] = float(p + 1)
-        dist.all_reduce(mine)
-        out[rank] = (float(cost), sk.nits, Cbar.numpy(), r0, r1, mine.numpy())
-    finally:
-        dist.destroy_process_group()
-
-
-@pytest.mark.parametrize("B,eps,L", [(12, 0.8, 25), (9, 1.0, 130)])
-def test_row_sharded_sinkhorn_two_ranks(B, eps, L):
-    from oracle import closed_form as cf
-    rng = np.random.default_rng(B)
-    C = (5.0 + rng.random((B, B)) * 3.0)
-    mgr = mp.Manager()
-    out = mgr.dict()
-    port = 29500 + (os.getpid() % 2000)
-    mp.spawn(_worker, args=(2, port, B, eps, L, C, out), nprocs=2, join=True)
-    ref, uh, vh, nits = cf.sinkhorn_forward(C, eps, L, Lmin=100, thresh=1e-2)
-    Cb = cf.sinkhorn_backward(C, eps, uh, vh, nits, gbar=1.5)
-    got = np.zeros_like(C)
-    for rank in (0, 1):
-        cost, n, Cbar, r0, r1, mine = out[rank]
-        assert n == nits
-        assert abs(cost - ref) < 1e-10 * abs(ref)
-        got[r0:r1] = Cbar
-        assert np.array_equal(mine, np.arange(1, 6, dtype=np.float64))
-    assert np.linalg.norm(got - Cb) < 1e-9 * np.linalg.norm(Cb)
 
 
 def _mixed_worker(rank, world, port, shape, inp, out):
