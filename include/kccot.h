@@ -144,6 +144,24 @@ int kccot_shard_cost_bwd(const float* Cbar3rows, const float* XYcol, const float
                          const float* h_real, const float* m_fake, int T, int J, float s,
                          float* g_fake_rows, float* gh_fake_rows, float* gm_real_part,
                          float* gh_real_rows, float* gm_fake_part, void* ws, size_t ws_bytes, void* stream);
+/* bf16 videos — the row-sharded cost for callers that keep their videos in bf16.  real / fake and g_fake_rows are
+ * raw bf16 bits (uint16_t), 16-byte aligned; everything else, including the workspace
+ * (kccot_shard_cost_workspace_bytes), is as in the fp32 entries above, and g_fake_rows may be NULL.
+ * Contract: the results are EXACTLY those of the fp32 entries on the widened videos (a bf16 value is exact in fp32):
+ * C3rows and the h / M gradients bit for bit, g_fake_rows the fp32 gradient rows rounded to nearest even.  The
+ * pre-pass widens on load and runs the fp32 instruction sequence; the adjoint GEMM rounds only at its store.  No fp32
+ * copy of a video is made.  Null pointers, a bad row range and a video or gradient pointer that is not 16-byte
+ * aligned are rejected (KCCOT_EINVAL) before any CUDA call.  The Sinkhorn entries below see only fp32 cost rows. */
+int kccot_shard_cost_fwd_bf16(const uint16_t* real, const uint16_t* fake, int B, long long K, int row0,
+                              int Brows, const float* h_fake, const float* m_real, const float* h_real,
+                              const float* m_fake, int T, int J, float s, float* C3rows, void* ws,
+                              size_t ws_bytes, void* stream);
+int kccot_shard_cost_bwd_bf16(const float* Cbar3rows, const float* XYcol, const float* YYcol, int B,
+                              long long K, int row0, int Brows, const float* h_fake, const float* m_real,
+                              const float* h_real, const float* m_fake, int T, int J, float s,
+                              uint16_t* g_fake_rows, float* gh_fake_rows, float* gm_real_part,
+                              float* gh_real_rows, float* gm_fake_part, void* ws, size_t ws_bytes,
+                              void* stream);
 size_t kccot_shard_sinkhorn_workspace_bytes(int np, int Brows, int B, int L);
 size_t kccot_shard_mailbox_bytes(int np, int nranks, int B);
 int kccot_shard_local_min(const float* Crows, int np, int Brows, int B, float* shift_out, void* stream);

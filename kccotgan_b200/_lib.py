@@ -40,6 +40,9 @@ SIGNATURES = {
     "kccot_shard_cost_fwd": (_I, [_P, _P, _I, _LL, _I, _I, _P, _P, _P, _P, _I, _I, _F, _P, _P, _SZ, _P]),
     "kccot_shard_cost_bwd": (_I, [_P, _P, _P, _I, _LL, _I, _I, _P, _P, _P, _P, _I, _I, _F, _P, _P, _P, _P, _P, _P, _SZ,
                                   _P]),
+    "kccot_shard_cost_fwd_bf16": (_I, [_P, _P, _I, _LL, _I, _I, _P, _P, _P, _P, _I, _I, _F, _P, _P, _SZ, _P]),
+    "kccot_shard_cost_bwd_bf16": (_I, [_P, _P, _P, _I, _LL, _I, _I, _P, _P, _P, _P, _I, _I, _F, _P, _P, _P, _P, _P, _P,
+                                       _SZ, _P]),
     "kccot_shard_sinkhorn_workspace_bytes": (_SZ, [_I, _I, _I, _I]),
     "kccot_shard_mailbox_bytes": (_SZ, [_I, _I, _I]),
     "kccot_shard_local_min": (_I, [_P, _I, _I, _I, _P, _P]),

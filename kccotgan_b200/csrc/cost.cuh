@@ -101,7 +101,7 @@ struct G3Job {
   int m, n;                // valid rows / columns of the block
   int tm, tn, ntiles;      // filled by g3_count_tiles_pair
   int tri;                 // symmetric block (a_row0 == b_row0): only tiles touching the upper triangle
-  float* out;              // [ksplit][m][ld]
+  float* out;              // [ksplit][m][ld] (bf16 bits for launch_gemm_f16x3_pair_bf16)
   long long ld, ks_stride;
 };
 struct G3Params {
@@ -120,6 +120,10 @@ void g3_plan_split(int ntiles, int nkb, int units, int* ksplit, int* kb_per_spli
 int launch_gemm_f16x3_pair(const __half* A1, const __half* A2, long long a_rows, long long a_pitch_elems,
                            const __half* B1, const __half* B2, long long b_rows, long long b_pitch_elems, long long kdim,
                            G3Params P, cudaStream_t st);
+// the same product stored as bf16 (the fp32 output value rounded to nearest even); P.accumulate must be 0
+int launch_gemm_f16x3_pair_bf16(const __half* A1, const __half* A2, long long a_rows, long long a_pitch_elems,
+                                const __half* B1, const __half* B2, long long b_rows, long long b_pitch_elems,
+                                long long kdim, G3Params P, cudaStream_t st);
 
 // large_abi.cu: true when the large-batch path takes the shape
 bool large_path_wanted(int Bx, int By, bool same);
@@ -142,6 +146,15 @@ int large_shard_cost_fwd(const float* real, const float* fake, int B, long long 
 int large_shard_cost_bwd(const float* Cbar3rows, const float* XYcol, const float* YYcol, int B, long long K, int row0,
                          int Brows, const float* h_fake, const float* m_real, const float* h_real, const float* m_fake,
                          int T, int J, float s, float* g_fake_rows, float* gh_fake_rows, float* gm_real_part,
+                         float* gh_real_rows, float* gm_fake_part, void* ws, size_t ws_bytes, cudaStream_t st);
+// bf16 videos and fake gradient rows (raw bits): the fp32 results on the widened videos, the gradient rows rounded to
+// nearest even; same workspace
+int large_shard_cost_fwd(const uint16_t* real, const uint16_t* fake, int B, long long K, int row0, int Brows,
+                         const float* h_fake, const float* m_real, const float* h_real, const float* m_fake, int T, int J,
+                         float s, float* C3rows, void* ws, size_t ws_bytes, cudaStream_t st);
+int large_shard_cost_bwd(const float* Cbar3rows, const float* XYcol, const float* YYcol, int B, long long K, int row0,
+                         int Brows, const float* h_fake, const float* m_real, const float* h_real, const float* m_fake,
+                         int T, int J, float s, uint16_t* g_fake_rows, float* gh_fake_rows, float* gm_real_part,
                          float* gh_real_rows, float* gm_fake_part, void* ws, size_t ws_bytes, cudaStream_t st);
 
 }  // namespace kccot

@@ -135,6 +135,9 @@ __device__ __forceinline__ bool decode_item(const G3Params& P, int w, Item& it) 
 }
 }  // namespace
 
+// Out = float: out (+)= alpha * acc.  Out = uint16_t: out = bf16(alpha * acc), the fp32 epilogue's value rounded to
+// nearest even (G3Job::out then holds bf16 bits; no accumulation).
+template <typename Out>
 __global__ void __launch_bounds__(kThreads, 1)
 gemm_f16x3_pair_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_constant__ CUtensorMap tmA2,
                        const __grid_constant__ CUtensorMap tmB1, const __grid_constant__ CUtensorMap tmB2,
@@ -279,8 +282,9 @@ gemm_f16x3_pair_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_co
         }
         if (last) {
           // cross accumulator, then the output tile (written once per work item)
-          float* orow = jb.out + (long long)it.ks * jb.ks_stride + (long long)row * jb.ld + it.n0 + half * 128;
-          const bool vec_ok = ((jb.ld & 3) == 0) && ((reinterpret_cast<uintptr_t>(jb.out) & 15) == 0) &&
+          Out* orow = reinterpret_cast<Out*>(jb.out) + (long long)it.ks * jb.ks_stride + (long long)row * jb.ld + it.n0 +
+                      half * 128;
+          const bool vec_ok = ((jb.ld & 3) == 0) && ((reinterpret_cast<uintptr_t>(jb.out) & (4 * sizeof(Out) - 1)) == 0) &&
                               (((long long)it.ks * jb.ks_stride & 3) == 0) && ((it.n0 & 3) == 0);
 #pragma unroll
           for (int cc = 0; cc < 4; ++cc) {
@@ -293,7 +297,25 @@ gemm_f16x3_pair_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_co
               if (lane == 0) mbar_arrive_cluster(free_leader);
             }
             const int ncols = ncols_left - cc * 32;
-            if (row_ok && ncols > 0) {
+            if constexpr (sizeof(Out) == 2) {
+              if (row_ok && ncols > 0) {
+                uint16_t* o = orow + cc * 32;
+                if (vec_ok && ncols >= 32) {                // 8-byte stores of four values
+#pragma unroll
+                  for (int j = 0; j < 8; ++j) {
+                    const float v0 = fmaf(alpha, racc[cc * 32 + 4 * j + 0] + x[4 * j + 0], 0.f);
+                    const float v1 = fmaf(alpha, racc[cc * 32 + 4 * j + 1] + x[4 * j + 1], 0.f);
+                    const float v2 = fmaf(alpha, racc[cc * 32 + 4 * j + 2] + x[4 * j + 2], 0.f);
+                    const float v3 = fmaf(alpha, racc[cc * 32 + 4 * j + 3] + x[4 * j + 3], 0.f);
+                    reinterpret_cast<uint2*>(o)[j] = make_uint2(pack_bf16x2(v0, v1), pack_bf16x2(v2, v3));
+                  }
+                } else {
+#pragma unroll
+                  for (int j = 0; j < 32; ++j)
+                    if (j < ncols) o[j] = __bfloat16_as_ushort(__float2bfloat16_rn(alpha * (racc[cc * 32 + j] + x[j])));
+                }
+              }
+            } else if (row_ok && ncols > 0) {
               float* o = orow + cc * 32;
               if (vec_ok && ncols >= 32) {
 #pragma unroll
@@ -357,9 +379,10 @@ void g3_plan_split(int ntiles, int nkb, int units, int* ksplit, int* kb_per_spli
   *kb_per_split = per;
 }
 
-int launch_gemm_f16x3_pair(const __half* A1, const __half* A2, long long a_rows, long long a_pitch_elems,
-                           const __half* B1, const __half* B2, long long b_rows, long long b_pitch_elems, long long kdim,
-                           G3Params P, cudaStream_t st) {
+namespace {
+template <typename Out>
+int launch_pair(const __half* A1, const __half* A2, long long a_rows, long long a_pitch_elems, const __half* B1,
+                const __half* B2, long long b_rows, long long b_pitch_elems, long long kdim, G3Params P, cudaStream_t st) {
   CUtensorMap tA1, tA2, tB1, tB2;
   if (int rc = encode_tmap_2d_f16(&tA1, A1, (uint64_t)kdim, (uint64_t)a_rows, (uint64_t)a_pitch_elems * 2, BK, 128)) return rc;
   if (int rc = encode_tmap_2d_f16(&tA2, A2, (uint64_t)kdim, (uint64_t)a_rows, (uint64_t)a_pitch_elems * 2, BK, 128)) return rc;
@@ -373,7 +396,7 @@ int launch_gemm_f16x3_pair(const __half* A1, const __half* A2, long long a_rows,
   const size_t smem = (size_t)kStages * kStageBytes + sizeof(Bars) + 1024;
   static size_t attr_set[kMaxDevices] = {};
   if (smem_attr_needed(attr_set, smem))
-    KCCOT_CUDA(cudaFuncSetAttribute(gemm_f16x3_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    KCCOT_CUDA(cudaFuncSetAttribute(gemm_f16x3_pair_kernel<Out>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const long long nitems = (long long)P.ntiles_total * P.ksplit;
   const int max_clusters = num_sms() / 2;
   const int nclusters = (int)(nitems < max_clusters ? nitems : max_clusters);
@@ -389,9 +412,22 @@ int launch_gemm_f16x3_pair(const __half* A1, const __half* A2, long long a_rows,
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  KCCOT_CUDA(cudaLaunchKernelEx(&cfg, gemm_f16x3_pair_kernel, tA1, tA2, tB1, tB2, P));
+  KCCOT_CUDA(cudaLaunchKernelEx(&cfg, gemm_f16x3_pair_kernel<Out>, tA1, tA2, tB1, tB2, P));
   KCCOT_LAUNCH_CHECK();
   return KCCOT_OK;
+}
+}  // namespace
+
+int launch_gemm_f16x3_pair(const __half* A1, const __half* A2, long long a_rows, long long a_pitch_elems,
+                           const __half* B1, const __half* B2, long long b_rows, long long b_pitch_elems, long long kdim,
+                           G3Params P, cudaStream_t st) {
+  return launch_pair<float>(A1, A2, a_rows, a_pitch_elems, B1, B2, b_rows, b_pitch_elems, kdim, P, st);
+}
+int launch_gemm_f16x3_pair_bf16(const __half* A1, const __half* A2, long long a_rows, long long a_pitch_elems,
+                                const __half* B1, const __half* B2, long long b_rows, long long b_pitch_elems,
+                                long long kdim, G3Params P, cudaStream_t st) {
+  KCCOT_CHECK_ARG(!P.accumulate, "bf16 GEMM output cannot accumulate");
+  return launch_pair<uint16_t>(A1, A2, a_rows, a_pitch_elems, B1, B2, b_rows, b_pitch_elems, kdim, P, st);
 }
 
 }  // namespace kccot

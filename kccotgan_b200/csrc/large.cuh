@@ -37,6 +37,12 @@ int large_launch_stats(const float* x, const float* y, int Bx, int By, long long
 int large_launch_split(const float* x, const float* y, int Bx, int By, long long K, long long Kp, int Rp,
                        const float* mean, const float* scal, __half* Zh1, __half* Zh2, __half* ZT1, __half* ZT2,
                        cudaStream_t st);
+// bf16 videos (raw bits): the same column sums, scale and split as the fp32 launchers on the widened videos
+int large_launch_stats(const uint16_t* x, const uint16_t* y, int Bx, int By, long long K, int nseg, float* part,
+                       float* mean, float* scal, cudaStream_t st);
+int large_launch_split(const uint16_t* x, const uint16_t* y, int Bx, int By, long long K, long long Kp, int Rp,
+                       const float* mean, const float* scal, __half* Zh1, __half* Zh2, __half* ZT1, __half* ZT2,
+                       cudaStream_t st);
 int large_launch_rownorm(const __half* Zh1, const __half* Zh2, int R, long long K, long long Kp, float* norms,
                          cudaStream_t st);
 int large_launch_finalize(const LargeFin& F, int nblocks, int T, int J, float s, const float* scal, cudaStream_t st);

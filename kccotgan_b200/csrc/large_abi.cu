@@ -257,9 +257,12 @@ ShardWs carve_shard(void* ws, int B, long long K, int Brows) {
 
 size_t large_shard_ws_bytes(int B, long long K, int Brows) { return carve_shard(nullptr, B, K, Brows).bytes; }
 
-int large_shard_cost_fwd(const float* real, const float* fake, int B, long long K, int row0, int Brows, const float* h_fake,
-                         const float* m_real, const float* h_real, const float* m_fake, int T, int J, float s,
-                         float* C3rows, void* ws, size_t ws_bytes, cudaStream_t st) {
+namespace {
+// Video element type V (float, or bf16 bits): only the pre-pass reads the videos, so only it depends on V.
+template <typename V>
+int shard_cost_fwd(const V* real, const V* fake, int B, long long K, int row0, int Brows, const float* h_fake,
+                   const float* m_real, const float* h_real, const float* m_fake, int T, int J, float s, float* C3rows,
+                   void* ws, size_t ws_bytes, cudaStream_t st) {
   KCCOT_CHECK_ARG(row0 >= 0 && Brows >= 1 && row0 + Brows <= B, "bad row range [%d, %d) of %d", row0, row0 + Brows, B);
   const ShardWs w = carve_shard(ws, B, K, Brows);
   KCCOT_CHECK_ARG(ws_bytes >= w.bytes, "workspace too small (row-shard cost path needs %zu bytes, got %zu)", w.bytes, ws_bytes);
@@ -289,12 +292,12 @@ int large_shard_cost_fwd(const float* real, const float* fake, int B, long long 
   return large_launch_finalize(F, 3, T, J, s, w.scal, st);
 }
 
-// g_fake_rows [Brows][K]; gh_* rows [Brows][T][J] (own samples); gm_* partial sums [B][T][J] over this rank's rows
-// (the caller all-reduces them).  `ws` is the workspace of the matching large_shard_cost_fwd call.
-int large_shard_cost_bwd(const float* Cbar3rows, const float* XYcol, const float* YYcol, int B, long long K, int row0,
-                         int Brows, const float* h_fake, const float* m_real, const float* h_real, const float* m_fake,
-                         int T, int J, float s, float* g_fake_rows, float* gh_fake_rows, float* gm_real_part,
-                         float* gh_real_rows, float* gm_fake_part, void* ws, size_t ws_bytes, cudaStream_t st) {
+// Gradient element type G (float, or bf16 bits): only the adjoint GEMM's store depends on G.
+template <typename G>
+int shard_cost_bwd(const float* Cbar3rows, const float* XYcol, const float* YYcol, int B, long long K, int row0, int Brows,
+                   const float* h_fake, const float* m_real, const float* h_real, const float* m_fake, int T, int J,
+                   float s, G* g_fake_rows, float* gh_fake_rows, float* gm_real_part, float* gh_real_rows,
+                   float* gm_fake_part, void* ws, size_t ws_bytes, cudaStream_t st) {
   const ShardWs w = carve_shard(ws, B, K, Brows);
   KCCOT_CHECK_ARG(ws_bytes >= w.bytes, "workspace too small (row-shard cost path needs %zu bytes, got %zu)", w.bytes, ws_bytes);
   const long long RB = (long long)Brows * B, hm = (long long)T * J;
@@ -312,7 +315,7 @@ int large_shard_cost_bwd(const float* Cbar3rows, const float* XYcol, const float
                                          w.Wh1, w.Wh2, st))
     return rc;
   G3Params P{};
-  P.job[0] = G3Job{0, 0, Brows, (int)K, 0, 0, 0, 0, g_fake_rows, K, 0};
+  P.job[0] = G3Job{0, 0, Brows, (int)K, 0, 0, 0, 0, reinterpret_cast<float*>(g_fake_rows), K, 0};
   g3_count_tiles_pair(&P.job[0]);
   P.njobs = 1;
   P.ksplit = 1;
@@ -320,7 +323,39 @@ int large_shard_cost_bwd(const float* Cbar3rows, const float* XYcol, const float
   P.alpha = -2.f * s;
   P.alpha_dev = w.scal + kScalGradAlpha;
   const int R = 2 * B;
-  return launch_gemm_f16x3_pair(w.Wh1, w.Wh2, Brows, w.Rp, w.ZT1, w.ZT2, K, w.Rp, R, P, st);
+  if constexpr (sizeof(G) == 2)
+    return launch_gemm_f16x3_pair_bf16(w.Wh1, w.Wh2, Brows, w.Rp, w.ZT1, w.ZT2, K, w.Rp, R, P, st);
+  else
+    return launch_gemm_f16x3_pair(w.Wh1, w.Wh2, Brows, w.Rp, w.ZT1, w.ZT2, K, w.Rp, R, P, st);
+}
+}  // namespace
+
+int large_shard_cost_fwd(const float* real, const float* fake, int B, long long K, int row0, int Brows, const float* h_fake,
+                         const float* m_real, const float* h_real, const float* m_fake, int T, int J, float s,
+                         float* C3rows, void* ws, size_t ws_bytes, cudaStream_t st) {
+  return shard_cost_fwd(real, fake, B, K, row0, Brows, h_fake, m_real, h_real, m_fake, T, J, s, C3rows, ws, ws_bytes, st);
+}
+int large_shard_cost_fwd(const uint16_t* real, const uint16_t* fake, int B, long long K, int row0, int Brows,
+                         const float* h_fake, const float* m_real, const float* h_real, const float* m_fake, int T, int J,
+                         float s, float* C3rows, void* ws, size_t ws_bytes, cudaStream_t st) {
+  return shard_cost_fwd(real, fake, B, K, row0, Brows, h_fake, m_real, h_real, m_fake, T, J, s, C3rows, ws, ws_bytes, st);
+}
+
+// g_fake_rows [Brows][K]; gh_* rows [Brows][T][J] (own samples); gm_* partial sums [B][T][J] over this rank's rows
+// (the caller all-reduces them).  `ws` is the workspace of the matching large_shard_cost_fwd call.
+int large_shard_cost_bwd(const float* Cbar3rows, const float* XYcol, const float* YYcol, int B, long long K, int row0,
+                         int Brows, const float* h_fake, const float* m_real, const float* h_real, const float* m_fake,
+                         int T, int J, float s, float* g_fake_rows, float* gh_fake_rows, float* gm_real_part,
+                         float* gh_real_rows, float* gm_fake_part, void* ws, size_t ws_bytes, cudaStream_t st) {
+  return shard_cost_bwd(Cbar3rows, XYcol, YYcol, B, K, row0, Brows, h_fake, m_real, h_real, m_fake, T, J, s, g_fake_rows,
+                        gh_fake_rows, gm_real_part, gh_real_rows, gm_fake_part, ws, ws_bytes, st);
+}
+int large_shard_cost_bwd(const float* Cbar3rows, const float* XYcol, const float* YYcol, int B, long long K, int row0,
+                         int Brows, const float* h_fake, const float* m_real, const float* h_real, const float* m_fake,
+                         int T, int J, float s, uint16_t* g_fake_rows, float* gh_fake_rows, float* gm_real_part,
+                         float* gh_real_rows, float* gm_fake_part, void* ws, size_t ws_bytes, cudaStream_t st) {
+  return shard_cost_bwd(Cbar3rows, XYcol, YYcol, B, K, row0, Brows, h_fake, m_real, h_real, m_fake, T, J, s, g_fake_rows,
+                        gh_fake_rows, gm_real_part, gh_real_rows, gm_fake_part, ws, ws_bytes, st);
 }
 
 }  // namespace kccot

@@ -145,6 +145,109 @@ __global__ void __launch_bounds__(256) split_kernel(const float* __restrict__ x,
   }
 }
 
+// ---- bf16 videos ---------------------------------------------------------------------------------
+// colsum_part_kernel and split_kernel for bf16 videos (raw bits).  A bf16 value widens exactly, so after the load
+// each runs the fp32 kernel's instruction sequence and summation order: the column sums, the scale and the fp16 split
+// equal the fp32 kernels' on the widened videos.  Separate kernels, so that the fp32 ones keep their code.
+__device__ __forceinline__ float ld1(const uint16_t* __restrict__ p, long long i) {
+  return __uint_as_float((unsigned)p[i] << 16);
+}
+
+__global__ void __launch_bounds__(128) colsum_part_bf16_kernel(const uint16_t* __restrict__ x,
+                                                               const uint16_t* __restrict__ y, int Bx, int By,
+                                                               long long K, int rows_per_seg, float* __restrict__ part,
+                                                               unsigned* __restrict__ absmax) {
+  const long long k = (long long)blockIdx.x * 128 + threadIdx.x;
+  const int R = Bx + By;
+  const int r0 = blockIdx.y * rows_per_seg, r1 = min(R, r0 + rows_per_seg);
+  float acc = 0.f, mx = 0.f;
+  if (k < K) {
+    int r = r0;
+    for (; r + 4 <= r1; r += 4) {
+      float v[4];
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        const int rr = r + u;
+        v[u] = (rr < Bx) ? ld1(x, (long long)rr * K + k) : ld1(y, (long long)(rr - Bx) * K + k);
+      }
+#pragma unroll
+      for (int u = 0; u < 4; ++u) { acc += v[u]; mx = fmaxf(mx, fabsf(v[u])); }
+    }
+    for (; r < r1; ++r) {
+      const float v = (r < Bx) ? ld1(x, (long long)r * K + k) : ld1(y, (long long)(r - Bx) * K + k);
+      acc += v;
+      mx = fmaxf(mx, fabsf(v));
+    }
+    part[(long long)blockIdx.y * K + k] = acc;
+  }
+  mx = warp_max(mx);
+  if ((threadIdx.x & 31) == 0 && mx > 0.f && mx < 3.0e38f) atomicMax(absmax, __float_as_uint(mx));
+}
+
+__global__ void __launch_bounds__(256) split_bf16_kernel(const uint16_t* __restrict__ x, const uint16_t* __restrict__ y,
+                                                         int Bx, int By, long long K, long long Kp, int Rp,
+                                                         const float* __restrict__ mean, const float* __restrict__ scal,
+                                                         __half* __restrict__ Zh1, __half* __restrict__ Zh2,
+                                                         __half* __restrict__ ZT1, __half* __restrict__ ZT2) {
+  __shared__ __half t1[64][72], t2[64][72];                 // [column][row] for the transposed copy
+  const int R = Bx + By;
+  const long long c0 = (long long)blockIdx.x * 64;
+  const int r0 = blockIdx.y * 64;
+  const int t = threadIdx.x;
+  const int cg = (t & 15) * 4;
+  const float zs = scal[kScalZscale];
+  float m[4];
+#pragma unroll
+  for (int e = 0; e < 4; ++e) m[e] = (c0 + cg + e < K) ? mean[c0 + cg + e] : 0.f;
+  const bool vec = ((K & 3) == 0) && ((reinterpret_cast<uintptr_t>(x) & 7) == 0) &&
+                   ((reinterpret_cast<uintptr_t>(y) & 7) == 0);
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int rl = (t >> 4) + 16 * i;
+    const int r = r0 + rl;
+    float v[4] = {0.f, 0.f, 0.f, 0.f};
+    if (r < R) {
+      const uint16_t* src = (r < Bx) ? x + (long long)r * K : y + (long long)(r - Bx) * K;
+      if (vec && c0 + cg + 3 < K) {
+        const float4 q = widen_bf16x4(*reinterpret_cast<const uint2*>(src + c0 + cg));
+        v[0] = q.x; v[1] = q.y; v[2] = q.z; v[3] = q.w;
+      } else {
+#pragma unroll
+        for (int e = 0; e < 4; ++e)
+          if (c0 + cg + e < K) v[e] = ld1(src, c0 + cg + e);
+      }
+    }
+    __half h1[4], h2[4];
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      const bool in = (r < R) && (c0 + cg + e < K);
+      const float z = in ? (v[e] - m[e]) * zs : 0.f;
+      h1[e] = __float2half_rn(z);
+      h2[e] = __float2half_rn(z - __half2float(h1[e]));
+    }
+    if (Zh1 != nullptr && r < R && c0 + cg < Kp) {          // Kp is a multiple of 64: the 4-group is inside the pitch
+      *reinterpret_cast<uint2*>(Zh1 + (long long)r * Kp + c0 + cg) = *reinterpret_cast<const uint2*>(h1);
+      *reinterpret_cast<uint2*>(Zh2 + (long long)r * Kp + c0 + cg) = *reinterpret_cast<const uint2*>(h2);
+    }
+    if (ZT1 != nullptr) {
+#pragma unroll
+      for (int e = 0; e < 4; ++e) { t1[cg + e][rl] = h1[e]; t2[cg + e][rl] = h2[e]; }
+    }
+  }
+  if (ZT1 == nullptr) return;
+  __syncthreads();
+  // transposed rows: 4 threads per video column, 16 stacked rows (32 bytes) each
+  const int c = t >> 2, seg = (t & 3) * 16;
+  if (c0 + c < Kp && r0 + seg < Rp) {                        // Rp is a multiple of 64
+    const uint4* s1 = reinterpret_cast<const uint4*>(&t1[c][seg]);
+    const uint4* s2 = reinterpret_cast<const uint4*>(&t2[c][seg]);
+    uint4* d1 = reinterpret_cast<uint4*>(ZT1 + (c0 + c) * (long long)Rp + r0 + seg);
+    uint4* d2 = reinterpret_cast<uint4*>(ZT2 + (c0 + c) * (long long)Rp + r0 + seg);
+    d1[0] = s1[0]; d1[1] = s1[1];
+    d2[0] = s2[0]; d2[1] = s2[1];
+  }
+}
+
 // ---- row norms of the represented values ----------------------------------------------------------
 __global__ void __launch_bounds__(256) rownorm_kernel(const __half* __restrict__ Zh1, const __half* __restrict__ Zh2,
                                                       long long K, long long Kp, float* __restrict__ norms) {
@@ -381,27 +484,64 @@ __global__ void __launch_bounds__(256) w_convert_kernel(const float* __restrict_
 // ------------------------------------------------------------------------------------------------
 // launchers
 // ------------------------------------------------------------------------------------------------
-int large_launch_stats(const float* x, const float* y, int Bx, int By, long long K, int nseg, float* part, float* mean,
-                       float* scal, cudaStream_t st) {
+namespace {
+// the pre-pass kernels of an input element type
+template <typename T>
+struct Prep;
+template <>
+struct Prep<float> {
+  static constexpr auto colsum = colsum_part_kernel;
+  static constexpr auto split = split_kernel;
+};
+template <>
+struct Prep<uint16_t> {
+  static constexpr auto colsum = colsum_part_bf16_kernel;
+  static constexpr auto split = split_bf16_kernel;
+};
+
+template <typename T>
+int launch_stats(const T* x, const T* y, int Bx, int By, long long K, int nseg, float* part, float* mean, float* scal,
+                 cudaStream_t st) {
   const int R = Bx + By;
   const int rps = (R + nseg - 1) / nseg;
   KCCOT_CUDA(cudaMemsetAsync(scal, 0, kScalCount * sizeof(float), st));
-  colsum_part_kernel<<<dim3((unsigned)((K + 127) / 128), nseg), 128, 0, st>>>(x, y, Bx, By, K, rps, part,
-                                                                              reinterpret_cast<unsigned*>(scal) + kScalAbsmax);
+  Prep<T>::colsum<<<dim3((unsigned)((K + 127) / 128), nseg), 128, 0, st>>>(
+      x, y, Bx, By, K, rps, part, reinterpret_cast<unsigned*>(scal) + kScalAbsmax);
   KCCOT_LAUNCH_CHECK();
   colmean_kernel<<<(unsigned)((K + 255) / 256), 256, 0, st>>>(part, (R + rps - 1) / rps, K, R, mean, scal);
   KCCOT_LAUNCH_CHECK();
   return KCCOT_OK;
 }
 
+template <typename T>
+int launch_split(const T* x, const T* y, int Bx, int By, long long K, long long Kp, int Rp, const float* mean,
+                 const float* scal, __half* Zh1, __half* Zh2, __half* ZT1, __half* ZT2, cudaStream_t st) {
+  const int R = Bx + By;
+  Prep<T>::split<<<dim3((unsigned)((K + 63) / 64), (R + 63) / 64), 256, 0, st>>>(x, y, Bx, By, K, Kp, Rp, mean,
+                                                                                        scal, Zh1, Zh2, ZT1, ZT2);
+  KCCOT_LAUNCH_CHECK();
+  return KCCOT_OK;
+}
+}  // namespace
+
+int large_launch_stats(const float* x, const float* y, int Bx, int By, long long K, int nseg, float* part, float* mean,
+                       float* scal, cudaStream_t st) {
+  return launch_stats(x, y, Bx, By, K, nseg, part, mean, scal, st);
+}
+int large_launch_stats(const uint16_t* x, const uint16_t* y, int Bx, int By, long long K, int nseg, float* part,
+                       float* mean, float* scal, cudaStream_t st) {
+  return launch_stats(x, y, Bx, By, K, nseg, part, mean, scal, st);
+}
+
 int large_launch_split(const float* x, const float* y, int Bx, int By, long long K, long long Kp, int Rp,
                        const float* mean, const float* scal, __half* Zh1, __half* Zh2, __half* ZT1, __half* ZT2,
                        cudaStream_t st) {
-  const int R = Bx + By;
-  split_kernel<<<dim3((unsigned)((K + 63) / 64), (R + 63) / 64), 256, 0, st>>>(x, y, Bx, By, K, Kp, Rp, mean, scal, Zh1, Zh2,
-                                                                            ZT1, ZT2);
-  KCCOT_LAUNCH_CHECK();
-  return KCCOT_OK;
+  return launch_split(x, y, Bx, By, K, Kp, Rp, mean, scal, Zh1, Zh2, ZT1, ZT2, st);
+}
+int large_launch_split(const uint16_t* x, const uint16_t* y, int Bx, int By, long long K, long long Kp, int Rp,
+                       const float* mean, const float* scal, __half* Zh1, __half* Zh2, __half* ZT1, __half* ZT2,
+                       cudaStream_t st) {
+  return launch_split(x, y, Bx, By, K, Kp, Rp, mean, scal, Zh1, Zh2, ZT1, ZT2, st);
 }
 
 int large_launch_rownorm(const __half* Zh1, const __half* Zh2, int R, long long K, long long Kp, float* norms,

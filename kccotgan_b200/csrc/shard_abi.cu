@@ -24,6 +24,8 @@ int fill_comm(ShardComm* c, int nranks, int rank, void* const* mbox_ptrs, void* 
   return KCCOT_OK;
 }
 
+bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
 __global__ void __launch_bounds__(256) shard_min_kernel(const float* __restrict__ C, long long n, float* __restrict__ out) {
   __shared__ float red[8];
   const float* Cp = C + (long long)blockIdx.x * n;
@@ -60,6 +62,30 @@ int kccot_shard_cost_bwd(const float* Cbar3rows, const float* XYcol, const float
                          int T, int J, float s, float* g_fake_rows, float* gh_fake_rows, float* gm_real_part,
                          float* gh_real_rows, float* gm_fake_part, void* ws, size_t ws_bytes, void* stream) {
   KCCOT_CHECK_ARG(Cbar3rows && XYcol && YYcol && h_fake && m_real && h_real && m_fake && ws, "null pointer");
+  return large_shard_cost_bwd(Cbar3rows, XYcol, YYcol, B, K, row0, Brows, h_fake, m_real, h_real, m_fake, T, J, s, g_fake_rows,
+                              gh_fake_rows, gm_real_part, gh_real_rows, gm_fake_part, ws, ws_bytes, (cudaStream_t)stream);
+}
+
+int kccot_shard_cost_fwd_bf16(const uint16_t* real, const uint16_t* fake, int B, long long K, int row0, int Brows,
+                              const float* h_fake, const float* m_real, const float* h_real, const float* m_fake, int T,
+                              int J, float s, float* C3rows, void* ws, size_t ws_bytes, void* stream) {
+  KCCOT_CHECK_ARG(real && fake && h_fake && m_real && h_real && m_fake && C3rows && ws, "null pointer");
+  KCCOT_CHECK_ARG(B >= 1 && K >= 1 && T >= 2 && J >= 1, "bad sizes");
+  KCCOT_CHECK_ARG(row0 >= 0 && Brows >= 1 && row0 + Brows <= B, "bad row range [%d, %d) of %d", row0, row0 + Brows, B);
+  KCCOT_CHECK_ARG(aligned16(real) && aligned16(fake), "bf16 videos must be 16-byte aligned");
+  return large_shard_cost_fwd(real, fake, B, K, row0, Brows, h_fake, m_real, h_real, m_fake, T, J, s, C3rows, ws, ws_bytes,
+                              (cudaStream_t)stream);
+}
+
+int kccot_shard_cost_bwd_bf16(const float* Cbar3rows, const float* XYcol, const float* YYcol, int B, long long K, int row0,
+                              int Brows, const float* h_fake, const float* m_real, const float* h_real,
+                              const float* m_fake, int T, int J, float s, uint16_t* g_fake_rows, float* gh_fake_rows,
+                              float* gm_real_part, float* gh_real_rows, float* gm_fake_part, void* ws, size_t ws_bytes,
+                              void* stream) {
+  KCCOT_CHECK_ARG(Cbar3rows && XYcol && YYcol && h_fake && m_real && h_real && m_fake && ws, "null pointer");
+  KCCOT_CHECK_ARG(B >= 1 && K >= 1 && T >= 2 && J >= 1, "bad sizes");
+  KCCOT_CHECK_ARG(row0 >= 0 && Brows >= 1 && row0 + Brows <= B, "bad row range [%d, %d) of %d", row0, row0 + Brows, B);
+  KCCOT_CHECK_ARG(aligned16(g_fake_rows), "bf16 gradient rows must be 16-byte aligned");
   return large_shard_cost_bwd(Cbar3rows, XYcol, YYcol, B, K, row0, Brows, h_fake, m_real, h_real, m_fake, T, J, s, g_fake_rows,
                               gh_fake_rows, gm_real_part, gh_real_rows, gm_fake_part, ws, ws_bytes, (cudaStream_t)stream);
 }

@@ -17,6 +17,7 @@ import torch
 import torch.distributed as dist
 
 from . import _lib
+from .functional import _as_dtypes, _check_hm, _videos
 
 
 def split_problems(nprob, rank, world):
@@ -67,7 +68,13 @@ class PeerMailbox:
 
 
 class CudaMixedShardBackend:
-    """The C-ABI stages of the fused row-sharded loss on this rank's samples [row0, row0 + Brows)."""
+    """The C-ABI stages of the fused row-sharded loss on this rank's samples [row0, row0 + Brows).
+
+    `cost_fwd` validates its inputs before any launch and raises ValueError for anything the kernels cannot read:
+    videos and h / m must be CUDA tensors on this backend's device with [B, K] and [B, T, J] elements.  Two bf16
+    videos go to the bf16 entry points (a view that is not 16-byte aligned is cloned) and `cost_bwd` then returns the
+    `fake` gradient rows in bf16: the fp32 rows on the widened videos, rounded to nearest even.  A bf16 video next to
+    an fp32 one, and bf16 h / m, are widened (exact).  Every other dtype is rejected."""
 
     def __init__(self, B, K, T, J, s, eps, L, row0, Brows, dev, group):
         self.B, self.K, self.T, self.J, self.s, self.eps, self.L = B, K, T, J, float(s), float(eps), int(L)
@@ -102,12 +109,26 @@ class CudaMixedShardBackend:
             return None, None, 0
         return self.mail.mbox_ptrs, self.mail.flag_ptrs, self.mail.next_epoch()
 
+    def _check(self, real, fake, hm):
+        real, fake, bf16 = _videos(real, fake)
+        hm = [_check_hm(t, n, 3) for t, n in zip(hm, ("h_fake", "m_real", "h_real", "m_fake"))]
+        for t, n, shape in [(real, "f_real", (self.B, self.K)), (fake, "f_fake", (self.B, self.K))] + \
+                [(t, n, (self.B, self.T, self.J)) for t, n in zip(hm, ("h_fake", "m_real", "h_real", "m_fake"))]:
+            if tuple(t.shape) != shape:
+                raise ValueError(f"{n}: expected shape {shape}, got {tuple(t.shape)}")
+            if t.device != self.ws_cost.device:
+                raise ValueError(f"{n}: expected a tensor on {self.ws_cost.device}, got {t.device}")
+        return real, fake, bf16, hm
+
     def cost_fwd(self, real, fake, h_fake, m_real, h_real, m_fake):
+        real, fake, self.bf16, hm = self._check(real, fake, (h_fake, m_real, h_real, m_fake))
+        h_fake, m_real, h_real, m_fake = hm
         self.inputs = (real, fake, h_fake, m_real, h_real, m_fake)
         p = self._p
         with torch.cuda.device(self.dev):
-            _lib.call("kccot_shard_cost_fwd", p(real), p(fake), self.B, self.K, self.row0, self.Brows, p(h_fake), p(m_real),
-                      p(h_real), p(m_fake), self.T, self.J, self.s, p(self.C3), p(self.ws_cost), self.ws_cost.numel(), self._st())
+            _lib.call("kccot_shard_cost_fwd_bf16" if self.bf16 else "kccot_shard_cost_fwd", p(real), p(fake), self.B,
+                      self.K, self.row0, self.Brows, p(h_fake), p(m_real), p(h_real), p(m_fake), self.T, self.J, self.s,
+                      p(self.C3), p(self.ws_cost), self.ws_cost.numel(), self._st())
             _lib.call("kccot_shard_local_min", p(self.C3), 3, self.Brows, self.B, p(self.shift), self._st())
         return self.shift
 
@@ -133,13 +154,13 @@ class CudaMixedShardBackend:
         p = self._p
         real, fake, h_fake, m_real, h_real, m_fake = self.inputs
         f32 = dict(dtype=torch.float32, device=self.dev)
-        g_fake = torch.empty((self.Brows, self.K), **f32)
+        g_fake = torch.empty((self.Brows, self.K), dtype=torch.bfloat16 if self.bf16 else torch.float32, device=self.dev)
         gh_fake = torch.empty((self.Brows, self.T, self.J), **f32)
         gh_real = torch.empty((self.Brows, self.T, self.J), **f32)
         gm_real = torch.empty((self.B, self.T, self.J), **f32)
         gm_fake = torch.empty((self.B, self.T, self.J), **f32)
         with torch.cuda.device(self.dev):
-            _lib.call("kccot_shard_cost_bwd", p(self.Cbar3), p(XYcol), p(YYcol), self.B, self.K, self.row0, self.Brows,
+            _lib.call("kccot_shard_cost_bwd_bf16" if self.bf16 else "kccot_shard_cost_bwd", p(self.Cbar3), p(XYcol), p(YYcol), self.B, self.K, self.row0, self.Brows,
                       p(h_fake), p(m_real), p(h_real), p(m_fake), self.T, self.J, self.s, p(g_fake), p(gh_fake), p(gm_real),
                       p(gh_real), p(gm_fake), p(self.ws_cost), self.ws_cost.numel(), self._st())
         return g_fake, gh_fake, gm_real, gh_real, gm_fake
@@ -152,7 +173,12 @@ class ShardedMixedLoss:
 
     forward()  -> (loss, terms[3]) replicated on all ranks.
     backward() -> gradients of this rank's own samples: `fake` [Brows, ...] and `h_fake`, `h_real` [Brows, T, J];
-                  `m_real`, `m_fake` [B, T, J] summed over ranks (every sample's M meets every row).
+                  `m_real`, `m_fake` [B, T, J] summed over ranks (every sample's M meets every row).  Each gradient
+                  comes back in the dtype of its input.
+    The CUDA backend takes fp32 or bf16 videos and h / m (see CudaMixedShardBackend).  With bf16 videos the results
+    are exactly those of fp32 videos widened from them: loss, terms and the h / m gradients bit for bit, the `fake`
+    rows the fp32 rows rounded to nearest even, with no fp32 copy of a video.  bf16 m gradients are rounded after
+    the fp32 all-reduce, so every rank holds the same bits.
     Collectives of one evaluation (all small except the two [Brows, B] all-to-alls): MIN of 3 floats, SUM of 6
     floats, all-to-all of Cbar_xy / Cbar_yy, SUM of two [B, T, J]; the 2 x L x 3 column-sum exchanges of the
     Sinkhorn iterations happen inside the persistent kernels.
@@ -191,6 +217,7 @@ class ShardedMixedLoss:
         if flat[0].shape[1] != self.K:
             raise ValueError(f"expected videos with {self.K} elements per sample, got {flat[0].shape[1]}")
         self.fake_shape = fake.shape
+        self.dtypes = [t.dtype for t in (fake, h_fake, m_real, h_real, m_fake)]
         shift = self.be.cost_fwd(flat[0].contiguous(), flat[1].contiguous(), h_fake.contiguous(), m_real.contiguous(),
                                  h_real.contiguous(), m_fake.contiguous())
         self._allreduce(shift, dist.ReduceOp.MIN)               # one cost shift per problem for all ranks
@@ -209,6 +236,7 @@ class ShardedMixedLoss:
         g_fake, gh_fake, gm_real, gh_real, gm_fake = self.be.cost_bwd(XYcol, YYcol)
         self._allreduce(gm_real, dist.ReduceOp.SUM)
         self._allreduce(gm_fake, dist.ReduceOp.SUM)
+        g_fake, gh_fake, gm_real, gh_real, gm_fake = _as_dtypes((g_fake, gh_fake, gm_real, gh_real, gm_fake), self.dtypes)
         return {"fake": g_fake.reshape((self.Brows,) + tuple(self.fake_shape[1:])), "h_fake": gh_fake, "m_real": gm_real,
                 "h_real": gh_real, "m_fake": gm_fake}
 
