@@ -297,6 +297,28 @@ int kccot_smooth_bwd_bf16(int mode, const uint16_t* gout, const uint16_t* out, c
                           int radius_t, const float* taps_s, int radius_s, uint16_t* gx, void* ws,
                           size_t ws_bytes, void* stream);
 
+/* Weights in device memory — the smoothing for a sigma that changes between replays of a captured CUDA graph (an
+ * annealed sigma, :584-586), which host weights cannot follow: a graph records kernel arguments once.  Each entry has
+ * the arguments of its twin above, except that the two host arrays (taps_t, radius_t, taps_s, radius_s) become one
+ * device array `taps_dev` of 2*radius+1 fp32 weights, 4-byte aligned, and its radius: mode 1 filters T with them,
+ * mode 3 filters H, T and W with them.  The kernels read taps_dev when they run, so it may be rewritten between
+ * replays; it must hold its values until the call's kernels have run.
+ * Contract, for the same weight values: out, maxval and the tie mask are bit-identical to the twin's; gx is
+ * bit-identical outside the adjoint stencil of the tied maxima, where S = sum(gout * out) is an order-dependent atomic
+ * sum in both.  The argument checks are the twin's (the backward entries also check the sizes, as the bf16 ones do)
+ * plus a null or misaligned taps_dev (KCCOT_EINVAL), all made before any CUDA call, with the twin's error codes. */
+int kccot_smooth_fwd_dev(int mode, const float* x, int B, int H, int T, int W, int C, const float* taps_dev,
+                         int radius, float* out, float* maxval, void* ws, size_t ws_bytes, void* stream);
+int kccot_smooth_bwd_dev(int mode, const float* gout, const float* out, const float* maxval, int B, int H,
+                         int T, int W, int C, const float* taps_dev, int radius, float* gx, void* ws,
+                         size_t ws_bytes, void* stream);
+int kccot_smooth_fwd_bf16_dev(int mode, const uint16_t* x, int B, int H, int T, int W, int C,
+                              const float* taps_dev, int radius, uint16_t* out, float* maxval, uint32_t* ties,
+                              void* ws, size_t ws_bytes, void* stream);
+int kccot_smooth_bwd_bf16_dev(int mode, const uint16_t* gout, const uint16_t* out, const float* maxval,
+                              const uint32_t* ties, int B, int H, int T, int W, int C, const float* taps_dev,
+                              int radius, uint16_t* gx, void* ws, size_t ws_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -72,6 +72,10 @@ SIGNATURES = {
     "kccot_smooth_ties_bytes": (_SZ, [_I, _I, _I, _I, _I]),
     "kccot_smooth_fwd_bf16": (_I, [_I, _P, _I, _I, _I, _I, _I, _P, _I, _P, _I, _P, _P, _P, _P, _SZ, _P]),
     "kccot_smooth_bwd_bf16": (_I, [_I, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _I, _P, _I, _P, _P, _SZ, _P]),
+    "kccot_smooth_fwd_dev": (_I, [_I, _P, _I, _I, _I, _I, _I, _P, _I, _P, _P, _P, _SZ, _P]),
+    "kccot_smooth_bwd_dev": (_I, [_I, _P, _P, _P, _I, _I, _I, _I, _I, _P, _I, _P, _P, _SZ, _P]),
+    "kccot_smooth_fwd_bf16_dev": (_I, [_I, _P, _I, _I, _I, _I, _I, _P, _I, _P, _P, _P, _P, _SZ, _P]),
+    "kccot_smooth_bwd_bf16_dev": (_I, [_I, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _I, _P, _P, _SZ, _P]),
 }
 
 _lib = None

@@ -31,13 +31,21 @@ struct Taps {                        // by value in the kernel parameters
   int r;
 };
 __device__ __forceinline__ int reflect(int q, int n) { return q < 0 ? -q : (q >= n ? 2 * (n - 1) - q : q); }
+// the 2R+1 weights of a pass: the kernel arguments, or, when wdev is set (the *_dev entries), device memory read as
+// the kernel starts, so that a replayed CUDA graph filters with the buffer's current values.  (These kernels use no
+// programmatic dependent launch; one that did would have to read wdev after griddepcontrol.wait.)
+template <int R>
+__device__ __forceinline__ void load_weights(float (&w)[2 * R + 1], const Taps& tp, const float* wdev) {
+#pragma unroll
+  for (int k = 0; k < 2 * R + 1; ++k) w[k] = wdev != nullptr ? wdev[k] : tp.w[k];
+}
 // A[p][q] of the REFLECT-padded filter (or its transpose)
 template <int R>
-__device__ __forceinline__ float band_coef(const Taps& tp, int n, int p, int q, bool transposed) {
+__device__ __forceinline__ float band_coef(const float (&w)[2 * R + 1], int n, int p, int q, bool transposed) {
   const int row = transposed ? q : p, col = transposed ? p : q;
   float a = 0.f;
 #pragma unroll
-  for (int k = 0; k < 2 * R + 1; ++k) a += (reflect(row + k - R, n) == col) ? tp.w[k] : 0.f;
+  for (int k = 0; k < 2 * R + 1; ++k) a += (reflect(row + k - R, n) == col) ? w[k] : 0.f;
   return a;
 }
 
@@ -85,13 +93,15 @@ template <> struct Vec<1> {
 template <int MODE, int V, int R>
 __global__ void __launch_bounds__(FT) axis_col_kernel(const float* __restrict__ in, float* __restrict__ out,
                                                       long long outer, int n, long long inner,
-                                                      const Taps tp, float* gmax,
+                                                      const Taps tp, const float* wdev, float* gmax,
                                                       const float* divisor, BwdIn bw) {
   constexpr int kR = R, kTaps = 2 * R + 1;
   extern __shared__ float coef[];                          // coef[p][d] = A[p][p + d - R] (0 outside the matrix)
+  float w[kTaps];
+  load_weights<R>(w, tp, wdev);
   for (int e = threadIdx.x; e < n * kTaps; e += FT) {
     const int p = e / kTaps, q = p + (e % kTaps) - kR;
-    coef[e] = (q >= 0 && q < n) ? band_coef<R>(tp, n, p, q, (MODE & 16) != 0) : 0.f;
+    coef[e] = (q >= 0 && q < n) ? band_coef<R>(w, n, p, q, (MODE & 16) != 0) : 0.f;
   }
   __syncthreads();
   const long long iv = inner / V;
@@ -145,7 +155,7 @@ __global__ void __launch_bounds__(FT) axis_col_kernel(const float* __restrict__ 
 template <int MODE, int R>
 __global__ void __launch_bounds__(1024) axis_tile_kernel(const float* __restrict__ in, float* __restrict__ out,
                                                          long long outer, int n, int inner, int o_chunk,
-                                                         const Taps tp, float* gmax,
+                                                         const Taps tp, const float* wdev, float* gmax,
                                                          const float* divisor, BwdIn bw) {
   constexpr int kR = R, kTaps = 2 * R + 1;
   extern __shared__ __align__(16) float tile[];            // [o_chunk][n][inner], contiguous like global memory
@@ -183,11 +193,13 @@ __global__ void __launch_bounds__(1024) axis_tile_kernel(const float* __restrict
   int off[kTaps];
   {
     const int p = min(t, ni - 1) / inner;
+    float w[kTaps];
+    load_weights<R>(w, tp, wdev);
 #pragma unroll
     for (int d = 0; d < kTaps; ++d) {
       const int q = p + d - kR;
       const bool ok = q >= 0 && q < n;
-      c[d] = ok ? band_coef<R>(tp, n, p, q, (MODE & 16) != 0) : 0.f;
+      c[d] = ok ? band_coef<R>(w, n, p, q, (MODE & 16) != 0) : 0.f;
       off[d] = ok ? (d - kR) * inner : 0;
     }
   }
@@ -332,12 +344,15 @@ __device__ __forceinline__ void mark_ties(uint32_t* bits, const VecF<V>& r, long
 template <typename TI, typename TO, int MODE, int V, int R>
 __global__ void __launch_bounds__(FT) axis_col_bf16_kernel(const TI* __restrict__ in, TO* __restrict__ out,
                                                            long long outer, int n, long long inner, const Taps tp,
-                                                           float* gmax, const float* divisor, Ties tie) {
+                                                           const float* wdev, float* gmax, const float* divisor,
+                                                           Ties tie) {
   constexpr int kR = R, kTaps = 2 * R + 1;
   extern __shared__ float coef[];                          // coef[p][d] = A[p][p + d - R] (0 outside the matrix)
+  float w[kTaps];
+  load_weights<R>(w, tp, wdev);
   for (int e = threadIdx.x; e < n * kTaps; e += FT) {
     const int p = e / kTaps, q = p + (e % kTaps) - kR;
-    coef[e] = (q >= 0 && q < n) ? band_coef<R>(tp, n, p, q, (MODE & 16) != 0) : 0.f;
+    coef[e] = (q >= 0 && q < n) ? band_coef<R>(w, n, p, q, (MODE & 16) != 0) : 0.f;
   }
   __syncthreads();
   const long long iv = inner / V;
@@ -412,8 +427,8 @@ __global__ void __launch_bounds__(FT) axis_col_bf16_kernel(const TI* __restrict_
 template <typename TI, typename TO, int MODE, int R>
 __global__ void __launch_bounds__(1024) axis_tile_bf16_kernel(const TI* __restrict__ in, TO* __restrict__ out,
                                                               long long outer, int n, int inner, int o_chunk,
-                                                              const Taps tp, float* gmax, const float* divisor,
-                                                              Ties tie) {
+                                                              const Taps tp, const float* wdev, float* gmax,
+                                                              const float* divisor, Ties tie) {
   constexpr int kR = R, kTaps = 2 * R + 1;
   extern __shared__ __align__(16) float tile[];            // [o_chunk][n][inner], contiguous like global memory
   const int ni = n * inner;
@@ -448,11 +463,13 @@ __global__ void __launch_bounds__(1024) axis_tile_bf16_kernel(const TI* __restri
   int off[kTaps];
   {
     const int p = min(t, ni - 1) / inner;
+    float w[kTaps];
+    load_weights<R>(w, tp, wdev);
 #pragma unroll
     for (int d = 0; d < kTaps; ++d) {
       const int q = p + d - kR;
       const bool ok = q >= 0 && q < n;
-      c[d] = ok ? band_coef<R>(tp, n, p, q, (MODE & 16) != 0) : 0.f;
+      c[d] = ok ? band_coef<R>(w, n, p, q, (MODE & 16) != 0) : 0.f;
       off[d] = ok ? (d - kR) * inner : 0;
     }
   }
@@ -541,14 +558,15 @@ AxisPlan plan_axis(long long outer, int n, long long inner) {
 }
 
 template <int MODE, int R>
-int run_axis_r(const float* in, float* out, const AxisPlan& p, const Taps& tp, float* gmax, const float* divisor,
-               BwdIn bw, cudaStream_t st) {
+int run_axis_r(const float* in, float* out, const AxisPlan& p, const Taps& tp, const float* wdev, float* gmax,
+               const float* divisor, BwdIn bw, cudaStream_t st) {
   if (p.tiled) {
     const int ni = p.n * (int)p.inner;
     const int threads = (ni + 31) / 32 * 32;
     const unsigned grid = (unsigned)((p.outer + p.o_chunk - 1) / p.o_chunk);
     const size_t smem = (size_t)p.o_chunk * ni * sizeof(float);
-    axis_tile_kernel<MODE, R><<<grid, threads, smem, st>>>(in, out, p.outer, p.n, (int)p.inner, p.o_chunk, tp, gmax, divisor, bw);
+    axis_tile_kernel<MODE, R><<<grid, threads, smem, st>>>(in, out, p.outer, p.n, (int)p.inner, p.o_chunk, tp, wdev, gmax,
+                                                           divisor, bw);
   } else {
     const bool v4 = (p.inner % 4 == 0) && (reinterpret_cast<uintptr_t>(in) & 15) == 0 &&
                     (!(MODE & 1) || (reinterpret_cast<uintptr_t>(out) & 15) == 0) &&
@@ -560,49 +578,53 @@ int run_axis_r(const float* in, float* out, const AxisPlan& p, const Taps& tp, f
       if (v4) KCCOT_CUDA(cudaFuncSetAttribute(axis_col_kernel<MODE, 4, R>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       else KCCOT_CUDA(cudaFuncSetAttribute(axis_col_kernel<MODE, 1, R>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     }
-    if (v4) axis_col_kernel<MODE, 4, R><<<grid, FT, smem, st>>>(in, out, p.outer, p.n, p.inner, tp, gmax, divisor, bw);
-    else axis_col_kernel<MODE, 1, R><<<grid, FT, smem, st>>>(in, out, p.outer, p.n, p.inner, tp, gmax, divisor, bw);
+    if (v4) axis_col_kernel<MODE, 4, R><<<grid, FT, smem, st>>>(in, out, p.outer, p.n, p.inner, tp, wdev, gmax, divisor,
+                                                                bw);
+    else axis_col_kernel<MODE, 1, R><<<grid, FT, smem, st>>>(in, out, p.outer, p.n, p.inner, tp, wdev, gmax, divisor, bw);
   }
   KCCOT_LAUNCH_CHECK();
   return KCCOT_OK;
 }
 template <int MODE>
-int run_axis(const float* in, float* out, const AxisPlan& p, const Taps& tp, float* gmax, const float* divisor,
-             BwdIn bw, cudaStream_t st) {
+int run_axis(const float* in, float* out, const AxisPlan& p, const Taps& tp, const float* wdev, float* gmax,
+             const float* divisor, BwdIn bw, cudaStream_t st) {
   switch (tp.r) {
-    case 1: return run_axis_r<MODE, 1>(in, out, p, tp, gmax, divisor, bw, st);
-    case 2: return run_axis_r<MODE, 2>(in, out, p, tp, gmax, divisor, bw, st);
-    case 3: return run_axis_r<MODE, 3>(in, out, p, tp, gmax, divisor, bw, st);
-    case 4: return run_axis_r<MODE, 4>(in, out, p, tp, gmax, divisor, bw, st);
-    case 5: return run_axis_r<MODE, 5>(in, out, p, tp, gmax, divisor, bw, st);
-    case 6: return run_axis_r<MODE, 6>(in, out, p, tp, gmax, divisor, bw, st);
+    case 1: return run_axis_r<MODE, 1>(in, out, p, tp, wdev, gmax, divisor, bw, st);
+    case 2: return run_axis_r<MODE, 2>(in, out, p, tp, wdev, gmax, divisor, bw, st);
+    case 3: return run_axis_r<MODE, 3>(in, out, p, tp, wdev, gmax, divisor, bw, st);
+    case 4: return run_axis_r<MODE, 4>(in, out, p, tp, wdev, gmax, divisor, bw, st);
+    case 5: return run_axis_r<MODE, 5>(in, out, p, tp, wdev, gmax, divisor, bw, st);
+    case 6: return run_axis_r<MODE, 6>(in, out, p, tp, wdev, gmax, divisor, bw, st);
   }
   set_error("smoothing radius %d not supported (1..%d)", tp.r, kMaxRadius);
   return KCCOT_EUNSUPPORTED;
 }
-int make_taps(Taps* tp, const float* w, int radius, const char* what) {
+// w: host weights, copied into the kernel arguments, or (on_device) a device array the kernels read as wdev
+int make_taps(Taps* tp, const float* w, int radius, const char* what, bool on_device = false) {
   KCCOT_CHECK_ARG(w != nullptr, "%s: null weights", what);
+  KCCOT_CHECK_ARG(!on_device || (reinterpret_cast<uintptr_t>(w) & 3) == 0, "%s: device weights must be 4-byte aligned",
+                  what);
   if (radius < 1 || radius > kMaxRadius) {
     set_error("%s: smoothing radius %d not supported (kernel sizes 2..%d, radius 1..%d)", what, radius, 2 * kMaxRadius + 1,
               kMaxRadius);
     return KCCOT_EUNSUPPORTED;
   }
   tp->r = radius;
-  for (int k = 0; k < 2 * kMaxRadius + 1; ++k) tp->w[k] = k < 2 * radius + 1 ? w[k] : 0.f;
+  for (int k = 0; k < 2 * kMaxRadius + 1; ++k) tp->w[k] = !on_device && k < 2 * radius + 1 ? w[k] : 0.f;
   return KCCOT_OK;
 }
 
 // run_axis for the bf16 passes (TI / TO as in axis_col_bf16_kernel; MODE 2 passes write nothing and take TO = uint16_t)
 template <typename TI, typename TO, int MODE, int R>
-int run_axis_bf16_r(const TI* in, TO* out, const AxisPlan& p, const Taps& tp, float* gmax, const float* divisor,
-                    Ties tie, cudaStream_t st) {
+int run_axis_bf16_r(const TI* in, TO* out, const AxisPlan& p, const Taps& tp, const float* wdev, float* gmax,
+                    const float* divisor, Ties tie, cudaStream_t st) {
   if (p.tiled) {
     const int ni = p.n * (int)p.inner;
     const int threads = (ni + 31) / 32 * 32;
     const unsigned grid = (unsigned)((p.outer + p.o_chunk - 1) / p.o_chunk);
     const size_t smem = (size_t)p.o_chunk * ni * sizeof(float);
     axis_tile_bf16_kernel<TI, TO, MODE, R><<<grid, threads, smem, st>>>(in, out, p.outer, p.n, (int)p.inner, p.o_chunk,
-                                                                       tp, gmax, divisor, tie);
+                                                                       tp, wdev, gmax, divisor, tie);
   } else {
     // widest access the shape and pointers allow, but 4 instead of 8 elements per thread while 8 would leave fewer
     // than ~1 000 threads per SM (config 3's T pass: 98 304 threads at 8, 196 608 at 4)
@@ -620,34 +642,34 @@ int run_axis_bf16_r(const TI* in, TO* out, const AxisPlan& p, const Taps& tp, fl
                          : v == 4 ? axis_col_bf16_kernel<TI, TO, MODE, 4, R> : axis_col_bf16_kernel<TI, TO, MODE, 1, R>;
     if (smem > 48 * 1024)
       KCCOT_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kernel<<<grid, FT, smem, st>>>(in, out, p.outer, p.n, p.inner, tp, gmax, divisor, tie);
+    kernel<<<grid, FT, smem, st>>>(in, out, p.outer, p.n, p.inner, tp, wdev, gmax, divisor, tie);
   }
   KCCOT_LAUNCH_CHECK();
   return KCCOT_OK;
 }
 template <typename TI, typename TO, int MODE>
-int run_axis_bf16(const TI* in, TO* out, const AxisPlan& p, const Taps& tp, float* gmax, const float* divisor, Ties tie,
-                  cudaStream_t st) {
+int run_axis_bf16(const TI* in, TO* out, const AxisPlan& p, const Taps& tp, const float* wdev, float* gmax,
+                  const float* divisor, Ties tie, cudaStream_t st) {
   switch (tp.r) {
-    case 1: return run_axis_bf16_r<TI, TO, MODE, 1>(in, out, p, tp, gmax, divisor, tie, st);
-    case 2: return run_axis_bf16_r<TI, TO, MODE, 2>(in, out, p, tp, gmax, divisor, tie, st);
-    case 3: return run_axis_bf16_r<TI, TO, MODE, 3>(in, out, p, tp, gmax, divisor, tie, st);
-    case 4: return run_axis_bf16_r<TI, TO, MODE, 4>(in, out, p, tp, gmax, divisor, tie, st);
-    case 5: return run_axis_bf16_r<TI, TO, MODE, 5>(in, out, p, tp, gmax, divisor, tie, st);
-    case 6: return run_axis_bf16_r<TI, TO, MODE, 6>(in, out, p, tp, gmax, divisor, tie, st);
+    case 1: return run_axis_bf16_r<TI, TO, MODE, 1>(in, out, p, tp, wdev, gmax, divisor, tie, st);
+    case 2: return run_axis_bf16_r<TI, TO, MODE, 2>(in, out, p, tp, wdev, gmax, divisor, tie, st);
+    case 3: return run_axis_bf16_r<TI, TO, MODE, 3>(in, out, p, tp, wdev, gmax, divisor, tie, st);
+    case 4: return run_axis_bf16_r<TI, TO, MODE, 4>(in, out, p, tp, wdev, gmax, divisor, tie, st);
+    case 5: return run_axis_bf16_r<TI, TO, MODE, 5>(in, out, p, tp, wdev, gmax, divisor, tie, st);
+    case 6: return run_axis_bf16_r<TI, TO, MODE, 6>(in, out, p, tp, wdev, gmax, divisor, tie, st);
   }
   set_error("smoothing radius %d not supported (1..%d)", tp.r, kMaxRadius);
   return KCCOT_EUNSUPPORTED;
 }
 
-// argument checks of the bf16 entries: those of kccot_smooth_fwd, all made before any CUDA call
-int smooth_bf16_args(int mode, int B, int H, int T, int W, int C, const float* taps_t, int radius_t,
-                     const float* taps_s, int radius_s, void* ws, size_t ws_bytes, Taps* tp) {
+// argument checks of the bf16 and the device-weight entries: those of kccot_smooth_fwd, all made before any CUDA call
+int smooth_args(int mode, int B, int H, int T, int W, int C, const float* taps_t, int radius_t, const float* taps_s,
+                int radius_s, bool taps_on_device, void* ws, size_t ws_bytes, Taps* tp) {
   KCCOT_CHECK_ARG(B >= 1 && H >= 1 && T >= 1 && W >= 1 && C >= 1, "bad sizes");
   KCCOT_CHECK_ARG(T <= kMaxAxis && H <= kMaxAxis && W <= kMaxAxis, "axis longer than %d not supported (H=%d T=%d W=%d)", kMaxAxis,
                   H, T, W);
-  if (int rc = mode == 1 ? make_taps(tp, taps_t, radius_t, "temporal_convolution") : make_taps(tp, taps_s, radius_s,
-                                                                                            "gaussian_convolution3D"))
+  if (int rc = mode == 1 ? make_taps(tp, taps_t, radius_t, "temporal_convolution", taps_on_device)
+                          : make_taps(tp, taps_s, radius_s, "gaussian_convolution3D", taps_on_device))
     return rc;
   KCCOT_CHECK_ARG(T > tp->r, "REFLECT padding by %d needs T > %d (T=%d)", tp->r, tp->r, T);
   if (mode == 3) {
@@ -655,6 +677,102 @@ int smooth_bf16_args(int mode, int B, int H, int T, int W, int C, const float* t
     KCCOT_CHECK_ARG(ws && ws_bytes >= kccot_smooth_workspace_bytes(mode, B, H, T, W, C), "workspace too small");
   }
   return KCCOT_OK;
+}
+
+// The passes of the four fp32 / bf16 entries, after their argument checks.  wdev == nullptr: the weights are tp.w
+// (host arrays, the existing entries); otherwise the 2 * tp.r + 1 floats at wdev (the *_dev entries).
+int smooth_fwd_f32(int mode, const float* x, int B, int H, int T, int W, int C, const Taps& tp, const float* wdev,
+                   float* out, float* maxval, void* ws, size_t ws_bytes, cudaStream_t st) {
+  init_max_kernel<<<1, 1, 0, st>>>(maxval);
+  KCCOT_LAUNCH_CHECK();
+  const AxisPlan pt = plan_axis((long long)B * H, T, (long long)W * C);
+  BwdIn none{};
+  if (mode == 1) {
+    if (int rc = run_axis<2>(x, nullptr, pt, tp, wdev, maxval, nullptr, none, st)) return rc;
+    return run_axis<1 | 4>(x, out, pt, tp, wdev, nullptr, maxval, none, st);
+  }
+  KCCOT_CHECK_ARG(H > tp.r && W > tp.r, "3-D smoothing needs H, W > %d (H=%d W=%d)", tp.r, H, W);
+  const size_t n = align_up((size_t)B * H * T * W * C * sizeof(float), 256);
+  KCCOT_CHECK_ARG(ws && ws_bytes >= 256 + 2 * n, "workspace too small");
+  float* t1 = (float*)((char*)ws + 256);
+  float* t2 = (float*)((char*)ws + 256 + n);
+  const AxisPlan ph = plan_axis(B, H, (long long)T * W * C);
+  const AxisPlan pw = plan_axis((long long)B * H * T, W, C);
+  if (int rc = run_axis<1>(x, t1, ph, tp, wdev, nullptr, nullptr, none, st)) return rc;
+  if (int rc = run_axis<1>(t1, t2, pt, tp, wdev, nullptr, nullptr, none, st)) return rc;
+  if (int rc = run_axis<2>(t2, nullptr, pw, tp, wdev, maxval, nullptr, none, st)) return rc;
+  return run_axis<1 | 4>(t2, out, pw, tp, wdev, nullptr, maxval, none, st);
+}
+
+int smooth_bwd_f32(int mode, const float* gout, const float* out, const float* maxval, int B, int H, int T, int W,
+                   int C, const Taps& tp, const float* wdev, float* gx, void* ws, size_t ws_bytes, cudaStream_t st) {
+  const long long nel = (long long)B * H * T * W * C;
+  float* sums = (float*)ws;
+  KCCOT_CUDA(cudaMemsetAsync(sums, 0, 2 * sizeof(float), st));
+  tie_sums_kernel<<<(unsigned)min((long long)4 * num_sms(), (nel / 4 + FT - 1) / FT + 1), FT, 0, st>>>(gout, out, nel, sums);
+  KCCOT_LAUNCH_CHECK();
+  BwdIn bw{out, maxval, sums};
+  BwdIn none{};
+  const AxisPlan pt = plan_axis((long long)B * H, T, (long long)W * C);
+  if (mode == 1) return run_axis<1 | 8 | 16>(gout, gx, pt, tp, wdev, nullptr, nullptr, bw, st);
+  const size_t n = align_up((size_t)nel * sizeof(float), 256);
+  KCCOT_CHECK_ARG(ws_bytes >= 256 + 2 * n, "workspace too small");
+  float* t1 = (float*)((char*)ws + 256);
+  float* t2 = (float*)((char*)ws + 256 + n);
+  const AxisPlan ph = plan_axis(B, H, (long long)T * W * C);
+  const AxisPlan pw = plan_axis((long long)B * H * T, W, C);
+  if (int rc = run_axis<1 | 8 | 16>(gout, t1, pw, tp, wdev, nullptr, nullptr, bw, st)) return rc;
+  if (int rc = run_axis<1 | 16>(t1, t2, pt, tp, wdev, nullptr, nullptr, none, st)) return rc;
+  return run_axis<1 | 16>(t2, gx, ph, tp, wdev, nullptr, nullptr, none, st);
+}
+
+int smooth_fwd_bf16(int mode, const uint16_t* x, int B, int H, int T, int W, int C, const Taps& tp, const float* wdev,
+                    uint16_t* out, float* maxval, uint32_t* ties, void* ws, cudaStream_t st) {
+  KCCOT_CUDA(cudaMemsetAsync(ties, 0, kccot_smooth_ties_bytes(B, H, T, W, C), st));
+  init_max_kernel<<<1, 1, 0, st>>>(maxval);
+  KCCOT_LAUNCH_CHECK();
+  const AxisPlan pt = plan_axis((long long)B * H, T, (long long)W * C);
+  const Ties tie{ties, nullptr, nullptr};
+  if (mode == 1) {
+    if (int rc = run_axis_bf16<uint16_t, uint16_t, 2>(x, nullptr, pt, tp, wdev, maxval, nullptr, tie, st)) return rc;
+    return run_axis_bf16<uint16_t, uint16_t, 1 | 4>(x, out, pt, tp, wdev, nullptr, maxval, tie, st);
+  }
+  // mode 3: bf16 -> fp32 H pass, the fp32 T pass and W max pass, fp32 -> bf16 W pass
+  const size_t n = align_up((size_t)B * H * T * W * C * sizeof(float), 256);
+  float* t1 = (float*)((char*)ws + 256);
+  float* t2 = (float*)((char*)ws + 256 + n);
+  const AxisPlan ph = plan_axis(B, H, (long long)T * W * C);
+  const AxisPlan pw = plan_axis((long long)B * H * T, W, C);
+  BwdIn none{};
+  if (int rc = run_axis_bf16<uint16_t, float, 1>(x, t1, ph, tp, wdev, nullptr, nullptr, tie, st)) return rc;
+  if (int rc = run_axis<1>(t1, t2, pt, tp, wdev, nullptr, nullptr, none, st)) return rc;
+  if (int rc = run_axis<2>(t2, nullptr, pw, tp, wdev, maxval, nullptr, none, st)) return rc;
+  return run_axis_bf16<float, uint16_t, 1 | 4>(t2, out, pw, tp, wdev, nullptr, maxval, tie, st);
+}
+
+int smooth_bwd_bf16(int mode, const uint16_t* gout, const uint16_t* out, const float* maxval, const uint32_t* ties,
+                    int B, int H, int T, int W, int C, const Taps& tp, const float* wdev, uint16_t* gx, void* ws,
+                    cudaStream_t st) {
+  const long long nel = (long long)B * H * T * W * C;
+  const long long nwords = (nel + 31) / 32;
+  float* sums = (float*)ws;
+  KCCOT_CUDA(cudaMemsetAsync(sums, 0, 2 * sizeof(float), st));
+  tie_sums_bf16_kernel<<<(unsigned)min((long long)4 * num_sms(), (nel / 8 + FT - 1) / FT + 1), FT, 0, st>>>(
+      gout, out, ties, nel, nwords, sums);
+  KCCOT_LAUNCH_CHECK();
+  const Ties tie{const_cast<uint32_t*>(ties), maxval, sums};     // read only: MODE & 4 is not set in the backward
+  const AxisPlan pt = plan_axis((long long)B * H, T, (long long)W * C);
+  if (mode == 1) return run_axis_bf16<uint16_t, uint16_t, 1 | 8 | 16>(gout, gx, pt, tp, wdev, nullptr, nullptr, tie, st);
+  // mode 3: bf16 -> fp32 W pass with the tie transform, the fp32 T pass, fp32 -> bf16 H pass
+  const size_t n = align_up((size_t)nel * sizeof(float), 256);
+  float* t1 = (float*)((char*)ws + 256);
+  float* t2 = (float*)((char*)ws + 256 + n);
+  const AxisPlan ph = plan_axis(B, H, (long long)T * W * C);
+  const AxisPlan pw = plan_axis((long long)B * H * T, W, C);
+  BwdIn none{};
+  if (int rc = run_axis_bf16<uint16_t, float, 1 | 8 | 16>(gout, t1, pw, tp, wdev, nullptr, nullptr, tie, st)) return rc;
+  if (int rc = run_axis<1 | 16>(t1, t2, pt, tp, wdev, nullptr, nullptr, none, st)) return rc;
+  return run_axis_bf16<float, uint16_t, 1 | 16>(t2, gx, ph, tp, wdev, nullptr, nullptr, tie, st);
 }
 }  // namespace
 }  // namespace kccot
@@ -676,31 +794,12 @@ int kccot_smooth_fwd(int mode, const float* x, int B, int H, int T, int W, int C
   KCCOT_CHECK_ARG(B >= 1 && H >= 1 && T >= 1 && W >= 1 && C >= 1, "bad sizes");
   KCCOT_CHECK_ARG(T <= kMaxAxis && H <= kMaxAxis && W <= kMaxAxis, "axis longer than %d not supported (H=%d T=%d W=%d)", kMaxAxis,
                   H, T, W);
-  cudaStream_t st = (cudaStream_t)stream;
   Taps tp;
   if (int rc = mode == 1 ? make_taps(&tp, taps_t, radius_t, "temporal_convolution") : make_taps(&tp, taps_s, radius_s,
                                                                                              "gaussian_convolution3D"))
     return rc;
   KCCOT_CHECK_ARG(T > tp.r, "REFLECT padding by %d needs T > %d (T=%d)", tp.r, tp.r, T);
-  init_max_kernel<<<1, 1, 0, st>>>(maxval);
-  KCCOT_LAUNCH_CHECK();
-  const AxisPlan pt = plan_axis((long long)B * H, T, (long long)W * C);
-  BwdIn none{};
-  if (mode == 1) {
-    if (int rc = run_axis<2>(x, nullptr, pt, tp, maxval, nullptr, none, st)) return rc;
-    return run_axis<1 | 4>(x, out, pt, tp, nullptr, maxval, none, st);
-  }
-  KCCOT_CHECK_ARG(H > tp.r && W > tp.r, "3-D smoothing needs H, W > %d (H=%d W=%d)", tp.r, H, W);
-  const size_t n = align_up((size_t)B * H * T * W * C * sizeof(float), 256);
-  KCCOT_CHECK_ARG(ws && ws_bytes >= 256 + 2 * n, "workspace too small");
-  float* t1 = (float*)((char*)ws + 256);
-  float* t2 = (float*)((char*)ws + 256 + n);
-  const AxisPlan ph = plan_axis(B, H, (long long)T * W * C);
-  const AxisPlan pw = plan_axis((long long)B * H * T, W, C);
-  if (int rc = run_axis<1>(x, t1, ph, tp, nullptr, nullptr, none, st)) return rc;
-  if (int rc = run_axis<1>(t1, t2, pt, tp, nullptr, nullptr, none, st)) return rc;
-  if (int rc = run_axis<2>(t2, nullptr, pw, tp, maxval, nullptr, none, st)) return rc;
-  return run_axis<1 | 4>(t2, out, pw, tp, nullptr, maxval, none, st);
+  return smooth_fwd_f32(mode, x, B, H, T, W, C, tp, nullptr, out, maxval, ws, ws_bytes, (cudaStream_t)stream);
 }
 
 int kccot_smooth_bwd(int mode, const float* gout, const float* out, const float* maxval, int B, int H, int T, int W,
@@ -708,29 +807,30 @@ int kccot_smooth_bwd(int mode, const float* gout, const float* out, const float*
                      size_t ws_bytes, void* stream) {
   KCCOT_CHECK_ARG(mode == 1 || mode == 3, "smoothing mode must be 1 or 3");
   KCCOT_CHECK_ARG(gout && out && maxval && gx && ws && ws_bytes >= 256, "null pointer / workspace");
-  cudaStream_t st = (cudaStream_t)stream;
   Taps tp;
   if (int rc = mode == 1 ? make_taps(&tp, taps_t, radius_t, "temporal_convolution") : make_taps(&tp, taps_s, radius_s,
                                                                                              "gaussian_convolution3D"))
     return rc;
-  const long long nel = (long long)B * H * T * W * C;
-  float* sums = (float*)ws;
-  KCCOT_CUDA(cudaMemsetAsync(sums, 0, 2 * sizeof(float), st));
-  tie_sums_kernel<<<(unsigned)min((long long)4 * num_sms(), (nel / 4 + FT - 1) / FT + 1), FT, 0, st>>>(gout, out, nel, sums);
-  KCCOT_LAUNCH_CHECK();
-  BwdIn bw{out, maxval, sums};
-  BwdIn none{};
-  const AxisPlan pt = plan_axis((long long)B * H, T, (long long)W * C);
-  if (mode == 1) return run_axis<1 | 8 | 16>(gout, gx, pt, tp, nullptr, nullptr, bw, st);
-  const size_t n = align_up((size_t)nel * sizeof(float), 256);
-  KCCOT_CHECK_ARG(ws_bytes >= 256 + 2 * n, "workspace too small");
-  float* t1 = (float*)((char*)ws + 256);
-  float* t2 = (float*)((char*)ws + 256 + n);
-  const AxisPlan ph = plan_axis(B, H, (long long)T * W * C);
-  const AxisPlan pw = plan_axis((long long)B * H * T, W, C);
-  if (int rc = run_axis<1 | 8 | 16>(gout, t1, pw, tp, nullptr, nullptr, bw, st)) return rc;
-  if (int rc = run_axis<1 | 16>(t1, t2, pt, tp, nullptr, nullptr, none, st)) return rc;
-  return run_axis<1 | 16>(t2, gx, ph, tp, nullptr, nullptr, none, st);
+  return smooth_bwd_f32(mode, gout, out, maxval, B, H, T, W, C, tp, nullptr, gx, ws, ws_bytes, (cudaStream_t)stream);
+}
+
+int kccot_smooth_fwd_dev(int mode, const float* x, int B, int H, int T, int W, int C, const float* taps_dev, int radius,
+                         float* out, float* maxval, void* ws, size_t ws_bytes, void* stream) {
+  KCCOT_CHECK_ARG(mode == 1 || mode == 3, "smoothing mode must be 1 (temporal) or 3 (3-D); the reference's '2d' "
+                                          "branch raises (data_utils.py:537-538)");
+  KCCOT_CHECK_ARG(x && out && maxval, "null pointer");
+  Taps tp;
+  if (int rc = smooth_args(mode, B, H, T, W, C, taps_dev, radius, taps_dev, radius, true, ws, ws_bytes, &tp)) return rc;
+  return smooth_fwd_f32(mode, x, B, H, T, W, C, tp, taps_dev, out, maxval, ws, ws_bytes, (cudaStream_t)stream);
+}
+
+int kccot_smooth_bwd_dev(int mode, const float* gout, const float* out, const float* maxval, int B, int H, int T, int W,
+                         int C, const float* taps_dev, int radius, float* gx, void* ws, size_t ws_bytes, void* stream) {
+  KCCOT_CHECK_ARG(mode == 1 || mode == 3, "smoothing mode must be 1 or 3");
+  KCCOT_CHECK_ARG(gout && out && maxval && gx && ws && ws_bytes >= 256, "null pointer / workspace");
+  Taps tp;
+  if (int rc = smooth_args(mode, B, H, T, W, C, taps_dev, radius, taps_dev, radius, true, ws, ws_bytes, &tp)) return rc;
+  return smooth_bwd_f32(mode, gout, out, maxval, B, H, T, W, C, tp, taps_dev, gx, ws, ws_bytes, (cudaStream_t)stream);
 }
 
 size_t kccot_smooth_ties_bytes(int B, int H, int T, int W, int C) {
@@ -747,28 +847,8 @@ int kccot_smooth_fwd_bf16(int mode, const uint16_t* x, int B, int H, int T, int 
   KCCOT_CHECK_ARG(x && out && maxval && ties, "null pointer");
   KCCOT_CHECK_ARG((reinterpret_cast<uintptr_t>(ties) & 3) == 0, "tie mask must be 4-byte aligned");
   Taps tp;
-  if (int rc = smooth_bf16_args(mode, B, H, T, W, C, taps_t, radius_t, taps_s, radius_s, ws, ws_bytes, &tp)) return rc;
-  cudaStream_t st = (cudaStream_t)stream;
-  KCCOT_CUDA(cudaMemsetAsync(ties, 0, kccot_smooth_ties_bytes(B, H, T, W, C), st));
-  init_max_kernel<<<1, 1, 0, st>>>(maxval);
-  KCCOT_LAUNCH_CHECK();
-  const AxisPlan pt = plan_axis((long long)B * H, T, (long long)W * C);
-  const Ties tie{ties, nullptr, nullptr};
-  if (mode == 1) {
-    if (int rc = run_axis_bf16<uint16_t, uint16_t, 2>(x, nullptr, pt, tp, maxval, nullptr, tie, st)) return rc;
-    return run_axis_bf16<uint16_t, uint16_t, 1 | 4>(x, out, pt, tp, nullptr, maxval, tie, st);
-  }
-  // mode 3: bf16 -> fp32 H pass, the fp32 T pass and W max pass, fp32 -> bf16 W pass
-  const size_t n = align_up((size_t)B * H * T * W * C * sizeof(float), 256);
-  float* t1 = (float*)((char*)ws + 256);
-  float* t2 = (float*)((char*)ws + 256 + n);
-  const AxisPlan ph = plan_axis(B, H, (long long)T * W * C);
-  const AxisPlan pw = plan_axis((long long)B * H * T, W, C);
-  BwdIn none{};
-  if (int rc = run_axis_bf16<uint16_t, float, 1>(x, t1, ph, tp, nullptr, nullptr, tie, st)) return rc;
-  if (int rc = run_axis<1>(t1, t2, pt, tp, nullptr, nullptr, none, st)) return rc;
-  if (int rc = run_axis<2>(t2, nullptr, pw, tp, maxval, nullptr, none, st)) return rc;
-  return run_axis_bf16<float, uint16_t, 1 | 4>(t2, out, pw, tp, nullptr, maxval, tie, st);
+  if (int rc = smooth_args(mode, B, H, T, W, C, taps_t, radius_t, taps_s, radius_s, false, ws, ws_bytes, &tp)) return rc;
+  return smooth_fwd_bf16(mode, x, B, H, T, W, C, tp, nullptr, out, maxval, ties, ws, (cudaStream_t)stream);
 }
 
 int kccot_smooth_bwd_bf16(int mode, const uint16_t* gout, const uint16_t* out, const float* maxval,
@@ -778,28 +858,31 @@ int kccot_smooth_bwd_bf16(int mode, const uint16_t* gout, const uint16_t* out, c
   KCCOT_CHECK_ARG(gout && out && maxval && ties && gx && ws && ws_bytes >= 256, "null pointer / workspace");
   KCCOT_CHECK_ARG((reinterpret_cast<uintptr_t>(ties) & 3) == 0, "tie mask must be 4-byte aligned");
   Taps tp;
-  if (int rc = smooth_bf16_args(mode, B, H, T, W, C, taps_t, radius_t, taps_s, radius_s, ws, ws_bytes, &tp)) return rc;
-  cudaStream_t st = (cudaStream_t)stream;
-  const long long nel = (long long)B * H * T * W * C;
-  const long long nwords = (nel + 31) / 32;
-  float* sums = (float*)ws;
-  KCCOT_CUDA(cudaMemsetAsync(sums, 0, 2 * sizeof(float), st));
-  tie_sums_bf16_kernel<<<(unsigned)min((long long)4 * num_sms(), (nel / 8 + FT - 1) / FT + 1), FT, 0, st>>>(
-      gout, out, ties, nel, nwords, sums);
-  KCCOT_LAUNCH_CHECK();
-  const Ties tie{const_cast<uint32_t*>(ties), maxval, sums};     // read only: MODE & 4 is not set in the backward
-  const AxisPlan pt = plan_axis((long long)B * H, T, (long long)W * C);
-  if (mode == 1) return run_axis_bf16<uint16_t, uint16_t, 1 | 8 | 16>(gout, gx, pt, tp, nullptr, nullptr, tie, st);
-  // mode 3: bf16 -> fp32 W pass with the tie transform, the fp32 T pass, fp32 -> bf16 H pass
-  const size_t n = align_up((size_t)nel * sizeof(float), 256);
-  float* t1 = (float*)((char*)ws + 256);
-  float* t2 = (float*)((char*)ws + 256 + n);
-  const AxisPlan ph = plan_axis(B, H, (long long)T * W * C);
-  const AxisPlan pw = plan_axis((long long)B * H * T, W, C);
-  BwdIn none{};
-  if (int rc = run_axis_bf16<uint16_t, float, 1 | 8 | 16>(gout, t1, pw, tp, nullptr, nullptr, tie, st)) return rc;
-  if (int rc = run_axis<1 | 16>(t1, t2, pt, tp, nullptr, nullptr, none, st)) return rc;
-  return run_axis_bf16<float, uint16_t, 1 | 16>(t2, gx, ph, tp, nullptr, nullptr, tie, st);
+  if (int rc = smooth_args(mode, B, H, T, W, C, taps_t, radius_t, taps_s, radius_s, false, ws, ws_bytes, &tp)) return rc;
+  return smooth_bwd_bf16(mode, gout, out, maxval, ties, B, H, T, W, C, tp, nullptr, gx, ws, (cudaStream_t)stream);
+}
+
+int kccot_smooth_fwd_bf16_dev(int mode, const uint16_t* x, int B, int H, int T, int W, int C, const float* taps_dev,
+                              int radius, uint16_t* out, float* maxval, uint32_t* ties, void* ws, size_t ws_bytes,
+                              void* stream) {
+  KCCOT_CHECK_ARG(mode == 1 || mode == 3, "smoothing mode must be 1 (temporal) or 3 (3-D); the reference's '2d' "
+                                          "branch raises (data_utils.py:537-538)");
+  KCCOT_CHECK_ARG(x && out && maxval && ties, "null pointer");
+  KCCOT_CHECK_ARG((reinterpret_cast<uintptr_t>(ties) & 3) == 0, "tie mask must be 4-byte aligned");
+  Taps tp;
+  if (int rc = smooth_args(mode, B, H, T, W, C, taps_dev, radius, taps_dev, radius, true, ws, ws_bytes, &tp)) return rc;
+  return smooth_fwd_bf16(mode, x, B, H, T, W, C, tp, taps_dev, out, maxval, ties, ws, (cudaStream_t)stream);
+}
+
+int kccot_smooth_bwd_bf16_dev(int mode, const uint16_t* gout, const uint16_t* out, const float* maxval,
+                              const uint32_t* ties, int B, int H, int T, int W, int C, const float* taps_dev, int radius,
+                              uint16_t* gx, void* ws, size_t ws_bytes, void* stream) {
+  KCCOT_CHECK_ARG(mode == 1 || mode == 3, "smoothing mode must be 1 or 3");
+  KCCOT_CHECK_ARG(gout && out && maxval && ties && gx && ws && ws_bytes >= 256, "null pointer / workspace");
+  KCCOT_CHECK_ARG((reinterpret_cast<uintptr_t>(ties) & 3) == 0, "tie mask must be 4-byte aligned");
+  Taps tp;
+  if (int rc = smooth_args(mode, B, H, T, W, C, taps_dev, radius, taps_dev, radius, true, ws, ws_bytes, &tp)) return rc;
+  return smooth_bwd_bf16(mode, gout, out, maxval, ties, B, H, T, W, C, tp, taps_dev, gx, ws, (cudaStream_t)stream);
 }
 
 }  // extern "C"

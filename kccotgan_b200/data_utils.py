@@ -6,11 +6,36 @@ schedules of the reference's data_utils are out of scope (SURVEY.md §2).
 The convolutions take CUDA fp32 or bf16 videos and return the input's dtype.  A bf16 video is smoothed by bf16
 kernels with fp32 arithmetic inside: the output is the fp32 output on the widened video rounded to nearest even, and
 the gradient is bf16 (kccot_smooth_fwd_bf16 / _bwd_bf16 in include/kccot.h).  Any other dtype raises ValueError.
+
+`sigma` is a number, or a SmoothingTaps: a device buffer of weights that the kernels read when they run, so that a
+CUDA graph captured with it follows an annealed sigma (the sigma changes between replays, the graph does not).
 """
 import numpy as np
 import torch
 
 from .functional import SmoothFn, _check_video
+
+
+class SmoothingTaps:
+    """The 2r+1 Gaussian weights of one radius in a fixed-address device buffer, for the convolutions of a captured
+    CUDA graph whose sigma changes between replays:
+
+        taps = SmoothingTaps(ks.temporal_radius).set(5.0)
+        (capture ks.temporal_convolution(x, taps) and its backward into a graph g)
+        taps.set(ks.annealing_sigma(5.0, it)); g.replay()
+
+    .set(sigma) writes KernelSmoothing._weights(radius, sigma), the host fp32 weights a float sigma uses, so the result
+    is the float-sigma call's at the same sigma.  It is ordered on the current stream and does not synchronise the
+    host (a pinned source copied with non_blocking=True)."""
+
+    def __init__(self, radius, device="cuda"):
+        self.radius = int(radius)
+        self.weights = torch.zeros(2 * self.radius + 1, dtype=torch.float32, device=device)
+
+    def set(self, sigma):
+        w = torch.from_numpy(KernelSmoothing._weights(self.radius, sigma))
+        self.weights.copy_(w.pin_memory() if self.weights.is_cuda else w, non_blocking=True)
+        return self
 
 
 class KernelSmoothing:
@@ -49,11 +74,22 @@ class KernelSmoothing:
         if n <= radius:
             raise ValueError(f"REFLECT padding by {radius} needs the {name} axis longer than {radius}, got {n}")
 
+    @staticmethod
+    def _taps(radius, sigma):
+        """the weights SmoothFn takes: a SmoothingTaps of this radius, or the host weights of a number"""
+        if isinstance(sigma, SmoothingTaps):
+            if sigma.radius != radius:
+                raise ValueError(f"SmoothingTaps of radius {sigma.radius} for a filter of radius {radius}")
+            return sigma
+        return tuple(KernelSmoothing._weights(radius, sigma))
+
     def temporal_convolution(self, inputs, sigma):
-        """data_utils.py:503-521 — (2r+1)-tap REFLECT filter along T, / global max."""
+        """data_utils.py:503-521 — (2r+1)-tap REFLECT filter along T, / global max.  `sigma`: a number or a
+        SmoothingTaps of radius temporal_radius."""
+        taps = self._taps(self.temporal_radius, sigma)
         inputs = _check_video(inputs, "inputs", 5)
         self._check_axis("T", inputs.shape[2], self.temporal_radius)
-        return SmoothFn.apply(inputs, 1, tuple(self._weights(self.temporal_radius, sigma)), None)
+        return SmoothFn.apply(inputs, 1, taps, None)
 
     def spatial_convolution(self, inputs, sigma):
         """data_utils.py:523-550 — BROKEN in the reference: the VALID conv2d shrinks H, W by 2r and the
@@ -66,12 +102,14 @@ class KernelSmoothing:
 
     def gaussian_convolution3D(self, inputs, sigma):
         """data_utils.py:552-582 — (2r+1)^3 REFLECT filter over (H,T,W) per channel (three separable
-        passes), / global max.  Uses the SPATIAL radius for all three axes (:553,562-564)."""
+        passes), / global max.  Uses the SPATIAL radius for all three axes (:553,562-564).  `sigma`: a number or a
+        SmoothingTaps of radius spatial_radius."""
+        taps = self._taps(self.spatial_radius, sigma)
         inputs = _check_video(inputs, "inputs", 5)
         _, H, T, W, _ = inputs.shape
         for name, n in (("H", H), ("T", T), ("W", W)):
             self._check_axis(name, n, self.spatial_radius)
-        return SmoothFn.apply(inputs, 3, None, tuple(self._weights(self.spatial_radius, sigma)))
+        return SmoothFn.apply(inputs, 3, None, taps)
 
     def annealing_sigma(self, init_sigma, step, decay_steps=500, decay_rate=0.975):
         """data_utils.py:584-586."""

@@ -441,10 +441,22 @@ def _taps(w):
 
 class SmoothFn(torch.autograd.Function):
     """mode 1: `taps_t` filters T; mode 3: `taps_s` filters H, T and W.  The weights are host sequences (they become
-    kernel arguments: nothing is copied to the device, so an annealed sigma costs nothing per step).
+    kernel arguments: nothing is copied to the device, so an annealed sigma costs nothing per step), or a
+    data_utils.SmoothingTaps, whose device buffer the kernels read when they run (the *_dev entry points): a captured
+    graph then follows its .set().  The forward snapshots that buffer (a device-to-device copy, capturable) and the
+    backward filters with the snapshot, so a .set() between the two cannot change the gradient.
     A bf16 x runs kccot_smooth_fwd_bf16 / _bwd_bf16: output and gradient are bf16, and the tie mask of the forward (the
     elements at the maximum, which the bf16 output cannot tell apart from values just below it) is saved for the
     backward."""
+
+    @staticmethod
+    def _weights(ctx, taps_t, taps_s):
+        """-> (entry-point suffix, weight arguments) for the taps saved on ctx"""
+        if ctx.taps_dev is not None:
+            return "_dev", (_ptr(ctx.taps_dev), ctx.radius)
+        at, rt = _taps(taps_t)
+        as_, rs = _taps(taps_s)
+        return "", (at, rt, as_, rs)
 
     @staticmethod
     def forward(ctx, x, mode, taps_t, taps_s):
@@ -453,19 +465,25 @@ class SmoothFn(torch.autograd.Function):
         B, H, T, W, C = x.shape
         dev = x.device
         lib = _lib.load()
+        from .data_utils import SmoothingTaps
+        taps = taps_t if mode == 1 else taps_s
+        ctx.taps_dev = None
+        if isinstance(taps, SmoothingTaps):
+            if taps.weights.device != dev:
+                raise ValueError(f"taps: the weights are on {taps.weights.device}, the video on {dev}")
+            ctx.taps_dev, ctx.radius = taps.weights.clone(), taps.radius
         out = torch.empty_like(x)
         maxval = torch.empty((1,), dtype=torch.float32, device=dev)
         ws = _ws(lib.kccot_smooth_workspace_bytes(mode, B, H, T, W, C), dev)
-        at, rt = _taps(taps_t)
-        as_, rs = _taps(taps_s)
+        suffix, wargs = SmoothFn._weights(ctx, taps_t, taps_s)
         with _on_device(dev):
             if bf16:
                 ties = torch.empty(lib.kccot_smooth_ties_bytes(B, H, T, W, C) // 4, dtype=torch.int32, device=dev)
-                _lib.call("kccot_smooth_fwd_bf16", mode, _ptr(x), B, H, T, W, C, at, rt, as_, rs, _ptr(out), _ptr(maxval),
-                          _ptr(ties), _ptr(ws), ws.numel(), _stream(dev))
+                _lib.call("kccot_smooth_fwd_bf16" + suffix, mode, _ptr(x), B, H, T, W, C, *wargs, _ptr(out),
+                          _ptr(maxval), _ptr(ties), _ptr(ws), ws.numel(), _stream(dev))
                 ctx.save_for_backward(out, maxval, ties)
             else:
-                _lib.call("kccot_smooth_fwd", mode, _ptr(x), B, H, T, W, C, at, rt, as_, rs, _ptr(out), _ptr(maxval),
+                _lib.call("kccot_smooth_fwd" + suffix, mode, _ptr(x), B, H, T, W, C, *wargs, _ptr(out), _ptr(maxval),
                           _ptr(ws), ws.numel(), _stream(dev))
                 ctx.save_for_backward(out, maxval)
         ctx.mode, ctx.taps = mode, (taps_t, taps_s)
@@ -479,13 +497,12 @@ class SmoothFn(torch.autograd.Function):
         gout = gout.contiguous().to(out.dtype)
         gx = torch.empty_like(out)
         ws = _ws(_lib.load().kccot_smooth_workspace_bytes(ctx.mode, B, H, T, W, C), dev)
-        at, rt = _taps(ctx.taps[0])
-        as_, rs = _taps(ctx.taps[1])
+        suffix, wargs = SmoothFn._weights(ctx, *ctx.taps)
         with _on_device(dev):
             if ties:
-                _lib.call("kccot_smooth_bwd_bf16", ctx.mode, _ptr(gout), _ptr(out), _ptr(maxval), _ptr(ties[0]), B, H, T,
-                          W, C, at, rt, as_, rs, _ptr(gx), _ptr(ws), ws.numel(), _stream(dev))
+                _lib.call("kccot_smooth_bwd_bf16" + suffix, ctx.mode, _ptr(gout), _ptr(out), _ptr(maxval),
+                          _ptr(ties[0]), B, H, T, W, C, *wargs, _ptr(gx), _ptr(ws), ws.numel(), _stream(dev))
             else:
-                _lib.call("kccot_smooth_bwd", ctx.mode, _ptr(gout), _ptr(out), _ptr(maxval), B, H, T, W, C, at, rt, as_,
-                          rs, _ptr(gx), _ptr(ws), ws.numel(), _stream(dev))
+                _lib.call("kccot_smooth_bwd" + suffix, ctx.mode, _ptr(gout), _ptr(out), _ptr(maxval), B, H, T, W, C,
+                          *wargs, _ptr(gx), _ptr(ws), ws.numel(), _stream(dev))
         return gx, None, None, None

@@ -13,7 +13,7 @@ import torch
 from torch import nn
 
 from . import gan_utils
-from .data_utils import KernelSmoothing
+from .data_utils import KernelSmoothing, SmoothingTaps
 
 
 class StubGenerator(nn.Module):
@@ -59,17 +59,22 @@ class StubDiscriminator(nn.Module):
         return torch.sigmoid(torch.cumsum(feat, dim=1) / steps)
 
 
+def _kernel_smoothing():
+    return KernelSmoothing(temporal_kernel_size=6, spatial_kernel_size=6)                  # kernel_train.py:216
+
+
 def make_training_steps(generator, discriminator_h, discriminator_m, batch_size, scaling_coef=1.0 / 15.0,
                         sinkhorn_eps=0.8, sinkhorn_l=100, reg_penalty=1.0, kernel_choice="none", gen_lr=1e-4,
                         disc_lr=1e-4, seed=1, capturable=False):
     """Returns (disc_training_step, gen_training_step), each `(real_in, real_pred, sigma) -> scalar tensor`,
-    mirroring kernel_train.py:219-292 (Adam with beta_1 = 0.5, beta_2 = 0.9 as at :62-63; the LR schedule is the caller's)."""
+    mirroring kernel_train.py:219-292 (Adam with beta_1 = 0.5, beta_2 = 0.9 as at :62-63; the LR schedule is the caller's).
+    `sigma` is a number or a data_utils.SmoothingTaps of the smoothing's radius (3)."""
     # capturable=True: the variant GraphedTrainingIteration records into a CUDA graph (Adam keeps its step count on
     # the device, the noise comes from the default CUDA generator, which graphs know how to advance)
     gen_opt = torch.optim.Adam(generator.parameters(), lr=gen_lr, betas=(0.5, 0.9), capturable=capturable)
     dischm_opt = torch.optim.Adam(list(discriminator_h.parameters()) + list(discriminator_m.parameters()), lr=disc_lr,
                                   betas=(0.5, 0.9), capturable=capturable)
-    gaussian_kernel = KernelSmoothing(temporal_kernel_size=6, spatial_kernel_size=6)      # kernel_train.py:216
+    gaussian_kernel = _kernel_smoothing()
     dev = next(generator.parameters()).device
     noise = torch.Generator(device=dev)
     noise.manual_seed(seed)
@@ -125,11 +130,11 @@ class GraphedTrainingIteration:
 
         it = GraphedTrainingIteration(gen, disc_h, disc_m, real_in_example, real_pred_example)
         it.real_in.copy_(x[:, :, :ctx]); it.real_pred.copy_(x[:, :, ctx:])
-        loss, pm = it.step()
+        loss, pm = it.step()                   # or it.step(sigma), e.g. sigma = annealing_sigma(init_sig, iteration)
 
-    Static-buffer contract as in graphed.GraphedSinkhornLoss.  `sigma` is fixed at capture time (the smoothing taps
-    are kernel arguments): use it with `kernel_choice="none"` or a constant sigma; an annealed sigma needs the eager
-    steps (or one capture per sigma)."""
+    Static-buffer contract as in graphed.GraphedSinkhornLoss.  With `kernel_choice` "1d" / "3d" the smoothing reads its
+    weights from a data_utils.SmoothingTaps captured with the graph: step(sigma) writes the weights of `sigma` there
+    before the replay (kernel_train.py's annealed sigma, :308-311), and step() replays the constructor's `sigma`."""
 
     def __init__(self, generator, discriminator_h, discriminator_m, real_in, real_pred, sigma=5.0, warmup=3, **kw):
         self.real_in = real_in.detach().clone()
@@ -137,6 +142,14 @@ class GraphedTrainingIteration:
         dev = self.real_in.device
         self._disc, self._gen = make_training_steps(generator, discriminator_h, discriminator_m, real_in.shape[0],
                                                     capturable=True, **kw)
+        self.sigma = self._sigma_set = sigma
+        self.taps = None
+        kernel_choice = kw.get("kernel_choice", "none")
+        if kernel_choice in ("1d", "3d"):
+            ks = _kernel_smoothing()
+            self.taps = SmoothingTaps(ks.temporal_radius if kernel_choice == "1d" else ks.spatial_radius,
+                                      device=dev).set(sigma)
+            sigma = self.taps
         side = torch.cuda.Stream(device=dev)
         side.wait_stream(torch.cuda.current_stream(dev))
         with torch.cuda.stream(side):                    # optimiser state and library attributes come to life here
@@ -150,6 +163,11 @@ class GraphedTrainingIteration:
             self.pm = self._disc(self.real_in, self.real_pred, sigma)
             self.loss = self._gen(self.real_in, self.real_pred, sigma)
 
-    def step(self):
+    def step(self, sigma=None):
+        """One replay at `sigma` (None: the constructor's); without smoothing sigma is unused, as in the eager steps."""
+        sigma = self.sigma if sigma is None else sigma
+        if self.taps is not None and sigma != self._sigma_set:
+            self.taps.set(sigma)
+            self._sigma_set = sigma
         self.graph.replay()
         return self.loss, self.pm
