@@ -319,6 +319,35 @@ int kccot_smooth_bwd_bf16_dev(int mode, const uint16_t* gout, const uint16_t* ou
                               const uint32_t* ties, int B, int H, int T, int W, int C, const float* taps_dev,
                               int radius, uint16_t* gx, void* ws, size_t ws_bytes, void* stream);
 
+/* Batched independent problems — nprob videos [B,H,T,W,C] that lie contiguously as [nprob,B,H,T,W,C] (x, out, gout,
+ * gx), smoothed in one call: problem p is filtered with its own weights, row p of `taps_dev` [nprob, 2*radius+1] (fp32,
+ * device memory, 4-byte aligned, read when the kernels run, as in the *_dev entries), and divided by its own maximum,
+ * maxval[p] [nprob], which the forward writes and the backward reads.  Mode 1 filters T, mode 3 filters H, T and W.
+ * The workspace (kccot_smooth_batched_workspace_bytes, 16-byte aligned) holds 2*nprob tie sums, and in mode 3 two fp32
+ * intermediates of nprob*B*H*T*W*C floats; the forward needs it in mode 3 only, the backward always.  The _bf16 twins
+ * take bf16 x / out / gout / gx (raw bits, any alignment) and one caller-owned tie mask over the whole batch,
+ * kccot_smooth_ties_bytes(nprob*B, H, T, W, C) bytes, 4-byte aligned: bit (p*n + e) % 32 of word (p*n + e) / 32 marks
+ * element e of problem p (n = B*H*T*W*C), so a word may hold bits of two problems.  The forward zeroes it first.
+ * Contract, for each problem p against the *_dev twin called on problem p's video with weights row p: out[p], maxval[p]
+ * and the tie-mask bits of problem p are bit-identical; gx[p] is bit-identical outside the adjoint stencil of p's
+ * tied maxima, where both sides form S_p = sum(gout * out) with atomics in a run-dependent order.  A tie in one problem
+ * changes no other problem's numbers.  The argument checks are the twin's plus 1 <= nprob <= 65535 (KCCOT_EINVAL), all
+ * made before any CUDA call, with the twin's error codes.  Both calls are graph-capturable. */
+size_t kccot_smooth_batched_workspace_bytes(int mode, int nprob, int B, int H, int T, int W, int C);
+int kccot_smooth_batched_fwd(int mode, const float* x, int nprob, int B, int H, int T, int W, int C,
+                             const float* taps_dev, int radius, float* out, float* maxval, void* ws,
+                             size_t ws_bytes, void* stream);
+int kccot_smooth_batched_bwd(int mode, const float* gout, const float* out, const float* maxval, int nprob, int B,
+                             int H, int T, int W, int C, const float* taps_dev, int radius, float* gx, void* ws,
+                             size_t ws_bytes, void* stream);
+int kccot_smooth_batched_fwd_bf16(int mode, const uint16_t* x, int nprob, int B, int H, int T, int W, int C,
+                                  const float* taps_dev, int radius, uint16_t* out, float* maxval, uint32_t* ties,
+                                  void* ws, size_t ws_bytes, void* stream);
+int kccot_smooth_batched_bwd_bf16(int mode, const uint16_t* gout, const uint16_t* out, const float* maxval,
+                                  const uint32_t* ties, int nprob, int B, int H, int T, int W, int C,
+                                  const float* taps_dev, int radius, uint16_t* gx, void* ws, size_t ws_bytes,
+                                  void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -76,6 +76,11 @@ SIGNATURES = {
     "kccot_smooth_bwd_dev": (_I, [_I, _P, _P, _P, _I, _I, _I, _I, _I, _P, _I, _P, _P, _SZ, _P]),
     "kccot_smooth_fwd_bf16_dev": (_I, [_I, _P, _I, _I, _I, _I, _I, _P, _I, _P, _P, _P, _P, _SZ, _P]),
     "kccot_smooth_bwd_bf16_dev": (_I, [_I, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _I, _P, _P, _SZ, _P]),
+    "kccot_smooth_batched_workspace_bytes": (_SZ, [_I, _I, _I, _I, _I, _I, _I]),
+    "kccot_smooth_batched_fwd": (_I, [_I, _P, _I, _I, _I, _I, _I, _I, _P, _I, _P, _P, _P, _SZ, _P]),
+    "kccot_smooth_batched_bwd": (_I, [_I, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P, _I, _P, _P, _SZ, _P]),
+    "kccot_smooth_batched_fwd_bf16": (_I, [_I, _P, _I, _I, _I, _I, _I, _I, _P, _I, _P, _P, _P, _P, _SZ, _P]),
+    "kccot_smooth_batched_bwd_bf16": (_I, [_I, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P, _I, _P, _P, _SZ, _P]),
 }
 
 _lib = None

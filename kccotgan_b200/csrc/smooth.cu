@@ -17,6 +17,8 @@
 //                    and row offsets in registers and produces out[o][p][i] for every o of the block.
 // (The first version used one generic tile kernel with three integer divisions per element: 190 us for a
 //  37.7 MB tensor, 20x off the HBM roofline.)
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace kccot {
@@ -774,6 +776,406 @@ int smooth_bwd_bf16(int mode, const uint16_t* gout, const uint16_t* out, const f
   if (int rc = run_axis<1 | 16>(t1, t2, pt, tp, wdev, nullptr, nullptr, none, st)) return rc;
   return run_axis_bf16<float, uint16_t, 1 | 16>(t2, gx, ph, tp, wdev, nullptr, nullptr, tie, st);
 }
+
+// ---- batched independent problems -----------------------------------------------------------------------------------
+// nprob videos [B,H,T,W,C], contiguous as [nprob, B,H,T,W,C], each filtered with its own 2R+1 device weights (row p of
+// taps) and divided by its own maximum (maxval[p]).  The problem is blockIdx.y, so a CTA never spans two problems: its
+// weights, its max atomic, its divisor and its tie sums are those of one problem, with no segmented reduction.  Every
+// pass is planned per problem with plan_axis and, per element, forms its sums with the coefficients and the FMA order of
+// the single-problem kernels, so problem p's numbers are those of a single-problem call on it.  One template serves
+// fp32 and bf16 through TI / TO, as axis_col_bf16_kernel does; they are kernels of their own so that the single-problem
+// kernels keep their code.  The backward's tie set is out == 1.0f where its first pass reads fp32 (TI = float) and the
+// tie mask where it reads bf16; bit p * n + e of the mask is element e of problem p (the bf16 forward's last pass sets
+// it, TO = uint16_t).
+struct Batch {
+  long long n;            // elements per problem
+  const float* taps;      // [nprob][2R+1]
+  float* maxval;          // [nprob]: reduced by MODE & 2, the divisor of MODE & 4, the m of MODE & 8
+  const float* sums;      // [nprob][2]: sum(gout*out), number of tied maxima (MODE & 8)
+  const float* out;       // fp32 forward output: the tie set of MODE & 8 with TI = float
+  uint32_t* bits;         // the bf16 tie mask over all problems
+};
+
+template <int R>
+__device__ __forceinline__ void load_batch_weights(float (&w)[2 * R + 1], const float* taps, int prob) {
+#pragma unroll
+  for (int k = 0; k < 2 * R + 1; ++k) w[k] = taps[prob * (2 * R + 1) + k];
+}
+// the BwdIn transform of the fp32 kernels on VecF
+template <int V>
+__device__ __forceinline__ void bwd_out_v(VecF<V>& r, float sc, float tie, const float* o) {
+  VecF<V> t;
+  load_v<V>(t, o);
+#pragma unroll
+  for (int j = 0; j < V; ++j) r.v[j] = r.v[j] * sc + ((t.v[j] == 1.0f) ? tie : 0.f);
+}
+// the input transform of a pass: the tie gradient on the first adjoint pass (MODE & 8); e: element index in the batch
+template <typename TI, int MODE, int V>
+__device__ __forceinline__ void batch_in(VecF<V>& r, float sc, float tie, const Batch& bt, long long e) {
+  if constexpr ((MODE & 8) != 0) {
+    if constexpr (sizeof(TI) == 4) bwd_out_v<V>(r, sc, tie, bt.out + e);
+    else bwd_v<V>(r, sc, tie, bt.bits, e);
+  }
+}
+
+template <typename TI, typename TO, int MODE, int V, int R>
+__global__ void __launch_bounds__(FT) axis_col_batched_kernel(const TI* __restrict__ in, TO* __restrict__ out,
+                                                              long long outer, int n, long long inner, Batch bt) {
+  constexpr int kR = R, kTaps = 2 * R + 1;
+  extern __shared__ float coef[];                          // coef[p][d] = A[p][p + d - R] (0 outside the matrix)
+  const int prob = blockIdx.y;
+  const long long off = (long long)prob * bt.n;
+  float w[kTaps];
+  load_batch_weights<R>(w, bt.taps, prob);
+  for (int e = threadIdx.x; e < n * kTaps; e += FT) {
+    const int p = e / kTaps, q = p + (e % kTaps) - kR;
+    coef[e] = (q >= 0 && q < n) ? band_coef<R>(w, n, p, q, (MODE & 16) != 0) : 0.f;
+  }
+  __syncthreads();
+  const long long iv = inner / V;
+  const long long gid = (long long)blockIdx.x * FT + threadIdx.x;
+  float lmax = -3.0e38f;
+  if (gid < outer * iv) {
+    const long long o = gid / iv;
+    const long long base = off + o * n * inner + (gid - o * iv) * V;
+    float gscale = 0.f, gtie = 0.f, inv = 1.f;
+    if (MODE & 8) {
+      const float m = bt.maxval[prob];
+      gscale = 1.f / m;
+      gtie = -(bt.sums[2 * prob] / m) / bt.sums[2 * prob + 1];
+    }
+    if (MODE & 4) inv = bt.maxval[prob];
+    auto fetch = [&](int q) {
+      VecF<V> r;
+      if (q < n) {
+        load_v<V>(r, in + base + (long long)q * inner);
+        batch_in<TI, MODE, V>(r, gscale, gtie, bt, base + (long long)q * inner);
+      } else {
+#pragma unroll
+        for (int j = 0; j < V; ++j) r.v[j] = 0.f;
+      }
+      return r;
+    };
+    VecF<V> win[kTaps];
+#pragma unroll
+    for (int d = 0; d < kR; ++d)
+#pragma unroll
+      for (int j = 0; j < V; ++j) win[d].v[j] = 0.f;
+#pragma unroll
+    for (int d = kR; d < kTaps; ++d) win[d] = fetch(d - kR);
+    constexpr bool kDeep = V * kTaps <= 64;
+    VecF<V> next = fetch(kR + 1), next2;
+    for (int p = 0; p < n; ++p) {
+      if constexpr (kDeep) next2 = fetch(p + kR + 2);
+      VecF<V> acc;
+#pragma unroll
+      for (int j = 0; j < V; ++j) acc.v[j] = 0.f;
+#pragma unroll
+      for (int d = 0; d < kTaps; ++d) {
+        const float c = coef[p * kTaps + d];
+#pragma unroll
+        for (int j = 0; j < V; ++j) acc.v[j] = fmaf(c, win[d].v[j], acc.v[j]);
+      }
+      if (MODE & 4) {
+#pragma unroll
+        for (int j = 0; j < V; ++j) acc.v[j] /= inv;
+        if constexpr (sizeof(TO) == 2) mark_ties<V>(bt.bits, acc, base + (long long)p * inner);
+      }
+      if (MODE & 2) {
+#pragma unroll
+        for (int j = 0; j < V; ++j) lmax = fmaxf(lmax, acc.v[j]);
+      }
+      if (MODE & 1) store_v<V>(out + base + (long long)p * inner, acc);
+#pragma unroll
+      for (int d = 0; d < kTaps - 1; ++d) win[d] = win[d + 1];
+      win[kTaps - 1] = next;
+      if constexpr (kDeep) next = next2;
+      else next = fetch(p + kR + 2);
+    }
+  }
+  if (MODE & 2) {
+    lmax = warp_max(lmax);
+    if ((threadIdx.x & 31) == 0) atomic_max_float(bt.maxval + prob, lmax);
+  }
+}
+
+template <typename TI, typename TO, int MODE, int R>
+__global__ void __launch_bounds__(1024) axis_tile_batched_kernel(const TI* __restrict__ in, TO* __restrict__ out,
+                                                                 long long outer, int n, int inner, int o_chunk,
+                                                                 Batch bt) {
+  constexpr int kR = R, kTaps = 2 * R + 1;
+  extern __shared__ __align__(16) float tile[];            // [o_chunk][n][inner], contiguous like global memory
+  const int prob = blockIdx.y;
+  const int ni = n * inner;
+  const long long o0 = (long long)blockIdx.x * o_chunk;
+  const int no = (int)min((long long)o_chunk, outer - o0);
+  const long long g0 = (long long)prob * bt.n + o0 * ni;    // element index in the batch
+  const int telems = no * ni;
+  float gscale = 0.f, gtie = 0.f, inv = 1.f;
+  if (MODE & 8) {
+    const float m = bt.maxval[prob];
+    gscale = 1.f / m;
+    gtie = -(bt.sums[2 * prob] / m) / bt.sums[2 * prob + 1];
+  }
+  if (MODE & 4) inv = bt.maxval[prob];
+  // the widest loads the tile's row length and the pointers allow (g0 % 8 == 0 whenever ni % 8 == 0)
+  auto fill = [&](auto vw) {
+    constexpr int VV = decltype(vw)::value;
+    for (int e = threadIdx.x * VV; e < telems; e += blockDim.x * VV) {
+      VecF<VV> r;
+      load_v<VV>(r, in + g0 + e);
+      batch_in<TI, MODE, VV>(r, gscale, gtie, bt, g0 + e);
+      store_v<VV>(tile + e, r);
+    }
+  };
+  auto aligned = [&](int v) {
+    const uintptr_t a = (uintptr_t)(v * sizeof(TI) < 16 ? v * sizeof(TI) : 16) - 1;
+    return ni % v == 0 && (reinterpret_cast<uintptr_t>(in + g0) & a) == 0 &&
+           (!(MODE & 8) || sizeof(TI) == 2 || (reinterpret_cast<uintptr_t>(bt.out + g0) & (v == 1 ? 3 : 15)) == 0);
+  };
+  if (aligned(8)) fill(std::integral_constant<int, 8>());
+  else if (aligned(4)) fill(std::integral_constant<int, 4>());
+  else fill(std::integral_constant<int, 1>());
+  const int t = threadIdx.x;
+  float c[kTaps];
+  int off[kTaps];
+  {
+    const int p = min(t, ni - 1) / inner;
+    float w[kTaps];
+    load_batch_weights<R>(w, bt.taps, prob);
+#pragma unroll
+    for (int d = 0; d < kTaps; ++d) {
+      const int q = p + d - kR;
+      const bool ok = q >= 0 && q < n;
+      c[d] = ok ? band_coef<R>(w, n, p, q, (MODE & 16) != 0) : 0.f;
+      off[d] = ok ? (d - kR) * inner : 0;
+    }
+  }
+  __syncthreads();
+  float lmax = -3.0e38f;
+  auto row_out = [&](int oo) {
+    const float* row = tile + oo * ni + t;
+    VecF<1> acc;
+    acc.v[0] = 0.f;
+#pragma unroll
+    for (int d = 0; d < kTaps; ++d) acc.v[0] = fmaf(c[d], row[off[d]], acc.v[0]);
+    const long long e = g0 + (long long)oo * ni + t;
+    if (MODE & 4) {
+      acc.v[0] = acc.v[0] / inv;
+      if constexpr (sizeof(TO) == 2) mark_ties<1>(bt.bits, acc, e);
+    }
+    if (MODE & 2) lmax = fmaxf(lmax, acc.v[0]);
+    if (MODE & 1) store_v<1>(out + e, acc);
+  };
+  if (t < ni) {
+    if constexpr ((MODE & 2) != 0) {
+#pragma unroll 1
+      for (int oo = 0; oo < no; ++oo) row_out(oo);
+    } else {
+      for (int oo = 0; oo < no; ++oo) row_out(oo);
+    }
+  }
+  if (MODE & 2) {
+    lmax = warp_max(lmax);
+    if ((threadIdx.x & 31) == 0) atomic_max_float(bt.maxval + prob, lmax);
+  }
+}
+
+__global__ void init_max_batched_kernel(float* m, int nprob) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < nprob) m[i] = __int_as_float(0xff800000);
+}
+
+// sums[2p] = sum gout * out over problem p (blockIdx.y), sums[2p+1] = its number of tied maxima: out == 1.0f in fp32,
+// the popcount of the mask bits p*n .. p*n + n - 1 in bf16 (a word may hold bits of two problems)
+template <typename T>
+__global__ void __launch_bounds__(FT) tie_sums_batched_kernel(const T* __restrict__ gout, const T* __restrict__ out,
+                                                              const uint32_t* __restrict__ bits, long long n,
+                                                              float* sums) {
+  constexpr int V = 16 / sizeof(T);                        // elements per 16-byte access
+  const int prob = blockIdx.y;
+  const long long off = (long long)prob * n;
+  gout += off;
+  out += off;
+  float s = 0.f, c = 0.f;
+  const long long stride = (long long)gridDim.x * FT;
+  const long long tid = (long long)blockIdx.x * FT + threadIdx.x;
+  const bool vec = ((reinterpret_cast<uintptr_t>(gout) | reinterpret_cast<uintptr_t>(out)) & 15) == 0;
+  const long long nv = vec ? n / V : 0;
+  auto acc = [&](const VecF<V>& g, const VecF<V>& o) {
+#pragma unroll
+    for (int j = 0; j < V; ++j) s = fmaf(g.v[j], o.v[j], s);
+    if constexpr (sizeof(T) == 4) {
+#pragma unroll
+      for (int j = 0; j < V; ++j) c += (o.v[j] == 1.0f ? 1.f : 0.f);
+    }
+  };
+  long long i = tid;
+  for (; i + 3 * stride < nv; i += 4 * stride) {
+    VecF<V> g[4], o[4];
+#pragma unroll
+    for (int u = 0; u < 4; ++u) { load_v<V>(g[u], gout + (i + u * stride) * V); load_v<V>(o[u], out + (i + u * stride) * V); }
+#pragma unroll
+    for (int u = 0; u < 4; ++u) acc(g[u], o[u]);
+  }
+  for (; i < nv; i += stride) {
+    VecF<V> g, o;
+    load_v<V>(g, gout + i * V);
+    load_v<V>(o, out + i * V);
+    acc(g, o);
+  }
+  for (long long k = V * nv + tid; k < n; k += stride) {
+    VecF<1> g, o;
+    load_v<1>(g, gout + k);
+    load_v<1>(o, out + k);
+    s = fmaf(g.v[0], o.v[0], s);
+    if constexpr (sizeof(T) == 4) c += (o.v[0] == 1.0f) ? 1.f : 0.f;
+  }
+  if constexpr (sizeof(T) == 2) {
+    const long long lo = off, hi = off + n, w0 = lo >> 5, w1 = (hi - 1) >> 5;
+    unsigned cnt = 0;
+    for (long long w = w0 + tid; w <= w1; w += stride) {
+      uint32_t b = bits[w];
+      if (w == w0) b &= ~0u << (lo & 31);
+      if (w == w1 && (hi & 31)) b &= (1u << (hi & 31)) - 1u;
+      cnt += __popc(b);
+    }
+    c = (float)cnt;
+  }
+  __shared__ float red[2][FT / 32];
+  s = warp_sum(s);
+  c = warp_sum(c);
+  if ((threadIdx.x & 31) == 0) { red[0][threadIdx.x >> 5] = s; red[1][threadIdx.x >> 5] = c; }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float ss = 0.f, cc = 0.f;
+#pragma unroll
+    for (int w = 0; w < FT / 32; ++w) { ss += red[0][w]; cc += red[1][w]; }
+    atomicAdd(&sums[2 * prob], ss);
+    atomicAdd(&sums[2 * prob + 1], cc);
+  }
+}
+
+// one pass over all problems; p is the plan of one problem, which a single-problem call of that shape would use (its
+// tile / column choice and vector width)
+template <typename TI, typename TO, int MODE, int R>
+int run_batched_r(const TI* in, TO* out, const AxisPlan& p, int nprob, const Batch& bt, cudaStream_t st) {
+  if (p.tiled) {
+    const int ni = p.n * (int)p.inner;
+    const int threads = (ni + 31) / 32 * 32;
+    const dim3 grid((unsigned)((p.outer + p.o_chunk - 1) / p.o_chunk), (unsigned)nprob);
+    const size_t smem = (size_t)p.o_chunk * ni * sizeof(float);
+    axis_tile_batched_kernel<TI, TO, MODE, R><<<grid, threads, smem, st>>>(in, out, p.outer, p.n, (int)p.inner,
+                                                                          p.o_chunk, bt);
+  } else {
+    // n % v == 0 when inner % v == 0, so every problem's rows have the alignment of problem 0's
+    auto fits = [&](int v) {
+      const uintptr_t a = (uintptr_t)(v * sizeof(TI) < 16 ? v * sizeof(TI) : 16) - 1;
+      const uintptr_t b = (uintptr_t)(v * sizeof(TO) < 16 ? v * sizeof(TO) : 16) - 1;
+      return p.inner % v == 0 && (reinterpret_cast<uintptr_t>(in) & a) == 0 &&
+             (!(MODE & 1) || (reinterpret_cast<uintptr_t>(out) & b) == 0) &&
+             (!(MODE & 8) || sizeof(TI) == 2 || (reinterpret_cast<uintptr_t>(bt.out) & a) == 0);
+    };
+    constexpr bool kF32 = sizeof(TI) == 4 && sizeof(TO) == 4;      // the fp32 kernels' widths: 4 or 1
+    const int v = kF32 ? (fits(4) ? 4 : 1)
+                       : fits(8) && p.outer * (p.inner / 8) >= 1024LL * num_sms() ? 8 : fits(4) ? 4 : fits(8) ? 8 : 1;
+    const long long total = p.outer * (p.inner / v);
+    const dim3 grid((unsigned)((total + FT - 1) / FT), (unsigned)nprob);
+    const size_t smem = (size_t)p.n * (2 * R + 1) * sizeof(float);
+    void (*kernel)(const TI*, TO*, long long, int, long long, Batch) =
+        v == 4 ? axis_col_batched_kernel<TI, TO, MODE, 4, R> : axis_col_batched_kernel<TI, TO, MODE, 1, R>;
+    if constexpr (!kF32) {
+      if (v == 8) kernel = axis_col_batched_kernel<TI, TO, MODE, 8, R>;
+    }
+    if (smem > 48 * 1024)
+      KCCOT_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kernel<<<grid, FT, smem, st>>>(in, out, p.outer, p.n, p.inner, bt);
+  }
+  KCCOT_LAUNCH_CHECK();
+  return KCCOT_OK;
+}
+template <typename TI, typename TO, int MODE>
+int run_batched(const TI* in, TO* out, const AxisPlan& p, int nprob, int radius, const Batch& bt, cudaStream_t st) {
+  switch (radius) {
+    case 1: return run_batched_r<TI, TO, MODE, 1>(in, out, p, nprob, bt, st);
+    case 2: return run_batched_r<TI, TO, MODE, 2>(in, out, p, nprob, bt, st);
+    case 3: return run_batched_r<TI, TO, MODE, 3>(in, out, p, nprob, bt, st);
+    case 4: return run_batched_r<TI, TO, MODE, 4>(in, out, p, nprob, bt, st);
+    case 5: return run_batched_r<TI, TO, MODE, 5>(in, out, p, nprob, bt, st);
+    case 6: return run_batched_r<TI, TO, MODE, 6>(in, out, p, nprob, bt, st);
+  }
+  set_error("smoothing radius %d not supported (1..%d)", radius, kMaxRadius);
+  return KCCOT_EUNSUPPORTED;
+}
+
+constexpr int kMaxProblems = 65535;                           // gridDim.y
+size_t batched_head_bytes(int nprob) { return align_up((size_t)nprob * 2 * sizeof(float), 256); }
+
+// argument checks of the batched entries: those of the *_dev entries plus the problem count and the batched workspace
+int smooth_batched_args(int mode, int nprob, int B, int H, int T, int W, int C, const float* taps, int radius,
+                        bool need_ws, void* ws, size_t ws_bytes, Taps* tp) {
+  KCCOT_CHECK_ARG(nprob >= 1 && nprob <= kMaxProblems, "nprob must be in 1..%d (nprob=%d)", kMaxProblems, nprob);
+  if (int rc = smooth_args(mode, B, H, T, W, C, taps, radius, taps, radius, true, ws, ws_bytes, tp)) return rc;
+  if (need_ws)
+    KCCOT_CHECK_ARG(ws && ws_bytes >= kccot_smooth_batched_workspace_bytes(mode, nprob, B, H, T, W, C),
+                    "workspace too small");
+  KCCOT_CHECK_ARG((reinterpret_cast<uintptr_t>(ws) & 15) == 0, "workspace must be 16-byte aligned");
+  return KCCOT_OK;
+}
+
+// T = float (fp32 videos) or uint16_t (bf16); ties is used by bf16 only
+template <typename T>
+int smooth_batched_fwd(int mode, const T* x, int nprob, int B, int H, int T_, int W, int C, const float* taps,
+                       int radius, T* out, float* maxval, uint32_t* ties, void* ws, cudaStream_t st) {
+  const long long n = (long long)B * H * T_ * W * C;
+  constexpr bool kBf16 = sizeof(T) == 2;
+  if (kBf16) KCCOT_CUDA(cudaMemsetAsync(ties, 0, ((size_t)nprob * n + 31) / 32 * sizeof(uint32_t), st));
+  init_max_batched_kernel<<<(nprob + 255) / 256, 256, 0, st>>>(maxval, nprob);
+  KCCOT_LAUNCH_CHECK();
+  const Batch bt{n, taps, maxval, nullptr, nullptr, ties};
+  const AxisPlan pt = plan_axis((long long)B * H, T_, (long long)W * C);
+  if (mode == 1) {
+    if (int rc = run_batched<T, T, 2>(x, nullptr, pt, nprob, radius, bt, st)) return rc;
+    return run_batched<T, T, 1 | 4>(x, out, pt, nprob, radius, bt, st);
+  }
+  const size_t head = batched_head_bytes(nprob), sz = align_up((size_t)nprob * n * sizeof(float), 256);
+  float* t1 = (float*)((char*)ws + head);
+  float* t2 = (float*)((char*)ws + head + sz);
+  const AxisPlan ph = plan_axis(B, H, (long long)T_ * W * C);
+  const AxisPlan pw = plan_axis((long long)B * H * T_, W, C);
+  if (int rc = run_batched<T, float, 1>(x, t1, ph, nprob, radius, bt, st)) return rc;
+  if (int rc = run_batched<float, float, 1>(t1, t2, pt, nprob, radius, bt, st)) return rc;
+  if (int rc = run_batched<float, float, 2>(t2, nullptr, pw, nprob, radius, bt, st)) return rc;
+  return run_batched<float, T, 1 | 4>(t2, out, pw, nprob, radius, bt, st);
+}
+
+template <typename T>
+int smooth_batched_bwd(int mode, const T* gout, const T* out, const float* maxval, const uint32_t* ties, int nprob,
+                       int B, int H, int T_, int W, int C, const float* taps, int radius, T* gx, void* ws,
+                       cudaStream_t st) {
+  const long long n = (long long)B * H * T_ * W * C;
+  float* sums = (float*)ws;
+  KCCOT_CUDA(cudaMemsetAsync(sums, 0, (size_t)nprob * 2 * sizeof(float), st));
+  {
+    const long long single = min((long long)4 * num_sms(), (n / (16 / (long long)sizeof(T)) + FT - 1) / FT + 1);
+    const long long per = max(1LL, min(single, (8LL * num_sms() + nprob - 1) / nprob));
+    tie_sums_batched_kernel<T><<<dim3((unsigned)per, (unsigned)nprob), FT, 0, st>>>(gout, out, ties, n, sums);
+    KCCOT_LAUNCH_CHECK();
+  }
+  // read only: no pass of the backward sets MODE & 4
+  const Batch bt{n, taps, const_cast<float*>(maxval), sums, sizeof(T) == 4 ? (const float*)out : nullptr,
+                 const_cast<uint32_t*>(ties)};
+  const AxisPlan pt = plan_axis((long long)B * H, T_, (long long)W * C);
+  if (mode == 1) return run_batched<T, T, 1 | 8 | 16>(gout, gx, pt, nprob, radius, bt, st);
+  const size_t head = batched_head_bytes(nprob), sz = align_up((size_t)nprob * n * sizeof(float), 256);
+  float* t1 = (float*)((char*)ws + head);
+  float* t2 = (float*)((char*)ws + head + sz);
+  const AxisPlan ph = plan_axis(B, H, (long long)T_ * W * C);
+  const AxisPlan pw = plan_axis((long long)B * H * T_, W, C);
+  if (int rc = run_batched<T, float, 1 | 8 | 16>(gout, t1, pw, nprob, radius, bt, st)) return rc;
+  if (int rc = run_batched<float, float, 1 | 16>(t1, t2, pt, nprob, radius, bt, st)) return rc;
+  return run_batched<float, T, 1 | 16>(t2, gx, ph, nprob, radius, bt, st);
+}
 }  // namespace
 }  // namespace kccot
 
@@ -883,6 +1285,63 @@ int kccot_smooth_bwd_bf16_dev(int mode, const uint16_t* gout, const uint16_t* ou
   Taps tp;
   if (int rc = smooth_args(mode, B, H, T, W, C, taps_dev, radius, taps_dev, radius, true, ws, ws_bytes, &tp)) return rc;
   return smooth_bwd_bf16(mode, gout, out, maxval, ties, B, H, T, W, C, tp, taps_dev, gx, ws, (cudaStream_t)stream);
+}
+
+size_t kccot_smooth_batched_workspace_bytes(int mode, int nprob, int B, int H, int T, int W, int C) {
+  if (nprob < 1 || B < 1 || H < 1 || T < 1 || W < 1 || C < 1) return 0;
+  const size_t n = (size_t)nprob * B * H * T * W * C * sizeof(float);
+  return batched_head_bytes(nprob) + (mode == 3 ? 2 * align_up(n, 256) : 0);
+}
+
+int kccot_smooth_batched_fwd(int mode, const float* x, int nprob, int B, int H, int T, int W, int C,
+                             const float* taps_dev, int radius, float* out, float* maxval, void* ws, size_t ws_bytes,
+                             void* stream) {
+  KCCOT_CHECK_ARG(mode == 1 || mode == 3, "smoothing mode must be 1 (temporal) or 3 (3-D); the reference's '2d' "
+                                          "branch raises (data_utils.py:537-538)");
+  KCCOT_CHECK_ARG(x && out && maxval, "null pointer");
+  Taps tp;
+  if (int rc = smooth_batched_args(mode, nprob, B, H, T, W, C, taps_dev, radius, mode == 3, ws, ws_bytes, &tp))
+    return rc;
+  return smooth_batched_fwd<float>(mode, x, nprob, B, H, T, W, C, taps_dev, radius, out, maxval, nullptr, ws,
+                                   (cudaStream_t)stream);
+}
+
+int kccot_smooth_batched_bwd(int mode, const float* gout, const float* out, const float* maxval, int nprob, int B,
+                             int H, int T, int W, int C, const float* taps_dev, int radius, float* gx, void* ws,
+                             size_t ws_bytes, void* stream) {
+  KCCOT_CHECK_ARG(mode == 1 || mode == 3, "smoothing mode must be 1 or 3");
+  KCCOT_CHECK_ARG(gout && out && maxval && gx && ws, "null pointer / workspace");
+  Taps tp;
+  if (int rc = smooth_batched_args(mode, nprob, B, H, T, W, C, taps_dev, radius, true, ws, ws_bytes, &tp)) return rc;
+  return smooth_batched_bwd<float>(mode, gout, out, maxval, nullptr, nprob, B, H, T, W, C, taps_dev, radius, gx, ws,
+                                   (cudaStream_t)stream);
+}
+
+int kccot_smooth_batched_fwd_bf16(int mode, const uint16_t* x, int nprob, int B, int H, int T, int W, int C,
+                                  const float* taps_dev, int radius, uint16_t* out, float* maxval, uint32_t* ties,
+                                  void* ws, size_t ws_bytes, void* stream) {
+  KCCOT_CHECK_ARG(mode == 1 || mode == 3, "smoothing mode must be 1 (temporal) or 3 (3-D); the reference's '2d' "
+                                          "branch raises (data_utils.py:537-538)");
+  KCCOT_CHECK_ARG(x && out && maxval && ties, "null pointer");
+  KCCOT_CHECK_ARG((reinterpret_cast<uintptr_t>(ties) & 3) == 0, "tie mask must be 4-byte aligned");
+  Taps tp;
+  if (int rc = smooth_batched_args(mode, nprob, B, H, T, W, C, taps_dev, radius, mode == 3, ws, ws_bytes, &tp))
+    return rc;
+  return smooth_batched_fwd<uint16_t>(mode, x, nprob, B, H, T, W, C, taps_dev, radius, out, maxval, ties, ws,
+                                      (cudaStream_t)stream);
+}
+
+int kccot_smooth_batched_bwd_bf16(int mode, const uint16_t* gout, const uint16_t* out, const float* maxval,
+                                  const uint32_t* ties, int nprob, int B, int H, int T, int W, int C,
+                                  const float* taps_dev, int radius, uint16_t* gx, void* ws, size_t ws_bytes,
+                                  void* stream) {
+  KCCOT_CHECK_ARG(mode == 1 || mode == 3, "smoothing mode must be 1 or 3");
+  KCCOT_CHECK_ARG(gout && out && maxval && ties && gx && ws, "null pointer / workspace");
+  KCCOT_CHECK_ARG((reinterpret_cast<uintptr_t>(ties) & 3) == 0, "tie mask must be 4-byte aligned");
+  Taps tp;
+  if (int rc = smooth_batched_args(mode, nprob, B, H, T, W, C, taps_dev, radius, true, ws, ws_bytes, &tp)) return rc;
+  return smooth_batched_bwd<uint16_t>(mode, gout, out, maxval, ties, nprob, B, H, T, W, C, taps_dev, radius, gx, ws,
+                                      (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -9,11 +9,16 @@ the gradient is bf16 (kccot_smooth_fwd_bf16 / _bwd_bf16 in include/kccot.h).  An
 
 `sigma` is a number, or a SmoothingTaps: a device buffer of weights that the kernels read when they run, so that a
 CUDA graph captured with it follows an annealed sigma (the sigma changes between replays, the graph does not).
+
+The *_batched convolutions smooth nprob independent videos [nprob, B, H, T, W, C] in one call, each with its own sigma
+and divided by its own maximum: the result is that of nprob separate calls.
 """
+import numbers
+
 import numpy as np
 import torch
 
-from .functional import SmoothFn, _check_video
+from .functional import SmoothBatchedFn, SmoothFn, _check_video
 
 
 class SmoothingTaps:
@@ -26,14 +31,28 @@ class SmoothingTaps:
 
     .set(sigma) writes KernelSmoothing._weights(radius, sigma), the host fp32 weights a float sigma uses, so the result
     is the float-sigma call's at the same sigma.  It is ordered on the current stream and does not synchronise the
-    host (a pinned source copied with non_blocking=True)."""
+    host (a pinned source copied with non_blocking=True).
 
-    def __init__(self, radius, device="cuda"):
+    With `nprob`, the weights of nprob problems for the *_batched convolutions: `weights` is [nprob, 2r+1] and .set()
+    takes one sigma for all of them or a sequence of nprob sigmas, row p holding KernelSmoothing._weights(radius,
+    sigma_p)."""
+
+    def __init__(self, radius, device="cuda", nprob=None):
         self.radius = int(radius)
-        self.weights = torch.zeros(2 * self.radius + 1, dtype=torch.float32, device=device)
+        self.nprob = None if nprob is None else int(nprob)
+        if self.nprob is not None and self.nprob < 1:
+            raise ValueError(f"nprob must be at least 1, got {nprob}")
+        shape = (2 * self.radius + 1,) if self.nprob is None else (self.nprob, 2 * self.radius + 1)
+        self.weights = torch.zeros(shape, dtype=torch.float32, device=device)
 
     def set(self, sigma):
-        w = torch.from_numpy(KernelSmoothing._weights(self.radius, sigma))
+        if self.nprob is None:
+            w = torch.from_numpy(KernelSmoothing._weights(self.radius, sigma))
+        else:
+            sig = [sigma] * self.nprob if isinstance(sigma, numbers.Real) else list(sigma)
+            if len(sig) != self.nprob:
+                raise ValueError(f"{len(sig)} sigmas for {self.nprob} problems")
+            w = torch.from_numpy(np.stack([KernelSmoothing._weights(self.radius, s) for s in sig]))
         self.weights.copy_(w.pin_memory() if self.weights.is_cuda else w, non_blocking=True)
         return self
 
@@ -110,6 +129,40 @@ class KernelSmoothing:
         for name, n in (("H", H), ("T", T), ("W", W)):
             self._check_axis(name, n, self.spatial_radius)
         return SmoothFn.apply(inputs, 3, None, taps)
+
+    # -- batched independent problems ----------------------------------------------------------------
+    def _batched(self, inputs, sigma, mode, radius):
+        """checks as in the single-problem methods, then one SmoothBatchedFn call.  A number or sequence sigma becomes a
+        SmoothingTaps whose weights are copied to the device on every call, which a CUDA graph cannot record."""
+        if isinstance(sigma, SmoothingTaps):
+            if sigma.radius != radius:
+                raise ValueError(f"SmoothingTaps of radius {sigma.radius} for a filter of radius {radius}")
+            nprob = inputs.shape[0] if isinstance(inputs, torch.Tensor) and inputs.dim() else None
+            if sigma.nprob != nprob:
+                raise ValueError(f"SmoothingTaps of {sigma.nprob} problems for a batch of {nprob} problems")
+        inputs = _check_video(inputs, "inputs", 6)
+        _, _, H, T, W, _ = inputs.shape
+        for name, n in ((("T", T),) if mode == 1 else (("H", H), ("T", T), ("W", W))):
+            self._check_axis(name, n, radius)
+        if not isinstance(sigma, SmoothingTaps):
+            if torch.cuda.is_current_stream_capturing():
+                raise ValueError("a number or sequence sigma is copied to the device on every call, which CUDA graph "
+                                 "capture cannot record: pass a SmoothingTaps(radius, nprob=...) and .set() it "
+                                 "between replays")
+            sigma = SmoothingTaps(radius, inputs.device, inputs.shape[0]).set(sigma)
+        return SmoothBatchedFn.apply(inputs, mode, sigma)
+
+    def temporal_convolution_batched(self, inputs, sigma):
+        """temporal_convolution of nprob independent videos in one call: `inputs` [nprob, B, H, T, W, C] (fp32 or
+        bf16), problem p filtered with sigma_p and divided by its own maximum.  `sigma`: a number, a sequence of nprob
+        numbers, or a SmoothingTaps(temporal_radius, nprob=nprob)."""
+        return self._batched(inputs, sigma, 1, self.temporal_radius)
+
+    def gaussian_convolution3D_batched(self, inputs, sigma):
+        """gaussian_convolution3D of nprob independent videos in one call: `inputs` [nprob, B, H, T, W, C] (fp32 or
+        bf16), problem p filtered with sigma_p and divided by its own maximum.  `sigma`: a number, a sequence of nprob
+        numbers, or a SmoothingTaps(spatial_radius, nprob=nprob)."""
+        return self._batched(inputs, sigma, 3, self.spatial_radius)
 
     def annealing_sigma(self, init_sigma, step, decay_steps=500, decay_rate=0.975):
         """data_utils.py:584-586."""

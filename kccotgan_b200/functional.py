@@ -7,6 +7,7 @@ of the library (the result is exactly the fp32 one on the widened videos, video 
 video next to an fp32 one, and bf16 h / m, are widened with .float() (exact).  Gradients come back in the dtype of
 their input.  The smoothing (SmoothFn) also takes bf16 videos: they run the bf16 entry points, whose output is the
 fp32 output on the widened video rounded to bf16, and whose gradient is bf16 (see kccot_smooth_fwd_bf16 in kccot.h).
+SmoothBatchedFn smooths nprob independent videos in one call, in fp32 or bf16 alike.
 """
 import ctypes
 
@@ -506,3 +507,57 @@ class SmoothFn(torch.autograd.Function):
                 _lib.call("kccot_smooth_bwd" + suffix, ctx.mode, _ptr(gout), _ptr(out), _ptr(maxval), B, H, T, W, C,
                           *wargs, _ptr(gx), _ptr(ws), ws.numel(), _stream(dev))
         return gx, None, None, None
+
+
+class SmoothBatchedFn(torch.autograd.Function):
+    """`nprob` independent smoothings in one call per direction (kccot_smooth_batched_fwd / _bwd): x is
+    [nprob, B, H, T, W, C], `taps` a data_utils.SmoothingTaps with nprob rows, row p the weights of problem p, which is
+    divided by its own maximum.  As in SmoothFn, mode 1 filters T and mode 3 filters H, T and W, the forward snapshots
+    the weights for the backward, and a bf16 x runs the _bf16 entries and saves the tie mask of the whole batch."""
+
+    @staticmethod
+    def forward(ctx, x, mode, taps):
+        x = _check_video(x, "inputs", 6)
+        bf16 = x.dtype == torch.bfloat16
+        P, B, H, T, W, C = x.shape
+        dev = x.device
+        if taps.weights.device != dev:
+            raise ValueError(f"taps: the weights are on {taps.weights.device}, the video on {dev}")
+        if tuple(taps.weights.shape) != (P, 2 * taps.radius + 1):
+            raise ValueError(f"taps: weights of shape {tuple(taps.weights.shape)} for {P} problems of radius "
+                             f"{taps.radius}; expected {(P, 2 * taps.radius + 1)}")
+        lib = _lib.load()
+        w = taps.weights.clone()
+        out = torch.empty_like(x)
+        maxval = torch.empty((P,), dtype=torch.float32, device=dev)
+        ws = _ws(lib.kccot_smooth_batched_workspace_bytes(mode, P, B, H, T, W, C), dev)
+        with _on_device(dev):
+            if bf16:
+                ties = torch.empty(lib.kccot_smooth_ties_bytes(P * B, H, T, W, C) // 4, dtype=torch.int32, device=dev)
+                _lib.call("kccot_smooth_batched_fwd_bf16", mode, _ptr(x), P, B, H, T, W, C, _ptr(w), taps.radius,
+                          _ptr(out), _ptr(maxval), _ptr(ties), _ptr(ws), ws.numel(), _stream(dev))
+                ctx.save_for_backward(out, maxval, w, ties)
+            else:
+                _lib.call("kccot_smooth_batched_fwd", mode, _ptr(x), P, B, H, T, W, C, _ptr(w), taps.radius, _ptr(out),
+                          _ptr(maxval), _ptr(ws), ws.numel(), _stream(dev))
+                ctx.save_for_backward(out, maxval, w)
+        ctx.mode, ctx.radius = mode, taps.radius
+        return out
+
+    @staticmethod
+    def backward(ctx, gout):
+        out, maxval, w, *ties = ctx.saved_tensors
+        P, B, H, T, W, C = out.shape
+        dev = out.device
+        gout = gout.contiguous().to(out.dtype)
+        gx = torch.empty_like(out)
+        ws = _ws(_lib.load().kccot_smooth_batched_workspace_bytes(ctx.mode, P, B, H, T, W, C), dev)
+        with _on_device(dev):
+            if ties:
+                _lib.call("kccot_smooth_batched_bwd_bf16", ctx.mode, _ptr(gout), _ptr(out), _ptr(maxval),
+                          _ptr(ties[0]), P, B, H, T, W, C, _ptr(w), ctx.radius, _ptr(gx), _ptr(ws), ws.numel(),
+                          _stream(dev))
+            else:
+                _lib.call("kccot_smooth_batched_bwd", ctx.mode, _ptr(gout), _ptr(out), _ptr(maxval), P, B, H, T, W, C,
+                          _ptr(w), ctx.radius, _ptr(gx), _ptr(ws), ws.numel(), _stream(dev))
+        return gx, None, None
