@@ -162,6 +162,45 @@ int kccot_shard_cost_bwd_bf16(const float* Cbar3rows, const float* XYcol, const 
                               uint16_t* g_fake_rows, float* gh_fake_rows, float* gm_real_part,
                               float* gh_real_rows, float* gm_fake_part, void* ws, size_t ws_bytes,
                               void* stream);
+/* Shared context frames in the row shards — the hint of kccot_mixed_loss_fwd_ctx for the sharded cost: every column c
+ * of the flattened [B, K] rows with (c % ctx_period) < ctx_len holds identical values in real and fake (for
+ * [B,H,T,W,C] videos ctx_period = T*W*C, ctx_len = ctx_frames*W*C).  Arguments as in the plain / _bf16 entries above,
+ * plus the hint; the workspace is kccot_shard_cost_workspace_bytes_ctx (0 for a bad hint), and the backward needs the
+ * workspace of the matching forward call with the same hint.
+ *   fwd: fake's context columns are never read; where a fake row's context value is needed (column statistics, row
+ *        norms) the real row's value stands in.  The Gram of the context columns is computed once (this rank's real
+ *        rows x all reals) and shared by the xy, xx and yy blocks, which add the Gram of the predicted columns to it.
+ *   results: equal to the plain entries' on inputs that keep the promise, within floating-point tolerance: not bit
+ *        for bit, because the context and predicted parts of each dot product are summed separately.
+ *   bwd: g_fake_rows is the gradient with respect to the PREDICTED columns; its context columns are written as zero
+ *        (as kccot_mixed_loss_bwd_ctx does).  The h / M gradients are those of the plain entry on the same cost
+ *        adjoints.  The _bf16_ctx twins keep the bf16 contract: the results of the fp32 _ctx entries on the widened
+ *        videos, g_fake_rows rounded to nearest even.
+ *   ctx_len == 0: no hint; the plain entries run, bit for bit.
+ *   Rejected with KCCOT_EINVAL before any CUDA call: ctx_period < 0, ctx_len < 0, ctx_len >= ctx_period (unless both
+ *   are 0), K % ctx_period != 0, K >= 2^31 - 64 with a hint, and every check of the plain / _bf16 entries, including
+ *   a bad row range in the backward. */
+size_t kccot_shard_cost_workspace_bytes_ctx(int B, long long K, int Brows, long long ctx_period, long long ctx_len);
+int kccot_shard_cost_fwd_ctx(const float* real, const float* fake, int B, long long K, int row0, int Brows,
+                             const float* h_fake, const float* m_real, const float* h_real,
+                             const float* m_fake, int T, int J, float s, float* C3rows, void* ws,
+                             size_t ws_bytes, void* stream, long long ctx_period, long long ctx_len);
+int kccot_shard_cost_bwd_ctx(const float* Cbar3rows, const float* XYcol, const float* YYcol, int B,
+                             long long K, int row0, int Brows, const float* h_fake, const float* m_real,
+                             const float* h_real, const float* m_fake, int T, int J, float s,
+                             float* g_fake_rows, float* gh_fake_rows, float* gm_real_part,
+                             float* gh_real_rows, float* gm_fake_part, void* ws, size_t ws_bytes,
+                             void* stream, long long ctx_period, long long ctx_len);
+int kccot_shard_cost_fwd_bf16_ctx(const uint16_t* real, const uint16_t* fake, int B, long long K, int row0,
+                                  int Brows, const float* h_fake, const float* m_real, const float* h_real,
+                                  const float* m_fake, int T, int J, float s, float* C3rows, void* ws,
+                                  size_t ws_bytes, void* stream, long long ctx_period, long long ctx_len);
+int kccot_shard_cost_bwd_bf16_ctx(const float* Cbar3rows, const float* XYcol, const float* YYcol, int B,
+                                  long long K, int row0, int Brows, const float* h_fake, const float* m_real,
+                                  const float* h_real, const float* m_fake, int T, int J, float s,
+                                  uint16_t* g_fake_rows, float* gh_fake_rows, float* gm_real_part,
+                                  float* gh_real_rows, float* gm_fake_part, void* ws, size_t ws_bytes,
+                                  void* stream, long long ctx_period, long long ctx_len);
 size_t kccot_shard_sinkhorn_workspace_bytes(int np, int Brows, int B, int L);
 size_t kccot_shard_mailbox_bytes(int np, int nranks, int B);
 int kccot_shard_local_min(const float* Crows, int np, int Brows, int B, float* shift_out, void* stream);

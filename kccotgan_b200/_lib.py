@@ -43,6 +43,14 @@ SIGNATURES = {
     "kccot_shard_cost_fwd_bf16": (_I, [_P, _P, _I, _LL, _I, _I, _P, _P, _P, _P, _I, _I, _F, _P, _P, _SZ, _P]),
     "kccot_shard_cost_bwd_bf16": (_I, [_P, _P, _P, _I, _LL, _I, _I, _P, _P, _P, _P, _I, _I, _F, _P, _P, _P, _P, _P, _P,
                                        _SZ, _P]),
+    "kccot_shard_cost_workspace_bytes_ctx": (_SZ, [_I, _LL, _I, _LL, _LL]),
+    "kccot_shard_cost_fwd_ctx": (_I, [_P, _P, _I, _LL, _I, _I, _P, _P, _P, _P, _I, _I, _F, _P, _P, _SZ, _P, _LL, _LL]),
+    "kccot_shard_cost_bwd_ctx": (_I, [_P, _P, _P, _I, _LL, _I, _I, _P, _P, _P, _P, _I, _I, _F, _P, _P, _P, _P, _P, _P,
+                                      _SZ, _P, _LL, _LL]),
+    "kccot_shard_cost_fwd_bf16_ctx": (_I, [_P, _P, _I, _LL, _I, _I, _P, _P, _P, _P, _I, _I, _F, _P, _P, _SZ, _P, _LL,
+                                           _LL]),
+    "kccot_shard_cost_bwd_bf16_ctx": (_I, [_P, _P, _P, _I, _LL, _I, _I, _P, _P, _P, _P, _I, _I, _F, _P, _P, _P, _P, _P,
+                                           _P, _SZ, _P, _LL, _LL]),
     "kccot_shard_sinkhorn_workspace_bytes": (_SZ, [_I, _I, _I, _I]),
     "kccot_shard_mailbox_bytes": (_SZ, [_I, _I, _I]),
     "kccot_shard_local_min": (_I, [_P, _I, _I, _I, _P, _P]),

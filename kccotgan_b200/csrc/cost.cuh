@@ -156,5 +156,27 @@ int large_shard_cost_bwd(const float* Cbar3rows, const float* XYcol, const float
                          int Brows, const float* h_fake, const float* m_real, const float* h_real, const float* m_fake,
                          int T, int J, float s, uint16_t* g_fake_rows, float* gh_fake_rows, float* gm_real_part,
                          float* gh_real_rows, float* gm_fake_part, void* ws, size_t ws_bytes, cudaStream_t st);
+// shared context frames (kccot_shard_cost_*_ctx; the caller has checked K < 2^31 - 64, K % period == 0 and
+// 0 < clen < period): fake's context columns are not read, g_fake_rows' context columns are written as zero.  Own
+// workspace size; the backward needs the workspace of the matching forward.
+size_t large_shard_ws_bytes_ctx(int B, long long K, int Brows, long long period, long long clen);
+int large_shard_cost_fwd_ctx(const float* real, const float* fake, int B, long long K, int row0, int Brows,
+                             const float* h_fake, const float* m_real, const float* h_real, const float* m_fake, int T,
+                             int J, float s, float* C3rows, void* ws, size_t ws_bytes, long long period, long long clen,
+                             cudaStream_t st);
+int large_shard_cost_fwd_ctx(const uint16_t* real, const uint16_t* fake, int B, long long K, int row0, int Brows,
+                             const float* h_fake, const float* m_real, const float* h_real, const float* m_fake, int T,
+                             int J, float s, float* C3rows, void* ws, size_t ws_bytes, long long period, long long clen,
+                             cudaStream_t st);
+int large_shard_cost_bwd_ctx(const float* Cbar3rows, const float* XYcol, const float* YYcol, int B, long long K, int row0,
+                             int Brows, const float* h_fake, const float* m_real, const float* h_real,
+                             const float* m_fake, int T, int J, float s, float* g_fake_rows, float* gh_fake_rows,
+                             float* gm_real_part, float* gh_real_rows, float* gm_fake_part, void* ws, size_t ws_bytes,
+                             long long period, long long clen, cudaStream_t st);
+int large_shard_cost_bwd_ctx(const float* Cbar3rows, const float* XYcol, const float* YYcol, int B, long long K, int row0,
+                             int Brows, const float* h_fake, const float* m_real, const float* h_real,
+                             const float* m_fake, int T, int J, float s, uint16_t* g_fake_rows, float* gh_fake_rows,
+                             float* gm_real_part, float* gh_real_rows, float* gm_fake_part, void* ws, size_t ws_bytes,
+                             long long period, long long clen, cudaStream_t st);
 
 }  // namespace kccot

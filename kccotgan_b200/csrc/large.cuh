@@ -43,6 +43,25 @@ int large_launch_stats(const uint16_t* x, const uint16_t* y, int Bx, int By, lon
 int large_launch_split(const uint16_t* x, const uint16_t* y, int Bx, int By, long long K, long long Kp, int Rp,
                        const float* mean, const float* scal, __half* Zh1, __half* Zh2, __half* ZT1, __half* ZT2,
                        cudaStream_t st);
+// Shared context frames of the row shards (B real rows x, B fake rows y; K < 2^31, K % period == 0,
+// 0 < clen < period): column c is a context column when c % period < clen, and y's values there are never read (x's
+// stand in).  The stats are those of large_launch_stats on inputs that keep that promise.  The split writes the columns
+// permuted: the nc = K / period * clen context columns in [0, Kcp), the predicted ones from Kcp on, each part
+// zero-padded to a multiple of 64; Zh [2B][Kpp], ZT [Kpp][Rp].  The scatter writes g_pred [nrows][nq] (the predicted
+// columns in order) back to the video columns of g [nrows][K] and zeroes the context columns.
+int large_launch_stats_ctx(const float* x, const float* y, int B, long long K, int period, int clen, int nseg,
+                           float* part, float* mean, float* scal, cudaStream_t st);
+int large_launch_stats_ctx(const uint16_t* x, const uint16_t* y, int B, long long K, int period, int clen, int nseg,
+                           float* part, float* mean, float* scal, cudaStream_t st);
+int large_launch_split_ctx(const float* x, const float* y, int B, long long K, int period, int clen, int Kcp,
+                           long long Kpp, int Rp, const float* mean, const float* scal, __half* Zh1, __half* Zh2,
+                           __half* ZT1, __half* ZT2, cudaStream_t st);
+int large_launch_split_ctx(const uint16_t* x, const uint16_t* y, int B, long long K, int period, int clen, int Kcp,
+                           long long Kpp, int Rp, const float* mean, const float* scal, __half* Zh1, __half* Zh2,
+                           __half* ZT1, __half* ZT2, cudaStream_t st);
+int large_launch_ctx_scatter(const float* g_pred, int nrows, int K, int period, int clen, float* g, cudaStream_t st);
+int large_launch_ctx_scatter(const uint16_t* g_pred, int nrows, int K, int period, int clen, uint16_t* g,
+                             cudaStream_t st);
 int large_launch_rownorm(const __half* Zh1, const __half* Zh2, int R, long long K, long long Kp, float* norms,
                          cudaStream_t st);
 int large_launch_finalize(const LargeFin& F, int nblocks, int T, int J, float s, const float* scal, cudaStream_t st);

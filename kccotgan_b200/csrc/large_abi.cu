@@ -221,18 +221,28 @@ int large_cost_bwd(const float* Cbar, const float* x, const float* y, int Bx, in
 // The workspace of the forward call carries the transposed split and the scales to the backward call.
 // ------------------------------------------------------------------------------------------------
 namespace {
+// Column layout of the shared-context split (large.cuh): nc context columns padded to Kcp, then nq predicted columns
+// padded to Kqp
+struct CtxCols {
+  int period, clen, nc, nq, Kcp, Kqp;
+  CtxCols(long long K, long long p, long long l)
+      : period((int)p), clen((int)l), nc((int)(K / p * l)), nq((int)(K - K / p * l)), Kcp((int)pad64(nc)),
+        Kqp((int)pad64(nq)) {}
+};
+
 struct ShardWs {
   float *scal, *part, *mean, *norms, *Wtmp, *rs_part, *rowsum;
   __half *Zh1, *Zh2, *ZT1, *ZT2, *Wh1, *Wh2;
   float* P[3];
+  float* g_pred;           // shared-context hint only: the adjoint GEMM's [Brows][nq] predicted-column rows
   int nseg, Rp;
-  long long Kp;
+  long long Kp;            // pitch of the split (padded permuted width under the hint)
   size_t bytes;
 };
-ShardWs carve_shard(void* ws, int B, long long K, int Brows) {
+ShardWs carve_shard(void* ws, int B, long long K, int Brows, const CtxCols* cc = nullptr) {
   ShardWs w{};
   const int R = 2 * B;
-  w.Kp = pad64(K);
+  w.Kp = cc ? (long long)cc->Kcp + cc->Kqp : pad64(K);
   w.Rp = (int)pad64(R);
   w.nseg = stats_segments(R, K);
   Carver c(ws);
@@ -250,26 +260,41 @@ ShardWs carve_shard(void* ws, int B, long long K, int Brows) {
   w.rowsum = c.take<float>((size_t)Brows);
   w.Wh1 = c.take<__half>((size_t)Brows * w.Rp);
   w.Wh2 = c.take<__half>((size_t)Brows * w.Rp);
+  if (cc) w.g_pred = c.take<float>((size_t)Brows * cc->nq);
   w.bytes = align_up(c.off, 256);
   return w;
 }
 }  // namespace
 
 size_t large_shard_ws_bytes(int B, long long K, int Brows) { return carve_shard(nullptr, B, K, Brows).bytes; }
+size_t large_shard_ws_bytes_ctx(int B, long long K, int Brows, long long period, long long clen) {
+  const CtxCols cc(K, period, clen);
+  return carve_shard(nullptr, B, K, Brows, &cc).bytes;
+}
 
 namespace {
 // Video element type V (float, or bf16 bits): only the pre-pass reads the videos, so only it depends on V.
+// cc != nullptr: the shared-context hint (large.cuh) — the context columns' Gram is computed once, real rows x all
+// reals, and the three blocks add their predicted columns' Gram to it.
 template <typename V>
 int shard_cost_fwd(const V* real, const V* fake, int B, long long K, int row0, int Brows, const float* h_fake,
                    const float* m_real, const float* h_real, const float* m_fake, int T, int J, float s, float* C3rows,
-                   void* ws, size_t ws_bytes, cudaStream_t st) {
+                   void* ws, size_t ws_bytes, cudaStream_t st, const CtxCols* cc = nullptr) {
   KCCOT_CHECK_ARG(row0 >= 0 && Brows >= 1 && row0 + Brows <= B, "bad row range [%d, %d) of %d", row0, row0 + Brows, B);
-  const ShardWs w = carve_shard(ws, B, K, Brows);
+  const ShardWs w = carve_shard(ws, B, K, Brows, cc);
   KCCOT_CHECK_ARG(ws_bytes >= w.bytes, "workspace too small (row-shard cost path needs %zu bytes, got %zu)", w.bytes, ws_bytes);
   const int R = 2 * B;
-  if (int rc = large_launch_stats(real, fake, B, B, K, w.nseg, w.part, w.mean, w.scal, st)) return rc;
-  if (int rc = large_launch_split(real, fake, B, B, K, w.Kp, w.Rp, w.mean, w.scal, w.Zh1, w.Zh2, w.ZT1, w.ZT2, st)) return rc;
-  if (int rc = large_launch_rownorm(w.Zh1, w.Zh2, R, K, w.Kp, w.norms, st)) return rc;
+  if (cc) {
+    if (int rc = large_launch_stats_ctx(real, fake, B, K, cc->period, cc->clen, w.nseg, w.part, w.mean, w.scal, st)) return rc;
+    if (int rc = large_launch_split_ctx(real, fake, B, K, cc->period, cc->clen, cc->Kcp, w.Kp, w.Rp, w.mean, w.scal, w.Zh1,
+                                        w.Zh2, w.ZT1, w.ZT2, st))
+      return rc;
+    if (int rc = large_launch_rownorm(w.Zh1, w.Zh2, R, w.Kp, w.Kp, w.norms, st)) return rc;
+  } else {
+    if (int rc = large_launch_stats(real, fake, B, B, K, w.nseg, w.part, w.mean, w.scal, st)) return rc;
+    if (int rc = large_launch_split(real, fake, B, B, K, w.Kp, w.Rp, w.mean, w.scal, w.Zh1, w.Zh2, w.ZT1, w.ZT2, st)) return rc;
+    if (int rc = large_launch_rownorm(w.Zh1, w.Zh2, R, K, w.Kp, w.norms, st)) return rc;
+  }
   G3Params P{};
   // xy: real rows x all fakes; xx: real rows x all reals; yy: fake rows x all fakes (no symmetry across ranks)
   P.job[0] = G3Job{row0, B, Brows, B, 0, 0, 0, 0, w.P[0], B, 0};
@@ -280,7 +305,28 @@ int shard_cost_fwd(const V* real, const V* fake, int B, long long K, int row0, i
   P.ksplit = 1;
   P.kb_per_split = (int)(w.Kp / G3_BK);
   P.alpha = 1.f;
-  if (int rc = launch_gemm_f16x3_pair(w.Zh1, w.Zh2, R, w.Kp, w.Zh1, w.Zh2, R, w.Kp, K, P, st)) return rc;
+  if (cc) {
+    // context columns: real and fake rows are the same there, so the three blocks share real rows x all reals
+    G3Params Pc{};
+    Pc.job[0] = P.job[1];
+    g3_count_tiles_pair(&Pc.job[0]);
+    Pc.njobs = 1;
+    Pc.ksplit = 1;
+    Pc.kb_per_split = cc->Kcp / G3_BK;
+    Pc.alpha = 1.f;
+    if (int rc = launch_gemm_f16x3_pair(w.Zh1, w.Zh2, R, w.Kp, w.Zh1, w.Zh2, R, w.Kp, cc->nc, Pc, st)) return rc;
+    const size_t pb = (size_t)Brows * B * sizeof(float);
+    KCCOT_CUDA(cudaMemcpyAsync(w.P[0], w.P[1], pb, cudaMemcpyDeviceToDevice, st));
+    KCCOT_CUDA(cudaMemcpyAsync(w.P[2], w.P[1], pb, cudaMemcpyDeviceToDevice, st));
+    // predicted columns: the three blocks, added to it
+    P.kb_per_split = cc->Kqp / G3_BK;
+    P.accumulate = 1;
+    if (int rc = launch_gemm_f16x3_pair(w.Zh1 + cc->Kcp, w.Zh2 + cc->Kcp, R, w.Kp, w.Zh1 + cc->Kcp, w.Zh2 + cc->Kcp, R, w.Kp,
+                                        cc->nq, P, st))
+      return rc;
+  } else {
+    if (int rc = launch_gemm_f16x3_pair(w.Zh1, w.Zh2, R, w.Kp, w.Zh1, w.Zh2, R, w.Kp, K, P, st)) return rc;
+  }
   const long long RB = (long long)Brows * B, hm = (long long)T * J;
   LargeFin F{};
   F.b[0] = LargeFinBlock{w.P[0], B, RB, 1, 0, w.norms + row0, w.norms + B, h_fake + row0 * hm, m_real, nullptr, nullptr,
@@ -297,8 +343,8 @@ template <typename G>
 int shard_cost_bwd(const float* Cbar3rows, const float* XYcol, const float* YYcol, int B, long long K, int row0, int Brows,
                    const float* h_fake, const float* m_real, const float* h_real, const float* m_fake, int T, int J,
                    float s, G* g_fake_rows, float* gh_fake_rows, float* gm_real_part, float* gh_real_rows,
-                   float* gm_fake_part, void* ws, size_t ws_bytes, cudaStream_t st) {
-  const ShardWs w = carve_shard(ws, B, K, Brows);
+                   float* gm_fake_part, void* ws, size_t ws_bytes, cudaStream_t st, const CtxCols* cc = nullptr) {
+  const ShardWs w = carve_shard(ws, B, K, Brows, cc);
   KCCOT_CHECK_ARG(ws_bytes >= w.bytes, "workspace too small (row-shard cost path needs %zu bytes, got %zu)", w.bytes, ws_bytes);
   const long long RB = (long long)Brows * B, hm = (long long)T * J;
   const float *Cxy = Cbar3rows, *Cxx = Cbar3rows + RB, *Cyy = Cbar3rows + 2 * RB;
@@ -316,6 +362,26 @@ int shard_cost_bwd(const float* Cbar3rows, const float* XYcol, const float* YYco
     return rc;
   G3Params P{};
   P.job[0] = G3Job{0, 0, Brows, (int)K, 0, 0, 0, 0, reinterpret_cast<float*>(g_fake_rows), K, 0};
+  if (cc) {
+    // the predicted columns only (rows [Kcp, Kcp + nq) of ZT) into g_pred, then back to the video columns
+    P.job[0] = G3Job{0, 0, Brows, cc->nq, 0, 0, 0, 0, w.g_pred, cc->nq, 0};
+    g3_count_tiles_pair(&P.job[0]);
+    P.njobs = 1;
+    P.ksplit = 1;
+    P.kb_per_split = (int)(w.Rp / G3_BK);
+    P.alpha = -2.f * s;
+    P.alpha_dev = w.scal + kScalGradAlpha;
+    const long long zoff = (long long)cc->Kcp * w.Rp;
+    const int R = 2 * B;
+    int rc;
+    if constexpr (sizeof(G) == 2)
+      rc = launch_gemm_f16x3_pair_bf16(w.Wh1, w.Wh2, Brows, w.Rp, w.ZT1 + zoff, w.ZT2 + zoff, cc->nq, w.Rp, R, P, st);
+    else
+      rc = launch_gemm_f16x3_pair(w.Wh1, w.Wh2, Brows, w.Rp, w.ZT1 + zoff, w.ZT2 + zoff, cc->nq, w.Rp, R, P, st);
+    if (rc) return rc;
+    return large_launch_ctx_scatter(reinterpret_cast<const G*>(w.g_pred), Brows, (int)K, cc->period, cc->clen, g_fake_rows,
+                                    st);
+  }
   g3_count_tiles_pair(&P.job[0]);
   P.njobs = 1;
   P.ksplit = 1;
@@ -356,6 +422,41 @@ int large_shard_cost_bwd(const float* Cbar3rows, const float* XYcol, const float
                          float* gh_real_rows, float* gm_fake_part, void* ws, size_t ws_bytes, cudaStream_t st) {
   return shard_cost_bwd(Cbar3rows, XYcol, YYcol, B, K, row0, Brows, h_fake, m_real, h_real, m_fake, T, J, s, g_fake_rows,
                         gh_fake_rows, gm_real_part, gh_real_rows, gm_fake_part, ws, ws_bytes, st);
+}
+
+int large_shard_cost_fwd_ctx(const float* real, const float* fake, int B, long long K, int row0, int Brows,
+                             const float* h_fake, const float* m_real, const float* h_real, const float* m_fake, int T,
+                             int J, float s, float* C3rows, void* ws, size_t ws_bytes, long long period, long long clen,
+                             cudaStream_t st) {
+  const CtxCols cc(K, period, clen);
+  return shard_cost_fwd(real, fake, B, K, row0, Brows, h_fake, m_real, h_real, m_fake, T, J, s, C3rows, ws, ws_bytes, st,
+                        &cc);
+}
+int large_shard_cost_fwd_ctx(const uint16_t* real, const uint16_t* fake, int B, long long K, int row0, int Brows,
+                             const float* h_fake, const float* m_real, const float* h_real, const float* m_fake, int T,
+                             int J, float s, float* C3rows, void* ws, size_t ws_bytes, long long period, long long clen,
+                             cudaStream_t st) {
+  const CtxCols cc(K, period, clen);
+  return shard_cost_fwd(real, fake, B, K, row0, Brows, h_fake, m_real, h_real, m_fake, T, J, s, C3rows, ws, ws_bytes, st,
+                        &cc);
+}
+int large_shard_cost_bwd_ctx(const float* Cbar3rows, const float* XYcol, const float* YYcol, int B, long long K, int row0,
+                             int Brows, const float* h_fake, const float* m_real, const float* h_real,
+                             const float* m_fake, int T, int J, float s, float* g_fake_rows, float* gh_fake_rows,
+                             float* gm_real_part, float* gh_real_rows, float* gm_fake_part, void* ws, size_t ws_bytes,
+                             long long period, long long clen, cudaStream_t st) {
+  const CtxCols cc(K, period, clen);
+  return shard_cost_bwd(Cbar3rows, XYcol, YYcol, B, K, row0, Brows, h_fake, m_real, h_real, m_fake, T, J, s, g_fake_rows,
+                        gh_fake_rows, gm_real_part, gh_real_rows, gm_fake_part, ws, ws_bytes, st, &cc);
+}
+int large_shard_cost_bwd_ctx(const float* Cbar3rows, const float* XYcol, const float* YYcol, int B, long long K, int row0,
+                             int Brows, const float* h_fake, const float* m_real, const float* h_real,
+                             const float* m_fake, int T, int J, float s, uint16_t* g_fake_rows, float* gh_fake_rows,
+                             float* gm_real_part, float* gh_real_rows, float* gm_fake_part, void* ws, size_t ws_bytes,
+                             long long period, long long clen, cudaStream_t st) {
+  const CtxCols cc(K, period, clen);
+  return shard_cost_bwd(Cbar3rows, XYcol, YYcol, B, K, row0, Brows, h_fake, m_real, h_real, m_fake, T, J, s, g_fake_rows,
+                        gh_fake_rows, gm_real_part, gh_real_rows, gm_fake_part, ws, ws_bytes, st, &cc);
 }
 
 }  // namespace kccot

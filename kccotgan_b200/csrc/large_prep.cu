@@ -479,6 +479,147 @@ __global__ void __launch_bounds__(256) w_convert_kernel(const float* __restrict_
   }
   if (blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == 0) scal[kScalGradAlpha] = pow2f(-e) * scal[kScalZinv];
 }
+
+// ---- shared context frames (row shards) ------------------------------------------------------------
+// Column c of the video rows is a CONTEXT column when c % period < clen: x (real) and y (fake) hold the same values
+// there, so y's are never read and x's stand in for them.  The split writes the columns permuted (the Gram and the
+// row norms do not depend on the column order): the nc context columns first, zero-padded to Kcp (a multiple of 64),
+// then the nq predicted columns, zero-padded as well.  K < 2^31 (checked by the callers): 32-bit column arithmetic.
+__device__ __forceinline__ float ld_video(const float* __restrict__ p, long long i) { return p[i]; }
+__device__ __forceinline__ float ld_video(const uint16_t* __restrict__ p, long long i) { return ld1(p, i); }
+__device__ __forceinline__ float4 ld_video4(const float* __restrict__ p) { return *reinterpret_cast<const float4*>(p); }
+__device__ __forceinline__ float4 ld_video4(const uint16_t* __restrict__ p) {
+  return widen_bf16x4(*reinterpret_cast<const uint2*>(p));
+}
+
+// colsum_part_kernel with y's context columns read from x: the same sums, in the same order, on inputs that keep the
+// promise
+template <typename T>
+__global__ void __launch_bounds__(128) colsum_part_ctx_kernel(const T* __restrict__ x, const T* __restrict__ y, int Bx,
+                                                              int By, long long K, int period, int clen,
+                                                              int rows_per_seg, float* __restrict__ part,
+                                                              unsigned* __restrict__ absmax) {
+  const long long k = (long long)blockIdx.x * 128 + threadIdx.x;
+  const int R = Bx + By;
+  const int r0 = blockIdx.y * rows_per_seg, r1 = min(R, r0 + rows_per_seg);
+  float acc = 0.f, mx = 0.f;
+  if (k < K) {
+    const T* yk = ((int)k % period < clen) ? x : y;
+    int r = r0;
+    for (; r + 4 <= r1; r += 4) {
+      float v[4];
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        const int rr = r + u;
+        v[u] = (rr < Bx) ? ld_video(x, (long long)rr * K + k) : ld_video(yk, (long long)(rr - Bx) * K + k);
+      }
+#pragma unroll
+      for (int u = 0; u < 4; ++u) { acc += v[u]; mx = fmaxf(mx, fabsf(v[u])); }
+    }
+    for (; r < r1; ++r) {
+      const float v = (r < Bx) ? ld_video(x, (long long)r * K + k) : ld_video(yk, (long long)(r - Bx) * K + k);
+      acc += v;
+      mx = fmaxf(mx, fabsf(v));
+    }
+    part[(long long)blockIdx.y * K + k] = acc;
+  }
+  mx = warp_max(mx);
+  if ((threadIdx.x & 31) == 0 && mx > 0.f && mx < 3.0e38f) atomicMax(absmax, __float_as_uint(mx));
+}
+
+// video column of permuted column j, or -1 for a padding column
+__device__ __forceinline__ int ctx_source_col(int j, int period, int clen, int nc, int nq, int Kcp) {
+  if (j < Kcp) return j < nc ? (j / clen) * period + j % clen : -1;
+  j -= Kcp;
+  const int pl = period - clen;
+  return j < nq ? (j / pl) * period + clen + j % pl : -1;
+}
+
+// split_kernel over the permuted columns: grid (Kpp / 64, ceil(R / 64)), Zh [R][Kpp], ZT [Kpp][Rp].  A 64-column tile
+// lies wholly in the context part or wholly in the predicted part (Kcp is a multiple of 64).
+template <typename T>
+__global__ void __launch_bounds__(256) split_ctx_kernel(const T* __restrict__ x, const T* __restrict__ y, int Bx, int By,
+                                                        long long K, int period, int clen, int Kcp, long long Kpp,
+                                                        int Rp, const float* __restrict__ mean,
+                                                        const float* __restrict__ scal, __half* __restrict__ Zh1,
+                                                        __half* __restrict__ Zh2, __half* __restrict__ ZT1,
+                                                        __half* __restrict__ ZT2) {
+  __shared__ __half t1[64][72], t2[64][72];                 // [column][row] for the transposed copy
+  const int R = Bx + By;
+  const int nc = (int)(K / period) * clen, nq = (int)K - nc;
+  const int c0 = blockIdx.x * 64;
+  const int r0 = blockIdx.y * 64;
+  const int t = threadIdx.x;
+  const int cg = (t & 15) * 4;
+  const float zs = scal[kScalZscale];
+  const T* yt = c0 < Kcp ? x : y;                           // source of the fake rows in this tile
+  int src[4];
+  float m[4];
+#pragma unroll
+  for (int e = 0; e < 4; ++e) {
+    src[e] = ctx_source_col(c0 + cg + e, period, clen, nc, nq, Kcp);
+    m[e] = src[e] >= 0 ? mean[src[e]] : 0.f;
+  }
+  // four permuted columns are four consecutive video columns when both part lengths are multiples of 4
+  const bool vec = ((clen & 3) == 0) && ((period & 3) == 0) && src[0] >= 0 &&
+                   ((reinterpret_cast<uintptr_t>(x) & (4 * sizeof(T) - 1)) == 0) &&
+                   ((reinterpret_cast<uintptr_t>(y) & (4 * sizeof(T) - 1)) == 0);
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int rl = (t >> 4) + 16 * i;
+    const int r = r0 + rl;
+    float v[4] = {0.f, 0.f, 0.f, 0.f};
+    if (r < R) {
+      const T* row = (r < Bx) ? x + (long long)r * K : yt + (long long)(r - Bx) * K;
+      if (vec) {
+        const float4 q = ld_video4(row + src[0]);
+        v[0] = q.x; v[1] = q.y; v[2] = q.z; v[3] = q.w;
+      } else {
+#pragma unroll
+        for (int e = 0; e < 4; ++e)
+          if (src[e] >= 0) v[e] = ld_video(row, src[e]);
+      }
+    }
+    __half h1[4], h2[4];
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      const bool in = (r < R) && src[e] >= 0;
+      const float z = in ? (v[e] - m[e]) * zs : 0.f;
+      h1[e] = __float2half_rn(z);
+      h2[e] = __float2half_rn(z - __half2float(h1[e]));
+    }
+    if (r < R) {
+      *reinterpret_cast<uint2*>(Zh1 + (long long)r * Kpp + c0 + cg) = *reinterpret_cast<const uint2*>(h1);
+      *reinterpret_cast<uint2*>(Zh2 + (long long)r * Kpp + c0 + cg) = *reinterpret_cast<const uint2*>(h2);
+    }
+#pragma unroll
+    for (int e = 0; e < 4; ++e) { t1[cg + e][rl] = h1[e]; t2[cg + e][rl] = h2[e]; }
+  }
+  __syncthreads();
+  // transposed rows: 4 threads per column, 16 stacked rows (32 bytes) each
+  const int c = t >> 2, seg = (t & 3) * 16;
+  if (r0 + seg < Rp) {                                      // Rp is a multiple of 64
+    const uint4* s1 = reinterpret_cast<const uint4*>(&t1[c][seg]);
+    const uint4* s2 = reinterpret_cast<const uint4*>(&t2[c][seg]);
+    uint4* d1 = reinterpret_cast<uint4*>(ZT1 + (c0 + c) * (long long)Rp + r0 + seg);
+    uint4* d2 = reinterpret_cast<uint4*>(ZT2 + (c0 + c) * (long long)Rp + r0 + seg);
+    d1[0] = s1[0]; d1[1] = s1[1];
+    d2[0] = s2[0]; d2[1] = s2[1];
+  }
+}
+
+// gradient rows of the predicted columns, g_pred [nrows][nq] (fp32 or bf16 bits), back to the video columns of
+// g [nrows][K]; the context columns are written as zero.  grid (ceil(K / 256), nrows)
+template <typename G>
+__global__ void __launch_bounds__(256) ctx_scatter_kernel(const G* __restrict__ g_pred, int K, int period, int clen,
+                                                          G* __restrict__ g) {
+  const int c = blockIdx.x * 256 + threadIdx.x;
+  if (c >= K) return;
+  const int pl = period - clen, nq = K / period * pl;
+  const int ph = c % period;
+  const long long r = blockIdx.y;
+  g[r * K + c] = ph < clen ? G(0) : g_pred[r * nq + (c / period) * pl + (ph - clen)];
+}
 }  // namespace
 
 // ------------------------------------------------------------------------------------------------
@@ -542,6 +683,65 @@ int large_launch_split(const uint16_t* x, const uint16_t* y, int Bx, int By, lon
                        const float* mean, const float* scal, __half* Zh1, __half* Zh2, __half* ZT1, __half* ZT2,
                        cudaStream_t st) {
   return launch_split(x, y, Bx, By, K, Kp, Rp, mean, scal, Zh1, Zh2, ZT1, ZT2, st);
+}
+
+namespace {
+template <typename T>
+int launch_stats_ctx(const T* x, const T* y, int B, long long K, int period, int clen, int nseg, float* part, float* mean,
+                     float* scal, cudaStream_t st) {
+  const int R = 2 * B;
+  const int rps = (R + nseg - 1) / nseg;
+  KCCOT_CUDA(cudaMemsetAsync(scal, 0, kScalCount * sizeof(float), st));
+  colsum_part_ctx_kernel<T><<<dim3((unsigned)((K + 127) / 128), nseg), 128, 0, st>>>(
+      x, y, B, B, K, period, clen, rps, part, reinterpret_cast<unsigned*>(scal) + kScalAbsmax);
+  KCCOT_LAUNCH_CHECK();
+  colmean_kernel<<<(unsigned)((K + 255) / 256), 256, 0, st>>>(part, (R + rps - 1) / rps, K, R, mean, scal);
+  KCCOT_LAUNCH_CHECK();
+  return KCCOT_OK;
+}
+
+template <typename T>
+int launch_split_ctx(const T* x, const T* y, int B, long long K, int period, int clen, int Kcp, long long Kpp, int Rp,
+                     const float* mean, const float* scal, __half* Zh1, __half* Zh2, __half* ZT1, __half* ZT2,
+                     cudaStream_t st) {
+  split_ctx_kernel<T><<<dim3((unsigned)(Kpp / 64), (2 * B + 63) / 64), 256, 0, st>>>(
+      x, y, B, B, K, period, clen, Kcp, Kpp, Rp, mean, scal, Zh1, Zh2, ZT1, ZT2);
+  KCCOT_LAUNCH_CHECK();
+  return KCCOT_OK;
+}
+
+template <typename G>
+int launch_ctx_scatter(const G* g_pred, int nrows, int K, int period, int clen, G* g, cudaStream_t st) {
+  ctx_scatter_kernel<G><<<dim3((unsigned)((K + 255) / 256), nrows), 256, 0, st>>>(g_pred, K, period, clen, g);
+  KCCOT_LAUNCH_CHECK();
+  return KCCOT_OK;
+}
+}  // namespace
+
+int large_launch_stats_ctx(const float* x, const float* y, int B, long long K, int period, int clen, int nseg,
+                           float* part, float* mean, float* scal, cudaStream_t st) {
+  return launch_stats_ctx(x, y, B, K, period, clen, nseg, part, mean, scal, st);
+}
+int large_launch_stats_ctx(const uint16_t* x, const uint16_t* y, int B, long long K, int period, int clen, int nseg,
+                           float* part, float* mean, float* scal, cudaStream_t st) {
+  return launch_stats_ctx(x, y, B, K, period, clen, nseg, part, mean, scal, st);
+}
+int large_launch_split_ctx(const float* x, const float* y, int B, long long K, int period, int clen, int Kcp,
+                           long long Kpp, int Rp, const float* mean, const float* scal, __half* Zh1, __half* Zh2,
+                           __half* ZT1, __half* ZT2, cudaStream_t st) {
+  return launch_split_ctx(x, y, B, K, period, clen, Kcp, Kpp, Rp, mean, scal, Zh1, Zh2, ZT1, ZT2, st);
+}
+int large_launch_split_ctx(const uint16_t* x, const uint16_t* y, int B, long long K, int period, int clen, int Kcp,
+                           long long Kpp, int Rp, const float* mean, const float* scal, __half* Zh1, __half* Zh2,
+                           __half* ZT1, __half* ZT2, cudaStream_t st) {
+  return launch_split_ctx(x, y, B, K, period, clen, Kcp, Kpp, Rp, mean, scal, Zh1, Zh2, ZT1, ZT2, st);
+}
+int large_launch_ctx_scatter(const float* g_pred, int nrows, int K, int period, int clen, float* g, cudaStream_t st) {
+  return launch_ctx_scatter(g_pred, nrows, K, period, clen, g, st);
+}
+int large_launch_ctx_scatter(const uint16_t* g_pred, int nrows, int K, int period, int clen, uint16_t* g,
+                             cudaStream_t st) {
+  return launch_ctx_scatter(g_pred, nrows, K, period, clen, g, st);
 }
 
 int large_launch_rownorm(const __half* Zh1, const __half* Zh2, int R, long long K, long long Kp, float* norms,

@@ -90,6 +90,88 @@ int kccot_shard_cost_bwd_bf16(const float* Cbar3rows, const float* XYcol, const 
                               gh_fake_rows, gm_real_part, gh_real_rows, gm_fake_part, ws, ws_bytes, (cudaStream_t)stream);
 }
 
+// ---- shared context frames -----------------------------------------------------------------------------------------
+// (ctx_period, ctx_len) with ctx_len == 0 is no hint (the plain entries run); otherwise 0 < ctx_len < ctx_period and
+// K % ctx_period == 0.  The column arithmetic of the hinted kernels is 32-bit.
+static bool ctx_hint_ok(long long K, long long period, long long len) {
+  if (period < 0 || len < 0 || (period == 0 && len != 0)) return false;
+  return period == 0 || (len < period && K % period == 0 && K < (1LL << 31) - 64);
+}
+#define KCCOT_CHECK_CTX(K, period, len) \
+  KCCOT_CHECK_ARG(ctx_hint_ok(K, period, len), "bad shared-context hint: period=%lld len=%lld K=%lld", period, len, K)
+
+size_t kccot_shard_cost_workspace_bytes_ctx(int B, long long K, int Brows, long long ctx_period, long long ctx_len) {
+  if (B < 1 || K < 1 || Brows < 1 || !ctx_hint_ok(K, ctx_period, ctx_len)) return 0;
+  return ctx_len == 0 ? large_shard_ws_bytes(B, K, Brows) : large_shard_ws_bytes_ctx(B, K, Brows, ctx_period, ctx_len);
+}
+
+int kccot_shard_cost_fwd_ctx(const float* real, const float* fake, int B, long long K, int row0, int Brows,
+                             const float* h_fake, const float* m_real, const float* h_real, const float* m_fake, int T,
+                             int J, float s, float* C3rows, void* ws, size_t ws_bytes, void* stream,
+                             long long ctx_period, long long ctx_len) {
+  KCCOT_CHECK_ARG(real && fake && h_fake && m_real && h_real && m_fake && C3rows && ws, "null pointer");
+  KCCOT_CHECK_ARG(B >= 1 && K >= 1 && T >= 2 && J >= 1, "bad sizes");
+  KCCOT_CHECK_ARG(row0 >= 0 && Brows >= 1 && row0 + Brows <= B, "bad row range [%d, %d) of %d", row0, row0 + Brows, B);
+  KCCOT_CHECK_CTX(K, ctx_period, ctx_len);
+  if (ctx_len == 0)
+    return kccot_shard_cost_fwd(real, fake, B, K, row0, Brows, h_fake, m_real, h_real, m_fake, T, J, s, C3rows, ws,
+                                ws_bytes, stream);
+  return large_shard_cost_fwd_ctx(real, fake, B, K, row0, Brows, h_fake, m_real, h_real, m_fake, T, J, s, C3rows, ws,
+                                  ws_bytes, ctx_period, ctx_len, (cudaStream_t)stream);
+}
+
+int kccot_shard_cost_bwd_ctx(const float* Cbar3rows, const float* XYcol, const float* YYcol, int B, long long K, int row0,
+                             int Brows, const float* h_fake, const float* m_real, const float* h_real,
+                             const float* m_fake, int T, int J, float s, float* g_fake_rows, float* gh_fake_rows,
+                             float* gm_real_part, float* gh_real_rows, float* gm_fake_part, void* ws, size_t ws_bytes,
+                             void* stream, long long ctx_period, long long ctx_len) {
+  KCCOT_CHECK_ARG(Cbar3rows && XYcol && YYcol && h_fake && m_real && h_real && m_fake && ws, "null pointer");
+  KCCOT_CHECK_ARG(B >= 1 && K >= 1 && T >= 2 && J >= 1, "bad sizes");
+  KCCOT_CHECK_ARG(row0 >= 0 && Brows >= 1 && row0 + Brows <= B, "bad row range [%d, %d) of %d", row0, row0 + Brows, B);
+  KCCOT_CHECK_CTX(K, ctx_period, ctx_len);
+  if (ctx_len == 0)
+    return kccot_shard_cost_bwd(Cbar3rows, XYcol, YYcol, B, K, row0, Brows, h_fake, m_real, h_real, m_fake, T, J, s,
+                                g_fake_rows, gh_fake_rows, gm_real_part, gh_real_rows, gm_fake_part, ws, ws_bytes, stream);
+  return large_shard_cost_bwd_ctx(Cbar3rows, XYcol, YYcol, B, K, row0, Brows, h_fake, m_real, h_real, m_fake, T, J, s,
+                                  g_fake_rows, gh_fake_rows, gm_real_part, gh_real_rows, gm_fake_part, ws, ws_bytes,
+                                  ctx_period, ctx_len, (cudaStream_t)stream);
+}
+
+int kccot_shard_cost_fwd_bf16_ctx(const uint16_t* real, const uint16_t* fake, int B, long long K, int row0, int Brows,
+                                  const float* h_fake, const float* m_real, const float* h_real, const float* m_fake,
+                                  int T, int J, float s, float* C3rows, void* ws, size_t ws_bytes, void* stream,
+                                  long long ctx_period, long long ctx_len) {
+  KCCOT_CHECK_ARG(real && fake && h_fake && m_real && h_real && m_fake && C3rows && ws, "null pointer");
+  KCCOT_CHECK_ARG(B >= 1 && K >= 1 && T >= 2 && J >= 1, "bad sizes");
+  KCCOT_CHECK_ARG(row0 >= 0 && Brows >= 1 && row0 + Brows <= B, "bad row range [%d, %d) of %d", row0, row0 + Brows, B);
+  KCCOT_CHECK_ARG(aligned16(real) && aligned16(fake), "bf16 videos must be 16-byte aligned");
+  KCCOT_CHECK_CTX(K, ctx_period, ctx_len);
+  if (ctx_len == 0)
+    return kccot_shard_cost_fwd_bf16(real, fake, B, K, row0, Brows, h_fake, m_real, h_real, m_fake, T, J, s, C3rows, ws,
+                                     ws_bytes, stream);
+  return large_shard_cost_fwd_ctx(real, fake, B, K, row0, Brows, h_fake, m_real, h_real, m_fake, T, J, s, C3rows, ws,
+                                  ws_bytes, ctx_period, ctx_len, (cudaStream_t)stream);
+}
+
+int kccot_shard_cost_bwd_bf16_ctx(const float* Cbar3rows, const float* XYcol, const float* YYcol, int B, long long K,
+                                  int row0, int Brows, const float* h_fake, const float* m_real, const float* h_real,
+                                  const float* m_fake, int T, int J, float s, uint16_t* g_fake_rows, float* gh_fake_rows,
+                                  float* gm_real_part, float* gh_real_rows, float* gm_fake_part, void* ws,
+                                  size_t ws_bytes, void* stream, long long ctx_period, long long ctx_len) {
+  KCCOT_CHECK_ARG(Cbar3rows && XYcol && YYcol && h_fake && m_real && h_real && m_fake && ws, "null pointer");
+  KCCOT_CHECK_ARG(B >= 1 && K >= 1 && T >= 2 && J >= 1, "bad sizes");
+  KCCOT_CHECK_ARG(row0 >= 0 && Brows >= 1 && row0 + Brows <= B, "bad row range [%d, %d) of %d", row0, row0 + Brows, B);
+  KCCOT_CHECK_ARG(aligned16(g_fake_rows), "bf16 gradient rows must be 16-byte aligned");
+  KCCOT_CHECK_CTX(K, ctx_period, ctx_len);
+  if (ctx_len == 0)
+    return kccot_shard_cost_bwd_bf16(Cbar3rows, XYcol, YYcol, B, K, row0, Brows, h_fake, m_real, h_real, m_fake, T, J, s,
+                                     g_fake_rows, gh_fake_rows, gm_real_part, gh_real_rows, gm_fake_part, ws, ws_bytes,
+                                     stream);
+  return large_shard_cost_bwd_ctx(Cbar3rows, XYcol, YYcol, B, K, row0, Brows, h_fake, m_real, h_real, m_fake, T, J, s,
+                                  g_fake_rows, gh_fake_rows, gm_real_part, gh_real_rows, gm_fake_part, ws, ws_bytes,
+                                  ctx_period, ctx_len, (cudaStream_t)stream);
+}
+
 size_t kccot_shard_sinkhorn_workspace_bytes(int np, int Brows, int B, int L) {
   if (np < 1 || Brows < 1 || B < 1 || L < 1 || !persist_supported(Brows, B, L)) return 0;
   return persist_workspace_bytes(np, Brows, B, L);

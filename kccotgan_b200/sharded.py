@@ -74,16 +74,28 @@ class CudaMixedShardBackend:
     videos and h / m must be CUDA tensors on this backend's device with [B, K] and [B, T, J] elements.  Two bf16
     videos go to the bf16 entry points (a view that is not 16-byte aligned is cloned) and `cost_bwd` then returns the
     `fake` gradient rows in bf16: the fp32 rows on the widened videos, rounded to nearest even.  A bf16 video next to
-    an fp32 one, and bf16 h / m, are widened (exact).  Every other dtype is rejected."""
+    an fp32 one, and bf16 h / m, are widened (exact).  Every other dtype is rejected.
 
-    def __init__(self, B, K, T, J, s, eps, L, row0, Brows, dev, group):
+    `ctx = (ctx_period, ctx_len)` is the shared-context hint of include/kccot.h, passed to the `_ctx` entry points: with
+    ctx_len > 0 the columns c with c % ctx_period < ctx_len of `fake` are never read (the `real` values stand in) and
+    the `fake` gradient rows are zero there; with ctx_len = 0 they run the plain computation.  (0, 0), the default,
+    calls the plain entry points."""
+
+    def __init__(self, B, K, T, J, s, eps, L, row0, Brows, dev, group, ctx=(0, 0)):
         self.B, self.K, self.T, self.J, self.s, self.eps, self.L = B, K, T, J, float(s), float(eps), int(L)
         self.row0, self.Brows, self.dev, self.group = row0, Brows, dev, group
+        self.ctx = (int(ctx[0]), int(ctx[1]))
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
         lib = _lib.load()
         f32 = dict(dtype=torch.float32, device=dev)
-        self.ws_cost = torch.empty(lib.kccot_shard_cost_workspace_bytes(B, K, Brows), dtype=torch.uint8, device=dev)
+        if self.ctx != (0, 0):
+            nb = lib.kccot_shard_cost_workspace_bytes_ctx(B, K, Brows, *self.ctx)
+            if nb == 0:
+                raise ValueError(f"bad shared-context hint (period, len) = {self.ctx} for K = {K}")
+        else:
+            nb = lib.kccot_shard_cost_workspace_bytes(B, K, Brows)
+        self.ws_cost = torch.empty(nb, dtype=torch.uint8, device=dev)
         nb = lib.kccot_shard_sinkhorn_workspace_bytes(3, Brows, B, self.L)
         if nb == 0:
             raise ValueError(f"row-sharded Sinkhorn needs 64 < B <= 8192 and B % 4 == 0, got B={B}")
@@ -125,10 +137,14 @@ class CudaMixedShardBackend:
         h_fake, m_real, h_real, m_fake = hm
         self.inputs = (real, fake, h_fake, m_real, h_real, m_fake)
         p = self._p
+        args = (p(real), p(fake), self.B, self.K, self.row0, self.Brows, p(h_fake), p(m_real), p(h_real), p(m_fake),
+                self.T, self.J, self.s, p(self.C3), p(self.ws_cost), self.ws_cost.numel(), self._st())
+        name = "kccot_shard_cost_fwd_bf16" if self.bf16 else "kccot_shard_cost_fwd"
         with torch.cuda.device(self.dev):
-            _lib.call("kccot_shard_cost_fwd_bf16" if self.bf16 else "kccot_shard_cost_fwd", p(real), p(fake), self.B,
-                      self.K, self.row0, self.Brows, p(h_fake), p(m_real), p(h_real), p(m_fake), self.T, self.J, self.s,
-                      p(self.C3), p(self.ws_cost), self.ws_cost.numel(), self._st())
+            if self.ctx != (0, 0):
+                _lib.call(name + "_ctx", *args, *self.ctx)
+            else:
+                _lib.call(name, *args)
             _lib.call("kccot_shard_local_min", p(self.C3), 3, self.Brows, self.B, p(self.shift), self._st())
         return self.shift
 
@@ -159,10 +175,15 @@ class CudaMixedShardBackend:
         gh_real = torch.empty((self.Brows, self.T, self.J), **f32)
         gm_real = torch.empty((self.B, self.T, self.J), **f32)
         gm_fake = torch.empty((self.B, self.T, self.J), **f32)
+        args = (p(self.Cbar3), p(XYcol), p(YYcol), self.B, self.K, self.row0, self.Brows, p(h_fake), p(m_real),
+                p(h_real), p(m_fake), self.T, self.J, self.s, p(g_fake), p(gh_fake), p(gm_real), p(gh_real), p(gm_fake),
+                p(self.ws_cost), self.ws_cost.numel(), self._st())
+        name = "kccot_shard_cost_bwd_bf16" if self.bf16 else "kccot_shard_cost_bwd"
         with torch.cuda.device(self.dev):
-            _lib.call("kccot_shard_cost_bwd_bf16" if self.bf16 else "kccot_shard_cost_bwd", p(self.Cbar3), p(XYcol), p(YYcol), self.B, self.K, self.row0, self.Brows,
-                      p(h_fake), p(m_real), p(h_real), p(m_fake), self.T, self.J, self.s, p(g_fake), p(gh_fake), p(gm_real),
-                      p(gh_real), p(gm_fake), p(self.ws_cost), self.ws_cost.numel(), self._st())
+            if self.ctx != (0, 0):
+                _lib.call(name + "_ctx", *args, *self.ctx)
+            else:
+                _lib.call(name, *args)
         return g_fake, gh_fake, gm_real, gh_real, gm_fake
 
 
@@ -179,12 +200,20 @@ class ShardedMixedLoss:
     are exactly those of fp32 videos widened from them: loss, terms and the h / m gradients bit for bit, the `fake`
     rows the fp32 rows rounded to nearest even, with no fp32 copy of a video.  bf16 m gradients are rounded after
     the fp32 all-reduce, so every rank holds the same bits.
+    `ctx_frames` > 0 states that the first ctx_frames frames of `fake` are those of `real` (kernel_train.py:268,
+    fake = concat(real_in, fake_pred)).  forward() then takes [B, H, T, W, C] videos, never reads fake's context
+    frames, and computes their share of the three cost blocks once; the result equals the plain one within
+    floating-point tolerance, and the `fake` gradient is that of the predicted frames, zero on the context frames.
     Collectives of one evaluation (all small except the two [Brows, B] all-to-alls): MIN of 3 floats, SUM of 6
     floats, all-to-all of Cbar_xy / Cbar_yy, SUM of two [B, T, J]; the 2 x L x 3 column-sum exchanges of the
     Sinkhorn iterations happen inside the persistent kernels.
     """
 
-    def __init__(self, B, K, T, J, scaling_coef, eps=1.0, L=100, group=None, device=None, backend=None):
+    def __init__(self, B, K, T, J, scaling_coef, eps=1.0, L=100, group=None, device=None, backend=None, ctx_frames=0):
+        if not 0 <= int(ctx_frames) < int(T):
+            raise ValueError(f"ctx_frames must be in [0, T = {T}), got {ctx_frames}")
+        if ctx_frames and backend is not None:
+            raise ValueError("ctx_frames > 0 needs the CUDA backend (a user-supplied backend takes no shared-context hint)")
         self.group = group
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
@@ -194,8 +223,12 @@ class ShardedMixedLoss:
         self.s, self.eps, self.L = float(scaling_coef), float(eps), int(L)
         self.row0, r1 = row_range(B, self.rank, self.world)
         self.Brows = r1 - self.row0
-        self.be = backend if backend is not None else CudaMixedShardBackend(
-            self.B, self.K, self.T, self.J, self.s, self.eps, self.L, self.row0, self.Brows, device, group)
+        self.ctx_frames, self.device = int(ctx_frames), device
+        if self.ctx_frames:
+            self.be = None                  # the hint needs the videos' frame size: the backend is made by forward()
+        else:
+            self.be = backend if backend is not None else CudaMixedShardBackend(
+                self.B, self.K, self.T, self.J, self.s, self.eps, self.L, self.row0, self.Brows, device, group)
 
     def _allreduce(self, t, op):
         if self.world > 1:
@@ -217,6 +250,8 @@ class ShardedMixedLoss:
         if flat[0].shape[1] != self.K:
             raise ValueError(f"expected videos with {self.K} elements per sample, got {flat[0].shape[1]}")
         self.fake_shape = fake.shape
+        if self.ctx_frames:
+            self._ctx_backend(real, fake)
         self.dtypes = [t.dtype for t in (fake, h_fake, m_real, h_real, m_fake)]
         shift = self.be.cost_fwd(flat[0].contiguous(), flat[1].contiguous(), h_fake.contiguous(), m_real.contiguous(),
                                  h_real.contiguous(), m_fake.contiguous())
@@ -227,6 +262,20 @@ class ShardedMixedLoss:
         self.terms = part[:, 1] / kscale + shift * part[:, 0]   # xy, xx, yy
         self.loss = 2.0 * self.terms[0] - self.terms[1] - self.terms[2]        # gan_utils.py:225
         return self.loss, self.terms
+
+    def _ctx_backend(self, real, fake):
+        """(ctx_period, ctx_len) = (T*W*C, ctx_frames*W*C) of [B, H, T, W, C] videos; a backend for that hint"""
+        for n, v in (("real", real), ("fake", fake)):
+            if v.dim() != 5 or v.shape[0] != self.B or v.shape[2] != self.T:
+                raise ValueError(f"{n}: ctx_frames > 0 needs [B, H, T, W, C] videos with B = {self.B}, T = {self.T}, "
+                                 f"got shape {tuple(v.shape)}")
+        if real.shape != fake.shape:
+            raise ValueError(f"real {tuple(real.shape)} and fake {tuple(fake.shape)} differ in shape")
+        frame = real.shape[3] * real.shape[4]
+        ctx = (self.T * frame, self.ctx_frames * frame)
+        if self.be is None or self.be.ctx != ctx:
+            self.be = CudaMixedShardBackend(self.B, self.K, self.T, self.J, self.s, self.eps, self.L, self.row0,
+                                            self.Brows, self.device, self.group, ctx=ctx)
 
     def backward(self, gloss=1.0):
         g3 = torch.tensor([2.0 * gloss, -gloss, -gloss], dtype=self.terms.dtype, device=self.terms.device)
