@@ -293,6 +293,22 @@ int kccot_pm_fwd(const float* M, int B, int T, int J, float reg_lam, float s, fl
 int kccot_pm_bwd(const float* M, int B, int T, int J, float reg_lam, float s, const float* stats,
                  const float* gpm /* device scalar */, float* gM, void* stream);
 
+/* Batched independent problems — nprob penalties in one call per direction (config 4's discriminator step: one p_M per
+ * problem; folding the problems into the batch axis would give one penalty over all of them, since the mean, sigma_j
+ * and A_tj are taken over the batch).  M [nprob,B,T,J] contiguous; pm [nprob]; stats [nprob, 2*J + (T-1)*J]
+ * (caller-owned, written by the forward, read by the backward; row p as in kccot_pm_fwd); gpm [nprob] on the device;
+ * gM [nprob,B,T,J].  The forward runs one CTA per problem, the backward one thread per element of the batch.
+ * Contract, for each problem p against kccot_pm_fwd / _bwd called on M[p] with upstream gradient gpm[p]: pm[p], stats
+ * row p and gM[p] are bit-identical (both sides run the same instructions in the same order).  A problem whose M is
+ * constant along some j (sigma_j = 0) takes the single call's sigma_j = 0 branch and changes no other problem's numbers.
+ * The argument checks are the single entries' (null pointers, B >= 1, T >= 2, J >= 1, and in the forward the
+ * shared-memory cap on T*J) plus 1 <= nprob <= 65535, all KCCOT_EINVAL and all made before any CUDA call.  Both calls
+ * only enqueue work (no allocation, no host synchronisation) and are graph-capturable. */
+int kccot_pm_batched_fwd(const float* M, int nprob, int B, int T, int J, float reg_lam, float s, float* pm,
+                         float* stats, void* stream);
+int kccot_pm_batched_bwd(const float* M, int nprob, int B, int T, int J, float reg_lam, float s, const float* stats,
+                         const float* gpm, float* gM, void* stream);
+
 /* ------------------------------------------------------------------------------------------
  * Gaussian kernel smoothing — data_utils.py:503-521 (temporal_convolution, mode 1) and
  * :552-582 (gaussian_convolution3D, mode 3).  x, out [B,H,T,W,C].  out = conv(x) / max(conv(x)) with REFLECT

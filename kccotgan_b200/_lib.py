@@ -74,6 +74,8 @@ SIGNATURES = {
                                        _P, _P, _P, _SZ, _I, _P, _LL, _LL]),
     "kccot_pm_fwd": (_I, [_P, _I, _I, _I, _F, _F, _P, _P, _P]),
     "kccot_pm_bwd": (_I, [_P, _I, _I, _I, _F, _F, _P, _P, _P, _P]),
+    "kccot_pm_batched_fwd": (_I, [_P, _I, _I, _I, _I, _F, _F, _P, _P, _P]),
+    "kccot_pm_batched_bwd": (_I, [_P, _I, _I, _I, _I, _F, _F, _P, _P, _P, _P]),
     "kccot_smooth_workspace_bytes": (_SZ, [_I, _I, _I, _I, _I, _I]),
     "kccot_smooth_fwd": (_I, [_I, _P, _I, _I, _I, _I, _I, _P, _I, _P, _I, _P, _P, _P, _SZ, _P]),
     "kccot_smooth_bwd": (_I, [_I, _P, _P, _P, _I, _I, _I, _I, _I, _P, _I, _P, _I, _P, _P, _SZ, _P]),

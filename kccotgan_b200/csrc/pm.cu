@@ -7,9 +7,10 @@ namespace kccot {
 namespace {
 constexpr int PT = 256;
 
-// one CTA; thread e walks column e of the [B, T*J] matrix (coalesced across e)
-__global__ void __launch_bounds__(PT) pm_fwd_kernel(const float* __restrict__ M, int B, int T, int J, float w,
-                                                    float* __restrict__ pm, float* __restrict__ stats) {
+// one CTA; thread e walks column e of the [B, T*J] matrix (coalesced across e).  The single and the batched
+// kernels inline this one body, so each problem of a batched call gets the single call's instructions and bits.
+__device__ __forceinline__ void pm_fwd_cta(const float* __restrict__ M, int B, int T, int J, float w,
+                                           float* __restrict__ pm, float* __restrict__ stats) {
   extern __shared__ float sh[];          // S[TJ] | V[TJ] | mean[J] | den[J] | red[32]
   const int TJ = T * J;
   float* S = sh;
@@ -67,12 +68,22 @@ __global__ void __launch_bounds__(PT) pm_fwd_kernel(const float* __restrict__ M,
   }
 }
 
-__global__ void __launch_bounds__(PT) pm_bwd_kernel(const float* __restrict__ M, int B, int T, int J, float w,
-                                                    const float* __restrict__ stats, const float* __restrict__ gpm,
-                                                    float* __restrict__ gM) {
-  const long long n = (long long)B * T * J;
-  const long long idx = (long long)blockIdx.x * PT + threadIdx.x;
-  if (idx >= n) return;
+__global__ void __launch_bounds__(PT) pm_fwd_kernel(const float* __restrict__ M, int B, int T, int J, float w,
+                                                    float* __restrict__ pm, float* __restrict__ stats) {
+  pm_fwd_cta(M, B, T, J, w, pm, stats);
+}
+
+// problem blockIdx.x of M [nprob, B, T, J]: pm[p] and stats row p [2J + (T-1)J]
+__global__ void __launch_bounds__(PT) pm_batched_fwd_kernel(const float* __restrict__ M, int B, int T, int J, float w,
+                                                            float* __restrict__ pm, float* __restrict__ stats) {
+  const int p = blockIdx.x;
+  pm_fwd_cta(M + (long long)p * B * T * J, B, T, J, w, pm + p, stats + (long long)p * (2 * J + (T - 1) * J));
+}
+
+// element idx < B*T*J of one problem
+__device__ __forceinline__ void pm_bwd_elem(const float* __restrict__ M, int B, int T, int J, float w,
+                                            const float* __restrict__ stats, const float* __restrict__ gpm,
+                                            float* __restrict__ gM, long long idx) {
   const int j = (int)(idx % J), t = (int)((idx / J) % T);
   const float mu = stats[j], sd = stats[J + j], den = sd + 1e-6f;
   const float* A = stats + 2 * J;
@@ -87,6 +98,26 @@ __global__ void __launch_bounds__(PT) pm_bwd_kernel(const float* __restrict__ M,
   const float gsig = -absA / den;
   if (sd > 0.f) v += gsig * (M[idx] - mu) / ((float)B * (float)T * sd);
   gM[idx] = g * v;
+}
+
+__global__ void __launch_bounds__(PT) pm_bwd_kernel(const float* __restrict__ M, int B, int T, int J, float w,
+                                                    const float* __restrict__ stats, const float* __restrict__ gpm,
+                                                    float* __restrict__ gM) {
+  const long long n = (long long)B * T * J;
+  const long long idx = (long long)blockIdx.x * PT + threadIdx.x;
+  if (idx >= n) return;
+  pm_bwd_elem(M, B, T, J, w, stats, gpm, gM, idx);
+}
+
+// grid (ceil(B*T*J / PT), nprob): problem blockIdx.y reads its own stats row and gpm[p]
+__global__ void __launch_bounds__(PT) pm_batched_bwd_kernel(const float* __restrict__ M, int B, int T, int J, float w,
+                                                            const float* __restrict__ stats,
+                                                            const float* __restrict__ gpm, float* __restrict__ gM) {
+  const long long n = (long long)B * T * J;
+  const long long idx = (long long)blockIdx.x * PT + threadIdx.x;
+  if (idx >= n) return;
+  const int p = blockIdx.y;
+  pm_bwd_elem(M + p * n, B, T, J, w, stats + (long long)p * (2 * J + (T - 1) * J), gpm + p, gM + p * n, idx);
 }
 }  // namespace
 }  // namespace kccot
@@ -109,6 +140,28 @@ int kccot_pm_bwd(const float* M, int B, int T, int J, float reg_lam, float s, co
   KCCOT_CHECK_ARG(B >= 1 && T >= 2 && J >= 1, "bad sizes");
   const long long n = (long long)B * T * J;
   pm_bwd_kernel<<<(unsigned)((n + PT - 1) / PT), PT, 0, (cudaStream_t)stream>>>(M, B, T, J, reg_lam * s, stats, gpm, gM);
+  KCCOT_LAUNCH_CHECK();
+  return KCCOT_OK;
+}
+int kccot_pm_batched_fwd(const float* M, int nprob, int B, int T, int J, float reg_lam, float s, float* pm,
+                         float* stats, void* stream) {
+  KCCOT_CHECK_ARG(M && pm && stats, "null pointer");
+  KCCOT_CHECK_ARG(nprob >= 1 && nprob <= 65535, "nprob=%d outside 1..65535", nprob);
+  KCCOT_CHECK_ARG(B >= 1 && T >= 2 && J >= 1, "bad sizes B=%d T=%d J=%d", B, T, J);
+  const size_t smem = (size_t)(2 * T * J + 2 * J + 32) * sizeof(float);
+  KCCOT_CHECK_ARG(smem <= 48 * 1024, "T*J too large for the p_M kernel (%d)", T * J);
+  pm_batched_fwd_kernel<<<nprob, PT, smem, (cudaStream_t)stream>>>(M, B, T, J, reg_lam * s, pm, stats);
+  KCCOT_LAUNCH_CHECK();
+  return KCCOT_OK;
+}
+int kccot_pm_batched_bwd(const float* M, int nprob, int B, int T, int J, float reg_lam, float s, const float* stats,
+                         const float* gpm, float* gM, void* stream) {
+  KCCOT_CHECK_ARG(M && stats && gpm && gM, "null pointer");
+  KCCOT_CHECK_ARG(nprob >= 1 && nprob <= 65535, "nprob=%d outside 1..65535", nprob);
+  KCCOT_CHECK_ARG(B >= 1 && T >= 2 && J >= 1, "bad sizes B=%d T=%d J=%d", B, T, J);
+  const long long n = (long long)B * T * J;
+  const dim3 grid((unsigned)((n + PT - 1) / PT), (unsigned)nprob);
+  pm_batched_bwd_kernel<<<grid, PT, 0, (cudaStream_t)stream>>>(M, B, T, J, reg_lam * s, stats, gpm, gM);
   KCCOT_LAUNCH_CHECK();
   return KCCOT_OK;
 }

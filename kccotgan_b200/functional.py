@@ -7,7 +7,9 @@ of the library (the result is exactly the fp32 one on the widened videos, video 
 video next to an fp32 one, and bf16 h / m, are widened with .float() (exact).  Gradients come back in the dtype of
 their input.  The smoothing (SmoothFn) also takes bf16 videos: they run the bf16 entry points, whose output is the
 fp32 output on the widened video rounded to bf16, and whose gradient is bf16 (see kccot_smooth_fwd_bf16 in kccot.h).
-SmoothBatchedFn smooths nprob independent videos in one call, in fp32 or bf16 alike.
+SmoothBatchedFn smooths nprob independent videos in one call, in fp32 or bf16 alike.  MartingalePenaltyBatchedFn
+computes nprob independent penalties in one call; a bf16 M is widened with .float() (exact) and its gradient comes back
+in bf16.
 """
 import ctypes
 
@@ -427,6 +429,41 @@ class MartingalePenaltyFn(torch.autograd.Function):
         with torch.cuda.device(M.device):
             _lib.call("kccot_pm_bwd", _ptr(M), B, T, J, lam, s, _ptr(stats), _ptr(gpm), _ptr(gM), _stream(M.device))
         return gM, None, None
+
+
+class MartingalePenaltyBatchedFn(torch.autograd.Function):
+    """`nprob` independent penalties in one C-ABI call per direction (kccot_pm_batched_fwd / _bwd): M is
+    [nprob, B, T, J], the result [nprob], entry p the penalty of M[p] alone with the bits of a single call on it.  A bf16
+    M is widened with .float() (exact) and its gradient comes back in bf16."""
+
+    @staticmethod
+    def forward(ctx, M, reg_lam, s):
+        dtype = M.dtype if isinstance(M, torch.Tensor) else None
+        M = _check_hm(M, "M", 4)
+        P, B, T, J = M.shape
+        if T < 2:
+            raise ValueError(f"M needs at least 2 time steps, got shape {tuple(M.shape)}")
+        dev = M.device
+        pm = torch.empty((P,), dtype=torch.float32, device=dev)
+        stats = torch.empty((P, 2 * J + (T - 1) * J), dtype=torch.float32, device=dev)
+        with _on_device(dev):
+            _lib.call("kccot_pm_batched_fwd", _ptr(M), P, B, T, J, float(reg_lam), float(s), _ptr(pm), _ptr(stats),
+                      _stream(dev))
+        ctx.save_for_backward(M, stats)
+        ctx.meta = (float(reg_lam), float(s), dtype)
+        return pm
+
+    @staticmethod
+    def backward(ctx, gpm):
+        M, stats = ctx.saved_tensors
+        lam, s, dtype = ctx.meta
+        P, B, T, J = M.shape
+        gM = torch.empty_like(M)
+        gpm = gpm.reshape(P).float().contiguous()
+        with _on_device(M.device):
+            _lib.call("kccot_pm_batched_bwd", _ptr(M), P, B, T, J, lam, s, _ptr(stats), _ptr(gpm), _ptr(gM),
+                      _stream(M.device))
+        return gM.to(dtype), None, None
 
 
 # ------------------------------------------------------------------------------------------------

@@ -8,7 +8,8 @@ exactly that of the fp32 call on the widened videos, the video gradients come ba
 gradient rounded to nearest even), and two bf16 videos are read as bf16 by the kernels (no fp32 copy
 at B <= 64 with B % 8 == 0 and K % 8 == 0, K >= 128).  So can a bf16 video smoothed first by
 data_utils.KernelSmoothing, which returns bf16 (the whole smoothing -> loss -> adjoints chain then makes no fp32
-copy of a video).  The other functions here stay fp32-only.
+copy of a video).  scale_invariante_martingale_regularization_batched widens a bf16 M (exact) and returns its gradient
+in bf16.  The other functions here stay fp32-only.
 
 Reference quirks are reproduced on purpose (SURVEY.md Appendix B):
   * compute_sinkhorn_loss passes `sinkhorn_eps, sinkhorn_l` positionally into compute_sinkhorn's
@@ -20,7 +21,8 @@ Reference quirks are reproduced on purpose (SURVEY.md Appendix B):
 """
 import torch
 
-from .functional import CostFn, MartingalePenaltyFn, MixedLossBatchedFn, MixedLossFn, SinkhornFn, _check_video
+from .functional import (CostFn, MartingalePenaltyBatchedFn, MartingalePenaltyFn, MixedLossBatchedFn, MixedLossFn,
+                         SinkhornFn, _check_video)
 
 __all__ = ["cost_xy", "modified_cost", "bi_causal_modified_cost", "benchmark_sinkhorn", "compute_sinkhorn",
            "compute_N", "scale_invariante_martingale_regularization", "compute_sinkhorn_loss"]
@@ -70,6 +72,14 @@ def compute_N(M):
 def scale_invariante_martingale_regularization(M, reg_lam, scaling_coef):
     """gan_utils.py:179-201 — p_M."""
     return MartingalePenaltyFn.apply(M, reg_lam, scaling_coef)
+
+
+def scale_invariante_martingale_regularization_batched(M, reg_lam, scaling_coef):
+    """Not in the reference: p_M of `nprob` independent problems in one call (BASELINE config 4's discriminator step,
+    kernel_train.py:249-250).  M is [nprob, B, T, J], fp32 or bf16; returns the [nprob] penalties, entry p bit-identical
+    to scale_invariante_martingale_regularization(M[p].float(), ...) and differentiable w.r.t. M[p] only.  Folding the
+    problems into the batch axis would not do: the mean, sigma_j and A_tj are taken over the batch."""
+    return MartingalePenaltyBatchedFn.apply(M, reg_lam, scaling_coef)
 
 
 def compute_sinkhorn_loss(f_real, f_fake, scaling_coef, sinkhorn_eps, sinkhorn_l, h_fake, m_real, h_real,
